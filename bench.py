@@ -294,15 +294,32 @@ def make_timed(world, dev, dist):
     return timed
 
 
+def dump_outputs(path, outputs, limit=64 << 20):
+    """Write every output as <path>/<name>.npy in float32 (float64 stays float64).  An array larger than its equal share
+    of half of `limit` bytes is replaced by a fixed, seeded sample of its elements, with their flat indices in
+    <name>_index.npy, so the directory stays below `limit`."""
+    os.makedirs(path, exist_ok=True)
+    share = limit // (2 * max(1, len(outputs)))
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.nbytes > share:
+            idx = np.sort(np.random.default_rng(1088).choice(a.size, share // 16, replace=False))
+            np.save(os.path.join(path, name + "_index.npy"), idx.astype(np.float64))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def synthetic_scene(cfg):
     from cmlpl_b200 import synth
     return synth.preprocessed_scene(cfg["R"], cfg["C"], cfg["B"], cfg["K"], 60, 1088, return_raw=True)
 
 
-def train_step_bench(cfg, dev, slab, spec_dev, truth, steps):
+def train_step_bench(cfg, dev, slab, spec_dev, truth, steps, outputs=None):
     """One mutual-learning step (train.py:149-278), 128 labelled + 128 unlabelled, dropout 0.8, noise 0.5:
     the fused tcgen05 step from a CUDA graph (inputs gathered from the cube inside the first kernel, Philox noise),
-    the fp32 reference-precision path, and the oracle's ref_step on the host cores."""
+    the fp32 reference-precision path, and the oracle's ref_step on the host cores.  When `outputs` is a dict, the
+    losses and both nets' parameters after the last timed fused step are stored in it."""
     from cmlpl_b200 import ops, train as T
     from cmlpl_b200.fused_step import FusedMutualStep
     from cmlpl_b200.tools.models import BaseNet2
@@ -323,7 +340,7 @@ def train_step_bench(cfg, dev, slab, spec_dev, truth, steps):
     for _ in range(5):
         fused()
     torch.cuda.synchronize()
-    n = max(steps, 200)
+    n = steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(n):
@@ -331,6 +348,10 @@ def train_step_bench(cfg, dev, slab, spec_dev, truth, steps):
     e1.record()
     torch.cuda.synchronize()
     fused_ms = e0.elapsed_time(e1) / n
+    if outputs is not None:
+        outputs["train_losses"] = fs.hist.cpu().numpy()
+        for e, net in enumerate(nets):
+            outputs.update({f"train_net{e}.{k}": p.detach().cpu().numpy() for k, p in net.named_parameters()})
     # per phase (eager C calls on the same state; forward / losses / backward / Adam)
     io = fs._io(slab, None, spec_dev, None, None, None, None)
     st = torch.cuda.current_stream().cuda_stream
@@ -411,11 +432,14 @@ def main():
     ap.add_argument("--config", default="c1", choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-train", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (float32, <= 64 MB)")
     args = ap.parse_args()
     cfg = CONFIGS[args.config]
-    # defaults that finish within minutes: 300 steps of ~1 ms on the GPU arm, 5 steps of ~5 s on the CPU arm
+    # defaults that finish within minutes: 300 steps of ~1 ms on the GPU arm (3 of ~0.2 s at c5), 5 steps of ~5 s on
+    # the CPU arm
     if args.steps is None:
-        args.steps = 5 if args.impl == "reference" else 300
+        args.steps = 5 if args.impl == "reference" else (3 if args.config == "c5" else 300)
     if args.warmup is None:
         args.warmup = 1 if args.impl == "reference" else 5
     if args.config == "c5":
@@ -485,7 +509,7 @@ def main():
                 # the counts are produced directly in its send buffer
                 self.exchange.local_cm.zero_()
                 ops.confusion(self.labels, self.truth, K, self.exchange.local_cm)
-                self.exchange()
+                self.result = self.exchange()
 
         def step_e2e(self):
             # the RAW uint16 band (+halo) in pinned host memory in, uint8 labels out (label map of the whole scene on
@@ -502,8 +526,17 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     band = Band(R)
+    outputs = {} if args.dump_outputs and rank == 0 else None
     ms_dev = timed(band.step_device, args.steps, args.warmup)
+    if outputs is not None:
+        # the label map of the whole scene (and the confusion counts when sharded), as the last timed step left them
+        if world > 1:
+            outputs["labels"], outputs["confusion"] = (t.cpu().numpy() for t in band.result)
+        else:
+            outputs["labels"] = band.labels.cpu().numpy()
     ms_e2e = timed(band.step_e2e, args.steps, args.warmup)
+    if outputs is not None:
+        outputs["labels_e2e"] = (band.map_host if world > 1 else band.streamed.labels_host).numpy().copy()
     ms_h2d = timed(band.step_h2d_only, args.steps, args.warmup)
     # a fixed >= 1 s window next to the K-step number (VERDICT r1: a 20-step region is 20 ms)
     n_steady = max(args.steps, int(math.ceil(1000.0 / max(ms_dev, 1e-3))))
@@ -573,7 +606,7 @@ def main():
     # ---- second half of the BASELINE metric: one mutual-learning train step (train.py:149-278), 128+128
     train = None
     if world == 1 and not args.no_train and args.config in ("c1", "c2", "c3"):
-        fs, fused_ms, phase_ms, fp32_ms = train_step_bench(cfg, dev, band.slab, band.spec, band.truth, args.steps)
+        fs, fused_ms, phase_ms, fp32_ms = train_step_bench(cfg, dev, band.slab, band.spec, band.truth, args.steps, outputs)
         train = {"fused_ms": fused_ms, "phase_ms": phase_ms, "fp32_ms": fp32_ms, "launches": fs.launches()}
     clocks = sampler.stop()
 
@@ -706,6 +739,8 @@ def main():
             line["cpu_baseline"]["ref_step_ms"] = cpu_ref_step_ms(cfg, cube_pca, spectra, gt, threads)
             line["cpu_baseline"]["ref_step_note"] = ("oracle ref_step (restatement of train.py:150-272 pinned against the "
                                                      "reference's train.main), median of 3, noise + dropout draws included")
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -23,6 +23,7 @@ from oracle import ref_shims  # noqa: E402
 
 ref_shims.install()
 from oracle import cmlpl_oracle as O  # noqa: E402
+from oracle import golden  # noqa: E402
 
 from tools import hyper_tools as RH  # noqa: E402  (reference)
 from tools import models as RM  # noqa: E402  (reference)
@@ -114,7 +115,7 @@ def gold_basenet2():
             for k, p in net.named_parameters():
                 if k in O.LIVE_KEYS:
                     out[f"grad.{k}"] = p.grad.numpy()
-    np.savez_compressed(os.path.join(GOLD, "basenet2.npz"), **out)
+    golden.save(os.path.join(GOLD, "basenet2.npz"), out)
     print("basenet2.npz ok")
 
 
@@ -237,14 +238,14 @@ def gold_train(num_epochs=2, num_unlabel=512):
         lab_ref, logit_ref = O.test_whole({k: torch.from_numpy(v) for k, v in ref_sd.items()},
                                           Xp, Xs, 20, return_logits=True)
         assert np.mean(lab_ref == loc["predict_label"]) >= 0.9995
-        np.savez_compressed(
+        golden.save(
             os.path.join(GOLD, "train_infer.npz"),
-            cube_pca=Xp.astype(np.float32), spectra=Xs.astype(np.float32), Y=Y, train_array=tr,
-            test_array=te, unlabel_array=un, loss_hist=ref_hist,
-            predict_label=loc["predict_label"].astype(np.uint8),
-            logits_trained=logit_ref.astype(np.float32),
-            OA=loc["OA"] / 100.0, Kappa=loc["Kappa"], producerA=loc["producerA"],
-            **{f"sd.{k}": v for k, v in ref_sd.items()})
+            dict(cube_pca=Xp.astype(np.float32), spectra=Xs.astype(np.float32), Y=Y, train_array=tr,
+                 test_array=te, unlabel_array=un, loss_hist=ref_hist,
+                 predict_label=loc["predict_label"].astype(np.uint8),
+                 logits_trained=logit_ref.astype(np.float32),
+                 OA=loc["OA"] / 100.0, Kappa=loc["Kappa"], producerA=loc["producerA"],
+                 **{f"sd.{k}": v for k, v in ref_sd.items()}))
         print("train_infer.npz ok  (OA=%.4f kappa=%.4f)" % (loc["OA"] / 100.0, loc["Kappa"]))
     finally:
         os.chdir(cwd)
@@ -351,7 +352,7 @@ def gold_loader():
                 if len(item) == 3:
                     assert item[2].dtype == np.int64 or item[2].dtype == int
             out[f"{name}.arity"] = np.array(len(ds[0]))
-        np.savez_compressed(os.path.join(GOLD, "loader.npz"), **out)
+        golden.save(os.path.join(GOLD, "loader.npz"), out)
         print("loader.npz ok:", {k: int(v) for k, v in out.items() if k.endswith(".len")})
     finally:
         os.chdir(cwd)
@@ -405,7 +406,7 @@ def gold_step():
     """One full-size (128+128) mutual-learning step through the oracle, with every input
     regenerable from the fixture (cube + indices + seeds).  The oracle's ref_step was
     pinned against train.main by gold_train(); this fixture freezes its outputs."""
-    z = np.load(os.path.join(GOLD, "train_infer.npz"))
+    z = golden.load(os.path.join(GOLD, "train_infer.npz"))
     Xp, Xs, Y = z["cube_pca"], z["spectra"], z["Y"].astype(np.int64) - 1
     tr, un = z["train_array"], z["unlabel_array"]
     K, B = 9, 103
@@ -436,7 +437,7 @@ def gold_step():
         out[f"grad.{k}"] = r["grads"][k].numpy()
         out[f"grad1.{k}"] = r["grads1"][k].numpy()
         out[f"new.{k}"] = st.sd[k].detach().numpy()
-    np.savez_compressed(os.path.join(GOLD, "step.npz"), **out)
+    golden.save(os.path.join(GOLD, "step.npz"), out)
     print("step.npz ok, hist =", r["hist"])
 
 

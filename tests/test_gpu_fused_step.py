@@ -21,6 +21,7 @@ import torch
 import torch.nn.functional as F
 
 from oracle import cmlpl_oracle as O
+from oracle import golden
 from test_oracle_cpu import replay_step
 
 pytestmark = pytest.mark.gpu
@@ -157,8 +158,8 @@ def compare_with_oracle(fs, hist, r, ost, w_before, patches, nb, sds_dev):
 
 def test_fused_step_matches_oracle_and_fixture(dev, golden_dir):
     """The 128+128 step of tests/golden/step.npz (PaviaU shape, B=103, 9 classes, epoch 1, bank smoothing on)."""
-    z = np.load(os.path.join(golden_dir, "step.npz"))
-    ti = np.load(os.path.join(golden_dir, "train_infer.npz"))
+    z = golden.load(os.path.join(golden_dir, "step.npz"))
+    ti = golden.load(os.path.join(golden_dir, "train_infer.npz"))
     r, ost = replay_step(z, ti)
     inp = ost.extras["inputs"]
     nz, a = inp["noise"], inp["args"]
@@ -182,7 +183,7 @@ def test_both_steps_at_the_indian_pines_shape_with_dropout_masks(dev, golden_dir
     step: the fp32 path (1e-5 / 1e-4 bars) and the fused tcgen05 path (bars in the module docstring) against the
     oracle's ref_step on the same inputs."""
     from cmlpl_b200 import train as T
-    ti = np.load(os.path.join(golden_dir, "train_infer.npz"))
+    ti = golden.load(os.path.join(golden_dir, "train_infer.npz"))
     Xp = ti["cube_pca"]
     B, K, bs = 200, 16, 128
     g = torch.Generator().manual_seed(123)
@@ -247,7 +248,7 @@ def test_fused_step_cube_mode_philox_and_graph(dev, golden_dir):
     steps; a CUDA-graph replay computes the same step as the eager launch sequence."""
     from cmlpl_b200.fused_step import FusedMutualStep
     from cmlpl_b200.tools.models import BaseNet2
-    ti = np.load(os.path.join(golden_dir, "train_infer.npz"))
+    ti = golden.load(os.path.join(golden_dir, "train_infer.npz"))
     cube = torch.from_numpy(ti["cube_pca"]).to(dev).contiguous()
     spectra = torch.from_numpy(ti["spectra"]).to(dev).contiguous()
     R, C = cube.shape[:2]
@@ -379,7 +380,7 @@ def test_fused_step_partial_batch_and_argument_checks(dev, golden_dir):
     """train.py's DataLoaders keep the last partial batch (10 000 samples / 128 -> a 16-row tail): a FusedMutualStep built
     for 128 + 128 runs a 16 + 16 step on the head of its buffers and matches the oracle; bad arguments fail loudly."""
     from cmlpl_b200 import _lib
-    ti = np.load(os.path.join(golden_dir, "train_infer.npz"))
+    ti = golden.load(os.path.join(golden_dir, "train_infer.npz"))
     Xp, Xs = ti["cube_pca"], ti["spectra"]
     B, K, bs = 103, 9, 16
     g = torch.Generator().manual_seed(77)

@@ -10,6 +10,7 @@ import torch
 import torch.nn.functional as F
 
 from oracle import cmlpl_oracle as O
+from oracle import golden
 
 pytestmark = pytest.mark.gpu
 
@@ -20,7 +21,7 @@ def rel(a, b):
 
 
 def g(golden_dir, name):
-    return np.load(os.path.join(golden_dir, name))
+    return golden.load(os.path.join(golden_dir, name))
 
 
 # ------------------------------------------------------------------ a1-a3 patch gather (bit-exact)
@@ -214,7 +215,7 @@ def _scene(dev, sd, cube, spectra, K, **kw):
 def test_scene_inference_trained_net_vs_reference_golden(dev, golden_dir):
     """Label map and logits of the net trained by the reference's own train.main."""
     z = g(golden_dir, "train_infer.npz")
-    sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")}
+    sd = {k[3:]: torch.from_numpy(z[k]) for k in z if k.startswith("sd.")}
     labels, logits = _scene(dev, sd, z["cube_pca"], z["spectra"], 9, want_logits=True)
     agree = np.mean(labels.cpu().numpy() == z["predict_label"])
     assert agree >= 0.999, agree
@@ -300,7 +301,7 @@ def test_test_whole_generic_loader(dev, golden_dir):
     from cmlpl_b200.tools.models import BaseNet2
     z = g(golden_dir, "train_infer.npz")
     net = BaseNet2(num_features=103, dropout=0.8, num_classes=9)
-    net.load_state_dict({k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")}, strict=False)
+    net.load_state_dict({k[3:]: torch.from_numpy(z[k]) for k in z if k.startswith("sd.")}, strict=False)
     net = net.to(dev)
     idx = np.arange(300, 700)
     XP = torch.from_numpy(O.extract_patches_at(z["cube_pca"], 20, idx))

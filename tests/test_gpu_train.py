@@ -11,6 +11,7 @@ import torch
 import torch.nn.functional as F
 
 from oracle import cmlpl_oracle as O
+from oracle import golden
 from test_oracle_cpu import replay_step
 
 pytestmark = pytest.mark.gpu
@@ -135,8 +136,8 @@ def test_fused_adam_matches_torch(dev):
 def test_mutual_step_matches_oracle_and_fixture(dev, golden_dir):
     """One full 128+128 step: forward, losses, both backward passes, both Adam updates, bank writes."""
     from cmlpl_b200 import train as T
-    z = np.load(os.path.join(golden_dir, "step.npz"))
-    ti = np.load(os.path.join(golden_dir, "train_infer.npz"))
+    z = golden.load(os.path.join(golden_dir, "step.npz"))
+    ti = golden.load(os.path.join(golden_dir, "train_infer.npz"))
     r, ost = replay_step(z, ti)
     inp = ost.extras["inputs"]
     nz, a = inp["noise"], inp["args"]

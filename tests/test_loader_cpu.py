@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 
 from oracle import cmlpl_oracle as O
+from oracle import golden
 
 CASES = {"label_tiled": dict(setindex="label", max_iters=137), "label_plain": dict(setindex="label"),
          "unlabel_head": dict(setindex="unlabel", max_iters=300, num_unlabel=200),
@@ -19,7 +20,7 @@ CASES = {"label_tiled": dict(setindex="label", max_iters=137), "label_plain": di
 
 @pytest.fixture(scope="module")
 def gold(golden_dir):
-    return np.load(os.path.join(golden_dir, "loader.npz")), np.load(os.path.join(golden_dir, "train_infer.npz"))
+    return golden.load(os.path.join(golden_dir, "loader.npz")), golden.load(os.path.join(golden_dir, "train_infer.npz"))
 
 
 def _write_dir(root, z, ti, materialise):

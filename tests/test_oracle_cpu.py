@@ -8,12 +8,13 @@ import pytest
 import torch
 
 from oracle import cmlpl_oracle as O
+from oracle import golden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _g(golden_dir, name):
-    return np.load(os.path.join(golden_dir, name))
+    return golden.load(os.path.join(golden_dir, name))
 
 
 def test_patches_match_reference_golden(golden_dir):
@@ -46,7 +47,7 @@ def test_band_sharding_reproduces_full_gather(golden_dir, world):
 
 def test_basenet2_matches_reference_golden(golden_dir):
     z = _g(golden_dir, "basenet2.npz")
-    sd = {k[3:]: torch.from_numpy(z[k]).requires_grad_(True) for k in z.files if k.startswith("sd.")}
+    sd = {k[3:]: torch.from_numpy(z[k]).requires_grad_(True) for k in z if k.startswith("sd.")}
     x, y = torch.from_numpy(z["x"]), torch.from_numpy(z["y"])
     lo, fe = O.basenet2_forward(sd, x, y)
     assert np.abs(lo.detach().numpy() - z["logits"]).max() <= 1e-5 * np.abs(z["logits"]).max()
@@ -88,7 +89,7 @@ def test_metrics_and_losses_match_reference_golden(golden_dir):
 def test_trained_inference_matches_reference_golden(golden_dir):
     """test_whole + CalAccuracy on the nets the reference's train.main produced."""
     z = _g(golden_dir, "train_infer.npz")
-    sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")}
+    sd = {k[3:]: torch.from_numpy(z[k]) for k in z if k.startswith("sd.")}
     rows = (10, 14)                                # a band keeps the CPU suite fast
     C = 36
     lab, logits = O.test_whole(sd, z["cube_pca"], z["spectra"], 20, rows=rows, return_logits=True)

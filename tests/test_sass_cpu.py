@@ -12,12 +12,14 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "cmlpl_b200", "libcmlpl_sm100.so")
+CUOBJDUMP = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
 
 
-@pytest.mark.skipif(shutil.which("cuobjdump") is None or not os.path.exists(LIB), reason="needs cuobjdump and the built library")
+@pytest.mark.skipif(not os.path.exists(CUOBJDUMP) or not os.path.exists(LIB), reason="needs cuobjdump and the built library")
 def test_tcgen05_and_tma_instructions_present():
+    env = dict(os.environ, PATH=os.path.dirname(CUOBJDUMP) + os.pathsep + os.environ.get("PATH", ""))
     out = subprocess.run([sys.executable, os.path.join(ROOT, "scripts", "sass_digest.py"), LIB], capture_output=True, text=True,
-                         check=True).stdout
+                         check=True, env=env).stdout
     rows = {}
     for line in out.splitlines():
         name = line[:62].strip()
