@@ -45,11 +45,11 @@ sim_tc_kernel(SimBatch sb) {
     fence_barrier_init();
   }
   if (warp == 8) tmem_alloc(sbase + S_TMEM, 128);
-  if (p.mode == 1) {   // queue_probs rows of this bank tile, zero beyond N
+  if (p.mode == 1) {   // queue_probs rows of this bank tile, zero beyond N and in the class slots C..31 the epilogue reads
     float* qs = reinterpret_cast<float*>(smem + S_QP);
-    for (int i = tid; i < 128 * p.C; i += kThreads) {
-      const int j = i / p.C, c = i - j * p.C;
-      qs[j * 32 + c] = (n0 + j < p.N) ? __ldg(p.qp + int64_t(n0 + j) * p.C + c) : 0.f;
+    for (int i = tid; i < 128 * 32; i += kThreads) {
+      const int j = i >> 5, c = i & 31;
+      qs[i] = (c < p.C && n0 + j < p.N) ? __ldg(p.qp + int64_t(n0 + j) * p.C + c) : 0.f;
     }
   }
   tc_fence_before();

@@ -262,13 +262,16 @@ def normalize(x: torch.Tensor) -> torch.Tensor:
     return x.div(x.pow(2).sum(1, keepdim=True).pow(0.5))
 
 
-def basenet2_forward(sd, x, y, dropout_mask=None, return_parts: bool = False):
+def basenet2_forward(sd, x, y, dropout_mask=None, return_parts: bool = False, relu_masks=None):
     """models.py:130-152.  ``dropout_mask`` (already scaled by 1/(1-p), or None) replaces
-    nn.Dropout so the test harness can inject it."""
+    nn.Dropout so the test harness can inject it.  ``relu_masks`` (the 0/1 masks of the two
+    trunk ReLUs, [n,64,20,20] and [n,64,10,10], or None) replaces ReLU's own sign test, so that a
+    reduced-precision forward's masks can be imposed on this one."""
+    relu = lambda z, i: F.relu(z) if relu_masks is None else z * relu_masks[i]
     x = F.conv2d(x, sd["conv0.weight"], sd["conv0.bias"])
-    x = F.relu(F.conv2d(x, sd["conv1.weight"], sd["conv1.bias"], padding=1) + x)
+    x = relu(F.conv2d(x, sd["conv1.weight"], sd["conv1.bias"], padding=1) + x, 0)
     x = F.avg_pool2d(x, 2, 2)
-    x = F.relu(F.conv2d(x, sd["conv2.weight"], sd["conv2.bias"], padding=1) + x)
+    x = relu(F.conv2d(x, sd["conv2.weight"], sd["conv2.bias"], padding=1) + x, 1)
     x = F.avg_pool2d(x, 2, 2)
     x = x.reshape(x.size(0), -1)
     y = F.relu(F.linear(y, sd["feat_spe.weight"], sd["feat_spe.bias"]))
@@ -458,11 +461,12 @@ def make_state(sd, sd1, num_classes, args: StepArgs) -> TrainState:
 
 
 def ref_step(st: TrainState, XP_l, X_l, Y_l, XP_u, X_u, noise, epoch, batch_index,
-             args: StepArgs, drop_masks=(None, None)):
+             args: StepArgs, drop_masks=(None, None), relu_masks=(None, None)):
     """train.py:150-278.  ``noise`` is a dict of the eight standard-normal tensors the
     reference draws (keys: xp_l1,x_l1,xp_l2,x_l2,xp_u1,x_u1,xp_u2,x_u2; in draw order
-    train.py:157,158,163,164,170,171,181,182).  Returns the five loss_hist columns plus
-    the tensors the parity tests compare."""
+    train.py:157,158,163,164,170,171,181,182).  ``relu_masks`` imposes the trunk ReLU masks
+    per net (see basenet2_forward).  Returns the five loss_hist columns plus the tensors the
+    parity tests compare."""
     T = args.temperature
     st.opt1.zero_grad()
     st.opt.zero_grad()
@@ -471,8 +475,8 @@ def ref_step(st: TrainState, XP_l, X_l, Y_l, XP_u, X_u, noise, epoch, batch_inde
     X_b_all = torch.cat([X_l + noise["x_l1"] * args.noise, X_u + noise["x_u1"] * args.noise], 0)
     XP_e_all = torch.cat([XP_l + noise["xp_l2"] * args.noise, XP_u + noise["xp_u2"] * args.noise], 0)
     X_e_all = torch.cat([X_l + noise["x_l2"] * args.noise, X_u + noise["x_u2"] * args.noise], 0)
-    out_b, feat_b = basenet2_forward(st.sd, XP_b_all, X_b_all, drop_masks[0])
-    out_e, feat_e = basenet2_forward(st.sd1, XP_e_all, X_e_all, drop_masks[1])
+    out_b, feat_b = basenet2_forward(st.sd, XP_b_all, X_b_all, drop_masks[0], relu_masks=relu_masks[0])
+    out_e, feat_e = basenet2_forward(st.sd1, XP_e_all, X_e_all, drop_masks[1], relu_masks=relu_masks[1])
     labeled_output, x_feature = out_b[:bs], feat_b[:bs]
     un_b_output, xs_feature = out_b[bs:], feat_b[bs:]
     labeled_output1, x_feature1 = out_e[:bs], feat_e[:bs]

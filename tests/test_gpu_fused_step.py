@@ -116,7 +116,9 @@ def mask_flips(fs, sds, patches, nb):
     return flips, flips / float(m1.numel() + m2.numel())
 
 
-def compare_with_oracle(fs, hist, r, ost, w_before, patches, nb, sds_dev):
+def compare_with_oracle(fs, hist, r, ost, w_before, patches, nb, sds_dev, adam=True):
+    """The step-1 bars.  ``adam=False`` skips the Adam block, which compares against the oracle's update from ITS
+    gradients and is only sound from a fresh Adam state (later steps: test_gpu_fused_step_shapes.check_adam_exact)."""
     h = hist.cpu().numpy()
     want = np.array([r["hist"][0], r["hist"][1], r["hist"][2], r["hist"][3], r["hist"][4], r["total1"], r["cls1"],
                      r["con1"], r["lc1"]])
@@ -144,7 +146,7 @@ def compare_with_oracle(fs, hist, r, ost, w_before, patches, nb, sds_dev):
             assert d[k] < 3e-2, (k, d[k])
     linearised_check(fs, w_before, nb)
     # Adam: compare where the gradient is not ~0 (the first step moves every weight by ~lr*sign(g))
-    for e, sd_new in enumerate((ost.sd, ost.sd1)):
+    for e, sd_new in enumerate((ost.sd, ost.sd1) if adam else ()):
         for i, k in enumerate(TENSORS):
             gr = (g, g1)[e][k].numpy()
             sel = np.abs(gr) > 5e-2 * np.abs(gr).max()
