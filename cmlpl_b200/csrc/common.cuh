@@ -98,22 +98,28 @@ struct PackedLayout {
   size_t bspe;    // f32 [1024]
   size_t wc_conv; // f32 [C][P*64]   classifier columns of the conv features, permuted to (pos, ch)
   size_t wc_spe;  // f32 [C][1024]
-  size_t bc;      // f32 [C] (padded to 16)
+  size_t bc;      // f32 [C] (padded to NC)
   size_t w1s;     // f16 [4 n-tiles][KC][256][8]  feat_spe weight, UMMA B operand tiles (K padded to 16)
-  size_t wc16;    // f16 [(P*8 + 128) k-chunks][16 classes][8]  classifier over [conv(pos,ch) | spectral]
-  size_t wcq;     // f16 per (Alpha,Beta) block [8 k-chunks][N = maps*16 rows = map*16+cls][8]: 0.25 * conv classifier
+  size_t wc16;    // f16 [(P*8 + 128) k-chunks][NC classes][8]  classifier over [conv(pos,ch) | spectral]
+  size_t wcq;     // f16 per (Alpha,Beta) block [8 k-chunks][N = maps*NC rows = map*NC+cls][8]: 0.25 * conv classifier
                   //     columns of pooled cell (I,J), per border block (Al,Be), rows J-major (w = 20 only; pool2_cls_kernel)
   size_t total;
   int conv_pos;   // P = (w/4)^2 pooled positions
   int kc_spe_in;  // KC = ceil(B/16)*2: 16-byte K-chunks of the spectral input
+  int nc;         // NC: class width of the tensor-core classifier blocks, 16 (C <= 16) or 32
 };
 
 __host__ __device__ inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
+
+// class width of the tensor-core classifier operands and of the dense path's partial maps: one MMA N of 16 up to 16
+// classes, 32 beyond (C > 32 has no tensor-core classifier; its packed blocks hold the first 32 classes and go unread)
+__host__ __device__ constexpr int class_width(int C) { return C <= 16 ? 16 : 32; }
 
 __host__ __device__ inline PackedLayout packed_layout(int B, int C, int w) {
   PackedLayout L;
   int p = (w / 2) / 2;
   L.conv_pos = p * p;
+  L.nc = class_width(C);
   size_t o = 0;
   L.w1 = o; o = align256(o + 9 * 8 * 64 * 8 * 2);
   L.w2 = o; o = align256(o + 9 * 8 * 64 * 8 * 2);
@@ -125,11 +131,11 @@ __host__ __device__ inline PackedLayout packed_layout(int B, int C, int w) {
   L.bspe = o; o = align256(o + 1024 * 4);
   L.wc_conv = o; o = align256(o + size_t(C) * L.conv_pos * 64 * 4);
   L.wc_spe = o; o = align256(o + size_t(C) * 1024 * 4);
-  L.bc = o; o = align256(o + size_t(C > 16 ? C : 16) * 4);
+  L.bc = o; o = align256(o + size_t(C > L.nc ? C : L.nc) * 4);
   L.kc_spe_in = ((B + 15) / 16) * 2;
   L.w1s = o; o = align256(o + size_t(4) * L.kc_spe_in * 256 * 16);
-  L.wc16 = o; o = align256(o + size_t(L.conv_pos * 8 + 128) * 16 * 16);
-  L.wcq = o; o = align256(o + size_t(400) * 128);
+  L.wc16 = o; o = align256(o + size_t(L.conv_pos * 8 + 128) * L.nc * 16);
+  L.wcq = o; o = align256(o + size_t(25) * L.nc * 128);
   L.total = o;
   return L;
 }

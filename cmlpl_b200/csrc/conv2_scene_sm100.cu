@@ -466,34 +466,49 @@ conv2_scene_kernel(const __grid_constant__ CUtensorMap tm_pm, const __half* __re
 // pooled row class Al and a pooled column J the tile of YP[Al][Be(J)] is loaded with its origin 2J columns to the right
 // (the column shift of the J-sum is a TMA coordinate), the remaining 2x2 pool of the middle classes is an A-descriptor
 // offset (u,v) inside the tile, and the maps I of the row class share the operand: (Al==1 ? 2 : 1) x (Be==1 ? 2 : 1)
-// shifts x 4 k-steps tcgen05.mma with M = 128 positions, N = 16 classes x (1 or 3) maps, all J accumulating into the
+// shifts x 4 k-steps tcgen05.mma with M = 128 positions, N = NC classes x (1 or 3) maps, all J accumulating into the
 // same TMEM columns.  The block weights carry 1/4, 1/2 or 1 (pack.cu).  Two accumulator stages: the MMAs of the next
 // tile run under the read-out of this one.
+// NC = class width: 16 for <= 16 classes; 32 for 17-32, whose 100 KB of weights leave room for 6 ring slots, and whose two
+// accumulator stages of 5 maps x 32 columns need 512 TMEM columns.
 namespace p2c {
 constexpr int TH = 4, TP = 32, TW = 31;              // outputs valid for tx = 0..30 (tx+1 must be in the tile)
 constexpr int CH = (TH + 1) * TP * 16;               // 2 560: one chunk plane of a tile, dense (written by TMA)
 constexpr int TBYTES = 8 * CH;                       // 20 480: one map tile
-constexpr int NSLOT = 8;                             // ring of map tiles (164 KB in flight per SM)
-constexpr int WBYTES = 400 * 128;                    // 25 maps x 16 classes x 64 channels, f16
-constexpr int S_W = 0, S_T = WBYTES, S_BAR = S_T + NSLOT * TBYTES + 128, S_TMEM = S_BAR + 256;   // +128: shifted A rows of the last slot
-constexpr int SMEM = (S_TMEM + 16 + 127) / 128 * 128;
 constexpr int kEpi = 256, kThreads = kEpi + 64;      // warps 0-7 epilogue, warp 8 loader, warp 9 MMA issuer
 constexpr int kLoadWarp = kEpi / 32, kMmaWarp = kLoadWarp + 1;
-enum { F0 = 0, E0 = NSLOT, DFULL0 = 2 * NSLOT, DEMPTY0 = 2 * NSLOT + 2, W_FULL = 2 * NSLOT + 4 };
-static_assert(SMEM <= 232448, "pool2_cls: shared memory over the 227 KB limit");
-static_assert(S_T % 128 == 0 && TBYTES % 128 == 0, "pool2_cls: TMA destinations must be 128-byte aligned");
+template <int NC>
+struct Plan {
+  static constexpr int NSLOT = NC == 16 ? 8 : 6;     // ring of map tiles (164 / 123 KB in flight per SM)
+  static constexpr int WBYTES = 25 * NC * 128;       // 25 maps x NC classes x 64 channels, f16
+  static constexpr int TCOLS = NC == 16 ? 256 : 512; // TMEM allocation; accumulator stage st at column st * TCOLS / 2
+  static constexpr int S_W = 0, S_T = WBYTES, S_BAR = S_T + NSLOT * TBYTES + 128, S_TMEM = S_BAR + 256;   // +128: shifted A rows of the last slot
+  static constexpr int SMEM = (S_TMEM + 16 + 127) / 128 * 128;
+  enum { F0 = 0, E0 = NSLOT, DFULL0 = 2 * NSLOT, DEMPTY0 = 2 * NSLOT + 2, W_FULL = 2 * NSLOT + 4 };
+  static_assert(SMEM <= 232448, "pool2_cls: shared memory over the 227 KB limit");
+  static_assert(S_T % 128 == 0 && TBYTES % 128 == 0, "pool2_cls: TMA destinations must be 128-byte aligned");
+  static_assert(2 * 5 * NC <= TCOLS && 5 * NC <= TCOLS / 2, "pool2_cls: two accumulator stages of 5 maps must fit TMEM");
+};
+static_assert(Plan<16>::SMEM <= 232448 && Plan<16>::NSLOT == 8, "pool2_cls<16>: 8-slot ring within 227 KB");
+static_assert(Plan<32>::SMEM <= 232448 && Plan<32>::NSLOT == 6, "pool2_cls<32>: 6-slot ring within 227 KB");
 }  // namespace p2c
 
-// yq f16 [9][4][8][PR2][PC2][8];  wcq f16 per block (Al,Be) [8 kchunks][N rows = ((J-J0)*nI + I-I0)*16 + cls][8];
-// lmap f32 [4 planes][5 = I][4 class quads][PR2][PC2][4]
+// yq f16 [9][4][8][PR2][PC2][8];  wcq f16 per block (Al,Be) [8 kchunks][N rows = ((J-J0)*nI + I-I0)*NC + cls][8];
+// lmap f32 [4 planes][5 = I][NC/4 class quads][PR2][PC2][4]
 // Every map tile ((TH+1) rows x 32 entries x 8 chunks, 20 KB) is ONE cp.async.bulk.tensor (TMA, 4-D tile mode, zero
-// fill outside the plane) into a ring of 8 slots, each with its own full / empty mbarrier, so a single loader thread
-// runs up to 8 tiles ahead of the MMAs; 15 loads per output tile (the three middle columns re-read their map at
+// fill outside the plane) into a ring of NSLOT slots, each with its own full / empty mbarrier, so a single loader thread
+// runs up to NSLOT tiles ahead of the MMAs; 15 loads per output tile (the three middle columns re-read their map at
 // three origins, from L2).
+template <int NC>
 __global__ void __launch_bounds__(p2c::kThreads, 1)
 pool2_cls_kernel(const __grid_constant__ CUtensorMap tm_y, int PR2, int PC2, int nq, int ncell /* pooled cells per side: 5 (w = 20) or 2 (w = 11) */,
                  const unsigned char* __restrict__ wcq, float* __restrict__ lmap) {
   using namespace p2c;
+  using P = Plan<NC>;
+  constexpr int NSLOT = P::NSLOT, WBYTES = P::WBYTES, TCOLS = P::TCOLS, S_W = P::S_W, S_T = P::S_T, S_BAR = P::S_BAR,
+                S_TMEM = P::S_TMEM;
+  constexpr int F0 = P::F0, E0 = P::E0, DFULL0 = P::DFULL0, DEMPTY0 = P::DEMPTY0, W_FULL = P::W_FULL;
+  constexpr int NQ = NC / 4;                           // class quads per lmap entry
   extern __shared__ __align__(128) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem);
@@ -517,7 +532,7 @@ pool2_cls_kernel(const __grid_constant__ CUtensorMap tm_y, int PR2, int PC2, int
     for (int s = 0; s < 2; ++s) { mbar_init(bars + 8 * (DFULL0 + s), 1); mbar_init(bars + 8 * (DEMPTY0 + s), kEpi); }
     fence_barrier_init();
   }
-  if (warp == kMmaWarp) tmem_alloc(sbase + S_TMEM, 256);
+  if (warp == kMmaWarp) tmem_alloc(sbase + S_TMEM, TCOLS);
   fence_proxy_async();
   tc_fence_before();
   __syncthreads();
@@ -547,23 +562,23 @@ pool2_cls_kernel(const __grid_constant__ CUtensorMap tm_y, int PR2, int PC2, int
     // ================================================================ MMA issuer
     constexpr uint64_t kHi = (uint64_t(128 >> 4) | (uint64_t(1) << 14)) << 32;
     uint32_t slot = 0, ph = 0, tj = 0;
-    mbar_wait(bars + 8 * p2c::W_FULL, 0, 70);                  // weights have landed
+    mbar_wait(bars + 8 * W_FULL, 0, 70);                       // weights have landed
     for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++tj) {
       const uint32_t st = tj & 1;
       mbar_wait(bars + 8 * (DEMPTY0 + st), ((tj >> 1) & 1) ^ 1, 72);   // this stage's previous tile has been read out
       tc_fence_after();
 #pragma unroll
       for (int Al = 0; Al < 3; ++Al) {
-        const int nI = blk_n(Al), N = nI * 16, nu = Al == 1 ? 2 : 1;
+        const int nI = blk_n(Al), N = nI * NC, nu = Al == 1 ? 2 : 1;
         const uint32_t idesc = make_idesc_f16(128, N);
-        const uint32_t dcol = tmem + st * 128 + uint32_t(blk_first(Al) * 16);
+        const uint32_t dcol = tmem + st * (TCOLS / 2) + uint32_t(blk_first(Al) * NC);
         if (Al >= nAl) continue;
 #pragma unroll
         for (int J = 0; J < 5; ++J) {
           if (J >= nJ) continue;
           const int Be = J == 0 ? 0 : (J == 4 ? 2 : 1), nv = Be == 1 ? 2 : 1;
-          const int Nb = nI * blk_n(Be) * 16;                  // rows of the block (Al, Be): its k-chunk stride
-          const uint32_t w_lo = ((sbase + S_W + blk_start(Al * 3 + Be) * 16 * 128 + (J - blk_first(Be)) * N * 16) >> 4) |
+          const int Nb = nI * blk_n(Be) * NC;                  // rows of the block (Al, Be): its k-chunk stride
+          const uint32_t w_lo = ((sbase + S_W + blk_start(Al * 3 + Be) * NC * 128 + (J - blk_first(Be)) * N * 16) >> 4) |
                                 (uint32_t((Nb * 16) >> 4) << 16);
           mbar_wait(bars + 8 * (F0 + slot), ph, 73);
           tc_fence_after();
@@ -602,14 +617,19 @@ pool2_cls_kernel(const __grid_constant__ CUtensorMap tm_y, int PR2, int PC2, int
       const int y = tr * TH + ty, x = tc * TW + tx;
       const bool valid = tx < TW && y < PR2 && x < PC2;
       const uint32_t st = tj & 1;
-      // lmap f32 [4 planes][5 maps][4 class quads][PR2][PC2][4]: a warp's store of one (map, quad) is 512 contiguous bytes
-      float4* dst = reinterpret_cast<float4*>(lmap) + int64_t(pl) * 20 * psz + (valid ? int64_t(y) * PC2 + x : 0);
+      // lmap f32 [4 planes][5 maps][NC/4 class quads][PR2][PC2][4]: a warp's store of one (map, quad) is 512 contiguous bytes
+      float4* dst = reinterpret_cast<float4*>(lmap) + int64_t(pl) * 5 * NQ * psz + (valid ? int64_t(y) * PC2 + x : 0);
       mbar_wait(bars + 8 * (DFULL0 + st), (tj >> 1) & 1, 74);
       tc_fence_after();
-      float v[3][16];
+      float v[3][NC];
 #pragma unroll
-      for (int m = 0; m < 3; ++m)
-        if (m0 + m < m1) tmem_ld16(lane_addr + st * 128 + uint32_t((m0 + m) * 16), v[m]);
+      for (int m = 0; m < 3; ++m) {
+        if (m0 + m < m1) {
+#pragma unroll
+          for (int h = 0; h < NC / 16; ++h)
+            tmem_ld16(lane_addr + st * (TCOLS / 2) + uint32_t((m0 + m) * NC + h * 16), v[m] + h * 16);
+        }
+      }
       tmem_ld_wait();
       tc_fence_before();
       mbar_arrive(bars + 8 * (DEMPTY0 + st));
@@ -618,8 +638,8 @@ pool2_cls_kernel(const __grid_constant__ CUtensorMap tm_y, int PR2, int PC2, int
         for (int m = 0; m < 3; ++m) {
           if (m0 + m < m1 && m0 + m < ncell) {
 #pragma unroll
-            for (int q = 0; q < 4; ++q)                         // class quads beyond the real classes are never read (head_sum_kernel)
-              if (q < nq) dst[int64_t((m0 + m) * 4 + q) * psz] = make_float4(v[m][4 * q], v[m][4 * q + 1], v[m][4 * q + 2], v[m][4 * q + 3]);
+            for (int q = 0; q < NQ; ++q)                        // class quads beyond the real classes are never read (head_sum_kernel)
+              if (q < nq) dst[int64_t((m0 + m) * NQ + q) * psz] = make_float4(v[m][4 * q], v[m][4 * q + 1], v[m][4 * q + 2], v[m][4 * q + 3]);
           }
         }
       }
@@ -627,7 +647,7 @@ pool2_cls_kernel(const __grid_constant__ CUtensorMap tm_y, int PR2, int PC2, int
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == kMmaWarp) { tc_fence_after(); tmem_dealloc(tmem, 256); }
+  if (warp == kMmaWarp) { tc_fence_after(); tmem_dealloc(tmem, TCOLS); }
 }
 
 }  // namespace cmlpl
@@ -680,19 +700,25 @@ extern "C" int cmlpl_conv2_scene_f16(const void* pmq, int cols, int w, int band_
 extern "C" int cmlpl_pool2_cls_f16(const void* yq, int cols, int w, int band_rows, int num_features, int num_classes,
                                    const void* packed, float* lmap, cmlpl_stream_t stream) {
   CMLPL_CHECK_ARG(yq && packed && lmap, "pool2_cls: null pointer");
-  CMLPL_CHECK_ARG((w == 20 || w == 11) && cols > 0 && band_rows > 0 && num_classes > 0 && num_classes <= 16,
-                  "pool2_cls: bad dims (w must be 20 or 11, <= 16 classes)");
+  CMLPL_CHECK_ARG((w == 20 || w == 11) && cols > 0 && band_rows > 0 && num_classes > 0 && num_classes <= 32,
+                  "pool2_cls: bad dims (w must be 20 or 11, <= 32 classes)");
   const int PR2 = (band_rows + w) / 2, PC2 = (cols + w) / 2;
   const PackedLayout L = packed_layout(num_features, num_classes, w);
   const unsigned char* pk = static_cast<const unsigned char*>(packed);
-  CMLPL_MAX_DYN_SMEM(pool2_cls_kernel, p2c::SMEM);
   const int ntiles = 4 * ((PR2 + p2c::TH - 1) / p2c::TH) * ((PC2 + p2c::TW - 1) / p2c::TW);
   int grid = sm_count(); if (grid > ntiles) grid = ntiles;
   CUtensorMap tm_y;
   const int trc = make_scene_tmap(&tm_y, yq, 36, PR2, PC2, p2c::TH + 1, p2c::TP);
   if (trc != CMLPL_OK) return trc;
-  pool2_cls_kernel<<<grid, p2c::kThreads, p2c::SMEM, static_cast<cudaStream_t>(stream)>>>(tm_y, PR2, PC2, (num_classes + 3) / 4,
-                                                                                          w == 20 ? 5 : 2, pk + L.wcq, lmap);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int nq = (num_classes + 3) / 4, ncell = w == 20 ? 5 : 2;
+  if (L.nc == 16) {
+    CMLPL_MAX_DYN_SMEM(pool2_cls_kernel<16>, p2c::Plan<16>::SMEM);
+    pool2_cls_kernel<16><<<grid, p2c::kThreads, p2c::Plan<16>::SMEM, s>>>(tm_y, PR2, PC2, nq, ncell, pk + L.wcq, lmap);
+  } else {
+    CMLPL_MAX_DYN_SMEM(pool2_cls_kernel<32>, p2c::Plan<32>::SMEM);
+    pool2_cls_kernel<32><<<grid, p2c::kThreads, p2c::Plan<32>::SMEM, s>>>(tm_y, PR2, PC2, nq, ncell, pk + L.wcq, lmap);
+  }
   CMLPL_CHECK_LAUNCH("pool2_cls");
   return CMLPL_OK;
 }

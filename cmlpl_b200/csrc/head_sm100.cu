@@ -277,24 +277,29 @@ head_kernel(const __half* __restrict__ p2t, int kc_conv, const __half* __restric
 //   epilogue                   bias + ReLU -> fp16, written back IN PLACE into the slot it came from (tcgen05.st): a thread
 //                              packs the 64 fp32 columns it has read into the first 32 of them, i.e. the half-tile sits in
 //                              columns [0,32) and [64,96) of the slot as a K-major A operand
-//   MMA2 (M=128, N=16, K=128)  classifier columns of those hidden features, A operand FROM TENSOR MEMORY, accumulated over
-//                              both halves -> TMEM; its commit hands the slot back to MMA1
-//   readout                    part[quarter][pixel][16] f32: the head adds the 4 quarter partials (53 MB instead of the
-//                              425 MB hidden tensor written and read back)
+//   MMA2 (M=128, N=NC, K=128)  classifier columns of those hidden features, A operand FROM TENSOR MEMORY, accumulated over
+//                              both halves -> TMEM; its commit hands the slot back to MMA1 (NC = 16, or 32 for 17-32 classes)
+//   readout                    part[quarter][pixel][NC] f32: the head adds the 4 quarter partials (53 MB at NC = 16 instead
+//                              of the 425 MB hidden tensor written and read back)
 // The hidden features touch neither HBM nor shared memory, whose space goes to the input-tile ring.
+// NC = 32 (17-32 classes): MMA2 is N = 32, and a logits stage holds ONE 32-column accumulator in place of two of 16 --
+// the 128 TMEM columns above the MMA1 ring keep four stages of 32 columns either way.
 namespace spl {
 constexpr int kEpi = 512, kThreads = kEpi + 96;      // warps 0-15 epilogue, warp 16 loader, warp 17 MMA1 issuer (+ TMEM), warp 18 MMA2 issuer
 constexpr int kLoadWarp = kEpi / 32, kMmaWarp = kLoadWarp + 1, kMma2Warp = kLoadWarp + 2;
-constexpr int WCBYTES = 32 * 256;                    // classifier columns of this quarter: 32 k-chunks x 16 classes x 16 B
-constexpr int D2COL = 384;                           // TMEM: MMA1 ring at 0/128/256, 4 stages x 2 logits accumulators at 384..511
+__host__ __device__ constexpr int wc_bytes(int NC) { return 32 * NC * 16; }   // classifier columns of this quarter: 32 k-chunks x NC classes x 16 B
+constexpr int D2COL = 384;                           // TMEM: MMA1 ring at 0/128/256, 4 logits stages x 32 columns at 384..511
 enum { A_FULL0 = 0, A_EMPTY0 = 4, D1_FULL0 = 8, D1_EMPTY0 = 11, H_FULL0 = 14, L_FULL0 = 20, L_EMPTY0 = 24, W_FULL = 28 };   // nA <= 4, 4 logits stages
 }  // namespace spl
 
+template <int NC>
 __global__ void __launch_bounds__(spl::kThreads, 1)
 spectral_logits_kernel(const __half* __restrict__ x16, int64_t mtiles, int KC, int nA,
                        const __half* __restrict__ w1t, const float* __restrict__ bspe,
                        const __half* __restrict__ wc_spe16, float* __restrict__ part) {
   using namespace spl;
+  static_assert(NC == 16 || NC == 32, "spectral_logits: class width 16 or 32");
+  constexpr int WCBYTES = wc_bytes(NC);
   extern __shared__ __align__(128) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem);
@@ -380,7 +385,8 @@ spectral_logits_kernel(const __half* __restrict__ x16, int64_t mtiles, int KC, i
   } else if (warp == kMma2Warp) {
     // ================================================================ MMA2 issuer: classifier columns over the hidden half-tiles (A from TMEM)
     constexpr uint64_t kHi = (uint64_t(128 >> 4) | (uint64_t(1) << 14)) << 32;
-    constexpr uint32_t idesc2 = make_idesc_f16(128, 16);
+    constexpr uint32_t idesc2 = make_idesc_f16(128, NC);
+    constexpr uint32_t kcb = NC * 16;                  // bytes per k-chunk of the classifier columns (LBO)
     mbar_wait(bars + 8 * W_FULL, 0, 90);
     [[maybe_unused]] uint32_t ntr = 0;
     for (uint32_t u = 0; u < U; ++u) {
@@ -391,14 +397,15 @@ spectral_logits_kernel(const __half* __restrict__ x16, int64_t mtiles, int KC, i
       tc_fence_after();
       if (lane == 0) CMLPL_TR(1, ntr, u * 4 + 2);
       if (elect_one_sync()) {
-        uint32_t b_lo = ((sbase + S_WC + hh * 16 * 256) >> 4) | (uint32_t(256 >> 4) << 16);
+        uint32_t b_lo = ((sbase + S_WC + hh * 16 * kcb) >> 4) | (uint32_t(kcb >> 4) << 16);
 #pragma unroll
         for (int ks = 0; ks < 8; ++ks) {
-          // k-step ks = hidden features 16 ks .. 16 ks + 15 of the half-tile = 8 packed columns; two independent
-          // accumulators (even / odd k-steps), the readout adds them
-          umma_f16_ta(D2COL + ls * 32 + (ks & 1) * 16, d * 128 + (ks >> 2) * 64 + (ks & 3) * 8, kHi | b_lo, idesc2,
-                      (hh | (ks >> 1)) ? 1u : 0u);
-          b_lo += 512 >> 4;
+          // k-step ks = hidden features 16 ks .. 16 ks + 15 of the half-tile = 8 packed columns; NC = 16: two independent
+          // accumulators (even / odd k-steps), the readout adds them; NC = 32: one accumulator
+          const uint32_t dcol = D2COL + ls * 32 + (NC == 16 ? (ks & 1) * 16 : 0);
+          const uint32_t acc = NC == 16 ? (hh | (ks >> 1)) : (hh | ks);
+          umma_f16_ta(dcol, d * 128 + (ks >> 2) * 64 + (ks & 3) * 8, kHi | b_lo, idesc2, acc ? 1u : 0u);
+          b_lo += (2 * kcb) >> 4;
         }
         umma_commit(bars + 8 * (D1_EMPTY0 + d));
         if (hh == 1) umma_commit(bars + 8 * (L_FULL0 + ls));
@@ -417,17 +424,19 @@ spectral_logits_kernel(const __half* __restrict__ x16, int64_t mtiles, int KC, i
       const uint32_t ls = ti & 3;
       mbar_wait(bars + 8 * (L_FULL0 + ls), (ti >> 2) & 1, 96);
       tc_fence_after();
-      float v[16], w1[16];
+      float v[32];
       tmem_ld16(lane_addr + D2COL + ls * 32, v);
-      tmem_ld16(lane_addr + D2COL + ls * 32 + 16, w1);
+      tmem_ld16(lane_addr + D2COL + ls * 32 + 16, v + 16);
       tmem_ld_wait();
       tc_fence_before();
       mbar_arrive(bars + 8 * (L_EMPTY0 + ls));
+      if (NC == 16) {
 #pragma unroll
-      for (int c = 0; c < 16; ++c) v[c] += w1[c];
-      float4* dst = reinterpret_cast<float4*>(part) + ((int64_t(ntile) * mtiles + (mt0 + int64_t(ti) * mstep)) * 128 + L) * 4;
+        for (int c = 0; c < 16; ++c) v[c] += v[16 + c];
+      }
+      float4* dst = reinterpret_cast<float4*>(part) + ((int64_t(ntile) * mtiles + (mt0 + int64_t(ti) * mstep)) * 128 + L) * (NC / 4);
 #pragma unroll
-      for (int k = 0; k < 4; ++k) dst[k] = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
+      for (int k = 0; k < NC / 4; ++k) dst[k] = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
     };
     [[maybe_unused]] uint32_t ntr = 0;
     const bool tracer = (warp & 7) == 0 && lane == 0;
@@ -475,27 +484,29 @@ spectral_logits_kernel(const __half* __restrict__ x16, int64_t mtiles, int KC, i
 // ------------------------------------------------------------------ head of the dense path: sums + argmax
 // logits(p) = bc + sum over the 4 hidden quarters of part[q][p] + the 5 gathered conv partials M[I][r'+2I, c'] of pixel p
 // (row maps of pool2_cls_kernel); first index wins ties (hyper_tools.py:426).  One thread per pixel:
-// adjacent lanes read adjacent 16-byte quads of the two parity planes of a row.
+// adjacent lanes read adjacent 16-byte quads of the two parity planes of a row.  NC = class width of part / lmap (16, 32).
+template <int NC>
 __global__ void __launch_bounds__(256)
 head_sum_kernel(const float* __restrict__ part, int64_t mtiles, const float* __restrict__ lmap, int cols, int PR2, int PC2,
                 int64_t n, int C, int ncell /* pooled rows: 5 (w = 20) or 2 (w = 11) */, const float* __restrict__ bc,
                 uint8_t* __restrict__ labels, float* __restrict__ logits) {
+  constexpr int NQ = NC / 4;                           // class quads per map entry
   const int64_t p = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
   if (p >= n) return;
   const int nq = (C + 3) >> 2;                         // class quads that hold real classes
-  float v[16];
+  float v[NC];
 #pragma unroll
-  for (int c = 0; c < 16; ++c) v[c] = 0.f;
+  for (int c = 0; c < NC; ++c) v[c] = 0.f;
   const int r = int(p / cols), c0 = int(p - int64_t(r) * cols);
   const int64_t psz = int64_t(PR2) * PC2;
-  const float4* base = reinterpret_cast<const float4*>(lmap) + int64_t((r & 1) * 2 + (c0 & 1)) * 20 * psz +
+  const float4* base = reinterpret_cast<const float4*>(lmap) + int64_t((r & 1) * 2 + (c0 & 1)) * 5 * NQ * psz +
                        int64_t(r >> 1) * PC2 + (c0 >> 1);
 #pragma unroll
   for (int I = 0; I < 5; ++I) {
     if (I >= ncell) break;
-    const float4* q = base + int64_t(I * 4) * psz + (2 * I) * PC2;
+    const float4* q = base + int64_t(I * NQ) * psz + (2 * I) * PC2;
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
+    for (int k = 0; k < NQ; ++k) {
       if (k < nq) {
         const float4 t = __ldg(q + int64_t(k) * psz);
         v[4 * k] += t.x; v[4 * k + 1] += t.y; v[4 * k + 2] += t.z; v[4 * k + 3] += t.w;
@@ -504,9 +515,9 @@ head_sum_kernel(const float* __restrict__ part, int64_t mtiles, const float* __r
   }
 #pragma unroll
   for (int qd = 0; qd < 4; ++qd) {
-    const float4* s = reinterpret_cast<const float4*>(part) + (int64_t(qd) * mtiles * 128 + p) * 4;
+    const float4* s = reinterpret_cast<const float4*>(part) + (int64_t(qd) * mtiles * 128 + p) * NQ;
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
+    for (int k = 0; k < NQ; ++k) {
       if (k < nq) {
         const float4 t = __ldg(s + k);
         v[4 * k] += t.x; v[4 * k + 1] += t.y; v[4 * k + 2] += t.z; v[4 * k + 3] += t.w;
@@ -515,7 +526,7 @@ head_sum_kernel(const float* __restrict__ part, int64_t mtiles, const float* __r
   }
   float best = -INFINITY; int arg = 0;
 #pragma unroll
-  for (int c = 0; c < 16; ++c) {
+  for (int c = 0; c < NC; ++c) {
     if (c < C) {
       const float z = v[c] + __ldg(bc + c);
       if (logits) logits[p * C + c] = z;
@@ -531,10 +542,11 @@ using namespace cmlpl;
 
 CMLPL_TRACE_EXPORT(cmlpl_debug_spl_trace)
 
-// shared-memory plan of spectral_logits_kernel for KC input k-chunks: as many input tiles in flight as fit (<= 4)
-static bool spectral_logits_plan(int KC, int* nA, size_t* smem) {
+// shared-memory plan of spectral_logits_kernel for KC input k-chunks and class width NC: as many input tiles in flight as
+// fit (<= 4).  224 bands (KC = 28) leave room for one at either width.
+static bool spectral_logits_plan(int KC, int NC, int* nA, size_t* smem) {
   for (int a = 4; a >= 1; --a) {
-    const size_t b = size_t(KC) * 4096 + size_t(a) * KC * 2048 + spl::WCBYTES + 1024 + 256 + 64;
+    const size_t b = size_t(KC) * 4096 + size_t(a) * KC * 2048 + spl::wc_bytes(NC) + 1024 + 256 + 64;
     if (b <= 232448) { *nA = a; *smem = b; return true; }
   }
   return false;
@@ -561,16 +573,23 @@ static int spectral_hidden_impl(const void* x, int dtype /* -1 = preprocessed f3
   CMLPL_CHECK_LAUNCH("x16_tile");
   if (fused_logits) {
     int nA = 0; size_t fsmem = 0;
-    CMLPL_CHECK_ARG(spectral_logits_plan(KC, &nA, &fsmem), "spectral_logits_tc: %d bands do not fit shared memory", num_features);
-    CMLPL_CHECK_ARG(num_classes <= 16, "spectral_logits_tc: needs <= 16 classes, got %d", num_classes);
-    CMLPL_MAX_DYN_SMEM(spectral_logits_kernel, int(fsmem));
+    CMLPL_CHECK_ARG(spectral_logits_plan(KC, L.nc, &nA, &fsmem), "spectral_logits_tc: %d bands do not fit shared memory", num_features);
+    CMLPL_CHECK_ARG(num_classes <= 32, "spectral_logits_tc: needs <= 32 classes, got %d", num_classes);
     int fgrid = sm_count() / 4 * 4;
     if (fgrid > mtiles * 4) fgrid = int(mtiles * 4);
     const unsigned char* fpk = static_cast<const unsigned char*>(packed);
-    spectral_logits_kernel<<<fgrid, spl::kThreads, fsmem, s>>>(
-        static_cast<const __half*>(x16), mtiles, KC, nA, reinterpret_cast<const __half*>(fpk + L.w1s),
-        reinterpret_cast<const float*>(fpk + L.bspe),
-        reinterpret_cast<const __half*>(fpk + L.wc16 + size_t(L.conv_pos) * 8 * 256), static_cast<float*>(h16));
+    const __half* w1s = reinterpret_cast<const __half*>(fpk + L.w1s);
+    const float* bspe = reinterpret_cast<const float*>(fpk + L.bspe);
+    const __half* wc_spe16 = reinterpret_cast<const __half*>(fpk + L.wc16 + size_t(L.conv_pos) * 8 * L.nc * 16);
+    if (L.nc == 16) {
+      CMLPL_MAX_DYN_SMEM(spectral_logits_kernel<16>, int(fsmem));
+      spectral_logits_kernel<16><<<fgrid, spl::kThreads, fsmem, s>>>(static_cast<const __half*>(x16), mtiles, KC, nA, w1s, bspe,
+                                                                     wc_spe16, static_cast<float*>(h16));
+    } else {
+      CMLPL_MAX_DYN_SMEM(spectral_logits_kernel<32>, int(fsmem));
+      spectral_logits_kernel<32><<<fgrid, spl::kThreads, fsmem, s>>>(static_cast<const __half*>(x16), mtiles, KC, nA, w1s, bspe,
+                                                                     wc_spe16, static_cast<float*>(h16));
+    }
     CMLPL_CHECK_LAUNCH("spectral_logits");
     return CMLPL_OK;
   }
@@ -620,8 +639,9 @@ extern "C" int cmlpl_head_tc(const void* p2t, const void* h16, int64_t n, int nu
   return CMLPL_OK;
 }
 
-// Fused spectral branch of the dense path: part f32 [4 hidden quarters][ceil(n/128)*128][16] partial spectral logits
-// (spectral_logits_kernel; the 1024 hidden features stay in shared memory).  x16 is scratch for the fp16 input tiles.
+// Fused spectral branch of the dense path: part f32 [4 hidden quarters][ceil(n/128)*128][NC] partial spectral logits, NC =
+// 16 for <= 16 classes and 32 for 17-32 (spectral_logits_kernel; the 1024 hidden features stay in shared memory).  x16 is
+// scratch for the fp16 input tiles.
 extern "C" int cmlpl_spectral_logits_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
                                         const void* packed, void* x16, float* part, cmlpl_stream_t stream) {
   return spectral_hidden_impl(spectra, -1, n, num_features, num_classes, w, nullptr, nullptr, packed, x16, part, stream, true);
@@ -641,13 +661,18 @@ extern "C" int cmlpl_head_sum_lmap(const float* part, const float* lmap, int col
                                    cmlpl_stream_t stream) {
   CMLPL_CHECK_ARG(part && lmap && packed && labels, "head_sum_lmap: null pointer");
   CMLPL_CHECK_ARG((w == 20 || w == 11) && cols > 0 && band_rows > 0, "head_sum_lmap: bad dims (w must be 20 or 11)");
-  CMLPL_CHECK_ARG(num_classes > 0 && num_classes <= 16, "head_sum_lmap: needs 1..16 classes, got %d", num_classes);
+  CMLPL_CHECK_ARG(num_classes > 0 && num_classes <= 32, "head_sum_lmap: needs 1..32 classes, got %d", num_classes);
   const PackedLayout L = packed_layout(num_features, num_classes, w);
   const int64_t n = int64_t(band_rows) * cols, mtiles = (n + 127) / 128;
   const unsigned char* pk = static_cast<const unsigned char*>(packed);
-  head_sum_kernel<<<unsigned((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      part, mtiles, lmap, cols, (band_rows + w) / 2, (cols + w) / 2, n, num_classes, w == 20 ? 5 : 2,
-      reinterpret_cast<const float*>(pk + L.bc), labels, logits);
+  const unsigned grid = unsigned((n + 255) / 256);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int PR2 = (band_rows + w) / 2, PC2 = (cols + w) / 2, ncell = w == 20 ? 5 : 2;
+  const float* bc = reinterpret_cast<const float*>(pk + L.bc);
+  if (L.nc == 16)
+    head_sum_kernel<16><<<grid, 256, 0, s>>>(part, mtiles, lmap, cols, PR2, PC2, n, num_classes, ncell, bc, labels, logits);
+  else
+    head_sum_kernel<32><<<grid, 256, 0, s>>>(part, mtiles, lmap, cols, PR2, PC2, n, num_classes, ncell, bc, labels, logits);
   CMLPL_CHECK_LAUNCH("head_sum");
   return CMLPL_OK;
 }

@@ -37,7 +37,7 @@ __global__ void pack_kernel(PackArgs a) {
       float* bc = reinterpret_cast<float*>(o + a.L.bc);
       for (int64_t i = t0; i < 64; i += step) { b1[i] = a.c1b[i]; b2[i] = a.c2b[i]; b0[i] = a.c0b[i]; }
       for (int64_t i = t0; i < 1024; i += step) bs[i] = a.sb[i];
-      for (int64_t i = t0; i < 16 || i < a.C; i += step) bc[i] = i < a.C ? a.cb[i] : 0.f;
+      for (int64_t i = t0; i < a.L.nc || i < a.C; i += step) bc[i] = i < a.C ? a.cb[i] : 0.f;
     } break;
     case 3: {  // conv0 -> f32 [ci][n]
       float* d = reinterpret_cast<float*>(o + a.L.w0);
@@ -72,11 +72,11 @@ __global__ void pack_kernel(PackArgs a) {
         d[i] = __float2half_rn(k < a.B ? a.sw[int64_t(nrow) * a.B + k] : 0.f);
       }
     } break;
-    case 7: {  // classifier -> f16 [(P*8 + 128)][16][8]; K order = (pos, ch) then spectral j
+    case 7: {  // classifier -> f16 [(P*8 + 128)][NC][8]; K order = (pos, ch) then spectral j
       __half* d = reinterpret_cast<__half*>(o + a.L.wc16);
-      const int P = a.P, in_f = 64 * P + 1024, kc_conv = P * 8;
-      for (int64_t i = t0; i < int64_t(kc_conv + 128) * 16 * 8; i += step) {
-        const int e = int(i & 7), cls = int((i >> 3) & 15), kc = int(i >> 7);
+      const int P = a.P, in_f = 64 * P + 1024, kc_conv = P * 8, NC = a.L.nc;
+      for (int64_t i = t0; i < int64_t(kc_conv + 128) * NC * 8; i += step) {
+        const int e = int(i & 7), cls = int((i >> 3) % NC), kc = int((i >> 3) / NC);
         float v = 0.f;
         if (cls < a.C) {
           if (kc < kc_conv) { const int pos = kc >> 3, ch = (kc & 7) * 8 + e; v = a.cw[int64_t(cls) * in_f + ch * P + pos]; }
@@ -85,23 +85,23 @@ __global__ void pack_kernel(PackArgs a) {
         d[i] = __float2half_rn(v);
       }
     } break;
-    case 8: {  // dense-path classifier: per block [8 kc][N][8], row = ((J-J0)*nI + (I-I0))*16 + cls, value = Wc[cls][ch,I,J] / 4 for the
-               // middle classes; a border class arrives averaged over its two variants (conv2_scene_kernel), so its factor
+    case 8: {  // dense-path classifier: per block [8 kc][N][8], row = ((J-J0)*nI + (I-I0))*NC + cls, value = Wc[cls][ch,I,J] / 4 for
+               // the middle classes; a border class arrives averaged over its two variants (conv2_scene_kernel), so its factor
                // doubles per border direction
       // w = 20: 5x5 pooled cells.  w = 11: 2x2 cells (I, J in {0, 1}) at the same border classes, every other map zero
       if (a.P != 25 && a.P != 4) break;
       __half* d = reinterpret_cast<__half*>(o + a.L.wcq);
       const int pw = a.P == 25 ? 5 : 2;                         // pooled cells per side
-      const int in_f = 64 * a.P + 1024;
-      for (int64_t i = t0; i < 400 * 64; i += step) {
+      const int in_f = 64 * a.P + 1024, NC = a.L.nc;
+      for (int64_t i = t0; i < int64_t(25) * NC * 64; i += step) {
         int b = 0;
-        while (b < 8 && i >= int64_t(blk_start(b + 1)) * 16 * 64) ++b;
-        const int Al = b / 3, Be = b % 3, N = blk_n(Al) * blk_n(Be) * 16;
-        const int64_t li = i - int64_t(blk_start(b)) * 16 * 64;
+        while (b < 8 && i >= int64_t(blk_start(b + 1)) * NC * 64) ++b;
+        const int Al = b / 3, Be = b % 3, N = blk_n(Al) * blk_n(Be) * NC;
+        const int64_t li = i - int64_t(blk_start(b)) * NC * 64;
         const int e = int(li & 7), row = int((li >> 3) % N), kc = int((li >> 3) / N);
         // rows J-major: the maps of one pooled column J (all I of the block) are one contiguous B operand
-        const int nI = blk_n(Al), cls = row & 15, ch = kc * 8 + e;
-        const int I = blk_first(Al) + (row >> 4) % nI, J = blk_first(Be) + (row >> 4) / nI;
+        const int nI = blk_n(Al), cls = row % NC, ch = kc * 8 + e;
+        const int I = blk_first(Al) + (row / NC) % nI, J = blk_first(Be) + (row / NC) / nI;
         const float sc = 0.25f * (Al != 1 ? 2.f : 1.f) * (Be != 1 ? 2.f : 1.f);
         d[i] = __float2half_rn(cls < a.C && I < pw && J < pw ? sc * a.cw[int64_t(cls) * in_f + ch * a.P + I * pw + J] : 0.f);
       }

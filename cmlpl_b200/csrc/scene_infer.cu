@@ -10,7 +10,7 @@
 //                    the avg-pool + conv columns of the classifier -> 25 class-partial maps (conv2_scene_sm100.cu)
 //   4. head          spectral columns of the classifier (models.py:150) + the pixel's 25 gathered conv
 //                    partials + bias, argmax (hyper_tools.py:426, first index wins ties)
-//   (> 16 classes / > 224 bands: the all-per-pixel patch_cnn_sm100.cu kernel + CUDA-core classify instead)
+//   (<= 32 classes and <= 224 bands; otherwise the all-per-pixel patch_cnn_sm100.cu kernel + CUDA-core classify instead)
 #include <mutex>
 
 #include "common.cuh"
@@ -35,7 +35,7 @@ int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0,
 template <int CMAX>
 __global__ void __launch_bounds__(256)
 classify_kernel(const __half* __restrict__ p2, const float* __restrict__ spe, const float* __restrict__ part,
-                int64_t part_stride, int64_t n, int K, int C,
+                int64_t part_stride, int part_width, int64_t n, int K, int C,
                 const float* __restrict__ wc, const float* __restrict__ bc,
                 uint8_t* __restrict__ labels, float* __restrict__ logits) {
   const int lane = threadIdx.x & 31;
@@ -72,9 +72,9 @@ classify_kernel(const __half* __restrict__ p2, const float* __restrict__ spe, co
       if (c < C) {
         float v = warp_sum(acc[c]);
         v += (spe ? spe[p * C + c] : 0.f) + bc[c];
-        if (part)      // spectral_logits_kernel: four hidden-quarter partials f32 [4][part_stride][16]
-          v += (part[p * 16 + c] + part[(part_stride + p) * 16 + c]) +
-               (part[(2 * part_stride + p) * 16 + c] + part[(3 * part_stride + p) * 16 + c]);
+        if (part)      // spectral_logits_kernel: four hidden-quarter partials f32 [4][part_stride][part_width]
+          v += (part[p * part_width + c] + part[(part_stride + p) * part_width + c]) +
+               (part[(2 * part_stride + p) * part_width + c] + part[(3 * part_stride + p) * part_width + c]);
         if (logits && lane == 0) logits[p * C + c] = v;
         if (v > best) { best = v; arg = c; }   // strict '>' : first index wins ties
       }
@@ -92,9 +92,10 @@ __global__ void argmax_kernel(const float* __restrict__ logits, int64_t n, int C
   }
 }
 
-// Tensor-core head (head_sm100.cu) applies for <= 16 classes and <= 208 bands; otherwise the
-// CUDA-core spectral_head + classify kernels above run (same C ABI, same results contract).
-static bool use_tc_head(int B, int C) { return C <= 16 && ((B + 15) / 16) * 2 <= 28; }   // <= 224 bands (spectral_logits_kernel)
+// The tensor-core spectral branch (spectral_logits_kernel, head_sm100.cu) takes <= 224 bands and <= 32 classes.  It runs
+// on the dense path, and in path mode 0 for <= 16 classes or from the raw cube; otherwise the CUDA-core spectral_head +
+// classify kernels above run (same C ABI, same results contract).
+static bool tc_spectral_fits(int B, int C) { return C <= 32 && ((B + 15) / 16) * 2 <= 28; }   // <= 224 bands
 
 // 1 (default): the exact-compute-sharing kernels where they apply; 0: the per-pixel tensor-core kernels everywhere (the
 // independent implementation the tests compare against).  Per host thread; the workspace layout follows the mode.
@@ -105,32 +106,35 @@ struct SceneWs {
   int64_t chunk;
   bool tc, dense;
 };
-// tensor-core path (<= 16 classes, <= 224 bands): conv0 map, spectral tiles, conv1 variants (fp32 scratch), pooled
-// parity planes, the 25 conv2 variants, the 25 class-partial maps.  CUDA-core path: conv0 map, per-pixel pooled
-// features, spectral logits, hidden chunk.
+// tensor-core path: conv0 map, spectral tiles, partial spectral logits, pooled parity planes, the 9 half-pooled conv2
+// maps, the 5 class-partial row maps.  CUDA-core path: conv0 map, per-pixel pooled features, spectral logits, hidden
+// chunk.  Path mode 0 at 17-32 classes holds both spectral branches: the cube entry point runs the CUDA-core one, the raw
+// entry point (which has no other) the tensor-core one.
 static SceneWs scene_ws(int band_rows, int cols, int B, int C, int w) {
   SceneWs s;
   const int64_t n = int64_t(band_rows) * cols;
   const int64_t mtiles = (n + 127) / 128;
   const int P = ((w / 2) / 2) * ((w / 2) / 2);
-  s.tc = use_tc_head(B, C);
+  const int NC = class_width(C);
+  const bool tc_fits = tc_spectral_fits(B, C);
   // the exact-compute-sharing kernels: w = 20 (9 / 25 border classes) and w = 11, whose 4 / 9 classes and 2x2 pooled cells
   // are a subset of them (conv1 rows 0..9 and conv2 rows 0..3 of an 11-window are top / mid class only)
-  s.dense = s.tc && (w == 20 || w == 11) && g_scene_path_mode == 1;
+  s.dense = tc_fits && (w == 20 || w == 11) && g_scene_path_mode == 1;
+  s.tc = s.dense || (tc_fits && C <= 16);
   size_t o = 0;
   s.f0pad = o; o = align256(o + size_t(band_rows + w - 1) * (cols + w - 1) * 64 * 2);
   s.p2 = s.spe = s.hidden = s.x16 = s.h16 = s.g = s.pm = s.yq = s.lmap = 0;
   s.chunk = n < 16384 ? n : 16384;
-  if (s.tc) {
+  if (tc_fits) {
     s.x16 = o; o = align256(o + size_t(mtiles) * (((B + 15) / 16) * 2) * 2048);
-    s.h16 = o; o = align256(o + size_t(4) * mtiles * 128 * 64);   // partial spectral logits f32 [4 quarters][mtiles*128][16]
+    s.h16 = o; o = align256(o + size_t(4) * mtiles * 128 * NC * 4);   // partial spectral logits f32 [4 quarters][mtiles*128][NC]
   }
   if (s.dense) {
     const size_t qpos = size_t(4) * ((band_rows + w) / 2) * ((cols + w) / 2);     // positions of the 4 parity planes
     s.g = o;                                               // (fp32 conv1 variants: not materialised any more)
     s.pm = o; o = align256(o + qpos * 9 * 64 * 2);         // pooled variants, f16 parity planes [9][4][8][PR2][PC2][8]
     s.yq = o; o = align256(o + qpos * 9 * 64 * 2);         // half-pooled conv2 maps, f16 [9][4][8][PR2][PC2][8]
-    s.lmap = o; o = align256(o + qpos * 5 * 16 * 4);       // class partials per pooled row, f32 [4][5][4][PR2][PC2][4]
+    s.lmap = o; o = align256(o + qpos * 5 * NC * 4);       // class partials per pooled row, f32 [4][5][NC/4][PR2][PC2][4]
   } else {
     s.p2 = o; o = align256(o + size_t(n) * P * 64 * 2);     // per-pixel pooled conv features (patch_cnn_sm100.cu)
     if (!s.tc) {
@@ -258,6 +262,7 @@ extern "C" int cmlpl_spectral_head_f32(const float* spectra, int64_t n, int num_
 static int classify_launch(const void* p2, const float* spe_logits, const float* part, int64_t part_stride, int64_t n,
                            int num_features, int num_classes, int w, const void* packed, uint8_t* labels, float* logits,
                            cmlpl_stream_t stream) {
+  const int part_width = class_width(num_classes);        // row width of spectral_logits_kernel's partials
   CMLPL_CHECK_ARG(p2 && packed && labels, "classify: null pointer");
   CMLPL_CHECK_ARG(n >= 0 && num_classes > 0 && num_classes <= 32 && w >= 4, "classify: bad dims (C=%d w=%d)",
                   num_classes, w);
@@ -272,11 +277,11 @@ static int classify_launch(const void* p2, const float* spe_logits, const float*
   if (grid > cap) grid = cap;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (num_classes <= 16)
-    classify_kernel<16><<<int(grid), 256, 0, s>>>(static_cast<const __half*>(p2), spe_logits, part, part_stride, n, K,
-                                                  num_classes, wc, bc, labels, logits);
+    classify_kernel<16><<<int(grid), 256, 0, s>>>(static_cast<const __half*>(p2), spe_logits, part, part_stride, part_width, n,
+                                                  K, num_classes, wc, bc, labels, logits);
   else
-    classify_kernel<32><<<int(grid), 256, 0, s>>>(static_cast<const __half*>(p2), spe_logits, part, part_stride, n, K,
-                                                  num_classes, wc, bc, labels, logits);
+    classify_kernel<32><<<int(grid), 256, 0, s>>>(static_cast<const __half*>(p2), spe_logits, part, part_stride, part_width, n,
+                                                  K, num_classes, wc, bc, labels, logits);
   CMLPL_CHECK_LAUNCH("classify");
   return CMLPL_OK;
 }
@@ -368,7 +373,7 @@ extern "C" int cmlpl_scene_infer_raw(const void* raw, int dtype, int scene_rows,
   CMLPL_CHECK_ARG(dtype == 0 || dtype == 1, "scene_infer_raw: dtype must be 0 (uint16) or 1 (float32)");
   CMLPL_CHECK_ARG(w == 20 || w == 11, "scene_infer_raw: w=%d unsupported (20, or 11 for the odd-window variant)", w);
   CMLPL_CHECK_ARG(band_rows > 0 && cols > 0 && num_classes > 0 && num_features > 0, "scene_infer_raw: bad dims");
-  CMLPL_CHECK_ARG(use_tc_head(num_features, num_classes), "scene_infer_raw: needs <= 16 classes and <= 224 bands");
+  CMLPL_CHECK_ARG(tc_spectral_fits(num_features, num_classes), "scene_infer_raw: needs <= 32 classes and <= 224 bands");
   CMLPL_CHECK_ARG(w / 2 <= scene_rows && w / 2 <= cols, "scene_infer_raw: window larger than the scene");
   CMLPL_CHECK_ARG(band_row0 >= 0 && band_row0 + band_rows <= scene_rows, "scene_infer_raw: band outside the scene");
   const int a = band_row0 + window_lo(w), b = band_row0 + band_rows - 1 + window_lo(w) + w - 1;

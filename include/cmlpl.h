@@ -103,8 +103,9 @@ int cmlpl_l2norm_bwd_f32(const float* y, const float* norm, const float* dy, flo
  * the classifier are evaluated ONCE PER SCENE POSITION in the 9 / 25 classes of how a patch border can
  * cut them (exact compute sharing; persistent tcgen05 kernels fed by TMA tile loads); the spectral
  * branch is one fused two-GEMM kernel; a sum head adds each pixel's 25 gathered conv partials to its
- * spectral partials and takes the argmax.  > 16 classes or > 224 bands fall back to the all-per-pixel
- * tcgen05 kernel (patch window staged in shared memory) and CUDA-core heads.
+ * spectral partials and takes the argmax.  This path takes up to 32 classes (class width 16 up to 16 classes, 32
+ * beyond); > 32 classes or > 224 bands fall back to the all-per-pixel tcgen05 kernel (patch window staged in shared
+ * memory) and CUDA-core heads, and cmlpl_scene_infer / cmlpl_scene_infer_raw refuse more than 32 classes.
  *
  * Packed weights: cmlpl_pack_basenet2() converts the reference state_dict tensors
  * (models.py:102-127: conv0/1/2.{weight,bias}, feat_spe.*, classifier.*) into the
@@ -119,17 +120,19 @@ int cmlpl_pack_basenet2(const float* conv0_w, const float* conv0_b,
                         int num_features, int num_classes, int w,
                         void* packed, cmlpl_stream_t stream);
 
-/* Which kernels cmlpl_scene_infer / cmlpl_scene_infer_raw run on the tensor-core path (<= 16 classes, <= 224 bands), per
+/* Which kernels cmlpl_scene_infer / cmlpl_scene_infer_raw run on the tensor-core path (<= 32 classes, <= 224 bands), per
  * calling host thread: 1 (default) = the scene-level kernels with exact compute sharing (w = 20 and w = 11), 0 = the
  * per-pixel kernels (patch_cnn_kernel<w> per pixel; the independent implementation the tests compare the default against,
- * models.py:133-150 per patch).  The workspace size and layout follow the mode: set it before sizing the workspace. */
+ * models.py:133-150 per patch; at 17-32 classes with the CUDA-core heads, the raw entry point with the tensor-core
+ * spectral branch).  The workspace size and layout follow the mode: set it before sizing the workspace. */
 int cmlpl_set_scene_path_mode(int mode);
 
 /* Workspace needed to infer `band_rows` rows of a scene with `cols` columns. */
 size_t cmlpl_scene_workspace_bytes(int band_rows, int cols, int num_features, int num_classes, int w);
 
 /* Byte offsets of the workspace regions (for stage-level profiling): offsets[12] =
- * {f0pad, x16, h16 (partial spectral logits f32 [4][ceil(n/128)*128][16] on the dense path), g (unused, zero-sized),
+ * {f0pad, x16, h16 (partial spectral logits f32 [4][ceil(n/128)*128][NC], NC = 16 for <= 16 classes, 32 for 17-32),
+ *  g (unused, zero-sized),
  *  pmq, yq, lmap, p2, spe_logits, hidden, total, uses_tensor_core_path}. */
 int cmlpl_scene_workspace_layout(int band_rows, int cols, int num_features, int num_classes, int w,
                                  size_t* offsets);
@@ -145,7 +148,7 @@ int cmlpl_scene_infer(const float* cube, int scene_rows, int cols, int slab_row0
                       void* workspace, size_t workspace_bytes,
                       uint8_t* labels, float* logits, cmlpl_stream_t stream);
 
-/* The same from the RAW cube (dtype 0 = uint16, 1 = float32; <= 16 classes, <= 224 bands): the PCA
+/* The same from the RAW cube (dtype 0 = uint16, 1 = float32; <= 32 classes, <= 224 bands): the PCA
  * projection and both z-scores of tools/hyper_tools.py:285-292 are folded into conv0
  * (wf f32 [B][64] = (W0 . (U/s)^T)^T, bf f32 [64] = b0 - W0 . m/s) and into the fp16 conversion of the
  * spectral branch (mu, inv_sigma f32 [B]); neither the PCA cube nor the z-scored spectra touch HBM.
@@ -200,7 +203,8 @@ int cmlpl_conv1_scene_f16(const void* f0pad, int cols, int w, int band_rows, con
  *                                   yq[Al][Be][y',x'] = mean over the border partners of Y[rho][kap][y'+u, x'+v]
  *   cmlpl_pool2_cls_f16           : rest of the 2x2 avg-pool (middle classes) + conv columns of the classifier per
  *                                   pooled cell (I,J), summed over the pooled columns J of a pooled row I:
- *                                   lmap f32 [4][5 = I][4 class quads][PR2][PC2][4],
+ *                                   lmap f32 [4][5 = I][NC/4 class quads][PR2][PC2][4] (NC = 16 up to 16 classes, 32 for
+ *                                   17-32),
  *                                   lmap[I][y',x'] = sum_J L[I][J][y', x'+2J] */
 int cmlpl_conv1_scene_variants_f32(const void* f0pad, int cols, int w, int band_rows, const void* packed, float* g,
                                    cmlpl_stream_t stream);
@@ -215,8 +219,9 @@ int cmlpl_conv2_scene_f16(const void* pmq, int cols, int w, int band_rows, const
 int cmlpl_pool2_cls_f16(const void* yq, int cols, int w, int band_rows, int num_features, int num_classes,
                         const void* packed, float* lmap, cmlpl_stream_t stream);
 /* Fused spectral branch + sum head (what cmlpl_scene_infer runs since the hidden features stopped going through HBM):
- *   cmlpl_spectral_logits_tc     : part f32 [4 hidden quarters][ceil(n/128)*128][16] = Wc_spe . relu(Wspe . x + b) per
- *                                  quarter of the 1024 hidden features (tools/models.py:142-143,150), <= 224 bands
+ *   cmlpl_spectral_logits_tc     : part f32 [4 hidden quarters][ceil(n/128)*128][NC] = Wc_spe . relu(Wspe . x + b) per
+ *                                  quarter of the 1024 hidden features (tools/models.py:142-143,150), <= 224 bands,
+ *                                  <= 32 classes (NC = 16 up to 16 classes, 32 for 17-32)
  *   cmlpl_spectral_logits_raw_tc : the same from the raw cube (z-score folded into the fp16 conversion)
  *   cmlpl_head_sum_lmap          : 4 quarter partials + the 5 gathered conv partials + bias, argmax */
 int cmlpl_spectral_logits_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
