@@ -92,7 +92,7 @@ constexpr int kEpiWarps = kEpiThreads / 32, kLoadWarp0 = kEpiWarps, kMmaWarp = k
   } while (0)
 
 // TRAIN = the forward trunk of the fused training step (tools/models.py:133-140 in batch mode): every "pixel" is one
-// sample of one of the two BaseNet2 peers whose conv0 output a0 [8 chunks][20x20][8] lies in the workspace.  The CTAs
+// sample of one of the two BaseNet2 peers whose conv0 output a0 [8 chunks][W x W][8] lies in the workspace.  The CTAs
 // are split between the nets (each keeps ONE net's weights, converted from the fp32 parameters in the prologue) and
 // the epilogues additionally save what the backward pass needs: the ReLU masks of both blocks as bits, the pooled
 // conv1 output p1 (B operand of conv2's weight gradient) and the pooled conv2 output as fp32 in the classifier's
@@ -104,6 +104,7 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
                  const float* __restrict__ b1g, const float* __restrict__ b2g, __half* __restrict__ p2out,
                  int p2_tiled, long long* __restrict__ trace, TrainCnnArgs ta) {
   using Cfg = PatchCfg<W>;
+  using G = TrainGeom<W>;
   extern __shared__ __align__(128) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem);
@@ -185,7 +186,7 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
     for (int64_t p = p_begin; p < p_end; ++p, ph ^= 1) {
       const __half* src;
       if constexpr (TRAIN) {
-        src = ta.a0 + p * int64_t(kActBytes / 2);
+        src = ta.a0 + p * int64_t(G::ActBytes / 2);
       } else {
         const int rb = int(p / cols), c = int(p - int64_t(rb) * cols);
         src = f0pad + (int64_t(rb) * pitch + c) * 8;
@@ -288,6 +289,18 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
       out_hi = *reinterpret_cast<uint4*>(&hv[4]);
     };
     for (int64_t p = p_begin; p < p_end; ++p, ph ^= 1) {
+      if constexpr (TRAIN && (W & 1)) {
+        // floor pooling drops the last row / column of both maps: no gradient reaches them, so their ReLU mask bits
+        // are stored as 0 (m1: 2W-1 positions, m2: 2*H2-1 positions, two words each)
+        if (tid < 2 * (2 * W - 1)) {
+          const int k = tid >> 1, y = k < W ? W - 1 : k - W, x = k < W ? k : W - 1;
+          ta.m1[(p * G::TPos + y * W + x) * 2 + (tid & 1)] = 0u;
+        }
+        if (tid < 2 * (2 * Cfg::H2 - 1)) {
+          const int k = tid >> 1, y = k < Cfg::H2 ? Cfg::H2 - 1 : k - Cfg::H2, x = k < Cfg::H2 ? k : Cfg::H2 - 1;
+          ta.m2[(p * G::TPos2 + y * Cfg::H2 + x) * 2 + (tid & 1)] = 0u;
+        }
+      }
       mbar_wait(bars + 8 * BAR_A1_FULL, ph, 9);             // the residuals are read back from A1
       // ------------------------------------------------ conv1 epilogue -> A2 (pooled, fp16)
 #pragma unroll 1
@@ -344,12 +357,12 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
         uint32_t me = mbits_e, mo = mbits_o;
         unsigned char* p1g = nullptr;
         if constexpr (TRAIN) {
-          // pooled conv1 output of this sample: p1 [8 chunks][10x10][8]
-          p1g = reinterpret_cast<unsigned char*>(ta.p1) + p * int64_t(kAct2Bytes) + (chalf * 4) * (kTPos2 * 16) +
+          // pooled conv1 output of this sample: p1 [8 chunks][(W/2)x(W/2)][8]
+          p1g = reinterpret_cast<unsigned char*>(ta.p1) + p * int64_t(G::Act2Bytes) + (chalf * 4) * (G::TPos2 * 16) +
                 (i * (W / 2) + (x >> 1)) * 16;
           if (writer) {
             *reinterpret_cast<uint4*>(p1g) = w0;
-            *reinterpret_cast<uint4*>(p1g + kTPos2 * 16) = w1;
+            *reinterpret_cast<uint4*>(p1g + G::TPos2 * 16) = w1;
           }
         }
         if (tid == 0 && h == 0) CMLPL_TRACE(15);
@@ -365,11 +378,11 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
         }
         if constexpr (TRAIN) {
           if (writer) {
-            *reinterpret_cast<uint4*>(p1g + 2 * kTPos2 * 16) = w0;
-            *reinterpret_cast<uint4*>(p1g + 3 * kTPos2 * 16) = w1;
+            *reinterpret_cast<uint4*>(p1g + 2 * G::TPos2 * 16) = w0;
+            *reinterpret_cast<uint4*>(p1g + 3 * G::TPos2 * 16) = w1;
           }
           if (valid) {   // m1 [sample][y][x][half]: bit c%32 of word c/32 = (a1[c][y][x] > 0), rows y = 2i, 2i+1
-            uint32_t* mg = ta.m1 + (p * kTPos + (2 * i) * W + x) * 2 + chalf;
+            uint32_t* mg = ta.m1 + (p * G::TPos + (2 * i) * W + x) * 2 + chalf;
             mg[0] = me | (mbits_e << 16);
             mg[2 * W] = mo | (mbits_o << 16);
           }
@@ -418,8 +431,8 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
         uint32_t me = mbits_e, mo = mbits_o;
         float* catg = nullptr;
         if constexpr (TRAIN) {
-          // flatten order of tools/models.py:141: feature = channel * 25 + pooled position
-          catg = ta.cat + p * int64_t(kCatDim) + (chalf * 32) * Cfg::P + pos;
+          // flatten order of tools/models.py:141: feature = channel * P + pooled position (P = 25, or 4 at W = 11)
+          catg = ta.cat + p * int64_t(G::CatDim) + (chalf * 32) * Cfg::P + pos;
           if (writer) {
 #pragma unroll
             for (int j = 0; j < 16; ++j) catg[j * Cfg::P] = pooled[j];
@@ -438,8 +451,8 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
 #pragma unroll
             for (int j = 0; j < 16; ++j) catg[(16 + j) * Cfg::P] = pooled[j];
           }
-          if (valid) {   // m2 [sample][y][x][half], rows y = 2i, 2i+1 of the 10x10 conv2 output
-            uint32_t* mg = ta.m2 + (p * kTPos2 + (2 * i) * Cfg::H2 + x) * 2 + chalf;
+          if (valid) {   // m2 [sample][y][x][half], rows y = 2i, 2i+1 of the H2 x H2 conv2 output
+            uint32_t* mg = ta.m2 + (p * G::TPos2 + (2 * i) * Cfg::H2 + x) * 2 + chalf;
             mg[0] = me | (mbits_e << 16);
             mg[2 * Cfg::H2] = mo | (mbits_o << 16);
           }
@@ -502,13 +515,18 @@ static int launch_patch_cnn(const void* f0pad, int cols, int w, int band_rows, c
 }
 
 namespace cmlpl {
-int launch_train_cnn(const TrainCnnArgs& ta, cudaStream_t st) {
-  using Cfg = PatchCfg<20>;
-  auto kern = patch_cnn_kernel<20, false, true>;
-  CMLPL_MAX_DYN_SMEM(kern, Cfg::SMEM);
+int launch_train_cnn(const TrainCnnArgs& ta, int w, cudaStream_t st) {
   int grid = sm_count() & ~1;                       // split evenly between the two nets
   if (grid > 2 * ta.nb) grid = 2 * ta.nb;
-  kern<<<grid, kThreads, Cfg::SMEM, st>>>(nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr, ta);
+  if (w == 11) {
+    auto kern = patch_cnn_kernel<11, false, true>;
+    CMLPL_MAX_DYN_SMEM(kern, PatchCfg<11>::SMEM);
+    kern<<<grid, kThreads, PatchCfg<11>::SMEM, st>>>(nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr, ta);
+  } else {
+    auto kern = patch_cnn_kernel<20, false, true>;
+    CMLPL_MAX_DYN_SMEM(kern, PatchCfg<20>::SMEM);
+    kern<<<grid, kThreads, PatchCfg<20>::SMEM, st>>>(nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr, ta);
+  }
   CMLPL_CHECK_LAUNCH("train_cnn");
   return CMLPL_OK;
 }

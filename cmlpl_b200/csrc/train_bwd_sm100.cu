@@ -15,6 +15,9 @@
 //   * the bias gradient, as one more N=8 MMA per K-step against a plane of ones.
 // Gradient operands are multiplied by a power of two S (grad_scale) so they sit in fp16's normal range; S is undone on
 // the fp32 results.  (Layout facts verified on hardware by scripts/micro/mn_major_probe.cu.)
+// H = 10 / 20 are conv2 / conv1 of the w = 20 net, H = 5 / 11 those of the w = 11 net.  Odd maps are pooled with floor
+// semantics (avg_pool2d): the last row / column gets no upstream gradient, but stays a conv output whose data gradient
+// (from its neighbours' taps) and residual fan-out are formed like any other position's.
 #include "common.cuh"
 #include "sm100_ptx.cuh"
 #include "train_common.cuh"
@@ -60,6 +63,9 @@ template <int H>
 __global__ void __launch_bounds__(kBwdThreads, 1)
 train_conv_bwd_kernel(ConvBwdArgs a) {
   using C = BwdCfg<H>;
+  constexpr bool kConv2 = H == 10 || H == 5;             // conv2 of the window W = 20 / 11; otherwise conv1, H = W
+  constexpr int W = H == 5 ? 11 : H == 10 ? 20 : H;
+  using G = TrainGeom<W>;
   extern __shared__ __align__(128) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem);
@@ -156,37 +162,49 @@ train_conv_bwd_kernel(ConvBwdArgs a) {
         mbar_wait(bars + 8 * BB_W_DONE, (k - 1) & 1, 52);              // every MMA of the previous sample has read the planes
         named_bar_sync(1, kBwdWorkers);                                // ... and every worker its residual entries
       }
-      if constexpr (H == 10) {
-        // dz2 = dL/dp2 / 4 * [a2 > 0] (pool + ReLU backward, tools/models.py:139-140), scaled, and the p1 planes
-        const float* dc = a.dcat + s * kCatDim;
-        const uint32_t* m2 = a.m2 + s * (kTPos2 * 2);
-        const unsigned char* pg = reinterpret_cast<const unsigned char*>(a.act) + s * kAct2Bytes;
+      if constexpr (kConv2) {
+        // dz2 = dL/dp2 / 4 * [a2 > 0] (pool + ReLU backward, tools/models.py:139-140), scaled, and the p1 planes.
+        // Odd H: the floor pool drops the last row / column, where dz2 = 0.
+        constexpr int NP = G::NP2, P = NP * NP;
+        const float* dc = a.dcat + s * G::CatDim;
+        const uint32_t* m2 = a.m2 + s * (G::TPos2 * 2);
+        const unsigned char* pg = reinterpret_cast<const unsigned char*>(a.act) + s * G::Act2Bytes;
         const float q = 0.25f * S;
-        for (int i = tid; i < 8 * kTPos2; i += kBwdWorkers) {
-          const int chunk = i / kTPos2, pos = i - chunk * kTPos2;
-          const int y = pos / 10, x = pos - y * 10;
+        for (int i = tid; i < 8 * G::TPos2; i += kBwdWorkers) {
+          const int chunk = i / G::TPos2, pos = i - chunk * G::TPos2;
+          const int y = pos / H, x = pos - y * H;
           const int ent = (y + 1) * C::PW + x + 1;
-          cp_async16(sbase + C::S_ACT + chunk * C::CH + ent * 16, pg + (chunk * kTPos2 + pos) * 16);
-          const uint32_t bits = m2[pos * 2 + (chunk >> 2)] >> ((chunk & 3) * 8);
-          const float* d = dc + (chunk * 8) * 25 + (y >> 1) * 5 + (x >> 1);
+          cp_async16(sbase + C::S_ACT + chunk * C::CH + ent * 16, pg + (chunk * G::TPos2 + pos) * 16);
+          const bool kept = H % 2 == 0 || (y < 2 * NP && x < 2 * NP);
+          const uint32_t bits = kept ? m2[pos * 2 + (chunk >> 2)] >> ((chunk & 3) * 8) : 0u;
+          const float* d = dc + (chunk * 8) * P + (y >> 1) * NP + (x >> 1);
           __half2 h[4];
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
-            const float v0 = (bits >> (2 * j)) & 1u ? __ldg(d + (2 * j) * 25) * q : 0.f;
-            const float v1 = (bits >> (2 * j + 1)) & 1u ? __ldg(d + (2 * j + 1) * 25) * q : 0.f;
+            const float v0 = (bits >> (2 * j)) & 1u ? __ldg(d + (2 * j) * P) * q : 0.f;
+            const float v1 = (bits >> (2 * j + 1)) & 1u ? __ldg(d + (2 * j + 1) * P) * q : 0.f;
             h[j] = __floats2half2_rn(v0, v1);
           }
           *reinterpret_cast<uint4*>(smem + C::S_DZ + chunk * C::CH + ent * 16) = *reinterpret_cast<uint4*>(h);
         }
+        if constexpr (W % 2 == 1) {
+          // conv1's last row / column feed no pooling window: dz1 there is 0 (written here, read by conv1's backward)
+          unsigned char* zg = reinterpret_cast<unsigned char*>(a.dz_out) + s * G::ActBytes;
+          for (int i = tid; i < 8 * (2 * W - 1); i += kBwdWorkers) {
+            const int chunk = i / (2 * W - 1), k = i - chunk * (2 * W - 1);
+            const int y = k < W ? W - 1 : k - W, x = k < W ? k : W - 1;
+            *reinterpret_cast<uint4*>(zg + (chunk * G::TPos + y * W + x) * 16) = make_uint4(0, 0, 0, 0);
+          }
+        }
       } else {
-        const unsigned char* zg = reinterpret_cast<const unsigned char*>(a.dz_in) + s * kActBytes;
-        const unsigned char* ag = reinterpret_cast<const unsigned char*>(a.act) + s * kActBytes;
-        for (int i = tid; i < 8 * kTPos; i += kBwdWorkers) {
-          const int chunk = i / kTPos, pos = i - chunk * kTPos;
-          const int y = pos / 20, x = pos - y * 20;
+        const unsigned char* zg = reinterpret_cast<const unsigned char*>(a.dz_in) + s * G::ActBytes;
+        const unsigned char* ag = reinterpret_cast<const unsigned char*>(a.act) + s * G::ActBytes;
+        for (int i = tid; i < 8 * G::TPos; i += kBwdWorkers) {
+          const int chunk = i / G::TPos, pos = i - chunk * G::TPos;
+          const int y = pos / H, x = pos - y * H;
           const int ent = (y + 1) * C::PW + x + 1;
-          cp_async16(sbase + C::S_DZ + chunk * C::CH + ent * 16, zg + (chunk * kTPos + pos) * 16);
-          cp_async16(sbase + C::S_ACT + chunk * C::CH + ent * 16, ag + (chunk * kTPos + pos) * 16);
+          cp_async16(sbase + C::S_DZ + chunk * C::CH + ent * 16, zg + (chunk * G::TPos + pos) * 16);
+          cp_async16(sbase + C::S_ACT + chunk * C::CH + ent * 16, ag + (chunk * G::TPos + pos) * 16);
         }
       }
       cp_async_wait_all();
@@ -221,13 +239,13 @@ train_conv_bwd_kernel(ConvBwdArgs a) {
           v[2 * j] += f.x; v[2 * j + 1] += f.y;
         }
         if (!valid) continue;
-        if constexpr (H == 10) {
-          // dL/dp1 (scaled) -> pool backward to the four 20x20 positions, ReLU mask of a1 -> dz1 (scaled)
-          unsigned char* og = reinterpret_cast<unsigned char*>(a.dz_out) + s * kActBytes + (chalf * 4) * (kTPos * 16);
-          const uint32_t* m1 = a.m1 + s * (kTPos * 2) + chalf;
+        if constexpr (kConv2) {
+          // dL/dp1 (scaled) -> pool backward to the four W x W positions, ReLU mask of a1 -> dz1 (scaled)
+          unsigned char* og = reinterpret_cast<unsigned char*>(a.dz_out) + s * G::ActBytes + (chalf * 4) * (G::TPos * 16);
+          const uint32_t* m1 = a.m1 + s * (G::TPos * 2) + chalf;
 #pragma unroll
           for (int ab = 0; ab < 4; ++ab) {
-            const int pos = (2 * y + (ab >> 1)) * 20 + 2 * x + (ab & 1);
+            const int pos = (2 * y + (ab >> 1)) * W + 2 * x + (ab & 1);
             const uint32_t bits = m1[pos * 2];
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
@@ -237,18 +255,18 @@ train_conv_bwd_kernel(ConvBwdArgs a) {
                 const int b = c * 8 + 2 * j;
                 h[j] = __floats2half2_rn((bits >> b) & 1u ? v[b] * 0.25f : 0.f, (bits >> (b + 1)) & 1u ? v[b + 1] * 0.25f : 0.f);
               }
-              *reinterpret_cast<uint4*>(og + c * (kTPos * 16) + pos * 16) = *reinterpret_cast<uint4*>(h);
+              *reinterpret_cast<uint4*>(og + c * (G::TPos * 16) + pos * 16) = *reinterpret_cast<uint4*>(h);
             }
           }
         } else {
-          unsigned char* og = reinterpret_cast<unsigned char*>(a.dz_out) + s * kActBytes + (chalf * 4) * (kTPos * 16) +
-                              (y * 20 + x) * 16;
+          unsigned char* og = reinterpret_cast<unsigned char*>(a.dz_out) + s * G::ActBytes + (chalf * 4) * (G::TPos * 16) +
+                              (y * H + x) * 16;
 #pragma unroll
           for (int c = 0; c < 4; ++c) {
             __half2 h[4];
 #pragma unroll
             for (int j = 0; j < 4; ++j) h[j] = __floats2half2_rn(v[c * 8 + 2 * j], v[c * 8 + 2 * j + 1]);
-            *reinterpret_cast<uint4*>(og + c * (kTPos * 16)) = *reinterpret_cast<uint4*>(h);
+            *reinterpret_cast<uint4*>(og + c * (G::TPos * 16)) = *reinterpret_cast<uint4*>(h);
           }
         }
       }
@@ -284,38 +302,57 @@ train_conv_bwd_kernel(ConvBwdArgs a) {
   if (warp == 8) { tc_fence_after(); tmem_dealloc(tmem, 512); }
 }
 
+template <int H>
+static int launch_conv_bwd_h(const ConvBwdArgs& a, int grid, cudaStream_t st) {
+  auto kern = train_conv_bwd_kernel<H>;
+  CMLPL_MAX_DYN_SMEM(kern, BwdCfg<H>::SMEM);
+  kern<<<grid, kBwdThreads, BwdCfg<H>::SMEM, st>>>(a);
+  return CMLPL_OK;
+}
+
+// H = 10 / 20: conv2 / conv1 of the w = 20 net; H = 5 / 11: of the w = 11 net
 int launch_train_conv_bwd(int H, const ConvBwdArgs& a, cudaStream_t st) {
   int grid = sm_count() & ~1;
   if (grid > 2 * a.nb) grid = 2 * a.nb;
-  if (H == 10) {
-    auto kern = train_conv_bwd_kernel<10>;
-    CMLPL_MAX_DYN_SMEM(kern, BwdCfg<10>::SMEM);
-    kern<<<grid, kBwdThreads, BwdCfg<10>::SMEM, st>>>(a);
-  } else {
-    auto kern = train_conv_bwd_kernel<20>;
-    CMLPL_MAX_DYN_SMEM(kern, BwdCfg<20>::SMEM);
-    kern<<<grid, kBwdThreads, BwdCfg<20>::SMEM, st>>>(a);
+  int rc;
+  switch (H) {
+    case 10: rc = launch_conv_bwd_h<10>(a, grid, st); break;
+    case 20: rc = launch_conv_bwd_h<20>(a, grid, st); break;
+    case 5: rc = launch_conv_bwd_h<5>(a, grid, st); break;
+    case 11: rc = launch_conv_bwd_h<11>(a, grid, st); break;
+    default: CMLPL_CHECK_ARG(false, "train_conv_bwd: H=%d unsupported", H);
   }
+  if (rc != CMLPL_OK) return rc;
   CMLPL_CHECK_LAUNCH("train_conv_bwd");
   return CMLPL_OK;
 }
 
 // ============================================================================ conv0 weight gradient
 // dW0[co][ci] = sum_{sample,pos} da0[pos][co] * x16[pos][ci], db0 = sum da0: both operands are unpadded chunk planes
-// in HBM, so a sample is two contiguous 51 200-byte bulk copies into a two-stage ring; 25 K-steps of one M=64 N=64
-// and one N=8 (ones) MMA.
-namespace c0b {
-constexpr int STAGE = 2 * kActBytes;
-constexpr int S_ONES = 2 * STAGE;
-constexpr int S_BAR = S_ONES + 256;
-constexpr int S_TMEM = S_BAR + 64;
-constexpr int SMEM = (S_TMEM + 16 + 127) / 128 * 128;
-enum { B_FULL0 = 0, B_FULL1, B_EMPTY0, B_EMPTY1, B_DONE };
-}  // namespace c0b
+// in HBM, so a sample is 2 x 8 bulk copies of its chunk planes into a two-stage ring; one M=64 N=64 and one N=8 (ones)
+// MMA per K-step of 16 positions (25 at W = 20).  At W = 11 the 121 positions take 8 K-steps: a staged plane is padded
+// to 128 positions whose zero tail (never written by the copies) adds nothing.
+template <int W>
+struct C0bCfg {
+  using G = TrainGeom<W>;
+  static constexpr int KS = (G::TPos + 15) / 16;        // K-steps per sample
+  static constexpr int GCH = G::TPos * 16;              // chunk plane in HBM (bytes)
+  static constexpr int PCH = KS * 256;                  // chunk plane in shared memory
+  static constexpr int STAGE = 2 * 8 * PCH;             // da0 planes, then x16 planes
+  static constexpr int S_ONES = 2 * STAGE;
+  static constexpr int S_BAR = S_ONES + 256;
+  static constexpr int S_TMEM = S_BAR + 64;
+  static constexpr int SMEM = (S_TMEM + 16 + 127) / 128 * 128;
+};
+enum { C0B_FULL0 = 0, C0B_FULL1, C0B_EMPTY0, C0B_EMPTY1, C0B_DONE };
 
+template <int W>
 __global__ void __launch_bounds__(128, 1)
 train_conv0_bwd_kernel(Conv0BwdArgs a) {
-  using namespace c0b;
+  using Cfg = C0bCfg<W>;
+  constexpr int STAGE = Cfg::STAGE, PCH = Cfg::PCH, GCH = Cfg::GCH, S_ONES = Cfg::S_ONES, S_BAR = Cfg::S_BAR,
+                S_TMEM = Cfg::S_TMEM;
+  enum { B_FULL0 = C0B_FULL0, B_FULL1 = C0B_FULL1, B_EMPTY0 = C0B_EMPTY0, B_EMPTY1 = C0B_EMPTY1, B_DONE = C0B_DONE };
   extern __shared__ __align__(128) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem);
@@ -328,6 +365,12 @@ train_conv0_bwd_kernel(Conv0BwdArgs a) {
   const int nsamp = k_end - k_begin;
   const int64_t s0 = int64_t(net) * a.nb + k_begin;
   reinterpret_cast<__half*>(smem + S_ONES)[tid] = __float2half_rn(1.f);
+  if constexpr (PCH > GCH) {
+    for (int i = tid; i < 2 * 2 * 8 * (PCH - GCH) / 16; i += 128) {     // zero tails of every staged plane
+      const int plane = i / ((PCH - GCH) / 16), j = i - plane * ((PCH - GCH) / 16);
+      reinterpret_cast<uint4*>(smem + plane * PCH + GCH)[j] = make_uint4(0, 0, 0, 0);
+    }
+  }
   // the 3x3 weight gradients train_conv_bwd_kernel staged as [net][conv][tap][co][ci] -> torch's [co][ci][3][3]
   for (int i = blockIdx.x * 128 + tid; i < 4 * 36864; i += int(gridDim.x) * 128) {
     const int t4 = i / 36864, j = i - t4 * 36864;                   // j = (tap * 64 + co) * 64 + ci, coalesced read
@@ -351,12 +394,12 @@ train_conv0_bwd_kernel(Conv0BwdArgs a) {
       const int st = k & 1;
       mbar_wait(bars + 8 * (B_EMPTY0 + st), ((k >> 1) & 1) ^ 1, 60);
       const uint32_t full = bars + 8 * (B_FULL0 + st);
-      mbar_arrive_expect_tx(full, STAGE);
-      const unsigned char* g0 = reinterpret_cast<const unsigned char*>(a.da0) + (s0 + k) * kActBytes;
-      const unsigned char* g1 = reinterpret_cast<const unsigned char*>(a.x16) + (s0 + k) * kActBytes;
-      for (int o = 0; o < kActBytes; o += 6400) {
-        bulk_g2s(sbase + st * STAGE + o, g0 + o, 6400, full);
-        bulk_g2s(sbase + st * STAGE + kActBytes + o, g1 + o, 6400, full);
+      mbar_arrive_expect_tx(full, 2 * 8 * GCH);
+      const unsigned char* g0 = reinterpret_cast<const unsigned char*>(a.da0) + (s0 + k) * (8 * GCH);
+      const unsigned char* g1 = reinterpret_cast<const unsigned char*>(a.x16) + (s0 + k) * (8 * GCH);
+      for (int c = 0; c < 8; ++c) {
+        bulk_g2s(sbase + st * STAGE + c * PCH, g0 + c * GCH, GCH, full);
+        bulk_g2s(sbase + st * STAGE + 8 * PCH + c * PCH, g1 + c * GCH, GCH, full);
       }
     }
   } else if (warp == 2 && lane == 0) {
@@ -367,10 +410,10 @@ train_conv0_bwd_kernel(Conv0BwdArgs a) {
       mbar_wait(bars + 8 * (B_FULL0 + st), (k >> 1) & 1, 61);
       tc_fence_after();
 #pragma unroll 1
-      for (int ks = 0; ks < 25; ++ks) {
+      for (int ks = 0; ks < Cfg::KS; ++ks) {
         const uint32_t acc = (k | ks) != 0 ? 1u : 0u;
-        const uint64_t da = make_desc(sbase + st * STAGE + ks * 256, 128, 6400);
-        umma_f16(tmem, da, make_desc(sbase + st * STAGE + kActBytes + ks * 256, 128, 6400), kIdW, acc);
+        const uint64_t da = make_desc(sbase + st * STAGE + ks * 256, 128, PCH);
+        umma_f16(tmem, da, make_desc(sbase + st * STAGE + 8 * PCH + ks * 256, 128, PCH), kIdW, acc);
         umma_f16(tmem + 64, da, make_desc(sbase + S_ONES, 128, 128), kIdB, acc);
       }
       umma_commit(bars + 8 * (B_EMPTY0 + st));
@@ -398,11 +441,18 @@ train_conv0_bwd_kernel(Conv0BwdArgs a) {
   if (warp == 0) { tc_fence_after(); tmem_dealloc(tmem, 128); }
 }
 
-int launch_train_conv0_bwd(const Conv0BwdArgs& a, cudaStream_t st) {
+int launch_train_conv0_bwd(const Conv0BwdArgs& a, int w, cudaStream_t st) {
   int grid = sm_count() & ~1;
   if (grid > 2 * a.nb) grid = 2 * a.nb;
-  CMLPL_MAX_DYN_SMEM(train_conv0_bwd_kernel, c0b::SMEM);
-  train_conv0_bwd_kernel<<<grid, 128, c0b::SMEM, st>>>(a);
+  if (w == 11) {
+    auto kern = train_conv0_bwd_kernel<11>;
+    CMLPL_MAX_DYN_SMEM(kern, C0bCfg<11>::SMEM);
+    kern<<<grid, 128, C0bCfg<11>::SMEM, st>>>(a);
+  } else {
+    auto kern = train_conv0_bwd_kernel<20>;
+    CMLPL_MAX_DYN_SMEM(kern, C0bCfg<20>::SMEM);
+    kern<<<grid, 128, C0bCfg<20>::SMEM, st>>>(a);
+  }
   CMLPL_CHECK_LAUNCH("train_conv0_bwd");
   return CMLPL_OK;
 }

@@ -14,10 +14,28 @@ namespace cmlpl {
 constexpr int kTW = 20, kTPos = kTW * kTW, kTPos2 = (kTW / 2) * (kTW / 2);
 constexpr int kActBytes = 8 * kTPos * 16;     // x16 / a0 / dz1 / da0 of one sample: 51 200 B
 constexpr int kAct2Bytes = 8 * kTPos2 * 16;   // p1 of one sample: 12 800 B
-constexpr int kCatDim = 64 * 25 + 1024;       // 2624 (tools/models.py:127)
-constexpr int kConvFeat = 64 * 25;
 constexpr int kHid = 1024;
+constexpr int kCatDim = 64 * 25 + kHid;       // 2624 (tools/models.py:127)
+constexpr int kConvFeat = 64 * 25;
 constexpr int kWPackBytes = 9 * 64 * 64 * 2;  // one 3x3 conv's weights in fp16: 73 728 B
+
+// Per-window geometry of the trunk kernels.  W = 20 is the reference's BaseNet2 (the constants above, which also size
+// the workspace); W = 11 is the odd window of ExtractPatches_for_base (hyper_tools.py:300-317), whose 2x2 average pools
+// floor 11 -> 5 -> 2 and drop the last row / column of each map.  A W = 11 step runs in the W = 20 workspace at the
+// same region offsets, each region packed densely at the per-sample strides below (include/cmlpl.h).
+template <int W>
+struct TrainGeom {
+  static constexpr int TPos = W * W;                     // conv0 / conv1 positions
+  static constexpr int H2 = W / 2;                       // conv2 map
+  static constexpr int TPos2 = H2 * H2;
+  static constexpr int NP2 = H2 / 2;                     // pooled conv2 map
+  static constexpr int ActBytes = 8 * TPos * 16;         // x16 / a0 / dz1 / da0 of one sample
+  static constexpr int Act2Bytes = 8 * TPos2 * 16;       // p1 of one sample
+  static constexpr int ConvFeat = 64 * NP2 * NP2;        // flattened pooled conv2 output (tools/models.py:141)
+  static constexpr int CatDim = ConvFeat + kHid;         // classifier input
+};
+static_assert(TrainGeom<20>::CatDim == kCatDim && TrainGeom<20>::ActBytes == kActBytes, "W = 20 geometry");
+static_assert(TrainGeom<11>::CatDim == 1280 && TrainGeom<11>::ActBytes <= kActBytes, "W = 11 fits the W = 20 workspace");
 
 struct TrainWs {
   size_t x16, a0, p1, m1, m2, cat, dmask, ynoisy, norm, dlogits, dfeat, dcat, dhp, dz1, da0, S, G, dG, probs_orig, wpack, gstage, total;

@@ -8,6 +8,8 @@
 //   MMA       16 tcgen05.mma (4 position tiles x 4 K-steps, M=128 N=64 K=16) against W0 (fp32 -> fp16 in the prologue)
 //   epilogue  TMEM -> +bias -> fp16 -> a0 chunk planes in HBM (input of conv1 and B operand of conv1's weight gradient)
 // The patch is never materialised in fp32 and the noise never exists as a tensor in the Philox mode.
+// W = 11 (ExtractPatches_for_base, hyper_tools.py:300-317: rows r-5 .. r+5, the same mirror) has 121 positions: one
+// position tile, 4 MMAs.
 #include "common.cuh"
 #include "sm100_ptx.cuh"
 #include "train_common.cuh"
@@ -15,20 +17,28 @@
 
 namespace cmlpl {
 
-namespace c0 {
-constexpr int CH = kTPos * 16;                 // bytes per chunk plane (6400)
-constexpr int S_X = 0;
-constexpr int S_W = 8 * CH + 2048;             // tile 3 reads rows 400..511 of plane 7: 1792 B of slack
-constexpr int S_BIAS = S_W + 8 * 64 * 16;
-constexpr int S_BAR = S_BIAS + 256;
-constexpr int S_TMEM = S_BAR + 16;
-constexpr int SMEM = (S_TMEM + 16 + 127) / 128 * 128;
-constexpr int THREADS = 256;
-}  // namespace c0
+template <int W>
+struct C0Cfg {
+  using G = TrainGeom<W>;
+  static constexpr int CH = G::TPos * 16;        // bytes per chunk plane (6400 at W = 20)
+  static constexpr int NT = (G::TPos + 127) / 128;   // 128-row position tiles (4 at W = 20, 1 at W = 11)
+  static constexpr int S_X = 0;
+  static constexpr int S_W = 8 * CH + 2048;      // the last tile reads rows up to NT*128-1 of plane 7: slack
+  static constexpr int S_BIAS = S_W + 8 * 64 * 16;
+  static constexpr int S_BAR = S_BIAS + 256;
+  static constexpr int S_TMEM = S_BAR + 16;
+  static constexpr int SMEM = (S_TMEM + 16 + 127) / 128 * 128;
+  static_assert((NT * 128 - G::TPos) * 16 <= 2048, "tile slack");
+};
+constexpr int kC0Threads = 256;
 
-__global__ void __launch_bounds__(c0::THREADS)
+template <int W>
+__global__ void __launch_bounds__(kC0Threads)
 train_conv0_kernel(Conv0Args a) {
-  using namespace c0;
+  using G = TrainGeom<W>;
+  using Cfg = C0Cfg<W>;
+  constexpr int CH = Cfg::CH, S_X = Cfg::S_X, S_W = Cfg::S_W, S_BIAS = Cfg::S_BIAS, S_BAR = Cfg::S_BAR,
+                S_TMEM = Cfg::S_TMEM, THREADS = kC0Threads;
   extern __shared__ __align__(128) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem);
@@ -89,29 +99,29 @@ train_conv0_kernel(Conv0Args a) {
     const unsigned long long seed = a.prm->seed, offset = a.prm->offset;
     int r = 0, c = 0;
     if (a.cube) { const int64_t pix = a.pix[row]; r = int(pix / a.cols); c = int(pix - int64_t(r) * a.cols); }
-    const float* nz = a.noise ? a.noise + int64_t(s) * 60 * kTPos : nullptr;
-    unsigned char* xg = reinterpret_cast<unsigned char*>(a.x16) + int64_t(s) * kActBytes;
+    const float* nz = a.noise ? a.noise + int64_t(s) * 60 * G::TPos : nullptr;
+    unsigned char* xg = reinterpret_cast<unsigned char*>(a.x16) + int64_t(s) * G::ActBytes;
     const bool draw = a.cube && !nz && sigma != 0.f;
     // 6400 items (16 channel quads x 400 positions) / 256 threads = 25 per thread, in batches of 5 with all global
     // loads of a batch issued before any is consumed
     constexpr int U = 5;
 #pragma unroll 1
-    for (int i0 = tid; i0 < 16 * kTPos; i0 += THREADS * U) {
+    for (int i0 = tid; i0 < 16 * G::TPos; i0 += THREADS * U) {
       float4 b[U], z[U];
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const int i = i0 + u * THREADS;
-        const int q = i / kTPos, p = i - q * kTPos;        // q: group of 4 channels, p: window position
+        const int q = i / G::TPos, p = i - q * G::TPos;        // q: group of 4 channels, p: window position
         b[u] = make_float4(0.f, 0.f, 0.f, 0.f);
         z[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (i < 15 * kTPos) {
+        if (i < 15 * G::TPos) {
           if (nz) {
-            z[u].x = __ldg(nz + (4 * q + 0) * kTPos + p); z[u].y = __ldg(nz + (4 * q + 1) * kTPos + p);
-            z[u].z = __ldg(nz + (4 * q + 2) * kTPos + p); z[u].w = __ldg(nz + (4 * q + 3) * kTPos + p);
+            z[u].x = __ldg(nz + (4 * q + 0) * G::TPos + p); z[u].y = __ldg(nz + (4 * q + 1) * G::TPos + p);
+            z[u].z = __ldg(nz + (4 * q + 2) * G::TPos + p); z[u].w = __ldg(nz + (4 * q + 3) * G::TPos + p);
           }
           if (a.cube) {
-            const int y = p / kTW, x = p - y * kTW;
-            const int sr = mirror_index(r - kTW / 2 + y, a.scene_rows), sc = mirror_index(c - kTW / 2 + x, a.cols);
+            const int y = p / W, x = p - y * W;
+            const int sr = mirror_index(r - W / 2 + y, a.scene_rows), sc = mirror_index(c - W / 2 + x, a.cols);
             b[u] = __ldg(reinterpret_cast<const float4*>(a.cube + (int64_t(sr) * a.cols + sc) * 60) + q);
           }
         }
@@ -119,8 +129,8 @@ train_conv0_kernel(Conv0Args a) {
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const int i = i0 + u * THREADS;
-        if (i >= 16 * kTPos) continue;
-        const int q = i / kTPos, p = i - q * kTPos;
+        if (i >= 16 * G::TPos) continue;
+        const int q = i / G::TPos, p = i - q * G::TPos;
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
         if (q < 15) {
           if (draw) z[u] = philox_normal4(seed, offset, PHILOX_PATCH, uint32_t(s) * 6000u + uint32_t(i));
@@ -149,7 +159,7 @@ train_conv0_kernel(Conv0Args a) {
   if (tid == 0) {
     constexpr uint32_t kI = make_idesc_f16(128, 64);
 #pragma unroll
-    for (int t = 0; t < 4; ++t)
+    for (int t = 0; t < Cfg::NT; ++t)
 #pragma unroll
       for (int ks = 0; ks < 4; ++ks)
         umma_f16(tmem + t * 64, make_desc(sbase + S_X + t * 2048 + ks * 2 * CH, CH, 128),
@@ -161,16 +171,16 @@ train_conv0_kernel(Conv0Args a) {
   {
     const int q4 = warp & 3, chalf = warp >> 2;
     const float* bias = reinterpret_cast<const float*>(smem + S_BIAS) + chalf * 32;
-    unsigned char* ag = reinterpret_cast<unsigned char*>(a.a0) + int64_t(s) * kActBytes;
+    unsigned char* ag = reinterpret_cast<unsigned char*>(a.a0) + int64_t(s) * G::ActBytes;
 #pragma unroll 1
-    for (int t = 0; t < 4; ++t) {
+    for (int t = 0; t < Cfg::NT; ++t) {
       const int p = t * 128 + q4 * 32 + lane;
       const uint32_t taddr = tmem + (uint32_t(q4 * 32) << 16) + t * 64 + chalf * 32;
       float v[32];
       tmem_ld16(taddr, v);
       tmem_ld16(taddr + 16, v + 16);
       tmem_ld_wait();
-      if (p < kTPos) {
+      if (p < G::TPos) {
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
           __half2 h[4];
@@ -187,9 +197,16 @@ train_conv0_kernel(Conv0Args a) {
   if (warp == 0) { tc_fence_after(); tmem_dealloc(tmem, 256); }
 }
 
-int launch_train_conv0(const Conv0Args& a, cudaStream_t st) {
-  CMLPL_MAX_DYN_SMEM(train_conv0_kernel, c0::SMEM);
-  train_conv0_kernel<<<2 * a.nb, c0::THREADS, c0::SMEM, st>>>(a);
+int launch_train_conv0(const Conv0Args& a, int w, cudaStream_t st) {
+  if (w == 11) {
+    auto kern = train_conv0_kernel<11>;
+    CMLPL_MAX_DYN_SMEM(kern, C0Cfg<11>::SMEM);
+    kern<<<2 * a.nb, kC0Threads, C0Cfg<11>::SMEM, st>>>(a);
+  } else {
+    auto kern = train_conv0_kernel<20>;
+    CMLPL_MAX_DYN_SMEM(kern, C0Cfg<20>::SMEM);
+    kern<<<2 * a.nb, kC0Threads, C0Cfg<20>::SMEM, st>>>(a);
+  }
   CMLPL_CHECK_LAUNCH("train_conv0");
   return CMLPL_OK;
 }

@@ -128,16 +128,17 @@ __device__ __forceinline__ void block_sum4(float (&v)[NV], float* red /* [4][NV]
   for (int i = 0; i < NV; ++i) v[i] = (red[i] + red[NV + i]) + (red[2 * NV + i] + red[3 * NV + i]);
 }
 
-// one CTA (4 warps) per row: 656 float4 groups of the 2624 features over 128 threads
-template <int CMAX>
+// one CTA (4 warps) per row: 656 float4 groups of the 2624 features (320 of 1280 at W = 11) over 128 threads
+template <int CMAX, int W>
 __global__ void __launch_bounds__(128)
 head_fwd_kernel(HeadArgs a) {
+  constexpr int CAT = TrainGeom<W>::CatDim, CONV = TrainGeom<W>::ConvFeat;
   __shared__ float red[4 * (CMAX + 1)];
   const int s = blockIdx.x;
   const int tid = threadIdx.x;
   const int e = s / a.nb;
-  const float* cat = a.cat + int64_t(s) * kCatDim;
-  float* dm = a.dmask + int64_t(s) * kCatDim;
+  const float* cat = a.cat + int64_t(s) * CAT;
+  float* dm = a.dmask + int64_t(s) * CAT;
   const float* wc = a.wc[e];
   const float p = a.prm->dropout_p;
   const float keep_scale = p > 0.f ? 1.f / (1.f - p) : 1.f;
@@ -145,24 +146,24 @@ head_fwd_kernel(HeadArgs a) {
   float acc[CMAX + 1];                                 // [CMAX] = sum of squares of the spectral features
 #pragma unroll
   for (int c = 0; c <= CMAX; ++c) acc[c] = 0.f;
-  for (int g = tid; g < kCatDim / 4; g += 128) {
+  for (int g = tid; g < CAT / 4; g += 128) {
     const float4 x = ld4(cat + 4 * g);
     float4 m = make_float4(1.f, 1.f, 1.f, 1.f);
     if (a.drop_mask) {
-      m = ld4(a.drop_mask + int64_t(s) * kCatDim + 4 * g);
+      m = ld4(a.drop_mask + int64_t(s) * CAT + 4 * g);
     } else if (p > 0.f && a.training) {
-      const uint4 u = philox_uniform4(seed, offset, PHILOX_DROP, uint32_t(s) * (kCatDim / 4) + uint32_t(g));
+      const uint4 u = philox_uniform4(seed, offset, PHILOX_DROP, uint32_t(s) * (CAT / 4) + uint32_t(g));
       const uint32_t thr = uint32_t(fminf(p, 1.f) * 4294967295.0f);
       m.x = u.x >= thr ? keep_scale : 0.f; m.y = u.y >= thr ? keep_scale : 0.f;
       m.z = u.z >= thr ? keep_scale : 0.f; m.w = u.w >= thr ? keep_scale : 0.f;
     }
     *reinterpret_cast<float4*>(dm + 4 * g) = m;
     const float4 xd = make_float4(x.x * m.x, x.y * m.y, x.z * m.z, x.w * m.w);
-    if (4 * g >= kConvFeat) acc[CMAX] += x.x * x.x + x.y * x.y + x.z * x.z + x.w * x.w;
+    if (4 * g >= CONV) acc[CMAX] += x.x * x.x + x.y * x.y + x.z * x.z + x.w * x.w;
 #pragma unroll
     for (int c = 0; c < CMAX; ++c) {
       if (c < a.C) {
-        const float4 w = ld4(wc + int64_t(c) * kCatDim + 4 * g);
+        const float4 w = ld4(wc + int64_t(c) * CAT + 4 * g);
         acc[c] += xd.x * w.x + xd.y * w.y + xd.z * w.z + xd.w * w.w;
       }
     }
@@ -177,13 +178,18 @@ head_fwd_kernel(HeadArgs a) {
     a.logits[int64_t(s) * a.C + tid] = v + a.bc[e][tid];
   }
   float* f = a.feat + int64_t(s) * kHid;
-  for (int j = tid; j < kHid; j += 128) f[j] = cat[kConvFeat + j] / nr;
+  for (int j = tid; j < kHid; j += 128) f[j] = cat[CONV + j] / nr;
 }
 
-int launch_head_fwd(const HeadArgs& a, cudaStream_t st) {
+int launch_head_fwd(const HeadArgs& a, int w, cudaStream_t st) {
   const int grid = 2 * a.nb;
-  if (a.C <= 16) head_fwd_kernel<16><<<grid, 128, 0, st>>>(a);
-  else head_fwd_kernel<32><<<grid, 128, 0, st>>>(a);
+  if (w == 11) {
+    if (a.C <= 16) head_fwd_kernel<16, 11><<<grid, 128, 0, st>>>(a);
+    else head_fwd_kernel<32, 11><<<grid, 128, 0, st>>>(a);
+  } else {
+    if (a.C <= 16) head_fwd_kernel<16, 20><<<grid, 128, 0, st>>>(a);
+    else head_fwd_kernel<32, 20><<<grid, 128, 0, st>>>(a);
+  }
   CMLPL_CHECK_LAUNCH("train_head_fwd");
   return CMLPL_OK;
 }
@@ -381,17 +387,18 @@ int launch_loss_graph(const LossArgs& a, cudaStream_t st) {
 }
 
 // ============================================================================ head backward
-template <int CMAX>
+template <int CMAX, int W>
 __global__ void __launch_bounds__(128)
 head_bwd_kernel(HeadArgs a) {
+  constexpr int CAT = TrainGeom<W>::CatDim, CONV = TrainGeom<W>::ConvFeat;
   __shared__ float red[4];
   const int s = blockIdx.x;
   const int tid = threadIdx.x;
   const int e = s / a.nb, r = s - e * a.nb;
   const float* wc = a.wc[e];
-  const float* cat = a.cat + int64_t(s) * kCatDim;
-  const float* dm = a.dmask + int64_t(s) * kCatDim;
-  float* dcat = a.dcat + int64_t(s) * kCatDim;
+  const float* cat = a.cat + int64_t(s) * CAT;
+  const float* dm = a.dmask + int64_t(s) * CAT;
+  float* dcat = a.dcat + int64_t(s) * CAT;
   float dl[CMAX];
 #pragma unroll
   for (int c = 0; c < CMAX; ++c) dl[c] = c < a.C ? a.dlogits[int64_t(s) * a.C + c] : 0.f;
@@ -405,22 +412,22 @@ head_bwd_kernel(HeadArgs a) {
   block_sum4<1>(dot, red);
   const float inv_norm = 1.f / a.norm[s];
   float amax = 0.f;
-  for (int g = tid; g < kCatDim / 4; g += 128) {
+  for (int g = tid; g < CAT / 4; g += 128) {
     float4 d = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int c = 0; c < CMAX; ++c) {
       if (c < a.C) {
-        const float4 w = ld4(wc + int64_t(c) * kCatDim + 4 * g);
+        const float4 w = ld4(wc + int64_t(c) * CAT + 4 * g);
         d.x = fmaf(dl[c], w.x, d.x); d.y = fmaf(dl[c], w.y, d.y); d.z = fmaf(dl[c], w.z, d.z); d.w = fmaf(dl[c], w.w, d.w);
       }
     }
     const float4 m = ld4(dm + 4 * g);
     d.x *= m.x; d.y *= m.y; d.z *= m.z; d.w *= m.w;
-    if (4 * g < kConvFeat) {
+    if (4 * g < CONV) {
       *reinterpret_cast<float4*>(dcat + 4 * g) = d;
       amax = fmaxf(amax, fmaxf(fmaxf(fabsf(d.x), fabsf(d.y)), fmaxf(fabsf(d.z), fabsf(d.w))));
     } else {
-      const int j = 4 * g - kConvFeat;
+      const int j = 4 * g - CONV;
       const float4 h = ld4(cat + 4 * g);
       if (unl) {
         const float4 f = ld4(ft + j), q = ld4(df + j);
@@ -436,10 +443,15 @@ head_bwd_kernel(HeadArgs a) {
   if ((tid & 31) == 0 && amax > 0.f) atomicMax(reinterpret_cast<unsigned int*>(&a.prm_rw->grad_amax), __float_as_uint(amax));
 }
 
-int launch_head_bwd(const HeadArgs& a, cudaStream_t st) {
+int launch_head_bwd(const HeadArgs& a, int w, cudaStream_t st) {
   const int grid = 2 * a.nb;
-  if (a.C <= 16) head_bwd_kernel<16><<<grid, 128, 0, st>>>(a);
-  else head_bwd_kernel<32><<<grid, 128, 0, st>>>(a);
+  if (w == 11) {
+    if (a.C <= 16) head_bwd_kernel<16, 11><<<grid, 128, 0, st>>>(a);
+    else head_bwd_kernel<32, 11><<<grid, 128, 0, st>>>(a);
+  } else {
+    if (a.C <= 16) head_bwd_kernel<16, 20><<<grid, 128, 0, st>>>(a);
+    else head_bwd_kernel<32, 20><<<grid, 128, 0, st>>>(a);
+  }
   CMLPL_CHECK_LAUNCH("train_head_bwd");
   return CMLPL_OK;
 }
@@ -447,9 +459,10 @@ int launch_head_bwd(const HeadArgs& a, cudaStream_t st) {
 // column reductions over the rows of one net: classifier weight gradient dWc[c][k] = sum_s dl[s][c] * cat[s][k] * mask[s][k],
 // classifier bias gradient, feat_spe bias gradient dbs[j] = sum_s dhp[s][j].  grid (col blocks, net, row splits).
 constexpr int kWgRows = 32;
-template <int CMAX>
+template <int CMAX, int W>
 __global__ void __launch_bounds__(256)
 head_wgrad_kernel(HeadArgs a) {
+  constexpr int CAT = TrainGeom<W>::CatDim;
   __shared__ float sdl[kWgRows][CMAX];
   const int e = blockIdx.y;
   const int r0 = blockIdx.z * kWgRows;
@@ -461,21 +474,21 @@ head_wgrad_kernel(HeadArgs a) {
     sdl[rr][c] = c < a.C ? a.dlogits[(sb + rr) * a.C + c] : 0.f;
   }
   __syncthreads();
-  constexpr int kCatBlocks = (kCatDim + 255) / 256;
+  constexpr int kCatBlocks = (CAT + 255) / 256;
   if (int(blockIdx.x) < kCatBlocks) {
     const int k = blockIdx.x * 256 + threadIdx.x;
-    if (k < kCatDim) {
+    if (k < CAT) {
       float acc[CMAX];
 #pragma unroll
       for (int c = 0; c < CMAX; ++c) acc[c] = 0.f;
       for (int rr = 0; rr < rows; ++rr) {
-        const float x = a.cat[(sb + rr) * kCatDim + k] * a.dmask[(sb + rr) * kCatDim + k];
+        const float x = a.cat[(sb + rr) * CAT + k] * a.dmask[(sb + rr) * CAT + k];
 #pragma unroll
         for (int c = 0; c < CMAX; ++c) acc[c] = fmaf(sdl[rr][c], x, acc[c]);
       }
 #pragma unroll
       for (int c = 0; c < CMAX; ++c)
-        if (c < a.C) atomicAdd(a.g_wc[e] + int64_t(c) * kCatDim + k, acc[c]);
+        if (c < a.C) atomicAdd(a.g_wc[e] + int64_t(c) * CAT + k, acc[c]);
     }
     if (blockIdx.x == 0 && threadIdx.x < a.C) {
       float b = 0.f;
@@ -492,10 +505,16 @@ head_wgrad_kernel(HeadArgs a) {
   }
 }
 
-int launch_head_wgrad(const HeadArgs& a, cudaStream_t st) {
-  const dim3 grid((kCatDim + 255) / 256 + kHid / 256, 2, (a.nb + kWgRows - 1) / kWgRows);
-  if (a.C <= 16) head_wgrad_kernel<16><<<grid, 256, 0, st>>>(a);
-  else head_wgrad_kernel<32><<<grid, 256, 0, st>>>(a);
+int launch_head_wgrad(const HeadArgs& a, int w, cudaStream_t st) {
+  const int cat = w == 11 ? TrainGeom<11>::CatDim : kCatDim;
+  const dim3 grid((cat + 255) / 256 + kHid / 256, 2, (a.nb + kWgRows - 1) / kWgRows);
+  if (w == 11) {
+    if (a.C <= 16) head_wgrad_kernel<16, 11><<<grid, 256, 0, st>>>(a);
+    else head_wgrad_kernel<32, 11><<<grid, 256, 0, st>>>(a);
+  } else {
+    if (a.C <= 16) head_wgrad_kernel<16, 20><<<grid, 256, 0, st>>>(a);
+    else head_wgrad_kernel<32, 20><<<grid, 256, 0, st>>>(a);
+  }
   CMLPL_CHECK_LAUNCH("train_head_wgrad");
   return CMLPL_OK;
 }

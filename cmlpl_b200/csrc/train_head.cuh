@@ -37,9 +37,10 @@ struct HeadArgs {
   const float* dlogits; const float* dfeat; float* dcat; float* dhp;
   float* g_wc[2]; float* g_bc[2]; float* g_bs[2];
 };
-int launch_head_fwd(const HeadArgs& a, cudaStream_t st);
-int launch_head_bwd(const HeadArgs& a, cudaStream_t st);
-int launch_head_wgrad(const HeadArgs& a, cudaStream_t st);
+// w = 20 or 11 selects the classifier input width (2624 / 1280; conv features 1600 / 256)
+int launch_head_fwd(const HeadArgs& a, int w, cudaStream_t st);
+int launch_head_bwd(const HeadArgs& a, int w, cudaStream_t st);
+int launch_head_wgrad(const HeadArgs& a, int w, cudaStream_t st);
 
 struct LossArgs {
   const cmlpl_train_params* prm;

@@ -5,11 +5,14 @@
 
 namespace cmlpl {
 
+// Every trunk kernel exists for the window w = 20 and w = 11 (TrainGeom); the layouts below are written for w = 20,
+// w = 11 packs the same regions at its own sizes (121 / 25 positions, cat width 1280).
+
 // gather + noise + conv0 (train_fwd_sm100.cu)
 struct Conv0Args {
   const float* cube; int scene_rows, cols;
   const int64_t* pix;              // [nb]
-  const float* noise;              // [2][nb][60][20][20] or nullptr
+  const float* noise;              // [2][nb][60][w][w] or nullptr
   const float* w0[2]; const float* b0[2];
   const cmlpl_train_params* prm;
   __half* x16; __half* a0;         // [2*nb][8][400][8]
@@ -22,7 +25,7 @@ struct Conv0Args {
   const float* w3[2][2];           // [net][conv1 | conv2] fp32 [64][64][3][3]
   unsigned char* wpack;
 };
-int launch_train_conv0(const Conv0Args& a, cudaStream_t st);
+int launch_train_conv0(const Conv0Args& a, int w, cudaStream_t st);
 
 // conv1 + pool + conv2 + pool (patch_cnn_sm100.cu, TRAIN instantiation)
 struct TrainCnnArgs {
@@ -35,16 +38,16 @@ struct TrainCnnArgs {
   float* cat;                      // [2*nb][2624], first 1600 written here
   int nb;
 };
-int launch_train_cnn(const TrainCnnArgs& a, cudaStream_t st);
+int launch_train_cnn(const TrainCnnArgs& a, int w, cudaStream_t st);
 
 // conv2 / conv1 backward: data gradient + weight gradient + bias gradient (train_bwd_sm100.cu)
 struct ConvBwdArgs {
   const cmlpl_train_params* prm;
   const unsigned char* wpack[2];   // fp16 [tap][ci chunk][co][8 ci] of this conv, per net
   float* g_stage[2]; float* g_b[2];   // weight gradient staging [tap][co][ci] / bias gradient: accumulated into (zeroed by the caller)
-  // H = 10 (conv2): dz2 is formed from dcat (dL/dcat, first 1600 columns), the ReLU mask m2; activation = p1;
-  //                 the epilogue applies the pool backward + mask m1 and writes dz1
-  // H = 20 (conv1): dz1 is read back; activation = a0; the epilogue writes da0
+  // H = 10 / 5 (conv2 of w = 20 / 11): dz2 is formed from dcat (dL/dcat, first 1600 / 256 columns), the ReLU mask
+  //                 m2; activation = p1; the epilogue applies the pool backward + mask m1 and writes dz1
+  // H = 20 / 11 (conv1): dz1 is read back; activation = a0; the epilogue writes da0
   const float* dcat; const uint32_t* m2; const uint32_t* m1;
   const __half* act;               // p1 or a0
   const __half* dz_in;             // dz1 (H = 20)
@@ -62,6 +65,6 @@ struct Conv0BwdArgs {
   // prologue: staged 3x3 weight gradients [net][conv][tap][co][ci] -> torch layout [co][ci][3][3]
   const float* gstage; float* g_w3[2][2];
 };
-int launch_train_conv0_bwd(const Conv0BwdArgs& a, cudaStream_t st);
+int launch_train_conv0_bwd(const Conv0BwdArgs& a, int w, cudaStream_t st);
 
 }  // namespace cmlpl

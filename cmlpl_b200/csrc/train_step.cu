@@ -26,10 +26,10 @@ StepStreams* step_streams() {
   }
   return &s;
 }
-constexpr int64_t kNumel[CMLPL_TRAIN_TENSORS] = {64 * 60, 64, 64 * 64 * 9, 64, 64 * 64 * 9, 64, 0 /*1024*B*/, 1024, 0 /*C*2624*/, 0 /*C*/};
-int64_t numel(int i, int B, int C) {
+constexpr int64_t kNumel[CMLPL_TRAIN_TENSORS] = {64 * 60, 64, 64 * 64 * 9, 64, 64 * 64 * 9, 64, 0 /*1024*B*/, 1024, 0 /*C*cat*/, 0 /*C*/};
+int64_t numel(int i, int B, int C, int cat) {
   if (i == 6) return int64_t(1024) * B;
-  if (i == 8) return int64_t(C) * kCatDim;
+  if (i == 8) return int64_t(C) * cat;
   if (i == 9) return C;
   return kNumel[i];
 }
@@ -55,7 +55,8 @@ extern "C" int cmlpl_train_step_launches(int phases) {
 
 extern "C" int cmlpl_train_step(const cmlpl_train_io* io, int phases, cmlpl_stream_t stream) {
   CMLPL_CHECK_ARG(io, "train_step: null io");
-  CMLPL_CHECK_ARG(io->w == 20, "train_step: w=%d unsupported (BaseNet2's classifier fixes w=20, tools/models.py:127)", io->w);
+  CMLPL_CHECK_ARG(io->w == 20 || io->w == 11, "train_step: w=%d unsupported (20 = the reference's BaseNet2, "
+                  "tools/models.py:127; 11 = the odd window of ExtractPatches_for_base)", io->w);
   CMLPL_CHECK_ARG(io->bs > 0 && io->btu > 0 && io->bands > 0 && io->bands <= 256 && io->classes > 0 && io->classes <= 32 &&
                       io->queue > 0, "train_step: bad dims (bs=%d btu=%d bands=%d classes=%d queue=%d)", io->bs, io->btu,
                   io->bands, io->classes, io->queue);
@@ -63,7 +64,10 @@ extern "C" int cmlpl_train_step(const cmlpl_train_io* io, int phases, cmlpl_stre
                       io->hist, "train_step: null pointer");
   CMLPL_CHECK_ARG(io->cube ? (io->pix != nullptr && io->scene_rows >= 10 && io->cols >= 10) : io->patch_noise != nullptr,
                   "train_step: pass the PCA cube + pixel indices, or the assembled patches in patch_noise");
-  const int bs = io->bs, btu = io->btu, nb = bs + btu, B = io->bands, C = io->classes, Q = io->queue;
+  const int bs = io->bs, btu = io->btu, nb = bs + btu, B = io->bands, C = io->classes, Q = io->queue, w = io->w;
+  // classifier input width and its conv-feature head (2624 / 1600 at w = 20, 1280 / 256 at w = 11); a w = 11 step
+  // uses the w = 20 workspace layout, packing each region at its own per-sample strides
+  const int cat = w == 11 ? TrainGeom<11>::CatDim : kCatDim, conv = cat - kHid;
   const TrainWs L = train_ws_layout(bs, btu, B, C, Q);
   CMLPL_CHECK_ARG(io->work_bytes >= L.total, "train_step: workspace of %zu bytes, need %zu", io->work_bytes, L.total);
   CMLPL_CHECK_ARG(reinterpret_cast<uintptr_t>(io->work) % 256 == 0, "train_step: workspace must be 256-byte aligned");
@@ -114,18 +118,18 @@ extern "C" int cmlpl_train_step(const cmlpl_train_io* io, int phases, cmlpl_stre
       t.b1[e] = io->net[e].p[3]; t.b2[e] = io->net[e].p[5];
       // h = relu(feat_spe(y)) into the tail of cat (models.py:142-144)
       mg.p[e] = GemmProb{f32(L.ynoisy) + int64_t(e) * nb * B, B, 1, io->net[e].p[6], 1, B,
-                         f32(L.cat) + int64_t(e) * nb * kCatDim + kConvFeat, kCatDim, 1, io->net[e].p[7], nullptr,
+                         f32(L.cat) + int64_t(e) * nb * cat + conv, cat, 1, io->net[e].p[7], nullptr,
                          nb, kHid, B, 1.f, 1};
     }
-    if ((rc = launch_train_conv0(a, st)) != CMLPL_OK) return rc;
+    if ((rc = launch_train_conv0(a, w, st)) != CMLPL_OK) return rc;
     // fork: the spectral GEMM (needs only the noisy spectra of kernel 1) next to the conv trunk
     CMLPL_CUDA(cudaEventRecord(ss->ev[0], st));
     CMLPL_CUDA(cudaStreamWaitEvent(ss->side, ss->ev[0], 0));
     if ((rc = launch_multi_gemm(mg, ss->side, "train_spectral_fwd")) != CMLPL_OK) return rc;
     CMLPL_CUDA(cudaEventRecord(ss->ev[1], ss->side));
-    if ((rc = launch_train_cnn(t, st)) != CMLPL_OK) return rc;
+    if ((rc = launch_train_cnn(t, w, st)) != CMLPL_OK) return rc;
     CMLPL_CUDA(cudaStreamWaitEvent(st, ss->ev[1], 0));
-    if ((rc = launch_head_fwd(ha, st)) != CMLPL_OK) return rc;
+    if ((rc = launch_head_fwd(ha, w, st)) != CMLPL_OK) return rc;
   }
 
   if (phases & 2) {
@@ -166,10 +170,10 @@ extern "C" int cmlpl_train_step(const cmlpl_train_io* io, int phases, cmlpl_stre
     } else {
       for (int e = 0; e < 2; ++e)
         for (int i = 0; i < CMLPL_TRAIN_TENSORS; ++i)
-          CMLPL_CUDA(cudaMemsetAsync(io->net[e].g[i], 0, size_t(numel(i, B, C)) * 4, st));
+          CMLPL_CUDA(cudaMemsetAsync(io->net[e].g[i], 0, size_t(numel(i, B, C, cat)) * 4, st));
     }
     CMLPL_CUDA(cudaMemsetAsync(ws + L.gstage, 0, size_t(4) * 36864 * 4, st));
-    if ((rc = launch_head_bwd(ha, st)) != CMLPL_OK) return rc;
+    if ((rc = launch_head_bwd(ha, w, st)) != CMLPL_OK) return rc;
     MultiGemm dws{};
     dws.count = 2;
     ConvBwdArgs b2{}, b1{};
@@ -194,12 +198,12 @@ extern "C" int cmlpl_train_step(const cmlpl_train_io* io, int phases, cmlpl_stre
     // fork: the head weight gradients (classifier, feat_spe) next to the conv backward chain
     CMLPL_CUDA(cudaEventRecord(ss->ev[2], st));
     CMLPL_CUDA(cudaStreamWaitEvent(ss->side, ss->ev[2], 0));
-    if ((rc = launch_head_wgrad(ha, ss->side)) != CMLPL_OK) return rc;
+    if ((rc = launch_head_wgrad(ha, w, ss->side)) != CMLPL_OK) return rc;
     if ((rc = launch_multi_gemm(dws, ss->side, "train_spectral_wgrad")) != CMLPL_OK) return rc;
     CMLPL_CUDA(cudaEventRecord(ss->ev[3], ss->side));
-    if ((rc = launch_train_conv_bwd(10, b2, st)) != CMLPL_OK) return rc;
-    if ((rc = launch_train_conv_bwd(20, b1, st)) != CMLPL_OK) return rc;
-    if ((rc = launch_train_conv0_bwd(b0, st)) != CMLPL_OK) return rc;
+    if ((rc = launch_train_conv_bwd(w / 2, b2, st)) != CMLPL_OK) return rc;      // conv2: 10 x 10 / 5 x 5
+    if ((rc = launch_train_conv_bwd(w, b1, st)) != CMLPL_OK) return rc;          // conv1: 20 x 20 / 11 x 11
+    if ((rc = launch_train_conv0_bwd(b0, w, st)) != CMLPL_OK) return rc;
     CMLPL_CUDA(cudaStreamWaitEvent(st, ss->ev[3], 0));
   }
 
@@ -211,7 +215,7 @@ extern "C" int cmlpl_train_step(const cmlpl_train_io* io, int phases, cmlpl_stre
       for (int i = 0; i < CMLPL_TRAIN_TENSORS; ++i) {
         const int k = t.count++;
         t.p[k] = io->net[e].p[i]; t.g[k] = io->net[e].g[i]; t.m[k] = io->net[e].m[i]; t.v[k] = io->net[e].v[i];
-        t.n[k] = numel(i, B, C);
+        t.n[k] = numel(i, B, C, cat);
       }
     if ((rc = launch_adam_all(t, st)) != CMLPL_OK) return rc;
   }

@@ -21,6 +21,8 @@ TENSORS = ("conv0.weight", "conv0.bias", "conv1.weight", "conv1.bias", "conv2.we
            "feat_spe.weight", "feat_spe.bias", "classifier.weight", "classifier.bias")
 HIST = ("lc", "total", "cls", "con", "acc", "total1", "cls1", "con1", "lc1")
 CAT = 2624
+# classifier input width per window: 64 pooled channels x (w // 4)^2 positions + the 1024 spectral features
+CAT_OF_W = {20: CAT, 11: 64 * 2 * 2 + 1024}
 
 
 class TrainNet(ctypes.Structure):
@@ -55,7 +57,8 @@ class FusedMutualStep:
     ``step(...)`` runs one step on the current stream and returns the device tensor ``hist`` (f32 [12]: lc, total,
     cls, con, acc, total1, cls1, con1, lc1) without any host synchronisation.  Inputs either come from the PCA cube
     (``cube``, ``pix``; noise / dropout from the device Philox stream unless tensors are injected) or are passed
-    assembled (``patches`` f32 [2, nb, 60, 20, 20], ``spectra`` f32 [2, nb, B]) -- the form the parity tests use.
+    assembled (``patches`` f32 [2, nb, 60, w, w], ``spectra`` f32 [2, nb, B]) -- the form the parity tests use.
+    The window w (20, or 11 for the odd window of ExtractPatches_for_base) is the peers' ``BaseNet2.w``.
     """
 
     def __init__(self, Base, Base1, bs=128, btu=128, lr=5e-4, betas=(0.9, 0.999), eps=1e-8, temperature=0.3,
@@ -67,6 +70,12 @@ class FusedMutualStep:
         self.dev = dev
         self.bs, self.btu, self.nb = bs, btu, bs + btu
         self.B, self.C = Base.num_features, Base.num_classes
+        self.w = int(getattr(Base, "w", 20))
+        if int(getattr(Base1, "w", 20)) != self.w:
+            raise _lib.CmlplError(f"the two peers have different windows ({self.w} and {Base1.w})")
+        if self.w not in CAT_OF_W:
+            raise _lib.CmlplError(f"FusedMutualStep: w={self.w} unsupported (20 or 11)")
+        self.cat = CAT_OF_W[self.w]
         self.lr, self.betas, self.eps = lr, betas, eps
         self.T, self.alpha, self.thr, self.num_epochs, self.queue_batch = temperature, alpha, thr, num_epochs, queue_batch
         self.noise = noise
@@ -132,7 +141,7 @@ class FusedMutualStep:
 
     def _io(self, cube, patches, spectra, spec_row, patch_noise, spec_noise, drop_mask):
         io = TrainIO()
-        io.bs, io.btu, io.bands, io.classes, io.w, io.queue = self.cur[0], self.cur[1], self.B, self.C, 20, self.queue
+        io.bs, io.btu, io.bands, io.classes, io.w, io.queue = self.cur[0], self.cur[1], self.B, self.C, self.w, self.queue
         if cube is not None:
             io.cube, io.scene_rows, io.cols = cube.data_ptr(), cube.shape[0], cube.shape[1]
             io.pix = self.pix.data_ptr()
@@ -194,7 +203,8 @@ class FusedMutualStep:
                  "dz1", "da0", "S", "G", "dG", "probs_orig", "total")
 
     def workspace_layout(self):
-        """{region: byte offset into self.work} (cmlpl_train_workspace_layout; tests and profiling)."""
+        """{region: byte offset into self.work} (cmlpl_train_workspace_layout; tests and profiling).  The offsets do not
+        depend on w; a w = 11 step packs each region at its own per-sample strides (include/cmlpl.h)."""
         off = (c_size_t * 20)()
         _lib.call("cmlpl_train_workspace_layout", self.bs, self.btu, self.B, self.C, self.queue, off)
         return dict(zip(self.WS_FIELDS, [int(v) for v in off]))
@@ -213,9 +223,9 @@ class FusedMutualStep:
              patch_noise=None, spec_noise=None, drop_masks=None, phases=15):
         """labels i64 [bs].  Cube mode: ``cube`` f32 [R, C, 60], ``pix`` i64 [nb] raster pixels ([labelled ; unlabelled]),
         ``spectra`` f32 [N, B] table (row ``spec_row[i]`` or ``pix[i]``).  Assembled mode: ``patches`` f32
-        [2, nb, 60, 20, 20] and ``spectra`` f32 [2, nb, B] (train.py:174,184 after the noise was added).
-        ``patch_noise`` [2, nb, 60, 20, 20], ``spec_noise`` [2, nb, B] and ``drop_masks`` [2, nb, 2624] (scaled) inject
-        the random draws; otherwise the device Philox stream (seed, step counter) is used."""
+        [2, nb, 60, w, w] and ``spectra`` f32 [2, nb, B] (train.py:174,184 after the noise was added).
+        ``patch_noise`` [2, nb, 60, w, w], ``spec_noise`` [2, nb, B] and ``drop_masks`` [2, nb, cat] (scaled; cat = 2624,
+        or 1280 at w = 11) inject the random draws; otherwise the device Philox stream (seed, step counter) is used."""
         def chk(t, shape, name):
             if t is None or not t.is_cuda or not t.is_contiguous() or tuple(t.shape) != tuple(shape):
                 raise _lib.CmlplError(f"{name}: expected a contiguous CUDA tensor of shape {tuple(shape)}, got "
@@ -239,18 +249,18 @@ class FusedMutualStep:
                 raise _lib.CmlplError("spectra must be a contiguous CUDA f32 [rows, B] tensor")
             self.pix[:nb].copy_(pix, non_blocking=True)
             if patch_noise is not None:
-                chk(patch_noise, (2, nb, 60, 20, 20), "patch_noise")
+                chk(patch_noise, (2, nb, 60, self.w, self.w), "patch_noise")
             if spec_noise is not None:
                 chk(spec_noise, (2, nb, self.B), "spec_noise")
         else:
-            chk(patches, (2, nb, 60, 20, 20), "patches")
+            chk(patches, (2, nb, 60, self.w, self.w), "patches")
             chk(spectra, (2, nb, self.B), "spectra")
         chk(labels, (bs,), "labels")
         self.labels[:bs].copy_(labels, non_blocking=True)
         dm = None
         if drop_masks is not None:
             dm = drop_masks if isinstance(drop_masks, torch.Tensor) else torch.stack(list(drop_masks))
-            chk(dm, (2, nb, CAT), "drop_masks")
+            chk(dm, (2, nb, self.cat), "drop_masks")
         self._set_params(epoch, batch_index, phases)
         stream = torch.cuda.current_stream().cuda_stream
         key = (phases, bs, nb, _ptr(cube), _ptr(patches), _ptr(spectra), _ptr(spec_row), _ptr(patch_noise), _ptr(spec_noise), _ptr(dm))

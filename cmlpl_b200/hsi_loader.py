@@ -111,5 +111,7 @@ class HSIDataSet(data.Dataset):
         if 'pix' not in self._dev:
             self._dev['pix'] = torch.from_numpy(self.index).cuda()
         pix = self._dev['pix'][positions].contiguous()
-        XP = ops.patch_gather(self.cube_device(), self.w, idx=pix, noise=noise, noise_scale=noise_scale)
+        # odd w: ExtractPatches_for_base (hyper_tools.py:300-317), the window the odd-w scene path and model use
+        XP = ops.patch_gather(self.cube_device(), self.w, idx=pix, noise=noise, noise_scale=noise_scale,
+                              odd_mode=self.w % 2 == 1)
         return XP, self.spectra_device()[positions], self.labels_device()[positions]

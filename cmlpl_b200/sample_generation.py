@@ -80,7 +80,7 @@ def main(args):
         step = 8192
         for s in range(0, row * col, step):
             n = min(step, row * col - s)
-            out[s:s + n] = ops.patch_gather(cube_d, args.w, first=s, n=n).cpu().numpy()
+            out[s:s + n] = ops.patch_gather(cube_d, args.w, first=s, n=n, odd_mode=args.w % 2 == 1).cpu().numpy()
         out.flush()
     return save_pre_dir
 

@@ -57,9 +57,10 @@ class MutualState:
     extras: dict = field(default_factory=dict)
 
 
-def make_state(num_features, num_classes, args, device) -> MutualState:
-    Base = BaseNet2(num_features=num_features, dropout=args.dropout, num_classes=num_classes).to(device)
-    Base1 = BaseNet2(num_features=num_features, dropout=args.dropout, num_classes=num_classes).to(device)
+def make_state(num_features, num_classes, args, device, w=20) -> MutualState:
+    """Both peers at window ``w`` (the dataset's: 20, or 11 for ``sample_generation --w 11``)."""
+    Base = BaseNet2(num_features=num_features, dropout=args.dropout, num_classes=num_classes, w=w).to(device)
+    Base1 = BaseNet2(num_features=num_features, dropout=args.dropout, num_classes=num_classes, w=w).to(device)
     qs = 5 * args.labeled_batch_size * 2                                        # train.py:138,142
     z = lambda *s: torch.zeros(*s, device=device)
     return MutualState(Base, Base1, losses.FusedAdam(Base.parameters(), lr=args.lr),
@@ -150,12 +151,12 @@ def main(args):
     unlabeled = HSIDataSet(dataID, 'unlabel', max_iters=args.num_unlabel, num_unlabel=args.num_unlabel, root=root)
     whole = HSIDataSet(dataID, 'wholeset', root=root)
     whole_loader = torch.utils.data.DataLoader(whole, batch_size=args.val_batch_size, shuffle=False)
-    st = make_state(num_features, num_classes, args, device)
+    st = make_state(num_features, num_classes, args, device, w=labeled.w)
     lb, ub = args.labeled_batch_size, args.unlabeled_batch_size
     num_batches = min(math.ceil(len(labeled) / lb), math.ceil(len(unlabeled) / ub))                 # :134
     hist_dev = []
     fused = None
-    if not getattr(args, "fp32_step", False) and labeled.scene_ready and labeled.w == 20:
+    if not getattr(args, "fp32_step", False) and labeled.scene_ready and labeled.w in (20, 11):
         # default: the whole step is cmlpl_train_step (gather + Philox noise inside the first kernel, tcgen05
         # convolutions, 15 launches replayed from a CUDA graph); --fp32_step keeps the fp32 reference path below
         from .fused_step import FusedMutualStep

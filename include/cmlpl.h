@@ -357,7 +357,9 @@ int cmlpl_comm_destroy(cmlpl_comm* comm);
  * Row order inside a net: [bs labelled ; btu unlabelled] (train.py:174,184); nb = bs + btu.
  * Tensor index order in cmlpl_train_net arrays: 0 conv0.weight [64,60,1,1], 1 conv0.bias, 2 conv1.weight
  * [64,64,3,3], 3 conv1.bias, 4 conv2.weight, 5 conv2.bias, 6 feat_spe.weight [1024,B], 7 feat_spe.bias,
- * 8 classifier.weight [C,2624], 9 classifier.bias (state-dict layouts, tools/models.py:102-127).
+ * 8 classifier.weight [C,cat], 9 classifier.bias (state-dict layouts, tools/models.py:102-127).
+ * Window w = 20 (the reference's BaseNet2, cat = 64*5*5 + 1024 = 2624) or w = 11 (ExtractPatches_for_base windows,
+ * hyper_tools.py:300-317; both 2x2 pools floor, 11 -> 5 -> 2, so cat = 64*2*2 + 1024 = 1280).
  */
 #define CMLPL_TRAIN_TENSORS 10
 typedef struct cmlpl_train_net {
@@ -379,12 +381,12 @@ typedef struct cmlpl_train_params {   /* lives in DEVICE memory; the host refres
   int smooth;             /* epoch > 0 or batch_index > queue_batch, train.py:212 */
   int queue_ptr[2];       /* write positions of the two banks for THIS step (train.py:232-237, host keeps the quirk) */
   unsigned long long seed, offset;   /* device Philox stream for noise / dropout when no tensors are injected */
-  float grad_amax;        /* scratch: max |dL/dcat[:, :1600]| of this step (written by the head backward) */
+  float grad_amax;        /* scratch: max |dL/dcat[:, :conv]| of this step, conv = cat - 1024 (head backward) */
   int pad_;
 } cmlpl_train_params;
 
 typedef struct cmlpl_train_io {
-  int bs, btu, bands, classes, w, queue;      /* w must be 20, classes <= 16, bands <= 256 */
+  int bs, btu, bands, classes, w, queue;      /* w = 20 or 11, classes <= 32, bands <= 256 */
   /* ---- inputs */
   const float* cube; int scene_rows, cols;    /* f32 [R, cols, 60] PCA cube, or NULL: patch_noise then HOLDS the input patches */
   const int64_t* pix;                         /* i64 [nb] raster pixel per row (both nets read the same pixels) */
@@ -393,7 +395,7 @@ typedef struct cmlpl_train_io {
   const int64_t* spec_row;                    /* i64 [nb] row of `spectra` per sample; NULL: row pix[i] (cube mode) or the
                                                  assembled inputs f32 [2, nb, B] themselves (cube == NULL) */
   const float* spec_noise;                    /* f32 [2, nb, B] or NULL -> Philox (none when cube == NULL) */
-  const float* drop_mask;                     /* f32 [2, nb, 2624] inverted-dropout mask (0 or 1/(1-p)) or NULL -> Philox */
+  const float* drop_mask;                     /* f32 [2, nb, cat] inverted-dropout mask (0 or 1/(1-p)) or NULL -> Philox */
   const int64_t* labels;                      /* i64 [bs] 0-based (train.py:159) */
   cmlpl_train_net net[2];
   cmlpl_train_params* params;                 /* device */
@@ -408,12 +410,19 @@ typedef struct cmlpl_train_io {
   void* work; size_t work_bytes;              /* cmlpl_train_workspace_bytes() */
 } cmlpl_train_io;
 
+/* The size of the w = 20 layout, which bounds a w = 11 step of the same (bs, btu, bands, classes, queue): both windows
+ * use this size and the same region offsets. */
 size_t cmlpl_train_workspace_bytes(int bs, int btu, int bands, int classes, int queue);
 /* Byte offsets of the workspace regions (tests / profiling): offsets[20] = {x16, a0, p1, m1, m2, cat, dmask, ynoisy,
  * norm, dlogits, dfeat, dcat, dhp, dz1, da0, S, G, dG, probs_orig, total}.  Per-sample activations x16 / a0 / dz1 / da0
- * are f16 [2*nb][8 chunks][400][8], p1 f16 [2*nb][8][100][8]; m1 / m2 are ReLU masks u32 [2*nb][positions][2] (bit c%32
- * of word c/32); cat / dmask / dcat f32 [2*nb][2624]; dz1 / da0 carry the power-of-two gradient scale
- * 2^(12 - exponent(grad_amax)). */
+ * are f16 [2*nb][8 chunks][P1][8], p1 f16 [2*nb][8][P2][8]; m1 / m2 are ReLU masks u32 [2*nb][P1 | P2][2] (bit c%32 of
+ * word c/32); cat / dmask / dcat f32 [2*nb][cat]; positions are row-major (y*side + x).  Each region is packed densely
+ * from its offset at the window's own sizes:
+ *   w = 20: P1 = 400 (20x20), P2 = 100 (10x10), cat = 2624 -- per sample 51 200 B (x16 / a0 / dz1 / da0),
+ *           12 800 B (p1), 3 200 B (m1), 800 B (m2); row stride of cat / dmask / dcat 2624 floats
+ *   w = 11: P1 = 121 (11x11), P2 = 25 (5x5), cat = 1280 -- per sample 15 488 B, 3 200 B, 968 B, 200 B; row stride 1280
+ * At w = 11 the pools drop the last row / column of each map: their m1 / m2 bits and dz1 entries are stored as 0.
+ * dz1 / da0 carry the power-of-two gradient scale 2^(12 - exponent(grad_amax)). */
 int cmlpl_train_workspace_layout(int bs, int btu, int bands, int classes, int queue, size_t* offsets);
 /* phases: bit 0 forward (gather+noise -> logits, feat), bit 1 losses (+ bank update, dlogits, dfeat),
  * bit 2 backward (all gradients), bit 3 Adam.  15 = the whole step. */
