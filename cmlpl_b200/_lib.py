@@ -35,25 +35,15 @@ SIGNATURES = {
     "cmlpl_scene_workspace_bytes": (Z, [I, I, I, I, I]),
     "cmlpl_scene_infer": (I, [P, I, I, I, I, P, I, I, I, I, I, P, P, Z, P, P, P]),
     "cmlpl_scene_infer_raw": (I, [P, I, I, I, I, I, I, I, I, I, I, P, P, P, P, P, P, Z, P, P, P]),
-    "cmlpl_spectral_hidden_raw_tc": (I, [P, I, L, I, I, I, P, P, P, P, P, P]),
     "cmlpl_conv0_map_f16": (I, [P, I, I, I, I, I, I, I, P, P, P]),
     "cmlpl_patch_cnn_f16": (I, [P, I, I, I, P, P, P]),
-    "cmlpl_debug_patch_cnn_trace": (I, [P, I, I, I, P, P, P, P]),
-    "cmlpl_patch_cnn_f16_tiled": (I, [P, I, I, I, P, P, P]),
-    "cmlpl_conv1_scene_f16": (I, [P, I, I, I, P, P, P, P]),
-    "cmlpl_patch_conv2_f16_tiled": (I, [P, I, I, I, P, P, P]),
     "cmlpl_scene_workspace_layout": (I, [I, I, I, I, I, P]),
-    "cmlpl_conv1_scene_variants_f32": (I, [P, I, I, I, P, P, P]),
-    "cmlpl_conv1_scene_planes_f16": (I, [P, I, I, I, P, P, P, P]),
     "cmlpl_conv1_pool_planes_f16": (I, [P, I, I, I, P, P, P]),
     "cmlpl_conv2_scene_f16": (I, [P, I, I, I, P, P, P]),
     "cmlpl_pool2_cls_f16": (I, [P, I, I, I, I, I, P, P, P]),
     "cmlpl_spectral_logits_tc": (I, [P, L, I, I, I, P, P, P, P]),
     "cmlpl_spectral_logits_raw_tc": (I, [P, I, L, I, I, I, P, P, P, P, P, P]),
     "cmlpl_head_sum_lmap": (I, [P, P, I, I, I, I, I, P, P, P, P]),
-    "cmlpl_debug_patch_conv2_trace": (I, [P, I, I, I, P, P, P, P]),
-    "cmlpl_spectral_hidden_tc": (I, [P, L, I, I, I, P, P, P, P]),
-    "cmlpl_head_tc": (I, [P, P, L, I, I, I, P, P, P, P]),
     "cmlpl_spectral_head_f32": (I, [P, L, I, I, I, P, P, L, P, P]),
     "cmlpl_classify_f16": (I, [P, P, L, I, I, I, P, P, P, P]),
     "cmlpl_argmax_u8": (I, [P, L, I, P, P]),

@@ -1,4 +1,4 @@
-// Scene-level conv1 with exact compute sharing (SURVEY section 7 / 8-f3, conv1 part).
+// Scene-level conv1 + pool1 with exact compute sharing (SURVEY section 7 / 8-f3, conv1 part).
 //
 // The reference applies conv1 (3x3, zero padding at the PATCH border, tools/models.py:104,134) to
 // every pixel's 20x20 window separately, but a window position's output only depends on (a) its
@@ -8,241 +8,21 @@
 //     G[a][b][p] = relu(b1 + F0[p] + sum_{dy in S_a, dx in S_b} W1[dy,dx] . F0[p + (dy-1, dx-1)])
 //     S_top/left = {1,2},  S_mid = {0,1,2},  S_bot/right = {0,1}
 // and the patch of pixel (r,c) reads G[a(y)][b(x)] at scene position (r+y, c+x): identical math up to
-// fp32 summation order, ~15x fewer conv1 FLOPs.  pool1_scene_kernel then forms the 2x2 average
-// pools (models.py:136) for every top-left position in the 9 pooled border classes.
+// fp32 summation order, ~15x fewer conv1 FLOPs.  The 2x2 average pools (models.py:136) are formed for
+// every top-left position in the 9 pooled border classes
+//     PM[A][B][pr,pc] = 1/4 sum_{u,v in {0,1}} G[a(A,u)][b(B,v)][pr+u, pc+v]
+//     a(top,0)=top a(top,1)=mid   a(mid,.)=mid   a(bot,0)=mid a(bot,1)=bot     (pooled row 0 / 1..8 / 9)
+// and likewise b(B,v) for columns.
 //
-// Kernel: persistent, warp-specialised tcgen05 implicit GEMM over 4x30-position tiles (M=128 rows =
+// conv1_pool_kernel does both in ONE kernel -- the fp32 variants G (2.3 KB per scene position) never touch
+// HBM.  It is a persistent, warp-specialised tcgen05 implicit GEMM over 4x30-position tiles (M=128 rows =
 // 4 rows x 32 columns incl. one halo column each side), taps = A-descriptor offsets in a row-major
-// zero-haloed shared-memory tile, three accumulators R_dy = sum_{dx in S_b} tap(dy,dx) per column
-// class b; the epilogue forms top = R1+R2, mid = R0+R1+R2, bot = R0+R1 in the same lane.
-#include "common.cuh"
-#include "sm100_ptx.cuh"
-#include "tma.cuh"
-
-namespace cmlpl {
-
-namespace c1s {
-constexpr int TH = 4, TP = 32, TW = 30;              // tile rows, row pitch (entries), valid columns
-constexpr int ENT = 1 + (TH + 2) * TP + 1;           // 194 entries per 16-byte chunk plane
-constexpr int CH = ENT * 16 + 16;                    // bytes between chunk planes (+16: bank spread)
-constexpr int ABYTES = 8 * CH;
-constexpr int WBYTES = 3 * 8 * 192 * 16;             // 73 728
-constexpr int S_W = 0, S_A = WBYTES, S_BIAS = S_A + 2 * ABYTES, S_BAR = S_BIAS + 256, S_TMEM = S_BAR + 128;
-constexpr int SMEM = (S_TMEM + 16 + 127) / 128 * 128;
-constexpr int kEpi = 256, kLoad = 64, kThreads = kEpi + kLoad + 32;
-constexpr int kWLbo = 192 * 16, kWDx = 8 * kWLbo;
-enum { A_FULL0 = 0, A_FULL1, A_EMPTY0, A_EMPTY1, D_FULL0, D_FULL1, D_EMPTY0, D_EMPTY1 };
-}  // namespace c1s
-
-// f0: f16 chunk-planar [8][PR][PC][8];  g: f32 [9 variants = a*3+b][PR*PC][64]
-__global__ void __launch_bounds__(c1s::kThreads, 1)
-conv1_scene_kernel(const __half* __restrict__ f0, int PR, int PC, const unsigned char* __restrict__ w1p,
-                   const float* __restrict__ b1g, float* __restrict__ g) {
-  using namespace c1s;
-  extern __shared__ __align__(128) unsigned char smem[];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const uint32_t sbase = smem_u32(smem);
-  const uint32_t bars = sbase + S_BAR;
-  float* sbias = reinterpret_cast<float*>(smem + S_BIAS);
-  const int tiles_c = (PC + TW - 1) / TW, tiles_r = (PR + TH - 1) / TH;
-  const int ntiles = tiles_r * tiles_c;
-  const int64_t plane = int64_t(PR) * PC;
-
-  {
-    const uint4* gw = reinterpret_cast<const uint4*>(w1p);
-    uint4* sw = reinterpret_cast<uint4*>(smem + S_W);
-    for (int i = tid; i < WBYTES / 16; i += kThreads) sw[i] = __ldg(gw + i);
-    uint4* z = reinterpret_cast<uint4*>(smem + S_A);
-    for (int i = tid; i < 2 * ABYTES / 16; i += kThreads) z[i] = make_uint4(0, 0, 0, 0);
-  }
-  if (tid < 64) sbias[tid] = b1g[tid];
-  if (tid == 0) {
-    mbar_init(bars + 8 * A_FULL0, kLoad); mbar_init(bars + 8 * A_FULL1, kLoad);
-    mbar_init(bars + 8 * A_EMPTY0, 1 + kEpi); mbar_init(bars + 8 * A_EMPTY1, 1 + kEpi);
-    mbar_init(bars + 8 * D_FULL0, 1); mbar_init(bars + 8 * D_FULL1, 1);
-    mbar_init(bars + 8 * D_EMPTY0, kEpi); mbar_init(bars + 8 * D_EMPTY1, kEpi);
-    fence_barrier_init();
-  }
-  if (warp == 10) tmem_alloc(sbase + S_TMEM, 512);
-  fence_proxy_async();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *reinterpret_cast<volatile uint32_t*>(smem + S_TMEM);
-
-  if (warp >= 8 && warp < 10) {
-    // ================================================================ loaders: (TH+2) x TP entries, zero outside the map
-    const int lt = tid - kEpi;
-    uint32_t j = 0;
-    for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++j) {
-      const uint32_t buf = j & 1, ph = (j >> 1) & 1;
-      const int tr = t / tiles_c, tc = t - tr * tiles_c;
-      const int pr0 = tr * TH - 1, pc0 = tc * TW - 1;          // map coords of entry (ry=0, rx=0)
-      mbar_wait(bars + 8 * (A_EMPTY0 + buf), ph ^ 1, 41);
-      for (int it = lt; it < (TH + 2) * TP * 8; it += kLoad) {
-        const int ch = it & 7, e = it >> 3;
-        const int ry = e / TP, rx = e - ry * TP;
-        const int pr = pr0 + ry, pc = pc0 + rx;
-        const bool in = pr >= 0 && pr < PR && pc >= 0 && pc < PC;
-        const __half* src = f0 + ((int64_t(ch) * PR + (in ? pr : 0)) * PC + (in ? pc : 0)) * 8;
-        cp_async16_zfill(sbase + S_A + buf * ABYTES + ch * CH + (1 + e) * 16, src, in ? 16u : 0u);
-      }
-      cp_async_wait_all();
-      fence_proxy_async();
-      mbar_arrive(bars + 8 * (A_FULL0 + buf));
-    }
-  } else if (warp == 10) {
-    // ================================================================ MMA issuer
-    if (tmem != 0) { printf("conv1_scene: unexpected TMEM base %u\n", tmem); __trap(); }
-    constexpr uint64_t kHi = (uint64_t(128 >> 4) | (uint64_t(1) << 14)) << 32;
-    constexpr uint32_t kI64 = make_idesc_f16(128, 64);
-    const uint32_t w_lo = ((sbase + S_W) >> 4) | (uint32_t(kWLbo >> 4) << 16);
-    uint32_t j = 0, pj = 0;
-    for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++j) {
-      const uint32_t buf = j & 1, ph = (j >> 1) & 1;
-      const uint32_t a_lo = ((sbase + S_A + buf * ABYTES) >> 4) | (uint32_t(CH >> 4) << 16);
-      mbar_wait(bars + 8 * (A_FULL0 + buf), ph, 42);
-#pragma unroll 1
-      for (int b = 0; b < 3; ++b, ++pj) {                     // column class: left {1,2}, mid {0,1,2}, right {0,1}
-        const uint32_t stage = pj & 1, dph = (pj >> 1) & 1;
-        mbar_wait(bars + 8 * (D_EMPTY0 + stage), dph ^ 1, 43);
-        tc_fence_after();
-        if (elect_one_sync()) {
-          const int dx_lo = b == 0 ? 1 : 0, dx_hi = b == 2 ? 1 : 2;
-#pragma unroll
-          for (int dy = 0; dy < 3; ++dy) {
-            const uint32_t d = stage * 192 + dy * 64;
-            uint32_t acc = 0;
-            for (int dx = dx_lo; dx <= dx_hi; ++dx) {
-#pragma unroll
-              for (int ks = 0; ks < 4; ++ks) {
-                const uint32_t a = a_lo + uint32_t(dy * TP + dx) + uint32_t(ks * 2 * CH / 16);
-                const uint32_t bb = w_lo + uint32_t((dx * kWDx + ks * 2 * kWLbo) / 16) + uint32_t((2 - dy) * 64);
-                umma_f16(d, kHi | uint64_t(a), kHi | uint64_t(bb), kI64, acc);
-                acc = 1;
-              }
-            }
-          }
-          umma_commit(bars + 8 * (D_FULL0 + stage));
-          if (b == 2) umma_commit(bars + 8 * (A_EMPTY0 + buf));
-        }
-        __syncwarp();
-      }
-    }
-  } else {
-    // ================================================================ epilogue (warps 0-7)
-    const int L = (warp & 3) * 32 + lane, chalf = warp >> 2;
-    const uint32_t lane_addr = (uint32_t((warp & 3) * 32) << 16) + chalf * 32;
-    const int ty = L >> 5, tx = L & 31;
-    uint32_t j = 0, pj = 0;
-    for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++j) {
-      const uint32_t buf = j & 1;
-      const int tr = t / tiles_c, tc = t - tr * tiles_c;
-      const int pr = tr * TH + ty, pc = tc * TW + tx - 1;
-      const bool valid = tx >= 1 && tx <= TW && pr < PR && pc < PC;
-      const int64_t pos = int64_t(pr) * PC + pc;
-      // residual = centre entry (ty+1, tx) of the tile, 32 channels of this warp's half
-      uint4 res[4];
-      {
-        const unsigned char* rp = smem + S_A + buf * ABYTES + (chalf * 4) * CH + (1 + (ty + 1) * TP + tx) * 16;
-        mbar_wait(bars + 8 * (A_FULL0 + buf), (j >> 1) & 1, 44);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) res[k] = *reinterpret_cast<const uint4*>(rp + k * CH);
-      }
-#pragma unroll 1
-      for (int b = 0; b < 3; ++b, ++pj) {
-        const uint32_t stage = pj & 1, dph = (pj >> 1) & 1;
-        mbar_wait(bars + 8 * (D_FULL0 + stage), dph, 45);
-        tc_fence_after();
-#pragma unroll
-        for (int hgrp = 0; hgrp < 2; ++hgrp) {               // 16 channels at a time
-          float r0[16], r1[16], r2[16];
-          tmem_ld16(lane_addr + stage * 192 + 0 * 64 + hgrp * 16, r0);
-          tmem_ld16(lane_addr + stage * 192 + 1 * 64 + hgrp * 16, r1);
-          tmem_ld16(lane_addr + stage * 192 + 2 * 64 + hgrp * 16, r2);
-          tmem_ld_wait();
-          if (hgrp == 1) { tc_fence_before(); mbar_arrive(bars + 8 * (D_EMPTY0 + stage)); }
-          if (valid) {
-            const __half2* hr = reinterpret_cast<const __half2*>(&res[hgrp * 2]);
-            float base[16];
-#pragma unroll
-            for (int e = 0; e < 8; ++e) {
-              const float2 f = __half22float2(hr[e]);
-              base[2 * e] = f.x + sbias[chalf * 32 + hgrp * 16 + 2 * e];
-              base[2 * e + 1] = f.y + sbias[chalf * 32 + hgrp * 16 + 2 * e + 1];
-            }
-#pragma unroll
-            for (int a = 0; a < 3; ++a) {                    // top = R1+R2, mid = R0+R1+R2, bot = R0+R1
-              float4* dst = reinterpret_cast<float4*>(g + (int64_t(a * 3 + b) * plane + pos) * 64 + chalf * 32 + hgrp * 16);
-#pragma unroll
-              for (int q = 0; q < 4; ++q) {
-                float o[4];
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                  const int c = q * 4 + e;
-                  const float s = a == 0 ? r1[c] + r2[c] : (a == 1 ? r0[c] + r1[c] + r2[c] : r0[c] + r1[c]);
-                  o[e] = fmaxf(s + base[c], 0.f);
-                }
-                dst[q] = make_float4(o[0], o[1], o[2], o[3]);
-              }
-            }
-          }
-        }
-      }
-      mbar_arrive(bars + 8 * (A_EMPTY0 + buf));               // residual (and the MMAs, by their commit) done with A
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 10) { tc_fence_after(); tmem_dealloc(tmem, 512); }
-}
-
-// 2x2 average pools of the conv1 variants for every top-left position (pr, pc), pr < PR-1, pc < PC-1:
-//   PM[A][B][pr,pc] = 1/4 sum_{u,v in {0,1}} G[a(A,u)][b(B,v)][pr+u, pc+v]
-//   a(top,0)=top a(top,1)=mid   a(mid,.)=mid   a(bot,0)=mid a(bot,1)=bot     (pooled row 0 / 1..8 / 9)
-// written f16 position-major [9][PR][PC][64]: one 128-byte line per pooled cell, which is what the
-// per-pixel conv2 gather (every other row / column) fetches -- 100 lines per pixel.
-__global__ void pool1_scene_kernel(const float* __restrict__ g, int PR, int PC, __half* __restrict__ pm) {
-  const int64_t plane = int64_t(PR) * PC;
-  const int64_t total = plane * 8;
-  for (int64_t t = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; t < total; t += int64_t(gridDim.x) * blockDim.x) {
-    const int64_t pos = t >> 3;
-    const int ch = int(t & 7);
-    const int pr = int(pos / PC), pc = int(pos - int64_t(pr) * PC);
-    if (pr >= PR - 1 || pc >= PC - 1) continue;
-#pragma unroll
-    for (int A = 0; A < 3; ++A) {
-      const int a0 = A == 0 ? 0 : 1, a1 = A == 2 ? 2 : 1;
-#pragma unroll
-      for (int B = 0; B < 3; ++B) {
-        const int b0 = B == 0 ? 0 : 1, b1 = B == 2 ? 2 : 1;
-        const float4* p00 = reinterpret_cast<const float4*>(g + (int64_t(a0 * 3 + b0) * plane + pos) * 64 + ch * 8);
-        const float4* p01 = reinterpret_cast<const float4*>(g + (int64_t(a0 * 3 + b1) * plane + pos + 1) * 64 + ch * 8);
-        const float4* p10 = reinterpret_cast<const float4*>(g + (int64_t(a1 * 3 + b0) * plane + pos + PC) * 64 + ch * 8);
-        const float4* p11 = reinterpret_cast<const float4*>(g + (int64_t(a1 * 3 + b1) * plane + pos + PC + 1) * 64 + ch * 8);
-        __half2 h[4];
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-          const float4 x00 = __ldg(p00 + q), x01 = __ldg(p01 + q), x10 = __ldg(p10 + q), x11 = __ldg(p11 + q);
-          // same association as the per-pixel kernel: (row y + row y+1) then + horizontal neighbour, * 0.25
-          h[2 * q] = __floats2half2_rn(((x00.x + x10.x) + (x01.x + x11.x)) * 0.25f, ((x00.y + x10.y) + (x01.y + x11.y)) * 0.25f);
-          h[2 * q + 1] = __floats2half2_rn(((x00.z + x10.z) + (x01.z + x11.z)) * 0.25f, ((x00.w + x10.w) + (x01.w + x11.w)) * 0.25f);
-        }
-        *reinterpret_cast<uint4*>(pm + (int64_t(A * 3 + B) * plane + pos) * 64 + ch * 8) = *reinterpret_cast<uint4*>(h);
-      }
-    }
-  }
-}
-
-
-// =================================================================================================
-// conv1_pool_kernel: the 9 conv1 border-class variants AND their 2x2 average pools in ONE kernel -- the fp32
-// variants G (2.3 KB per scene position) never touch HBM.  Same tile / tap-as-descriptor-offset machinery as
-// conv1_scene_kernel, but
+// zero-haloed shared-memory tile loaded by TMA:
 //   * the tensor core produces the nine single-tap-column sums  T[dy][dx] = sum_ci W1[dy,dx] . F0[p+(dy-1,dx-1)]
 //     separately (N = 32 channels at a time: sub-stage (h, dy) = T[dy][0..2] in 96 TMEM columns, ring of 5), so
 //     that all three column classes  R[dy][left|mid|right] = T1+T2 | T0+T1+T2 | T0+T1  are formed in the
-//     epilogue from one TMEM read (36 MMAs per 32 channels instead of 84);
+//     epilogue from one TMEM read (36 MMAs per 32 channels), and the row classes from them as
+//     top = R1+R2, mid = R0+R1+R2, bot = R0+R1;
 //   * a tile's 4 conv rows give 3 pooled rows and its 30 conv columns 29 pooled columns: the vertical 2x2
 //     partner (ty+1, tx) lives in another warp (TMEM lane quarter) and comes through a double-buffered
 //     shared-memory exchange, the horizontal partner (tx+1) through a warp shuffle;
@@ -250,6 +30,12 @@ __global__ void pool1_scene_kernel(const float* __restrict__ g, int PR, int PC, 
 //     per thread and pass.
 //   V[A][b]  = G[a0(A)][b](y,x) + G[a1(A)][b](y+1,x)                 (a0,a1 = top,mid | mid,mid | mid,bot)
 //   PM[A][B] = 1/4 (V[A][b0(B)](x) + V[A][b1(B)](x+1))               (b0,b1 = left,mid | mid,mid | mid,right)
+#include "common.cuh"
+#include "sm100_ptx.cuh"
+#include "tma.cuh"
+
+namespace cmlpl {
+
 namespace c1p {
 constexpr int TH = 4, TP = 32, OH = 3, OW = 29;      // conv rows, row pitch; pooled rows / columns per tile
 constexpr int CH = (TH + 2) * TP * 16;               // 3 072: one chunk plane of the conv0 tile, dense (written by TMA)
@@ -491,36 +277,6 @@ conv1_pool_kernel(const __grid_constant__ CUtensorMap tm_f0, int PR, int PC, int
 using namespace cmlpl;
 
 CMLPL_TRACE_EXPORT(cmlpl_debug_c1p_trace)
-
-extern "C" int cmlpl_conv1_scene_variants_f32(const void* f0pad, int cols, int w, int band_rows, const void* packed,
-                                              float* g, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(f0pad && packed && g, "conv1_scene: null pointer");
-  CMLPL_CHECK_ARG(w == 20 && cols > 0 && band_rows > 0, "conv1_scene: bad dims (w must be 20)");
-  const int PR = band_rows + w - 1, PC = cols + w - 1;
-  const PackedLayout L = packed_layout(1, 1, w);
-  const unsigned char* pk = static_cast<const unsigned char*>(packed);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  CMLPL_MAX_DYN_SMEM(conv1_scene_kernel, c1s::SMEM);
-  const int ntiles = ((PR + c1s::TH - 1) / c1s::TH) * ((PC + c1s::TW - 1) / c1s::TW);
-  int grid = sm_count(); if (grid > ntiles) grid = ntiles;
-  conv1_scene_kernel<<<grid, c1s::kThreads, c1s::SMEM, s>>>(static_cast<const __half*>(f0pad), PR, PC, pk + L.w1,
-                                                            reinterpret_cast<const float*>(pk + L.b1), g);
-  CMLPL_CHECK_LAUNCH("conv1_scene");
-  return CMLPL_OK;
-}
-
-extern "C" int cmlpl_conv1_scene_f16(const void* f0pad, int cols, int w, int band_rows, const void* packed, float* g,
-                                     void* pm, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(pm, "conv1_scene: null pointer");
-  const int rc = cmlpl_conv1_scene_variants_f32(f0pad, cols, w, band_rows, packed, g, stream);
-  if (rc != CMLPL_OK) return rc;
-  const int PR = band_rows + w - 1, PC = cols + w - 1;
-  const int64_t total = int64_t(PR) * PC * 8;
-  int64_t pg = (total + 255) / 256; const int64_t cap = int64_t(sm_count()) * 16; if (pg > cap) pg = cap;
-  pool1_scene_kernel<<<int(pg), 256, 0, static_cast<cudaStream_t>(stream)>>>(g, PR, PC, static_cast<__half*>(pm));
-  CMLPL_CHECK_LAUNCH("pool1_scene");
-  return CMLPL_OK;
-}
 
 // conv1 variants + pooling fused (conv1_pool_kernel): f0pad -> pooled parity planes, no fp32 scratch
 extern "C" int cmlpl_conv1_pool_planes_f16(const void* f0pad, int cols, int w, int band_rows, const void* packed,

@@ -1,6 +1,6 @@
 // Scene-level conv2 + pool + classifier with exact compute sharing (SURVEY section 7 / 8-f3, second half).
 //
-// After conv1_scene the pooled conv1 window of pixel (r,c) is  PM[A(i)][B(j)][r+2i, c+2j]  (i,j = 0..9,
+// After conv1_pool_kernel (conv1_scene_sm100.cu) the pooled conv1 window of pixel (r,c) is  PM[A(i)][B(j)][r+2i, c+2j]  (i,j = 0..9,
 // A/B = top/mid/bot border class of the pooled row/column).  Everything downstream of it
 // (tools/models.py:137-150: conv2 3x3 with zero padding at the PATCH border, +residual, ReLU, 2x2
 // average pool, the conv columns of the classifier) again depends only on the scene position and on
@@ -30,53 +30,6 @@
 #include "tma.cuh"
 
 namespace cmlpl {
-
-// 2x2 average pools of the conv1 variants (see pool1_scene_kernel) written as PARITY PLANES, chunk-planar:
-//   pmq f16 [9 variants][4 planes = (pr&1)*2 + (pc&1)][8 chunks][PR2][PC2][8 channels]
-// entries without a pooled cell (pr >= PR-1 or pc >= PC-1) are zero.
-__global__ void pool1q_scene_kernel(const float* __restrict__ g, int PR, int PC, int PR2, int PC2,
-                                    __half* __restrict__ pmq) {
-  const int64_t plane = int64_t(PR) * PC;
-  const int64_t psz = int64_t(PR2) * PC2;
-  const int64_t total = 4 * psz * 8;
-  for (int64_t t = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; t < total; t += int64_t(gridDim.x) * blockDim.x) {
-    // 8 consecutive threads = the 8 channel chunks of one position: 256-B contiguous reads of g, and a warp's
-    // four positions write 64 contiguous bytes into each chunk plane
-    const int ch = int(t & 7);
-    int64_t r = t >> 3;
-    const int x2 = int(r % PC2); r /= PC2;
-    const int y2 = int(r % PR2), pl = int(r / PR2);
-    const int pr = 2 * y2 + (pl >> 1), pc = 2 * x2 + (pl & 1);
-    const bool valid = pr < PR - 1 && pc < PC - 1;
-    const int64_t pos = int64_t(pr) * PC + pc;
-#pragma unroll
-    for (int A = 0; A < 3; ++A) {
-      const int a0 = A == 0 ? 0 : 1, a1 = A == 2 ? 2 : 1;
-#pragma unroll
-      for (int B = 0; B < 3; ++B) {
-        const int b0 = B == 0 ? 0 : 1, b1 = B == 2 ? 2 : 1;
-        __half2 h[4];
-        if (valid) {
-          const float4* p00 = reinterpret_cast<const float4*>(g + (int64_t(a0 * 3 + b0) * plane + pos) * 64 + ch * 8);
-          const float4* p01 = reinterpret_cast<const float4*>(g + (int64_t(a0 * 3 + b1) * plane + pos + 1) * 64 + ch * 8);
-          const float4* p10 = reinterpret_cast<const float4*>(g + (int64_t(a1 * 3 + b0) * plane + pos + PC) * 64 + ch * 8);
-          const float4* p11 = reinterpret_cast<const float4*>(g + (int64_t(a1 * 3 + b1) * plane + pos + PC + 1) * 64 + ch * 8);
-#pragma unroll
-          for (int q = 0; q < 2; ++q) {
-            const float4 x00 = __ldg(p00 + q), x01 = __ldg(p01 + q), x10 = __ldg(p10 + q), x11 = __ldg(p11 + q);
-            h[2 * q] = __floats2half2_rn(((x00.x + x10.x) + (x01.x + x11.x)) * 0.25f, ((x00.y + x10.y) + (x01.y + x11.y)) * 0.25f);
-            h[2 * q + 1] = __floats2half2_rn(((x00.z + x10.z) + (x01.z + x11.z)) * 0.25f, ((x00.w + x10.w) + (x01.w + x11.w)) * 0.25f);
-          }
-        } else {
-#pragma unroll
-          for (int q = 0; q < 4; ++q) h[q] = __floats2half2_rn(0.f, 0.f);
-        }
-        *reinterpret_cast<uint4*>(pmq + ((int64_t((A * 3 + B) * 4 + pl) * 8 + ch) * psz + int64_t(y2) * PC2 + x2) * 8) =
-            *reinterpret_cast<uint4*>(h);
-      }
-    }
-  }
-}
 
 // =================================================================================================
 // conv2_scene_kernel: persistent, warp-specialised tcgen05 implicit GEMM over 4x30-position tiles of a
@@ -653,20 +606,6 @@ pool2_cls_kernel(const __grid_constant__ CUtensorMap tm_y, int PR2, int PC2, int
 }  // namespace cmlpl
 
 using namespace cmlpl;
-
-extern "C" int cmlpl_conv1_scene_planes_f16(const void* f0pad, int cols, int w, int band_rows, const void* packed,
-                                            float* g, void* pmq, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(f0pad && packed && g && pmq, "conv1_scene_planes: null pointer");
-  CMLPL_CHECK_ARG(w == 20 && cols > 0 && band_rows > 0, "conv1_scene_planes: bad dims (w must be 20)");
-  const int rc = cmlpl_conv1_scene_variants_f32(f0pad, cols, w, band_rows, packed, g, stream);
-  if (rc != CMLPL_OK) return rc;
-  const int PR = band_rows + w - 1, PC = cols + w - 1, PR2 = (PR + 1) / 2, PC2 = (PC + 1) / 2;
-  const int64_t total = int64_t(4) * PR2 * PC2 * 8;
-  int64_t pg = (total + 255) / 256; const int64_t cap = int64_t(sm_count()) * 16; if (pg > cap) pg = cap;
-  pool1q_scene_kernel<<<int(pg), 256, 0, static_cast<cudaStream_t>(stream)>>>(g, PR, PC, PR2, PC2, static_cast<__half*>(pmq));
-  CMLPL_CHECK_LAUNCH("pool1q_scene");
-  return CMLPL_OK;
-}
 
 CMLPL_TRACE_EXPORT(cmlpl_debug_c2s_trace)
 

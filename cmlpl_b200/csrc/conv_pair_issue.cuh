@@ -1,4 +1,4 @@
-// Issue helper shared by the per-pixel tcgen05 conv kernels (patch_cnn_sm100.cu, patch_conv2_sm100.cu).
+// Issue helper of the per-pixel tcgen05 conv kernel (patch_cnn_sm100.cu: conv1 and conv2, inference and training).
 #pragma once
 #include "sm100_ptx.cuh"
 

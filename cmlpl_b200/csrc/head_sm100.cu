@@ -1,16 +1,11 @@
-// Tensor-core head of the scene path (sm_100a): the spectral branch relu(feat_spe(x))
-// (tools/models.py:142-143) and the classifier over [conv features | spectral features] + argmax
-// (models.py:144,150; hyper_tools.py:426) as two tcgen05 GEMMs with fp16 operands / fp32 accumulate.
-//
-// Every A operand lives in HBM already in the UMMA "no-swizzle K-major" tile layout
-//     [m-tile][K/8 chunks][128 rows][8 halves]
-// so that a K-slab of a tile is one contiguous block: the loader is a single thread issuing
-// cp.async.bulk (UBLKCP) copies that complete on an mbarrier, and a chunk needs no repacking
-// before tcgen05.mma reads it.  x16_tile_kernel writes the spectra in this layout,
-// spectral_hidden_kernel writes the 1024 hidden features in it, and patch_cnn writes the pooled
-// conv features in it (p2_tiled).
-//   spectral_hidden_kernel: H = relu(X . Wspe^T + b)    M=128 x N=256 tiles, K = B (padded to 16)
-//   head_kernel           : logits = [P2 | H] . Wc^T + bc, argmax     M=128 x N=16, K = 1600 + 1024
+// Tensor-core head of the scene path (sm_100a): the spectral branch relu(feat_spe(x)) (tools/models.py:142-143)
+// and its classifier columns (models.py:150) as two chained tcgen05 GEMMs with fp16 operands / fp32 accumulate,
+// then the sum of all logit partials + argmax (models.py:144,150; hyper_tools.py:426).
+//   x16_tile(_raw)_kernel  : spectra (or the z-scored raw cube) -> fp16 A-operand tiles in the UMMA "no-swizzle
+//                            K-major" layout [m-tile][K/8 chunks][128 rows][8 halves], so that a tile is one
+//                            contiguous block the loader moves with cp.async.bulk (UBLKCP) and tcgen05.mma reads as is
+//   spectral_logits_kernel : part = Wc_spe . relu(Wspe . x + b) per hidden quarter, the hidden features never in HBM
+//   head_sum_kernel        : logits = bc + spectral partials + the gathered conv partials of pool2_cls_kernel, argmax
 #include "common.cuh"
 #include "sm100_ptx.cuh"
 
@@ -57,218 +52,6 @@ __global__ void x16_tile_raw_kernel(const T* __restrict__ X, int64_t n, int B, i
     *reinterpret_cast<uint4*>(out + t * 8) = *reinterpret_cast<uint4*>(h);
   }
 }
-
-// ------------------------------------------------------------------ H = relu(X . W^T + b)
-constexpr int kHidThreads = 320;   // warps 0-7 epilogue, warp 8 loader, warp 9 MMA issuer
-
-__global__ void __launch_bounds__(kHidThreads, 1)
-spectral_hidden_kernel(const __half* __restrict__ x16, int64_t mtiles, int KC, const __half* __restrict__ w1t,
-                       const float* __restrict__ bspe, __half* __restrict__ h16) {
-  extern __shared__ __align__(128) unsigned char smem[];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const uint32_t sbase = smem_u32(smem);
-  const uint32_t wbytes = uint32_t(KC) * 4096, abytes = uint32_t(KC) * 2048;
-  const uint32_t S_W = 0, S_A = wbytes, S_BIAS = S_A + 2 * abytes, S_BAR = S_BIAS + 1024, S_TMEM = S_BAR + 64;
-  const uint32_t bars = sbase + S_BAR;
-  enum { A_FULL0 = 0, A_FULL1, A_EMPTY0, A_EMPTY1, D_FULL0, D_FULL1, D_EMPTY0, D_EMPTY1 };
-  const int ntile = blockIdx.x & 3;
-  const int64_t mt0 = blockIdx.x >> 2, mstep = gridDim.x >> 2;
-
-  {  // weights of this N tile (already in UMMA layout) and its bias slice
-    const uint4* g = reinterpret_cast<const uint4*>(w1t) + size_t(ntile) * (wbytes / 16);
-    uint4* s = reinterpret_cast<uint4*>(smem + S_W);
-    for (uint32_t i = tid; i < wbytes / 16; i += kHidThreads) s[i] = __ldg(g + i);
-    float* sb = reinterpret_cast<float*>(smem + S_BIAS);
-    if (tid < 256) sb[tid] = bspe[ntile * 256 + tid];
-  }
-  if (tid == 0) {
-    mbar_init(bars + 8 * A_FULL0, 1); mbar_init(bars + 8 * A_FULL1, 1);
-    mbar_init(bars + 8 * A_EMPTY0, 1); mbar_init(bars + 8 * A_EMPTY1, 1);
-    mbar_init(bars + 8 * D_FULL0, 1); mbar_init(bars + 8 * D_FULL1, 1);
-    mbar_init(bars + 8 * D_EMPTY0, 256); mbar_init(bars + 8 * D_EMPTY1, 256);
-    fence_barrier_init();
-  }
-  if (warp == 9) tmem_alloc(sbase + S_TMEM, 512);
-  fence_proxy_async();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *reinterpret_cast<volatile uint32_t*>(smem + S_TMEM);
-
-  if (warp == 8) {
-    if (lane == 0) {
-      uint32_t j = 0;
-      for (int64_t mt = mt0; mt < mtiles; mt += mstep, ++j) {
-        const uint32_t s = j & 1, ph = (j >> 1) & 1;
-        mbar_wait(bars + 8 * (A_EMPTY0 + s), ph ^ 1, 21);
-        mbar_arrive_expect_tx(bars + 8 * (A_FULL0 + s), abytes);
-        bulk_g2s(sbase + S_A + s * abytes, x16 + mt * int64_t(KC) * 1024, abytes, bars + 8 * (A_FULL0 + s));
-      }
-    }
-  } else if (warp == 9) {
-    if (tmem != 0) { printf("spectral_hidden: unexpected TMEM base %u\n", tmem); __trap(); }
-    constexpr uint64_t kHi = (uint64_t(128 >> 4) | (uint64_t(1) << 14)) << 32;
-    constexpr uint32_t idesc = make_idesc_f16(128, 256);
-    uint32_t j = 0;
-    for (int64_t mt = mt0; mt < mtiles; mt += mstep, ++j) {
-      const uint32_t s = j & 1, ph = (j >> 1) & 1;
-      mbar_wait(bars + 8 * (A_FULL0 + s), ph, 22);
-      mbar_wait(bars + 8 * (D_EMPTY0 + s), ph ^ 1, 23);
-      tc_fence_after();
-      if (elect_one_sync()) {
-        uint32_t a_lo = ((sbase + S_A + s * abytes) >> 4) | (uint32_t(2048 >> 4) << 16);
-        uint32_t b_lo = ((sbase + S_W) >> 4) | (uint32_t(4096 >> 4) << 16);
-        for (int ks = 0; ks < KC / 2; ++ks) {
-          umma_f16(s * 256, kHi | a_lo, kHi | b_lo, idesc, ks ? 1u : 0u);
-          a_lo += 4096 >> 4; b_lo += 8192 >> 4;
-        }
-        umma_commit(bars + 8 * (A_EMPTY0 + s));
-        umma_commit(bars + 8 * (D_FULL0 + s));
-      }
-      __syncwarp();
-    }
-  } else {
-    const int L = (warp & 3) * 32 + lane, chalf = warp >> 2;
-    const uint32_t lane_addr = (uint32_t((warp & 3) * 32) << 16) + chalf * 128;
-    const float* sb = reinterpret_cast<const float*>(smem + S_BIAS) + chalf * 128;
-    uint32_t j = 0;
-    for (int64_t mt = mt0; mt < mtiles; mt += mstep, ++j) {
-      const uint32_t s = j & 1, ph = (j >> 1) & 1;
-      __half* dst = h16 + ((mt * 128 + (ntile * 32 + chalf * 16)) * 128 + L) * 8;
-      mbar_wait(bars + 8 * (D_FULL0 + s), ph, 24);
-      tc_fence_after();
-#pragma unroll 1
-      for (int g = 0; g < 8; g += 2) {
-        float v0[16], v1[16];
-        tmem_ld16(lane_addr + s * 256 + g * 16, v0);
-        tmem_ld16(lane_addr + s * 256 + g * 16 + 16, v1);
-        tmem_ld_wait();
-        if (g == 6) { tc_fence_before(); mbar_arrive(bars + 8 * (D_EMPTY0 + s)); }
-        __half2 h[16];
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-          h[e] = __floats2half2_rn(fmaxf(v0[2 * e] + sb[g * 16 + 2 * e], 0.f), fmaxf(v0[2 * e + 1] + sb[g * 16 + 2 * e + 1], 0.f));
-          h[8 + e] = __floats2half2_rn(fmaxf(v1[2 * e] + sb[g * 16 + 16 + 2 * e], 0.f),
-                                        fmaxf(v1[2 * e + 1] + sb[g * 16 + 16 + 2 * e + 1], 0.f));
-        }
-        const uint4* hv = reinterpret_cast<const uint4*>(h);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) *reinterpret_cast<uint4*>(dst + (g * 2 + q) * 1024) = hv[q];
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 9) { tc_fence_after(); tmem_dealloc(tmem, 512); }
-}
-
-// ------------------------------------------------------------------ logits = [P2 | H] . Wc^T + bc ; argmax
-constexpr int kHeadThreads = 192;   // warps 0-3 epilogue, warp 4 loader, warp 5 MMA issuer
-constexpr int kHeadStages = 6, kHeadChunkKc = 8, kHeadChunkBytes = kHeadChunkKc * 2048;
-
-__global__ void __launch_bounds__(kHeadThreads, 1)
-head_kernel(const __half* __restrict__ p2t, int kc_conv, const __half* __restrict__ h16, int kc_spe, int64_t mtiles,
-            int64_t n, int C, const __half* __restrict__ wc16, const float* __restrict__ bc,
-            uint8_t* __restrict__ labels, float* __restrict__ logits) {
-  extern __shared__ __align__(128) unsigned char smem[];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const uint32_t sbase = smem_u32(smem);
-  const int kc_all = kc_conv + kc_spe;
-  const uint32_t wbytes = uint32_t(kc_all) * 256;
-  const uint32_t S_W = 0, S_A = (wbytes + 127) / 128 * 128, S_BAR = S_A + kHeadStages * kHeadChunkBytes, S_TMEM = S_BAR + 256;
-  const uint32_t bars = sbase + S_BAR;
-  // barriers: full[0..5], empty[6..11], d_full[12,13], d_empty[14,15]
-  {
-    const uint4* g = reinterpret_cast<const uint4*>(wc16);
-    uint4* s = reinterpret_cast<uint4*>(smem + S_W);
-    for (uint32_t i = tid; i < wbytes / 16; i += kHeadThreads) s[i] = __ldg(g + i);
-  }
-  if (tid == 0) {
-    for (int i = 0; i < kHeadStages; ++i) { mbar_init(bars + 8 * i, 1); mbar_init(bars + 8 * (kHeadStages + i), 1); }
-    mbar_init(bars + 8 * 12, 1); mbar_init(bars + 8 * 13, 1);
-    mbar_init(bars + 8 * 14, 128); mbar_init(bars + 8 * 15, 128);
-    fence_barrier_init();
-  }
-  if (warp == 5) tmem_alloc(sbase + S_TMEM, 32);
-  fence_proxy_async();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *reinterpret_cast<volatile uint32_t*>(smem + S_TMEM);
-  const int nch_conv = kc_conv / kHeadChunkKc, nch = nch_conv + kc_spe / kHeadChunkKc;
-
-  if (warp == 4) {
-    if (lane == 0) {
-      uint32_t it = 0;
-      for (int64_t mt = blockIdx.x; mt < mtiles; mt += gridDim.x) {
-        for (int c = 0; c < nch; ++c, ++it) {
-          const uint32_t s = it % kHeadStages, ph = (it / kHeadStages) & 1;
-          mbar_wait(bars + 8 * (kHeadStages + s), ph ^ 1, 31);
-          mbar_arrive_expect_tx(bars + 8 * s, kHeadChunkBytes);
-          const __half* src = c < nch_conv ? p2t + (mt * kc_conv + int64_t(c) * kHeadChunkKc) * 1024
-                                           : h16 + (mt * kc_spe + int64_t(c - nch_conv) * kHeadChunkKc) * 1024;
-          bulk_g2s(sbase + S_A + s * kHeadChunkBytes, src, kHeadChunkBytes, bars + 8 * s);
-        }
-      }
-    }
-  } else if (warp == 5) {
-    constexpr uint64_t kHi = (uint64_t(128 >> 4) | (uint64_t(1) << 14)) << 32;
-    constexpr uint32_t idesc = make_idesc_f16(128, 16);
-    uint32_t it = 0, tj = 0;
-    for (int64_t mt = blockIdx.x; mt < mtiles; mt += gridDim.x, ++tj) {
-      const uint32_t acc = tj & 1, aph = (tj >> 1) & 1;
-      mbar_wait(bars + 8 * (14 + acc), aph ^ 1, 32);
-      tc_fence_after();
-      for (int c = 0; c < nch; ++c, ++it) {
-        const uint32_t s = it % kHeadStages, ph = (it / kHeadStages) & 1;
-        mbar_wait(bars + 8 * s, ph, 33);
-        tc_fence_after();
-        if (elect_one_sync()) {
-          uint32_t a_lo = ((sbase + S_A + s * kHeadChunkBytes) >> 4) | (uint32_t(2048 >> 4) << 16);
-          uint32_t b_lo = ((sbase + S_W + uint32_t(c) * kHeadChunkKc * 256) >> 4) | (uint32_t(256 >> 4) << 16);
-#pragma unroll
-          for (int ks = 0; ks < kHeadChunkKc / 2; ++ks) {
-            umma_f16(tmem + acc * 16, kHi | a_lo, kHi | b_lo, idesc, (c | ks) ? 1u : 0u);
-            a_lo += 4096 >> 4; b_lo += 512 >> 4;
-          }
-          umma_commit(bars + 8 * (kHeadStages + s));
-          if (c == nch - 1) umma_commit(bars + 8 * (12 + acc));
-        }
-        __syncwarp();
-      }
-    }
-  } else {
-    const int L = warp * 32 + lane;
-    uint32_t tj = 0;
-    for (int64_t mt = blockIdx.x; mt < mtiles; mt += gridDim.x, ++tj) {
-      const uint32_t acc = tj & 1, aph = (tj >> 1) & 1;
-      mbar_wait(bars + 8 * (12 + acc), aph, 34);
-      tc_fence_after();
-      float v[16];
-      tmem_ld16(tmem + (uint32_t(warp * 32) << 16) + acc * 16, v);
-      tmem_ld_wait();
-      tc_fence_before();
-      mbar_arrive(bars + 8 * (14 + acc));
-      const int64_t p = mt * 128 + L;
-      if (p < n) {
-        float best = -INFINITY; int arg = 0;
-#pragma unroll
-        for (int c = 0; c < 16; ++c) {
-          if (c < C) {
-            const float z = v[c] + __ldg(bc + c);
-            if (logits) logits[p * C + c] = z;
-            if (z > best) { best = z; arg = c; }        // strict '>': first index wins ties (hyper_tools.py:426)
-          }
-        }
-        labels[p] = uint8_t(arg);
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 5) { tc_fence_after(); tmem_dealloc(tmem, 32); }
-}
-
 
 // ------------------------------------------------------------------ spectral logits: Wc_spe . relu(Wspe . x + b), hidden never in HBM
 // spectral_logits_kernel fuses the two GEMMs of the spectral branch (models.py:142-143 and the spectral columns of
@@ -552,16 +335,18 @@ static bool spectral_logits_plan(int KC, int NC, int* nA, size_t* smem) {
   return false;
 }
 
-static int spectral_hidden_impl(const void* x, int dtype /* -1 = preprocessed f32 spectra */, int64_t n, int num_features,
-                                int num_classes, int w, const float* mu, const float* inv_sigma, const void* packed,
-                                void* x16, void* h16, cmlpl_stream_t stream, bool fused_logits = false) {
-  CMLPL_CHECK_ARG(x && packed && x16 && h16, "spectral_hidden_tc: null pointer");
-  CMLPL_CHECK_ARG(n > 0 && num_features > 0, "spectral_hidden_tc: bad dims");
+// x16_tile(_raw) + spectral_logits_kernel: x16 is scratch for the fp16 input tiles, part f32 [4][ceil(n/128)*128][NC].
+static int launch_spectral_logits(const void* x, int dtype /* -1 = preprocessed f32 spectra */, int64_t n, int num_features,
+                                  int num_classes, int w, const float* mu, const float* inv_sigma, const void* packed,
+                                  void* x16, float* part, cmlpl_stream_t stream) {
+  CMLPL_CHECK_ARG(x && packed && x16 && part, "spectral_logits_tc: null pointer");
+  CMLPL_CHECK_ARG(n > 0 && num_features > 0, "spectral_logits_tc: bad dims");
+  CMLPL_CHECK_ARG(num_classes <= 32, "spectral_logits_tc: needs <= 32 classes, got %d", num_classes);
   const PackedLayout L = packed_layout(num_features, num_classes, w);
-  CMLPL_CHECK_ARG(L.kc_spe_in <= (fused_logits ? 28 : 26), "spectral_hidden_tc: %d bands exceed what the tensor-core tile supports",
-                  num_features);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
   const int KC = L.kc_spe_in;
+  int nA = 0; size_t smem = 0;
+  CMLPL_CHECK_ARG(spectral_logits_plan(KC, L.nc, &nA, &smem), "spectral_logits_tc: %d bands do not fit shared memory", num_features);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
   const int64_t mtiles = (n + 127) / 128, total = mtiles * KC * 128;
   int64_t g = (total + 255) / 256; const int64_t cap = int64_t(sm_count()) * 16; if (g > cap) g = cap;
   if (dtype < 0)
@@ -571,87 +356,38 @@ static int spectral_hidden_impl(const void* x, int dtype /* -1 = preprocessed f3
   else
     x16_tile_raw_kernel<float><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), n, num_features, KC, total, mu, inv_sigma, static_cast<__half*>(x16));
   CMLPL_CHECK_LAUNCH("x16_tile");
-  if (fused_logits) {
-    int nA = 0; size_t fsmem = 0;
-    CMLPL_CHECK_ARG(spectral_logits_plan(KC, L.nc, &nA, &fsmem), "spectral_logits_tc: %d bands do not fit shared memory", num_features);
-    CMLPL_CHECK_ARG(num_classes <= 32, "spectral_logits_tc: needs <= 32 classes, got %d", num_classes);
-    int fgrid = sm_count() / 4 * 4;
-    if (fgrid > mtiles * 4) fgrid = int(mtiles * 4);
-    const unsigned char* fpk = static_cast<const unsigned char*>(packed);
-    const __half* w1s = reinterpret_cast<const __half*>(fpk + L.w1s);
-    const float* bspe = reinterpret_cast<const float*>(fpk + L.bspe);
-    const __half* wc_spe16 = reinterpret_cast<const __half*>(fpk + L.wc16 + size_t(L.conv_pos) * 8 * L.nc * 16);
-    if (L.nc == 16) {
-      CMLPL_MAX_DYN_SMEM(spectral_logits_kernel<16>, int(fsmem));
-      spectral_logits_kernel<16><<<fgrid, spl::kThreads, fsmem, s>>>(static_cast<const __half*>(x16), mtiles, KC, nA, w1s, bspe,
-                                                                     wc_spe16, static_cast<float*>(h16));
-    } else {
-      CMLPL_MAX_DYN_SMEM(spectral_logits_kernel<32>, int(fsmem));
-      spectral_logits_kernel<32><<<fgrid, spl::kThreads, fsmem, s>>>(static_cast<const __half*>(x16), mtiles, KC, nA, w1s, bspe,
-                                                                     wc_spe16, static_cast<float*>(h16));
-    }
-    CMLPL_CHECK_LAUNCH("spectral_logits");
-    return CMLPL_OK;
-  }
-  const size_t smem = size_t(KC) * 8192 + 1024 + 64 + 64;
-  CMLPL_MAX_DYN_SMEM(spectral_hidden_kernel, int(smem));
   int grid = sm_count() / 4 * 4;
   if (grid > mtiles * 4) grid = int(mtiles * 4);
   const unsigned char* pk = static_cast<const unsigned char*>(packed);
-  spectral_hidden_kernel<<<grid, kHidThreads, smem, s>>>(static_cast<const __half*>(x16), mtiles, KC,
-                                                         reinterpret_cast<const __half*>(pk + L.w1s),
-                                                         reinterpret_cast<const float*>(pk + L.bspe),
-                                                         static_cast<__half*>(h16));
-  CMLPL_CHECK_LAUNCH("spectral_hidden");
-  return CMLPL_OK;
-}
-
-extern "C" int cmlpl_spectral_hidden_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
-                                        const void* packed, void* x16, void* h16, cmlpl_stream_t stream) {
-  return spectral_hidden_impl(spectra, -1, n, num_features, num_classes, w, nullptr, nullptr, packed, x16, h16, stream);
-}
-
-extern "C" int cmlpl_spectral_hidden_raw_tc(const void* raw, int dtype, int64_t n, int num_features, int num_classes, int w,
-                                            const float* mu, const float* inv_sigma, const void* packed, void* x16,
-                                            void* h16, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG((dtype == 0 || dtype == 1) && mu && inv_sigma, "spectral_hidden_raw_tc: bad args");
-  return spectral_hidden_impl(raw, dtype, n, num_features, num_classes, w, mu, inv_sigma, packed, x16, h16, stream);
-}
-
-extern "C" int cmlpl_head_tc(const void* p2t, const void* h16, int64_t n, int num_features, int num_classes, int w,
-                             const void* packed, uint8_t* labels, float* logits, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(p2t && h16 && packed && labels, "head_tc: null pointer");
-  CMLPL_CHECK_ARG(n > 0 && num_classes > 0 && num_classes <= 16, "head_tc: needs 1..16 classes, got %d", num_classes);
-  const PackedLayout L = packed_layout(num_features, num_classes, w);
-  const int kc_conv = L.conv_pos * 8, kc_spe = 128;
-  CMLPL_CHECK_ARG(kc_conv % kHeadChunkKc == 0, "head_tc: conv feature width %d not a multiple of 64", kc_conv * 8);
-  const size_t wbytes = size_t(kc_conv + kc_spe) * 256;
-  const size_t smem = (wbytes + 127) / 128 * 128 + size_t(kHeadStages) * kHeadChunkBytes + 256 + 64;
-  CMLPL_CHECK_ARG(smem <= 227 * 1024, "head_tc: shared memory %zu too large", smem);
-  CMLPL_MAX_DYN_SMEM(head_kernel, int(smem));
-  const int64_t mtiles = (n + 127) / 128;
-  int grid = sm_count(); if (grid > mtiles) grid = int(mtiles);
-  const unsigned char* pk = static_cast<const unsigned char*>(packed);
-  head_kernel<<<grid, kHeadThreads, smem, static_cast<cudaStream_t>(stream)>>>(
-      static_cast<const __half*>(p2t), kc_conv, static_cast<const __half*>(h16), kc_spe, mtiles, n, num_classes,
-      reinterpret_cast<const __half*>(pk + L.wc16), reinterpret_cast<const float*>(pk + L.bc), labels, logits);
-  CMLPL_CHECK_LAUNCH("head");
+  const __half* w1s = reinterpret_cast<const __half*>(pk + L.w1s);
+  const float* bspe = reinterpret_cast<const float*>(pk + L.bspe);
+  const __half* wc_spe16 = reinterpret_cast<const __half*>(pk + L.wc16 + size_t(L.conv_pos) * 8 * L.nc * 16);
+  if (L.nc == 16) {
+    CMLPL_MAX_DYN_SMEM(spectral_logits_kernel<16>, int(smem));
+    spectral_logits_kernel<16><<<grid, spl::kThreads, smem, s>>>(static_cast<const __half*>(x16), mtiles, KC, nA, w1s, bspe,
+                                                                 wc_spe16, part);
+  } else {
+    CMLPL_MAX_DYN_SMEM(spectral_logits_kernel<32>, int(smem));
+    spectral_logits_kernel<32><<<grid, spl::kThreads, smem, s>>>(static_cast<const __half*>(x16), mtiles, KC, nA, w1s, bspe,
+                                                                 wc_spe16, part);
+  }
+  CMLPL_CHECK_LAUNCH("spectral_logits");
   return CMLPL_OK;
 }
 
 // Fused spectral branch of the dense path: part f32 [4 hidden quarters][ceil(n/128)*128][NC] partial spectral logits, NC =
-// 16 for <= 16 classes and 32 for 17-32 (spectral_logits_kernel; the 1024 hidden features stay in shared memory).  x16 is
+// 16 for <= 16 classes and 32 for 17-32 (spectral_logits_kernel; the 1024 hidden features stay on chip).  x16 is
 // scratch for the fp16 input tiles.
 extern "C" int cmlpl_spectral_logits_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
                                         const void* packed, void* x16, float* part, cmlpl_stream_t stream) {
-  return spectral_hidden_impl(spectra, -1, n, num_features, num_classes, w, nullptr, nullptr, packed, x16, part, stream, true);
+  return launch_spectral_logits(spectra, -1, n, num_features, num_classes, w, nullptr, nullptr, packed, x16, part, stream);
 }
 
 extern "C" int cmlpl_spectral_logits_raw_tc(const void* raw, int dtype, int64_t n, int num_features, int num_classes, int w,
                                             const float* mu, const float* inv_sigma, const void* packed, void* x16,
                                             float* part, cmlpl_stream_t stream) {
   CMLPL_CHECK_ARG((dtype == 0 || dtype == 1) && mu && inv_sigma, "spectral_logits_raw_tc: bad args");
-  return spectral_hidden_impl(raw, dtype, n, num_features, num_classes, w, mu, inv_sigma, packed, x16, part, stream, true);
+  return launch_spectral_logits(raw, dtype, n, num_features, num_classes, w, mu, inv_sigma, packed, x16, part, stream);
 }
 
 // Head of the dense path without a GEMM: quarter partials of cmlpl_spectral_logits_tc + the 5 gathered conv partials

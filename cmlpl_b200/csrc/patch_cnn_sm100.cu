@@ -84,25 +84,18 @@ enum { BAR_A1_FULL = 0, BAR_A1_EMPTY, BAR_C1_FULL0, BAR_C1_FULL1, BAR_C1_EMPTY0,
 constexpr int kEpiThreads = 256, kLoadThreads = 64, kThreads = kEpiThreads + kLoadThreads + 32;
 constexpr int kEpiWarps = kEpiThreads / 32, kLoadWarp0 = kEpiWarps, kMmaWarp = kEpiWarps + kLoadThreads / 32;
 
-// TRACE: CTA 0 records clock64() at the protocol points of its first 64 patches into
-// trace[patch][16] (diagnostics only; see cmlpl_debug_patch_cnn_trace).
-#define CMLPL_TRACE(slot)                                                                  \
-  do {                                                                                     \
-    if (TRACE && blockIdx.x == 0 && (p - p_begin) < 64) trace[(p - p_begin) * 16 + (slot)] = clock64(); \
-  } while (0)
-
 // TRAIN = the forward trunk of the fused training step (tools/models.py:133-140 in batch mode): every "pixel" is one
 // sample of one of the two BaseNet2 peers whose conv0 output a0 [8 chunks][W x W][8] lies in the workspace.  The CTAs
 // are split between the nets (each keeps ONE net's weights, converted from the fp32 parameters in the prologue) and
 // the epilogues additionally save what the backward pass needs: the ReLU masks of both blocks as bits, the pooled
 // conv1 output p1 (B operand of conv2's weight gradient) and the pooled conv2 output as fp32 in the classifier's
 // flatten order (tools/models.py:141).
-template <int W, bool TRACE, bool TRAIN>
+template <int W, bool TRAIN>
 __global__ void __launch_bounds__(kThreads, 1)
 patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
                  const unsigned char* __restrict__ packed_w1, const unsigned char* __restrict__ packed_w2,
                  const float* __restrict__ b1g, const float* __restrict__ b2g, __half* __restrict__ p2out,
-                 int p2_tiled, long long* __restrict__ trace, TrainCnnArgs ta) {
+                 TrainCnnArgs ta) {
   using Cfg = PatchCfg<W>;
   using G = TrainGeom<W>;
   extern __shared__ __align__(128) unsigned char smem[];
@@ -195,7 +188,6 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
       // hold the copies back until the previous patch's conv1 epilogue has finished: the LSU queue is
       // shared with the epilogue's shared-memory traffic, and the load still hides under conv2
       if (p > p_begin) mbar_wait(bars + 8 * BAR_A2_FULL, ph ^ 1, 10);
-      if (lt == 0) CMLPL_TRACE(0);
       if constexpr (kPairs) {
 #pragma unroll
         for (int g = 0; g < W / 2; ++g) {
@@ -210,7 +202,6 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
       }
       cp_async_wait_all();
       fence_proxy_async();                                   // generic-proxy writes -> visible to the MMA
-      if (lt == 0) CMLPL_TRACE(1);
       mbar_arrive(bars + 8 * BAR_A1_FULL);
     }
   } else if (warp == kMmaWarp) {
@@ -225,7 +216,6 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
     uint32_t ph = 0;
     for (int64_t p = p_begin; p < p_end; ++p, ph ^= 1) {
       mbar_wait(bars + 8 * BAR_A1_FULL, ph, 2);
-      if (lane == 0) CMLPL_TRACE(2);
       // ---- conv1: NT1 halves x 2 parities
 #pragma unroll
       for (int h = 0; h < Cfg::NT1; ++h) {
@@ -238,18 +228,15 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
         }
         __syncwarp();
       }
-      if (lane == 0) CMLPL_TRACE(3);
       // ---- conv2: 2 parities, one 128-row tile each
       mbar_wait(bars + 8 * BAR_A2_FULL, ph, 4);
       mbar_wait(bars + 8 * BAR_C2_EMPTY, ph ^ 1, 5);
       tc_fence_after();
-      if (lane == 0) CMLPL_TRACE(4);
       if (elect_one_sync()) {
         issue_conv_pair<Cfg::PW2, Cfg::CH2, Cfg::PLANE2>(Cfg::TM_C2, a2_lo, w2_lo);
         umma_commit(bars + 8 * BAR_C2_FULL);
       }
       __syncwarp();
-      if (lane == 0) CMLPL_TRACE(5);
     }
   } else {
     // ================================================================ EPILOGUE (warps 0-7)
@@ -339,7 +326,6 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
         unsigned char* dst = smem + Cfg::S_A2 + q2 * Cfg::PLANE2 + (chalf * 4) * Cfg::CH2 +
                              (1 + prow2 * Cfg::PW2 + (x >> 1)) * 16;
         mbar_wait(bars + 8 * (BAR_C1_FULL0 + h), ph, 6);
-        if (tid == 0) CMLPL_TRACE(6 + 2 * h);
         tc_fence_after();
         // two 16-channel groups one after the other keeps only 32 accumulators live
         float e[16], o[16];
@@ -347,9 +333,7 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
         tmem_ld16(lane_addr + Cfg::TM_C1 + (h * 2 + 0) * 64, e);
         tmem_ld16(lane_addr + Cfg::TM_C1 + (h * 2 + 1) * 64, o);
         tmem_ld_wait();
-        if (tid == 0 && h == 0) CMLPL_TRACE(13);
         pool16(e, o, &re[0], &ro[0], bias1, w0, w1);
-        if (tid == 0 && h == 0) CMLPL_TRACE(14);
         if (writer) {
           *reinterpret_cast<uint4*>(dst) = w0;
           *reinterpret_cast<uint4*>(dst + Cfg::CH2) = w1;
@@ -365,7 +349,6 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
             *reinterpret_cast<uint4*>(p1g + G::TPos2 * 16) = w1;
           }
         }
-        if (tid == 0 && h == 0) CMLPL_TRACE(15);
         tmem_ld16(lane_addr + Cfg::TM_C1 + (h * 2 + 0) * 64 + 16, e);
         tmem_ld16(lane_addr + Cfg::TM_C1 + (h * 2 + 1) * 64 + 16, o);
         tmem_ld_wait();
@@ -387,7 +370,6 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
             mg[2 * W] = mo | (mbits_o << 16);
           }
         }
-        if (tid == 0) CMLPL_TRACE(7 + 2 * h);
       }
       fence_proxy_async();
       mbar_arrive(bars + 8 * BAR_A2_FULL);
@@ -412,14 +394,10 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
             ro[k] = *reinterpret_cast<const uint4*>(rO + k * Cfg::CH2);
           }
         }
-        // row-major [pixel][pos][64]  or  UMMA A-operand tiles [pixel/128][pos*8 + chunk][pixel%128][8]
+        // row-major [pixel][pos][64]
         const int pos = i * Cfg::NP2 + (x >> 1);
-        __half* dst = p2_tiled ? p2out + (((p >> 7) * (Cfg::P * 8) + pos * 8 + chalf * 4) * 128 + (p & 127)) * 8
-                               : p2out + (p * Cfg::P + pos) * 64 + chalf * 32;
-        const int dstep = p2_tiled ? 128 : 1;                  // uint4 stride between consecutive 8-channel chunks
-        if (tid == 0) CMLPL_TRACE(10);
+        __half* dst = p2out + (p * Cfg::P + pos) * 64 + chalf * 32;
         mbar_wait(bars + 8 * BAR_C2_FULL, ph, 8);
-        if (tid == 0) CMLPL_TRACE(11);
         tc_fence_after();
         float e[16], o[16];
         uint4 w0, w1;
@@ -438,7 +416,7 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
             for (int j = 0; j < 16; ++j) catg[j * Cfg::P] = pooled[j];
           }
         } else {
-          if (writer) { __stcs(d4, w0); __stcs(d4 + dstep, w1); }
+          if (writer) { __stcs(d4, w0); __stcs(d4 + 1, w1); }
         }
         tmem_ld16(lane_addr + Cfg::TM_C2 + 0 * 64 + 16, e);
         tmem_ld16(lane_addr + Cfg::TM_C2 + 1 * 64 + 16, o);
@@ -457,10 +435,9 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
             mg[2 * Cfg::H2] = mo | (mbits_o << 16);
           }
         } else {
-          if (writer) { __stcs(d4 + 2 * dstep, w0); __stcs(d4 + 3 * dstep, w1); }
+          if (writer) { __stcs(d4 + 2, w0); __stcs(d4 + 3, w1); }
         }
       }
-      if (tid == 0) CMLPL_TRACE(12);
       // A2 is rewritten by the next patch's conv1 epilogue: all residual reads must be done
       asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");
     }
@@ -480,7 +457,7 @@ patch_cnn_kernel(const __half* __restrict__ f0pad, int cols, int band_rows,
 using namespace cmlpl;
 
 static int launch_patch_cnn(const void* f0pad, int cols, int w, int band_rows, const void* packed, void* p2,
-                            int p2_tiled, long long* trace, int grid_override, cudaStream_t stream) {
+                            cudaStream_t stream) {
   CMLPL_CHECK_ARG(f0pad && packed && p2, "patch_cnn: null pointer");
   CMLPL_CHECK_ARG(w == 20 || w == 11, "patch_cnn: w=%d unsupported (20 = the reference's BaseNet2, tools/models.py:127; "
                   "11 = the odd-window variant of BASELINE configs[4])", w);
@@ -490,25 +467,24 @@ static int launch_patch_cnn(const void* f0pad, int cols, int w, int band_rows, c
   const PackedLayout L = packed_layout(1, 1, w);   // conv offsets do not depend on B, C
   const unsigned char* pk = static_cast<const unsigned char*>(packed);
   const int64_t npix = int64_t(band_rows) * cols;
-  int64_t grid = grid_override > 0 ? grid_override : sm_count();
+  int64_t grid = sm_count();
   if (grid > npix) grid = npix;
   if (w == 11) {
-    CMLPL_CHECK_ARG(!trace, "patch_cnn: the trace build exists for w=20 only");
     using Cfg = PatchCfg<11>;
-    auto kern = patch_cnn_kernel<11, false, false>;
+    auto kern = patch_cnn_kernel<11, false>;
     CMLPL_MAX_DYN_SMEM(kern, Cfg::SMEM);
     kern<<<int(grid), kThreads, Cfg::SMEM, stream>>>(
         static_cast<const __half*>(f0pad), cols, band_rows, pk + L.w1, pk + L.w2,
         reinterpret_cast<const float*>(pk + L.b1), reinterpret_cast<const float*>(pk + L.b2),
-        static_cast<__half*>(p2), p2_tiled, trace, TrainCnnArgs{});
+        static_cast<__half*>(p2), TrainCnnArgs{});
   } else {
     using Cfg = PatchCfg<20>;
-    auto kern = trace ? patch_cnn_kernel<20, true, false> : patch_cnn_kernel<20, false, false>;
+    auto kern = patch_cnn_kernel<20, false>;
     CMLPL_MAX_DYN_SMEM(kern, Cfg::SMEM);
     kern<<<int(grid), kThreads, Cfg::SMEM, stream>>>(
         static_cast<const __half*>(f0pad), cols, band_rows, pk + L.w1, pk + L.w2,
         reinterpret_cast<const float*>(pk + L.b1), reinterpret_cast<const float*>(pk + L.b2),
-        static_cast<__half*>(p2), p2_tiled, trace, TrainCnnArgs{});
+        static_cast<__half*>(p2), TrainCnnArgs{});
   }
   CMLPL_CHECK_LAUNCH("patch_cnn");
   return CMLPL_OK;
@@ -519,13 +495,13 @@ int launch_train_cnn(const TrainCnnArgs& ta, int w, cudaStream_t st) {
   int grid = sm_count() & ~1;                       // split evenly between the two nets
   if (grid > 2 * ta.nb) grid = 2 * ta.nb;
   if (w == 11) {
-    auto kern = patch_cnn_kernel<11, false, true>;
+    auto kern = patch_cnn_kernel<11, true>;
     CMLPL_MAX_DYN_SMEM(kern, PatchCfg<11>::SMEM);
-    kern<<<grid, kThreads, PatchCfg<11>::SMEM, st>>>(nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr, ta);
+    kern<<<grid, kThreads, PatchCfg<11>::SMEM, st>>>(nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, ta);
   } else {
-    auto kern = patch_cnn_kernel<20, false, true>;
+    auto kern = patch_cnn_kernel<20, true>;
     CMLPL_MAX_DYN_SMEM(kern, PatchCfg<20>::SMEM);
-    kern<<<grid, kThreads, PatchCfg<20>::SMEM, st>>>(nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr, ta);
+    kern<<<grid, kThreads, PatchCfg<20>::SMEM, st>>>(nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, ta);
   }
   CMLPL_CHECK_LAUNCH("train_cnn");
   return CMLPL_OK;
@@ -534,18 +510,5 @@ int launch_train_cnn(const TrainCnnArgs& ta, int w, cudaStream_t st) {
 
 extern "C" int cmlpl_patch_cnn_f16(const void* f0pad, int cols, int w, int band_rows, const void* packed, void* p2,
                                    cmlpl_stream_t stream) {
-  return launch_patch_cnn(f0pad, cols, w, band_rows, packed, p2, 0, nullptr, 0, static_cast<cudaStream_t>(stream));
-}
-
-// Same, writing the pooled features as UMMA A-operand tiles [ceil(n/128)][P*8][128][8] for cmlpl_head_tc.
-extern "C" int cmlpl_patch_cnn_f16_tiled(const void* f0pad, int cols, int w, int band_rows, const void* packed,
-                                         void* p2t, cmlpl_stream_t stream) {
-  return launch_patch_cnn(f0pad, cols, w, band_rows, packed, p2t, 1, nullptr, 0, static_cast<cudaStream_t>(stream));
-}
-
-// Diagnostics: same kernel, CTA 0 writes clock64() stamps of its first 64 patches to trace[64][16].
-extern "C" int cmlpl_debug_patch_cnn_trace(const void* f0pad, int cols, int w, int band_rows, const void* packed,
-                                           void* p2, long long* trace, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(trace, "patch_cnn_trace: null trace buffer");
-  return launch_patch_cnn(f0pad, cols, w, band_rows, packed, p2, 0, trace, 0, static_cast<cudaStream_t>(stream));
+  return launch_patch_cnn(f0pad, cols, w, band_rows, packed, p2, static_cast<cudaStream_t>(stream));
 }

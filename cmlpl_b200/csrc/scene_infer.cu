@@ -4,7 +4,7 @@
 //                    halo-padded fp16 map F0pad[8 chunks][(rows+w-1)][(cols+w-1)][8 channels]; a pixel's patch
 //                    is then a plain w x w window of this map (hyper_tools.py:35-55,226-243)
 //   2. spectral_head relu(feat_spe(x)) (models.py:142-143) and its classifier columns
-//   3. conv1_scene   conv1 + residual + ReLU once per scene position in 9 patch-border classes and the
+//   3. conv1_pool    conv1 + residual + ReLU once per scene position in 9 patch-border classes and the
 //                    pooled maps as parity planes (conv1_scene_sm100.cu); conv2_scene: conv2 + residual +
 //                    ReLU once per position in 25 classes, border classes pooled in its epilogue; pool2_cls: rest of
 //                    the avg-pool + conv columns of the classifier -> 25 class-partial maps (conv2_scene_sm100.cu)
@@ -92,9 +92,9 @@ __global__ void argmax_kernel(const float* __restrict__ logits, int64_t n, int C
   }
 }
 
-// The tensor-core spectral branch (spectral_logits_kernel, head_sm100.cu) takes <= 224 bands and <= 32 classes.  It runs
-// on the dense path, and in path mode 0 for <= 16 classes or from the raw cube; otherwise the CUDA-core spectral_head +
-// classify kernels above run (same C ABI, same results contract).
+// Scene inference runs the tensor-core spectral branch (spectral_logits_kernel, head_sm100.cu) for <= 224 bands and <= 32
+// classes: on the dense path, and in path mode 0 for <= 16 classes or from the raw cube; otherwise the CUDA-core
+// spectral_head + classify kernels above run (same C ABI, same results contract).
 static bool tc_spectral_fits(int B, int C) { return C <= 32 && ((B + 15) / 16) * 2 <= 28; }   // <= 224 bands
 
 // 1 (default): the exact-compute-sharing kernels where they apply; 0: the per-pixel tensor-core kernels everywhere (the

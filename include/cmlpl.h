@@ -104,8 +104,10 @@ int cmlpl_l2norm_bwd_f32(const float* y, const float* norm, const float* dy, flo
  * cut them (exact compute sharing; persistent tcgen05 kernels fed by TMA tile loads); the spectral
  * branch is one fused two-GEMM kernel; a sum head adds each pixel's 25 gathered conv partials to its
  * spectral partials and takes the argmax.  This path takes up to 32 classes (class width 16 up to 16 classes, 32
- * beyond); > 32 classes or > 224 bands fall back to the all-per-pixel tcgen05 kernel (patch window staged in shared
- * memory) and CUDA-core heads, and cmlpl_scene_infer / cmlpl_scene_infer_raw refuse more than 32 classes.
+ * beyond) and up to 224 bands.  The per-pixel path (patch_cnn_kernel: conv1 + conv2 per patch window staged in shared
+ * memory, then the classifier heads) is the independent implementation selected by cmlpl_set_scene_path_mode(0); it
+ * also serves > 224 bands in cmlpl_scene_infer, with the CUDA-core spectral head.  cmlpl_scene_infer / cmlpl_scene_infer_raw
+ * refuse more than 32 classes, and cmlpl_scene_infer_raw more than 224 bands.
  *
  * Packed weights: cmlpl_pack_basenet2() converts the reference state_dict tensors
  * (models.py:102-127: conv0/1/2.{weight,bias}, feat_spe.*, classifier.*) into the
@@ -158,9 +160,6 @@ int cmlpl_scene_infer_raw(const void* raw, int dtype, int scene_rows, int cols, 
                           const float* wf, const float* bf, const float* mu, const float* inv_sigma,
                           const void* packed, void* workspace, size_t workspace_bytes,
                           uint8_t* labels, float* logits, cmlpl_stream_t stream);
-int cmlpl_spectral_hidden_raw_tc(const void* raw, int dtype, int64_t n, int num_features, int num_classes, int w,
-                                 const float* mu, const float* inv_sigma, const void* packed, void* x16,
-                                 void* h16, cmlpl_stream_t stream);
 
 /* Individual stages of cmlpl_scene_infer (exposed for tests / profiling). */
 int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, int slab_row0, int slab_rows,
@@ -174,29 +173,15 @@ int cmlpl_spectral_head_f32(const float* spectra, int64_t n, int num_features, i
 int cmlpl_classify_f16(const void* p2, const float* spe_logits /* may be NULL */, int64_t n,
                        int num_features, int num_classes, int w, const void* packed,
                        uint8_t* labels, float* logits /* may be NULL */, cmlpl_stream_t stream);
-/* Tensor-core head (<= 16 classes, <= 208 bands), fp16 operands / fp32 accumulate.  A operands are
- * "UMMA tiles": f16 [ceil(n/128)][K/8][128 rows][8], pixel p = tile p/128, row p%128.
- *   cmlpl_patch_cnn_f16_tiled : as cmlpl_patch_cnn_f16 but p2t is tiled with K = (w/4)^2*64 (pos, ch)
- *   cmlpl_spectral_hidden_tc  : x16 (scratch, K = B padded to 16) and h16 = relu(feat_spe(x)) tiles, K = 1024
- *   cmlpl_head_tc             : classifier over [p2t | h16] + bias, argmax -> labels (and logits) */
-int cmlpl_patch_cnn_f16_tiled(const void* f0pad, int cols, int w, int band_rows, const void* packed,
-                              void* p2t, cmlpl_stream_t stream);
-int cmlpl_spectral_hidden_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
-                             const void* packed, void* x16, void* h16, cmlpl_stream_t stream);
-int cmlpl_head_tc(const void* p2t, const void* h16, int64_t n, int num_features, int num_classes, int w,
-                  const void* packed, uint8_t* labels, float* logits, cmlpl_stream_t stream);
-/* Exact compute sharing of conv1 (SURVEY section 7): conv1 + bias + residual + ReLU evaluated once per
- * position of the conv0 map in 3x3 = 9 patch-border classes, then the 2x2 average pools of every
- * top-left position in the 9 pooled border classes (tools/models.py:133-136 for all patches at once).
- *   f0pad f16 [8][PR][PC][8] (PR = band_rows+w-1, PC = cols+w-1), g f32 [9][PR*PC][64] scratch,
- *   pm f16 [9][PR][PC][64]: pooled maps, variant = A*3+B (A,B in top/mid/bot, left/mid/right). */
-int cmlpl_conv1_scene_f16(const void* f0pad, int cols, int w, int band_rows, const void* packed, float* g,
-                          void* pm, cmlpl_stream_t stream);
-/* Dense (scene-level) rest of the conv tower, exact compute sharing of conv2 / pool / classifier
- * (tools/models.py:137-150 for all patches at once; csrc/conv2_scene_sm100.cu).  PR2 = (band_rows+w)/2,
- * PC2 = (cols+w)/2; "planes" = the 4 parity planes (pr&1)*2+(pc&1) of the padded map, y' = pr>>1, x' = pc>>1.
- *   cmlpl_conv1_scene_variants_f32: g f32 [9][PR*PC][64] only (no pooling)
- *   cmlpl_conv1_scene_planes_f16  : + pooled maps as planes   pmq f16 [9][4][8 chunks][PR2][PC2][8]
+/* Dense (scene-level) conv tower, exact compute sharing of conv1 / conv2 / pools / classifier (SURVEY section 7;
+ * tools/models.py:133-150 for all patches at once; csrc/conv1_scene_sm100.cu, csrc/conv2_scene_sm100.cu).
+ * PR = band_rows+w-1, PC = cols+w-1, PR2 = (band_rows+w)/2, PC2 = (cols+w)/2; "planes" = the 4 parity planes
+ * (pr&1)*2+(pc&1) of the padded map, y' = pr>>1, x' = pc>>1.
+ *   cmlpl_conv1_pool_planes_f16   : conv1 + bias + residual + ReLU once per position of the conv0 map f0pad
+ *                                   f16 [8][PR][PC][8] in 3x3 = 9 patch-border classes, and their 2x2 average pools for
+ *                                   every top-left position in the 9 pooled border classes, in ONE kernel (no fp32
+ *                                   scratch in HBM):  pmq f16 [9 = A*3+B][4][8 chunks][PR2][PC2][8] (A,B in top/mid/bot,
+ *                                   left/mid/right; entries without a pooled cell are 0; w = 11 stores A,B in top/mid)
  *   cmlpl_conv2_scene_f16         : conv2+bias+residual+ReLU in 25 border classes (rho, kap in {i=0, 1, 2..7, 8, 9}); the
  *                                   border halves of the 2x2 pool (rho 0 + rho 1 one row down, rho 3 + rho 4, same for
  *                                   kap) are averaged in the epilogue:  yq f16 [9 = Al*3+Be][4][8][PR2][PC2][8],
@@ -206,22 +191,17 @@ int cmlpl_conv1_scene_f16(const void* f0pad, int cols, int w, int band_rows, con
  *                                   lmap f32 [4][5 = I][NC/4 class quads][PR2][PC2][4] (NC = 16 up to 16 classes, 32 for
  *                                   17-32),
  *                                   lmap[I][y',x'] = sum_J L[I][J][y', x'+2J] */
-int cmlpl_conv1_scene_variants_f32(const void* f0pad, int cols, int w, int band_rows, const void* packed, float* g,
-                                   cmlpl_stream_t stream);
-int cmlpl_conv1_scene_planes_f16(const void* f0pad, int cols, int w, int band_rows, const void* packed, float* g,
-                                 void* pmq, cmlpl_stream_t stream);
-/* cmlpl_conv1_pool_planes_f16: the same pooled planes from ONE kernel (conv1 variants pooled in the epilogue through a
- * shared-memory / shuffle exchange; no fp32 scratch in HBM) -- what cmlpl_scene_infer runs. */
 int cmlpl_conv1_pool_planes_f16(const void* f0pad, int cols, int w, int band_rows, const void* packed, void* pmq,
                                 cmlpl_stream_t stream);
 int cmlpl_conv2_scene_f16(const void* pmq, int cols, int w, int band_rows, const void* packed, void* yq,
                           cmlpl_stream_t stream);
 int cmlpl_pool2_cls_f16(const void* yq, int cols, int w, int band_rows, int num_features, int num_classes,
                         const void* packed, float* lmap, cmlpl_stream_t stream);
-/* Fused spectral branch + sum head (what cmlpl_scene_infer runs since the hidden features stopped going through HBM):
+/* Fused spectral branch + sum head:
  *   cmlpl_spectral_logits_tc     : part f32 [4 hidden quarters][ceil(n/128)*128][NC] = Wc_spe . relu(Wspe . x + b) per
- *                                  quarter of the 1024 hidden features (tools/models.py:142-143,150), <= 224 bands,
- *                                  <= 32 classes (NC = 16 up to 16 classes, 32 for 17-32)
+ *                                  quarter of the 1024 hidden features (tools/models.py:142-143,150), <= 32 classes
+ *                                  (NC = 16 up to 16 classes, 32 for 17-32), as many bands as the kernel's input tiles
+ *                                  fit shared memory for (cmlpl_scene_infer uses it up to 224)
  *   cmlpl_spectral_logits_raw_tc : the same from the raw cube (z-score folded into the fp16 conversion)
  *   cmlpl_head_sum_lmap          : 4 quarter partials + the 5 gathered conv partials + bias, argmax */
 int cmlpl_spectral_logits_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
@@ -232,16 +212,6 @@ int cmlpl_spectral_logits_raw_tc(const void* raw, int dtype, int64_t n, int num_
 int cmlpl_head_sum_lmap(const float* part, const float* lmap, int cols, int band_rows, int num_features,
                         int num_classes, int w, const void* packed, uint8_t* labels, float* logits,
                         cmlpl_stream_t stream);
-/* Per-pixel conv2 stage on the pooled conv1 maps of cmlpl_conv1_scene_f16 (models.py:137-140 per patch):
- * pm f16 [9][PR][PC][64] -> p2t UMMA tiles [ceil(n/128)][(w/4)^2*8][128][8] for cmlpl_head_tc. */
-int cmlpl_patch_conv2_f16_tiled(const void* pm, int cols, int w, int band_rows, const void* packed,
-                                void* p2t, cmlpl_stream_t stream);
-int cmlpl_debug_patch_conv2_trace(const void* pm, int cols, int w, int band_rows, const void* packed,
-                                  void* p2t, long long* trace, cmlpl_stream_t stream);
-/* Diagnostics: cmlpl_patch_cnn_f16 with CTA 0 writing clock64() stamps of its first 64 patches
- * (16 slots each: loader / MMA issuer / epilogue protocol points) to trace i64 [64,16]. */
-int cmlpl_debug_patch_cnn_trace(const void* f0pad, int cols, int w, int band_rows, const void* packed,
-                                void* p2, long long* trace, cmlpl_stream_t stream);
 /* hyper_tools.py:426 torch.max(outputs, 1): first index on ties.  logits f32 [n, C] -> u8 [n]. */
 int cmlpl_argmax_u8(const float* logits, int64_t n, int num_classes, uint8_t* labels,
                     cmlpl_stream_t stream);

@@ -85,69 +85,6 @@ def test_confusion_and_gather_empty_inputs(dev):
     assert cm.sum() == 2 and cm[0, 0] == 1 and cm[2, 2] == 1
 
 
-def test_fused_conv1_pool_matches_two_kernel_planes(dev):
-    """conv1_pool_kernel (variants pooled in the epilogue) against conv1_scene_kernel + pool1q_scene_kernel on the same
-    conv0 map: identical up to the fp32 summation order of the 2x2 pool, i.e. at most one fp16 ulp."""
-    from cmlpl_b200 import _lib, ops
-    R, C, w = 41, 67, 20
-    rng = np.random.default_rng(11)
-    cube = torch.from_numpy(rng.standard_normal((R, C, 60)).astype(np.float32)).to(dev)
-    torch.manual_seed(11)
-    packed = ops.pack_basenet2({k: v.to(dev) for k, v in O.basenet2_init(103, 9).items()}, 103, 9, w)
-    st = torch.cuda.current_stream().cuda_stream
-    PR, PC = R + w - 1, C + w - 1
-    PR2, PC2 = (PR + 1) // 2, (PC + 1) // 2
-    f0 = torch.empty(8 * PR * PC * 8, dtype=torch.float16, device=dev)
-    g = torch.empty(9 * PR * PC * 64, dtype=torch.float32, device=dev)
-    two = torch.full((9, 4, 8, PR2, PC2, 8), float("nan"), dtype=torch.float16, device=dev)
-    one = torch.full((9, 4, 8, PR2, PC2, 8), float("nan"), dtype=torch.float16, device=dev)
-    _lib.call("cmlpl_conv0_map_f16", cube.data_ptr(), R, C, 0, R, w, 0, R, packed.data_ptr(), f0.data_ptr(), st)
-    _lib.call("cmlpl_conv1_scene_planes_f16", f0.data_ptr(), C, w, R, packed.data_ptr(), g.data_ptr(), two.data_ptr(), st)
-    _lib.call("cmlpl_conv1_pool_planes_f16", f0.data_ptr(), C, w, R, packed.data_ptr(), one.data_ptr(), st)
-    torch.cuda.synchronize()
-    a, b = one.float(), two.float()
-    assert not torch.isnan(a).any() and not torch.isnan(b).any()
-    ulp = (b.abs() * 2.0 ** -10).clamp_min(2.0 ** -24)
-    assert float(((a - b).abs() / ulp).max()) <= 1.0
-    assert float((one == two).float().mean()) > 0.999
-
-
-@pytest.mark.parametrize("B,K", [(103, 9), (200, 16)])
-def test_dense_tail_matches_per_pixel_tail(dev, B, K):
-    """The whole dense tail (fused conv1+pool -> conv2 in shifted row-class frames -> pool/classifier partial maps ->
-    fused spectral logits -> sum head) against the independent per-pixel tail (conv1_scene + patch_conv2 + spectral
-    GEMM + GEMM head) on the same inputs: logits within 5e-4 of each other, labels = argmax of the logits."""
-    from cmlpl_b200 import _lib, ops
-    R, C, w = 37, 45, 20
-    n = R * C
-    rng = np.random.default_rng(B)
-    cube = torch.from_numpy(rng.standard_normal((R, C, 60)).astype(np.float32)).to(dev)
-    spectra = torch.from_numpy(rng.standard_normal((n, B)).astype(np.float32)).to(dev)
-    torch.manual_seed(B)
-    packed = ops.pack_basenet2({k: v.to(dev) for k, v in O.basenet2_init(B, K).items()}, B, K, w)
-    labels, logits = ops.scene_infer(cube, spectra, packed, K, w, want_logits=True)
-    st = torch.cuda.current_stream().cuda_stream
-    PR, PC = R + w - 1, C + w - 1
-    mt, kc = (n + 127) // 128, ((B + 15) // 16) * 2
-    f0 = torch.empty(8 * PR * PC * 8, dtype=torch.float16, device=dev)
-    g = torch.empty(9 * PR * PC * 64, dtype=torch.float32, device=dev)
-    pm = torch.zeros(9 * PR * PC * 64, dtype=torch.float16, device=dev)
-    p2 = torch.empty(mt * 200 * 128 * 8, dtype=torch.float16, device=dev)
-    x16 = torch.empty(mt * kc * 1024, dtype=torch.float16, device=dev)
-    h16 = torch.empty(mt * 128 * 1024, dtype=torch.float16, device=dev)
-    lab2 = torch.empty(n, dtype=torch.uint8, device=dev)
-    log2 = torch.empty(n, K, dtype=torch.float32, device=dev)
-    _lib.call("cmlpl_conv0_map_f16", cube.data_ptr(), R, C, 0, R, w, 0, R, packed.data_ptr(), f0.data_ptr(), st)
-    _lib.call("cmlpl_conv1_scene_f16", f0.data_ptr(), C, w, R, packed.data_ptr(), g.data_ptr(), pm.data_ptr(), st)
-    _lib.call("cmlpl_patch_conv2_f16_tiled", pm.data_ptr(), C, w, R, packed.data_ptr(), p2.data_ptr(), st)
-    _lib.call("cmlpl_spectral_hidden_tc", spectra.data_ptr(), n, B, K, w, packed.data_ptr(), x16.data_ptr(), h16.data_ptr(), st)
-    _lib.call("cmlpl_head_tc", p2.data_ptr(), h16.data_ptr(), n, B, K, w, packed.data_ptr(), lab2.data_ptr(), log2.data_ptr(), st)
-    torch.cuda.synchronize()
-    assert rel(logits.cpu().numpy(), log2.cpu().numpy()) < 5e-4
-    assert torch.equal(labels.cpu(), logits.argmax(1).to(torch.uint8).cpu())
-    assert float((labels == lab2).float().mean()) > 0.995
-
-
 def test_full_size_scene_properties(dev):
     """BASELINE.json's headline shape (610 x 340 x 103, 9 classes) at full size, through size-independent properties:
     labels are the argmax of the returned logits, an uneven 4-band walk with read-only halos reproduces the one-shot
