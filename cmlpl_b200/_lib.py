@@ -42,10 +42,7 @@ SIGNATURES = {
     "cmlpl_conv2_scene_f16": (I, [P, I, I, I, P, P, P]),
     "cmlpl_pool2_cls_f16": (I, [P, I, I, I, I, I, P, P, P]),
     "cmlpl_spectral_logits_tc": (I, [P, L, I, I, I, P, P, P, P]),
-    "cmlpl_spectral_logits_raw_tc": (I, [P, I, L, I, I, I, P, P, P, P, P, P]),
     "cmlpl_head_sum_lmap": (I, [P, P, I, I, I, I, I, P, P, P, P]),
-    "cmlpl_spectral_head_f32": (I, [P, L, I, I, I, P, P, L, P, P]),
-    "cmlpl_classify_f16": (I, [P, P, L, I, I, I, P, P, P, P]),
     "cmlpl_argmax_u8": (I, [P, L, I, P, P]),
     "cmlpl_preprocess_fit_f64": (I, [P, I, L, I, P, P, P]),
     "cmlpl_preprocess_apply": (I, [P, I, L, I, I, P, P, P, P, P, P, P]),

@@ -1,4 +1,4 @@
-// Error plumbing and device queries for the C ABI (include/cmlpl.h).
+// Error plumbing, device queries and the per-device side stream for the C ABI (include/cmlpl.h).
 #include <stdarg.h>
 #include <string.h>
 
@@ -30,6 +30,28 @@ int sm_count() {
   return cached[dev];
 }
 
+SideStream* side_stream() {
+  static SideStream per_dev[64];
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
+  SideStream& x = per_dev[dev];
+  std::lock_guard<std::mutex> lock(x.mu);
+  if (x.s) return &x;
+  // complete or nothing: a failed creation releases what it made and leaves the slot empty for the next call
+  cudaStream_t s = nullptr;
+  cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+  bool ok = cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking) == cudaSuccess;
+  for (cudaEvent_t& e : ev) ok = ok && cudaEventCreateWithFlags(&e, cudaEventDisableTiming) == cudaSuccess;
+  if (!ok) {
+    for (cudaEvent_t e : ev)
+      if (e) cudaEventDestroy(e);
+    if (s) cudaStreamDestroy(s);
+    return nullptr;
+  }
+  x.fork[0] = ev[0]; x.join[0] = ev[1]; x.fork[1] = ev[2]; x.join[1] = ev[3];
+  x.s = s;
+  return &x;
+}
 
 int make_scene_tmap(CUtensorMap* out, const void* base, int outer, int rows, int cols, int box_rows, int box_cols) {
   static PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;

@@ -5,6 +5,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <mutex>
+
 #include "../../include/cmlpl.h"
 
 namespace cmlpl {
@@ -52,6 +54,21 @@ void set_error(const char* fmt, ...);
 
 // number of SMs of the current device (cached)
 int sm_count();
+
+// Fork / join inside one C call: kernels without a mutual dependency (the scene's spectral branch next to its conv tower;
+// in the training step the spectral GEMM next to the conv trunk and the head weight gradients next to the conv backward
+// chain) run on a side stream between a fork and a join event.  Works the same in eager mode and under stream capture
+// (the events become graph edges).  One side stream and two event pairs per device, created together on first use and
+// kept for the life of the process -- the only persistent resources the library owns.  A caller holds `mu` from its
+// first fork to its last join, so host threads that drive the same device from several streams take turns (the
+// launches are microseconds) and never enqueue onto a side stream that another thread's capture has forked.
+struct SideStream {
+  cudaStream_t s = nullptr;
+  cudaEvent_t fork[2] = {nullptr, nullptr}, join[2] = {nullptr, nullptr};
+  std::mutex mu;
+};
+// the current device's side stream, or nullptr if it cannot be created
+SideStream* side_stream();
 
 // a1 index map (tools/hyper_tools.py:35-55 == symmetric padding): single reflection.
 __host__ __device__ __forceinline__ int mirror_index(int o, int n) {

@@ -325,6 +325,8 @@ using namespace cmlpl;
 
 CMLPL_TRACE_EXPORT(cmlpl_debug_spl_trace)
 
+namespace cmlpl {
+
 // shared-memory plan of spectral_logits_kernel for KC input k-chunks and class width NC: as many input tiles in flight as
 // fit (<= 4).  224 bands (KC = 28) leave room for one at either width.
 static bool spectral_logits_plan(int KC, int NC, int* nA, size_t* smem) {
@@ -336,9 +338,9 @@ static bool spectral_logits_plan(int KC, int NC, int* nA, size_t* smem) {
 }
 
 // x16_tile(_raw) + spectral_logits_kernel: x16 is scratch for the fp16 input tiles, part f32 [4][ceil(n/128)*128][NC].
-static int launch_spectral_logits(const void* x, int dtype /* -1 = preprocessed f32 spectra */, int64_t n, int num_features,
-                                  int num_classes, int w, const float* mu, const float* inv_sigma, const void* packed,
-                                  void* x16, float* part, cmlpl_stream_t stream) {
+int launch_spectral_logits(const void* x, int dtype /* -1 = preprocessed f32 spectra */, int64_t n, int num_features,
+                           int num_classes, int w, const float* mu, const float* inv_sigma, const void* packed, void* x16,
+                           float* part, cmlpl_stream_t stream) {
   CMLPL_CHECK_ARG(x && packed && x16 && part, "spectral_logits_tc: null pointer");
   CMLPL_CHECK_ARG(n > 0 && num_features > 0, "spectral_logits_tc: bad dims");
   CMLPL_CHECK_ARG(num_classes <= 32, "spectral_logits_tc: needs <= 32 classes, got %d", num_classes);
@@ -375,19 +377,14 @@ static int launch_spectral_logits(const void* x, int dtype /* -1 = preprocessed 
   return CMLPL_OK;
 }
 
+}  // namespace cmlpl
+
 // Fused spectral branch of the dense path: part f32 [4 hidden quarters][ceil(n/128)*128][NC] partial spectral logits, NC =
 // 16 for <= 16 classes and 32 for 17-32 (spectral_logits_kernel; the 1024 hidden features stay on chip).  x16 is
 // scratch for the fp16 input tiles.
 extern "C" int cmlpl_spectral_logits_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
                                         const void* packed, void* x16, float* part, cmlpl_stream_t stream) {
   return launch_spectral_logits(spectra, -1, n, num_features, num_classes, w, nullptr, nullptr, packed, x16, part, stream);
-}
-
-extern "C" int cmlpl_spectral_logits_raw_tc(const void* raw, int dtype, int64_t n, int num_features, int num_classes, int w,
-                                            const float* mu, const float* inv_sigma, const void* packed, void* x16,
-                                            float* part, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG((dtype == 0 || dtype == 1) && mu && inv_sigma, "spectral_logits_raw_tc: bad args");
-  return launch_spectral_logits(raw, dtype, n, num_features, num_classes, w, mu, inv_sigma, packed, x16, part, stream);
 }
 
 // Head of the dense path without a GEMM: quarter partials of cmlpl_spectral_logits_tc + the 5 gathered conv partials

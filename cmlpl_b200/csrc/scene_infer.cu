@@ -11,8 +11,6 @@
 //   4. head          spectral columns of the classifier (models.py:150) + the pixel's 25 gathered conv
 //                    partials + bias, argmax (hyper_tools.py:426, first index wins ties)
 //   (<= 32 classes and <= 224 bands; otherwise the all-per-pixel patch_cnn_sm100.cu kernel + CUDA-core classify instead)
-#include <mutex>
-
 #include "common.cuh"
 #include "gemm_core.cuh"
 
@@ -29,6 +27,11 @@ namespace cmlpl {
 template <typename T, bool kVec4, bool kSplit>
 int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0, int prow_n, int pcol_n,
                     const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad, cudaStream_t s);
+
+// x16_tile(_raw) + spectral_logits_kernel (head_sm100.cu): x is the f32 z-scored spectra (dtype -1) or the raw cube's
+// rows (dtype 0 = uint16, 1 = float32, z-scored with mu / inv_sigma in the conversion)
+int launch_spectral_logits(const void* x, int dtype, int64_t n, int num_features, int num_classes, int w, const float* mu,
+                           const float* inv_sigma, const void* packed, void* x16, float* part, cmlpl_stream_t stream);
 
 // ------------------------------------------------------------------ classifier + argmax
 // one warp per pixel; lanes stride over the K = P*64 pooled features in 8-half chunks.
@@ -102,7 +105,7 @@ static bool tc_spectral_fits(int B, int C) { return C <= 32 && ((B + 15) / 16) *
 static thread_local int g_scene_path_mode = 1;
 
 struct SceneWs {
-  size_t f0pad, p2, spe, hidden, x16, h16, g, pm, yq, lmap, total;
+  size_t f0pad, p2, spe, hidden, x16, h16, pm, yq, lmap, total;
   int64_t chunk;
   bool tc, dense;
 };
@@ -123,7 +126,7 @@ static SceneWs scene_ws(int band_rows, int cols, int B, int C, int w) {
   s.tc = s.dense || (tc_fits && C <= 16);
   size_t o = 0;
   s.f0pad = o; o = align256(o + size_t(band_rows + w - 1) * (cols + w - 1) * 64 * 2);
-  s.p2 = s.spe = s.hidden = s.x16 = s.h16 = s.g = s.pm = s.yq = s.lmap = 0;
+  s.p2 = s.spe = s.hidden = s.x16 = s.h16 = s.pm = s.yq = s.lmap = 0;
   s.chunk = n < 16384 ? n : 16384;
   if (tc_fits) {
     s.x16 = o; o = align256(o + size_t(mtiles) * (((B + 15) / 16) * 2) * 2048);
@@ -131,7 +134,6 @@ static SceneWs scene_ws(int band_rows, int cols, int B, int C, int w) {
   }
   if (s.dense) {
     const size_t qpos = size_t(4) * ((band_rows + w) / 2) * ((cols + w) / 2);     // positions of the 4 parity planes
-    s.g = o;                                               // (fp32 conv1 variants: not materialised any more)
     s.pm = o; o = align256(o + qpos * 9 * 64 * 2);         // pooled variants, f16 parity planes [9][4][8][PR2][PC2][8]
     s.yq = o; o = align256(o + qpos * 9 * 64 * 2);         // half-pooled conv2 maps, f16 [9][4][8][PR2][PC2][8]
     s.lmap = o; o = align256(o + qpos * 5 * NC * 4);       // class partials per pooled row, f32 [4][5][NC/4][PR2][PC2][4]
@@ -166,45 +168,66 @@ extern "C" int cmlpl_scene_workspace_layout(int band_rows, int cols, int num_fea
   CMLPL_CHECK_ARG(offsets && band_rows > 0 && cols > 0 && num_classes > 0 && num_features > 0 && w >= 4,
                   "scene_workspace_layout: bad args");
   const SceneWs s = scene_ws(band_rows, cols, num_features, num_classes, w);
-  const size_t v[12] = {s.f0pad, s.x16, s.h16, s.g, s.pm, s.yq, s.lmap, s.p2, s.spe, s.hidden, s.total, size_t(s.dense)};
+  // offset 3 (g, an empty region that keeps the 12 offsets in place) starts where pm does
+  const size_t v[12] = {s.f0pad, s.x16, s.h16, s.pm, s.pm, s.yq, s.lmap, s.p2, s.spe, s.hidden, s.total, size_t(s.dense)};
   for (int i = 0; i < 12; ++i) offsets[i] = v[i];
   return CMLPL_OK;
 }
 
-// The spectral branch (fp16 tiles of the spectra + the two spectral GEMMs) does not depend on the conv tower until the
-// head: it runs on a side stream forked off the caller's, so that its conversion kernel shares the SMs with conv0 and
-// its tail with the head of conv1_pool; the head waits for both.  One side stream and two events per device; host threads
-// that drive the same device from several streams take turns (the launches are microseconds).
-struct SideStream { cudaStream_t s = nullptr; cudaEvent_t fork = nullptr, join = nullptr; std::mutex mu; };   // mu: one fork/join sequence at a time
-static SideStream* side_stream() {
-  static SideStream per_dev[64];
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
-  SideStream& x = per_dev[dev];
-  std::lock_guard<std::mutex> lock(x.mu);
-  if (!x.join) {                                             // `join` is created last: set only when all three exist
-    if (!x.s && cudaStreamCreateWithFlags(&x.s, cudaStreamNonBlocking) != cudaSuccess) { x.s = nullptr; return nullptr; }
-    if (!x.fork && cudaEventCreateWithFlags(&x.fork, cudaEventDisableTiming) != cudaSuccess) { x.fork = nullptr; return nullptr; }
-    if (cudaEventCreateWithFlags(&x.join, cudaEventDisableTiming) != cudaSuccess) { x.join = nullptr; return nullptr; }
-  }
-  return &x;
+// Where a scene call reads the scene from.  The two entry points differ only in their first two launches, conv0 and the
+// spectral branch's conversion (and the raw entry point has no CUDA-core spectral head).
+struct SceneSrc {
+  const char* fn;                          // the entry point, named in the error messages
+  bool from_raw;
+  const float* cube;                       // cmlpl_scene_infer: the PCA cube slab and the band's z-scored spectra
+  const float* spectra;
+  const void* raw;                         // cmlpl_scene_infer_raw: the raw slab (dtype 0 = uint16, 1 = float32) and the
+  int dtype;                               // preprocessing folded into conv0 and into the spectral branch (include/cmlpl.h)
+  const float *wf, *bf, *mu, *inv_sigma;
+};
+
+// The conv0 map's conditions on the scene geometry (`fn` names the caller): the window fits the scene, the band lies
+// inside it, and the slab holds every (mirrored) source row of the band's halo.  The halo holds the band's own rows,
+// so the band's spectra, which the raw entry point reads from the slab, are inside the slab too.
+static int check_band(const char* fn, int scene_rows, int cols, int slab_row0, int slab_rows, int w, int band_row0,
+                      int band_rows) {
+  CMLPL_CHECK_ARG(w / 2 <= scene_rows && w / 2 <= cols, "%s: window larger than the scene", fn);
+  CMLPL_CHECK_ARG(band_row0 >= 0 && band_row0 + band_rows <= scene_rows, "%s: band outside the scene", fn);
+  const int a = band_row0 + window_lo(w), b = band_row0 + band_rows - 1 + window_lo(w) + w - 1;
+  int rmin = a < 0 ? 0 : a, rmax = b >= scene_rows ? scene_rows - 1 : b;
+  if (a < 0 && -a - 1 > rmax) rmax = -a - 1;                          // rows -1..a reflect to 0..-a-1
+  if (b >= scene_rows && 2 * scene_rows - 1 - b < rmin) rmin = 2 * scene_rows - 1 - b;
+  CMLPL_CHECK_ARG(rmin >= slab_row0 && rmax < slab_row0 + slab_rows, "%s: slab rows [%d,%d) do not cover the band's halo [%d,%d]",
+                  fn, slab_row0, slab_row0 + slab_rows, rmin, rmax);
+  return CMLPL_OK;
 }
 
-// conv1 (9 border classes) -> pooled parity planes -> conv2 (25 classes) -> pool + conv classifier columns ->
-// spectral classifier columns + gathered conv partials + argmax: everything after conv0 / the spectral GEMM
-static int dense_tail(unsigned char* wsb, const SceneWs& ws, int cols, int w, int band_rows, int num_features,
-                      int num_classes, const void* packed, uint8_t* labels, float* logits, cmlpl_stream_t stream,
-                      cudaEvent_t spectral_done = nullptr) {
-  int rc = cmlpl_conv1_pool_planes_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.pm, stream);
+// Every condition of a scene call, checked before it enqueues anything.  Pure host arithmetic without a CUDA call, so a
+// rejected call leaves the caller's buffers and streams untouched.  *ws receives the workspace layout.
+static int check_scene(const SceneSrc& src, int scene_rows, int cols, int slab_row0, int slab_rows, int B, int C, int w,
+                       int band_row0, int band_rows, const void* packed, const void* workspace, size_t workspace_bytes,
+                       const uint8_t* labels, SceneWs* ws) {
+  const char* fn = src.fn;
+  CMLPL_CHECK_ARG(packed && workspace && labels &&
+                      (src.from_raw ? src.raw && src.wf && src.bf && src.mu && src.inv_sigma : src.cube && src.spectra),
+                  "%s: null pointer", fn);
+  CMLPL_CHECK_ARG(!src.from_raw || src.dtype == 0 || src.dtype == 1, "%s: dtype must be 0 (uint16) or 1 (float32)", fn);
+  // w = 20: the reference's BaseNet2 (classifier hard-wired to 2624 inputs, tools/models.py:127).  w = 11: the odd-window
+  // variant BASELINE configs[4] names (ExtractPatches_for_base windows, hyper_tools.py:300-317; pooled 5 -> 2, classifier
+  // over 64*2*2 + 1024 = 1280 inputs) -- a documented extension; its border classes and pooled cells are a subset of the
+  // w = 20 ones, so the same scene-level kernels run (DESIGN 4.5); patch_cnn_kernel<11> per pixel behind path mode 0.
+  CMLPL_CHECK_ARG(w == 20 || w == 11, "%s: w=%d unsupported (20, or 11 for the odd-window variant)", fn, w);
+  CMLPL_CHECK_ARG(band_rows > 0 && cols > 0 && B > 0, "%s: bad dims (band_rows=%d cols=%d bands=%d)", fn, band_rows, cols, B);
+  CMLPL_CHECK_ARG(C > 0 && C <= 32, "%s: needs 1..32 classes, got %d", fn, C);
+  CMLPL_CHECK_ARG(!src.from_raw || tc_spectral_fits(B, C), "%s: needs <= 224 bands, got %d", fn, B);
+  const int rc = check_band(fn, scene_rows, cols, slab_row0, slab_rows, w, band_row0, band_rows);
   if (rc != CMLPL_OK) return rc;
-  rc = cmlpl_conv2_scene_f16(wsb + ws.pm, cols, w, band_rows, packed, wsb + ws.yq, stream);
-  if (rc != CMLPL_OK) return rc;
-  rc = cmlpl_pool2_cls_f16(wsb + ws.yq, cols, w, band_rows, num_features, num_classes, packed,
-                           reinterpret_cast<float*>(wsb + ws.lmap), stream);
-  if (rc != CMLPL_OK) return rc;
-  if (spectral_done) CMLPL_CUDA(cudaStreamWaitEvent(static_cast<cudaStream_t>(stream), spectral_done, 0));
-  return cmlpl_head_sum_lmap(reinterpret_cast<const float*>(wsb + ws.h16), reinterpret_cast<const float*>(wsb + ws.lmap), cols,
-                             band_rows, num_features, num_classes, w, packed, labels, logits, stream);
+  CMLPL_CHECK_ARG(src.from_raw || reinterpret_cast<uintptr_t>(src.cube) % 16 == 0, "%s: cube must be 16-byte aligned", fn);
+  CMLPL_CHECK_ARG(reinterpret_cast<uintptr_t>(packed) % 16 == 0, "%s: packed weights must be 16-byte aligned", fn);
+  *ws = scene_ws(band_rows, cols, B, C, w);
+  CMLPL_CHECK_ARG(workspace_bytes >= ws->total, "%s: workspace %zu < required %zu", fn, workspace_bytes, ws->total);
+  CMLPL_CHECK_ARG(reinterpret_cast<uintptr_t>(workspace) % 256 == 0, "%s: workspace must be 256-byte aligned", fn);
+  return CMLPL_OK;
 }
 
 extern "C" int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, int slab_row0, int slab_rows, int w,
@@ -212,17 +235,9 @@ extern "C" int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, 
                                    cmlpl_stream_t stream) {
   CMLPL_CHECK_ARG(cube && packed && f0pad, "conv0_map: null pointer");
   CMLPL_CHECK_ARG(scene_rows > 0 && cols > 0 && w >= 2 && band_rows > 0, "conv0_map: bad dims");
-  CMLPL_CHECK_ARG(w / 2 <= scene_rows && w / 2 <= cols, "conv0_map: window larger than the scene");
-  CMLPL_CHECK_ARG(band_row0 >= 0 && band_row0 + band_rows <= scene_rows, "conv0_map: band outside the scene");
+  const int rc = check_band("conv0_map", scene_rows, cols, slab_row0, slab_rows, w, band_row0, band_rows);
+  if (rc != CMLPL_OK) return rc;
   CMLPL_CHECK_ARG(reinterpret_cast<uintptr_t>(cube) % 16 == 0, "conv0_map: cube must be 16-byte aligned");
-  // the slab must hold every (mirrored) source row of the band's halo
-  const int a = band_row0 + window_lo(w), b = band_row0 + band_rows - 1 + window_lo(w) + w - 1;
-  int rmin = a < 0 ? 0 : a, rmax = b >= scene_rows ? scene_rows - 1 : b;
-  if (a < 0 && -a - 1 > rmax) rmax = -a - 1;                          // rows -1..a reflect to 0..-a-1
-  if (b >= scene_rows && 2 * scene_rows - 1 - b < rmin) rmin = 2 * scene_rows - 1 - b;
-  CMLPL_CHECK_ARG(rmin >= slab_row0 && rmax < slab_row0 + slab_rows,
-                  "conv0_map: slab rows [%d,%d) do not cover the band's halo [%d,%d]", slab_row0,
-                  slab_row0 + slab_rows, rmin, rmax);
   const PackedLayout L = packed_layout(1, 1, w);  // w0/b0 offsets do not depend on B, C
   const unsigned char* pk = static_cast<const unsigned char*>(packed);
   const int prow_n = band_rows + w - 1, pcol_n = cols + w - 1;
@@ -231,12 +246,10 @@ extern "C" int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, 
                                       nullptr, static_cast<__half*>(f0pad), static_cast<cudaStream_t>(stream));
 }
 
-extern "C" int cmlpl_spectral_head_f32(const float* spectra, int64_t n, int num_features, int num_classes, int w,
-                                       const void* packed, float* hidden, int64_t chunk, float* spe_logits,
-                                       cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(spectra && packed && hidden && spe_logits, "spectral_head: null pointer");
-  CMLPL_CHECK_ARG(n >= 0 && chunk > 0 && num_features > 0 && num_classes > 0, "spectral_head: bad dims");
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
+// CUDA-core spectral head of the per-pixel path: spe_logits f32 [n][C] = Wc_spe . relu(Wspe . x + bspe), over chunks of
+// `chunk` pixels through the f32 scratch hidden [chunk][1024]
+static int spectral_head(const float* spectra, int64_t n, int num_features, int num_classes, int w, const void* packed,
+                         float* hidden, int64_t chunk, float* spe_logits, cudaStream_t s) {
   const unsigned char* pk = static_cast<const unsigned char*>(packed);
   const PackedLayout L = packed_layout(num_features, num_classes, w);
   const float* wspe = reinterpret_cast<const float*>(pk + L.wspe);
@@ -259,14 +272,12 @@ extern "C" int cmlpl_spectral_head_f32(const float* spectra, int64_t n, int num_
   return CMLPL_OK;
 }
 
+// classify_kernel over the per-pixel pooled features p2, adding the spectral logits spe_logits f32 [n][C] (CUDA-core
+// head) or the tensor-core branch's four quarter partials `part`
 static int classify_launch(const void* p2, const float* spe_logits, const float* part, int64_t part_stride, int64_t n,
                            int num_features, int num_classes, int w, const void* packed, uint8_t* labels, float* logits,
-                           cmlpl_stream_t stream) {
+                           cudaStream_t s) {
   const int part_width = class_width(num_classes);        // row width of spectral_logits_kernel's partials
-  CMLPL_CHECK_ARG(p2 && packed && labels, "classify: null pointer");
-  CMLPL_CHECK_ARG(n >= 0 && num_classes > 0 && num_classes <= 32 && w >= 4, "classify: bad dims (C=%d w=%d)",
-                  num_classes, w);
-  if (n == 0) return CMLPL_OK;
   const unsigned char* pk = static_cast<const unsigned char*>(packed);
   const PackedLayout L = packed_layout(num_features, num_classes, w);
   const int K = L.conv_pos * 64;
@@ -275,7 +286,6 @@ static int classify_launch(const void* p2, const float* spe_logits, const float*
   int64_t grid = (n + 7) / 8;
   const int64_t cap = int64_t(sm_count()) * 8;
   if (grid > cap) grid = cap;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (num_classes <= 16)
     classify_kernel<16><<<int(grid), 256, 0, s>>>(static_cast<const __half*>(p2), spe_logits, part, part_stride, part_width, n,
                                                   K, num_classes, wc, bc, labels, logits);
@@ -284,12 +294,6 @@ static int classify_launch(const void* p2, const float* spe_logits, const float*
                                                   K, num_classes, wc, bc, labels, logits);
   CMLPL_CHECK_LAUNCH("classify");
   return CMLPL_OK;
-}
-
-extern "C" int cmlpl_classify_f16(const void* p2, const float* spe_logits, int64_t n, int num_features,
-                                  int num_classes, int w, const void* packed, uint8_t* labels, float* logits,
-                                  cmlpl_stream_t stream) {
-  return classify_launch(p2, spe_logits, nullptr, 0, n, num_features, num_classes, w, packed, labels, logits, stream);
 }
 
 extern "C" int cmlpl_argmax_u8(const float* logits, int64_t n, int num_classes, uint8_t* labels, cmlpl_stream_t stream) {
@@ -303,58 +307,78 @@ extern "C" int cmlpl_argmax_u8(const float* logits, int64_t n, int num_classes, 
   return CMLPL_OK;
 }
 
+// One scene call of either entry point: check_scene, then the path the workspace layout was sized for.
+static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_row0, int slab_rows, int B, int C, int w,
+                       int band_row0, int band_rows, const void* packed, void* workspace, size_t workspace_bytes,
+                       uint8_t* labels, float* logits, cmlpl_stream_t stream) {
+  SceneWs ws;
+  int rc = check_scene(src, scene_rows, cols, slab_row0, slab_rows, B, C, w, band_row0, band_rows, packed, workspace,
+                       workspace_bytes, labels, &ws);
+  if (rc != CMLPL_OK) return rc;
+  unsigned char* wsb = static_cast<unsigned char*>(workspace);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int64_t n = int64_t(band_rows) * cols;
+  float* part = reinterpret_cast<float*>(wsb + ws.h16);
+  // the tensor-core spectral branch reads the band's z-scored spectra, or the band's rows of the raw slab
+  const void* band_spectra =
+      src.from_raw ? static_cast<const unsigned char*>(src.raw) + size_t(band_row0 - slab_row0) * cols * B * (src.dtype == 0 ? 2 : 4)
+                   : static_cast<const void*>(src.spectra);
+  auto spectral_tc = [&](cudaStream_t st) {
+    return launch_spectral_logits(band_spectra, src.from_raw ? src.dtype : -1, n, B, C, w, src.mu, src.inv_sigma, packed,
+                                  wsb + ws.x16, part, st);
+  };
+  auto conv0 = [&]() {
+    if (!src.from_raw)
+      return cmlpl_conv0_map_f16(src.cube, scene_rows, cols, slab_row0, slab_rows, w, band_row0, band_rows, packed,
+                                 wsb + ws.f0pad, stream);
+    const int prow_n = band_rows + w - 1, pcol_n = cols + w - 1;
+    __half* f0 = reinterpret_cast<__half*>(wsb + ws.f0pad);
+    return src.dtype == 0
+        ? launch_conv0_tc<uint16_t, false, true>(static_cast<const uint16_t*>(src.raw), B, scene_rows, cols, slab_row0, w,
+                                                 band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, s)
+        : launch_conv0_tc<float, false, true>(static_cast<const float*>(src.raw), B, scene_rows, cols, slab_row0, w,
+                                              band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, s);
+  };
+  if (ws.dense) {
+    // The spectral branch (fp16 tiles of the spectra + the two spectral GEMMs) does not depend on the conv tower until
+    // the head: forked onto the side stream, its conversion kernel shares the SMs with conv0 and its tail with the head
+    // of conv1_pool.  Then conv1 (9 border classes) -> pooled parity planes -> conv2 (25 classes) -> pool + conv
+    // classifier columns, and the head joins the branch: spectral partials + gathered conv partials + argmax.
+    SideStream* sd = side_stream();
+    CMLPL_CHECK_ARG(sd, "%s: cannot create the side stream", src.fn);
+    std::lock_guard<std::mutex> lock(sd->mu);
+    CMLPL_CUDA(cudaEventRecord(sd->fork[0], s));
+    CMLPL_CUDA(cudaStreamWaitEvent(sd->s, sd->fork[0], 0));
+    if ((rc = spectral_tc(sd->s)) != CMLPL_OK) return rc;
+    CMLPL_CUDA(cudaEventRecord(sd->join[0], sd->s));
+    if ((rc = conv0()) != CMLPL_OK) return rc;
+    if ((rc = cmlpl_conv1_pool_planes_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.pm, stream)) != CMLPL_OK) return rc;
+    if ((rc = cmlpl_conv2_scene_f16(wsb + ws.pm, cols, w, band_rows, packed, wsb + ws.yq, stream)) != CMLPL_OK) return rc;
+    float* lmap = reinterpret_cast<float*>(wsb + ws.lmap);
+    if ((rc = cmlpl_pool2_cls_f16(wsb + ws.yq, cols, w, band_rows, B, C, packed, lmap, stream)) != CMLPL_OK) return rc;
+    CMLPL_CUDA(cudaStreamWaitEvent(s, sd->join[0], 0));
+    return cmlpl_head_sum_lmap(part, lmap, cols, band_rows, B, C, w, packed, labels, logits, stream);
+  }
+  // per pixel: the tensor-core spectral branch, or the CUDA-core spectral head beyond 224 bands and in path mode 0 at
+  // 17-32 classes on the cube entry point (the raw entry point has only the tensor-core branch)
+  if ((rc = conv0()) != CMLPL_OK) return rc;
+  const bool tc = ws.tc || src.from_raw;
+  float* spe = reinterpret_cast<float*>(wsb + ws.spe);
+  rc = tc ? spectral_tc(s)
+          : spectral_head(src.spectra, n, B, C, w, packed, reinterpret_cast<float*>(wsb + ws.hidden), ws.chunk, spe, s);
+  if (rc != CMLPL_OK) return rc;
+  if ((rc = cmlpl_patch_cnn_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.p2, stream)) != CMLPL_OK) return rc;
+  return classify_launch(wsb + ws.p2, tc ? nullptr : spe, tc ? part : nullptr, ((n + 127) / 128) * 128, n, B, C, w, packed,
+                         labels, logits, s);
+}
+
 extern "C" int cmlpl_scene_infer(const float* cube, int scene_rows, int cols, int slab_row0, int slab_rows,
                                  const float* spectra, int num_features, int num_classes, int w, int band_row0,
                                  int band_rows, const void* packed, void* workspace, size_t workspace_bytes,
                                  uint8_t* labels, float* logits, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(cube && spectra && packed && workspace && labels, "scene_infer: null pointer");
-  // w = 20: the reference's BaseNet2 (classifier hard-wired to 2624 inputs, tools/models.py:127).  w = 11: the odd-window
-  // variant BASELINE configs[4] names (ExtractPatches_for_base windows, hyper_tools.py:300-317; pooled 5 -> 2, classifier
-  // over 64*2*2 + 1024 = 1280 inputs) -- a documented extension; its border classes and pooled cells are a subset of the
-  // w = 20 ones, so the same scene-level kernels run (DESIGN 4.5); patch_cnn_kernel<11> per pixel behind path mode 0.
-  CMLPL_CHECK_ARG(w == 20 || w == 11, "scene_infer: w=%d unsupported (20, or 11 for the odd-window variant)", w);
-  CMLPL_CHECK_ARG(band_rows > 0 && cols > 0 && num_classes > 0 && num_classes <= 32, "scene_infer: bad dims");
-  const SceneWs ws = scene_ws(band_rows, cols, num_features, num_classes, w);
-  CMLPL_CHECK_ARG(workspace_bytes >= ws.total, "scene_infer: workspace %zu < required %zu", workspace_bytes, ws.total);
-  CMLPL_CHECK_ARG(reinterpret_cast<uintptr_t>(workspace) % 256 == 0, "scene_infer: workspace must be 256-byte aligned");
-  unsigned char* wsb = static_cast<unsigned char*>(workspace);
-  const int64_t n = int64_t(band_rows) * cols;
-  int rc = CMLPL_OK;
-  if (ws.tc && ws.dense) {
-    SideStream* sd = side_stream();
-    CMLPL_CHECK_ARG(sd, "scene_infer: cannot create the side stream");
-    std::lock_guard<std::mutex> lock(sd->mu);
-    cudaStream_t ms = static_cast<cudaStream_t>(stream);
-    CMLPL_CUDA(cudaEventRecord(sd->fork, ms));
-    CMLPL_CUDA(cudaStreamWaitEvent(sd->s, sd->fork, 0));
-    rc = cmlpl_spectral_logits_tc(spectra, n, num_features, num_classes, w, packed, wsb + ws.x16,
-                                  reinterpret_cast<float*>(wsb + ws.h16), sd->s);
-    if (rc != CMLPL_OK) return rc;
-    CMLPL_CUDA(cudaEventRecord(sd->join, sd->s));
-    rc = cmlpl_conv0_map_f16(cube, scene_rows, cols, slab_row0, slab_rows, w, band_row0, band_rows, packed, wsb + ws.f0pad, stream);
-    if (rc != CMLPL_OK) return rc;
-    return dense_tail(wsb, ws, cols, w, band_rows, num_features, num_classes, packed, labels, logits, stream, sd->join);
-  }
-  rc = cmlpl_conv0_map_f16(cube, scene_rows, cols, slab_row0, slab_rows, w, band_row0, band_rows, packed,
-                           wsb + ws.f0pad, stream);
-  if (rc != CMLPL_OK) return rc;
-  if (ws.tc) {
-    rc = cmlpl_spectral_logits_tc(spectra, n, num_features, num_classes, w, packed, wsb + ws.x16,
-                                  reinterpret_cast<float*>(wsb + ws.h16), stream);
-    if (rc != CMLPL_OK) return rc;
-    rc = cmlpl_patch_cnn_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.p2, stream);
-    if (rc != CMLPL_OK) return rc;
-    return classify_launch(wsb + ws.p2, nullptr, reinterpret_cast<const float*>(wsb + ws.h16), ((n + 127) / 128) * 128, n,
-                           num_features, num_classes, w, packed, labels, logits, stream);
-  }
-  rc = cmlpl_spectral_head_f32(spectra, n, num_features, num_classes, w, packed,
-                               reinterpret_cast<float*>(wsb + ws.hidden), ws.chunk,
-                               reinterpret_cast<float*>(wsb + ws.spe), stream);
-  if (rc != CMLPL_OK) return rc;
-  rc = cmlpl_patch_cnn_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.p2, stream);
-  if (rc != CMLPL_OK) return rc;
-  return cmlpl_classify_f16(wsb + ws.p2, reinterpret_cast<const float*>(wsb + ws.spe), n, num_features, num_classes,
-                            w, packed, labels, logits, stream);
+  const SceneSrc src{"scene_infer", false, cube, spectra};
+  return scene_infer(src, scene_rows, cols, slab_row0, slab_rows, num_features, num_classes, w, band_row0, band_rows, packed,
+                     workspace, workspace_bytes, labels, logits, stream);
 }
 
 
@@ -369,58 +393,7 @@ extern "C" int cmlpl_scene_infer_raw(const void* raw, int dtype, int scene_rows,
                                      const float* wf, const float* bf, const float* mu, const float* inv_sigma,
                                      const void* packed, void* workspace, size_t workspace_bytes, uint8_t* labels,
                                      float* logits, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(raw && wf && bf && mu && inv_sigma && packed && workspace && labels, "scene_infer_raw: null pointer");
-  CMLPL_CHECK_ARG(dtype == 0 || dtype == 1, "scene_infer_raw: dtype must be 0 (uint16) or 1 (float32)");
-  CMLPL_CHECK_ARG(w == 20 || w == 11, "scene_infer_raw: w=%d unsupported (20, or 11 for the odd-window variant)", w);
-  CMLPL_CHECK_ARG(band_rows > 0 && cols > 0 && num_classes > 0 && num_features > 0, "scene_infer_raw: bad dims");
-  CMLPL_CHECK_ARG(tc_spectral_fits(num_features, num_classes), "scene_infer_raw: needs <= 32 classes and <= 224 bands");
-  CMLPL_CHECK_ARG(w / 2 <= scene_rows && w / 2 <= cols, "scene_infer_raw: window larger than the scene");
-  CMLPL_CHECK_ARG(band_row0 >= 0 && band_row0 + band_rows <= scene_rows, "scene_infer_raw: band outside the scene");
-  const int a = band_row0 + window_lo(w), b = band_row0 + band_rows - 1 + window_lo(w) + w - 1;
-  int rmin = a < 0 ? 0 : a, rmax = b >= scene_rows ? scene_rows - 1 : b;
-  if (a < 0 && -a - 1 > rmax) rmax = -a - 1;
-  if (b >= scene_rows && 2 * scene_rows - 1 - b < rmin) rmin = 2 * scene_rows - 1 - b;
-  CMLPL_CHECK_ARG(rmin >= slab_row0 && rmax < slab_row0 + slab_rows && band_row0 >= slab_row0,
-                  "scene_infer_raw: slab rows [%d,%d) do not cover the band's halo [%d,%d]", slab_row0,
-                  slab_row0 + slab_rows, rmin, rmax);
-  const SceneWs ws = scene_ws(band_rows, cols, num_features, num_classes, w);
-  CMLPL_CHECK_ARG(workspace_bytes >= ws.total, "scene_infer_raw: workspace %zu < required %zu", workspace_bytes, ws.total);
-  unsigned char* wsb = static_cast<unsigned char*>(workspace);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const int64_t n = int64_t(band_rows) * cols;
-  const int prow_n = band_rows + w - 1, pcol_n = cols + w - 1;
-  auto conv0_raw = [&]() {
-    __half* f0 = reinterpret_cast<__half*>(wsb + ws.f0pad);
-    return dtype == 0
-        ? launch_conv0_tc<uint16_t, false, true>(static_cast<const uint16_t*>(raw), num_features, scene_rows, cols, slab_row0, w,
-                                                 band_row0, prow_n, pcol_n, wf, bf, mu, inv_sigma, f0, s)
-        : launch_conv0_tc<float, false, true>(static_cast<const float*>(raw), num_features, scene_rows, cols, slab_row0, w,
-                                              band_row0, prow_n, pcol_n, wf, bf, mu, inv_sigma, f0, s);
-  };
-  const size_t esz = dtype == 0 ? 2 : 4;
-  const void* band_raw = static_cast<const unsigned char*>(raw) + size_t(band_row0 - slab_row0) * cols * num_features * esz;
-  int rc = CMLPL_OK;
-  if (ws.dense) {                                          // spectral branch beside the conv tower (see side_stream())
-    SideStream* sd = side_stream();
-    CMLPL_CHECK_ARG(sd, "scene_infer_raw: cannot create the side stream");
-    std::lock_guard<std::mutex> lock(sd->mu);
-    CMLPL_CUDA(cudaEventRecord(sd->fork, s));
-    CMLPL_CUDA(cudaStreamWaitEvent(sd->s, sd->fork, 0));
-    rc = cmlpl_spectral_logits_raw_tc(band_raw, dtype, n, num_features, num_classes, w, mu, inv_sigma, packed,
-                                      wsb + ws.x16, reinterpret_cast<float*>(wsb + ws.h16), sd->s);
-    if (rc != CMLPL_OK) return rc;
-    CMLPL_CUDA(cudaEventRecord(sd->join, sd->s));
-    rc = conv0_raw();
-    if (rc != CMLPL_OK) return rc;
-    return dense_tail(wsb, ws, cols, w, band_rows, num_features, num_classes, packed, labels, logits, stream, sd->join);
-  }
-  rc = conv0_raw();
-  if (rc != CMLPL_OK) return rc;
-  rc = cmlpl_spectral_logits_raw_tc(band_raw, dtype, n, num_features, num_classes, w, mu, inv_sigma, packed,
-                                    wsb + ws.x16, reinterpret_cast<float*>(wsb + ws.h16), stream);
-  if (rc != CMLPL_OK) return rc;
-  rc = cmlpl_patch_cnn_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.p2, stream);
-  if (rc != CMLPL_OK) return rc;
-  return classify_launch(wsb + ws.p2, nullptr, reinterpret_cast<const float*>(wsb + ws.h16), ((n + 127) / 128) * 128, n,
-                         num_features, num_classes, w, packed, labels, logits, stream);
+  const SceneSrc src{"scene_infer_raw", true, nullptr, nullptr, raw, dtype, wf, bf, mu, inv_sigma};
+  return scene_infer(src, scene_rows, cols, slab_row0, slab_rows, num_features, num_classes, w, band_row0, band_rows, packed,
+                     workspace, workspace_bytes, labels, logits, stream);
 }

@@ -9,23 +9,6 @@
 using namespace cmlpl;
 
 namespace {
-// Fork / join inside the step: kernels without a mutual dependency (the spectral GEMM next to the conv trunk; the head
-// weight gradients next to the conv backward chain) run on a side stream between two events.  Works the same in eager
-// mode and under stream capture (the events become graph edges).  One side stream + four events per device, created
-// on first use and kept for the life of the process -- the only persistent resources the library owns.
-struct StepStreams { cudaStream_t side = nullptr; cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr}; };
-StepStreams* step_streams() {
-  static StepStreams per_dev[64];
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
-  StepStreams& s = per_dev[dev];
-  if (!s.side) {
-    if (cudaStreamCreateWithFlags(&s.side, cudaStreamNonBlocking) != cudaSuccess) return nullptr;
-    for (auto& e : s.ev)
-      if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) return nullptr;
-  }
-  return &s;
-}
 constexpr int64_t kNumel[CMLPL_TRAIN_TENSORS] = {64 * 60, 64, 64 * 64 * 9, 64, 64 * 64 * 9, 64, 0 /*1024*B*/, 1024, 0 /*C*cat*/, 0 /*C*/};
 int64_t numel(int i, int B, int C, int cat) {
   if (i == 6) return int64_t(1024) * B;
@@ -82,8 +65,10 @@ extern "C" int cmlpl_train_step(const cmlpl_train_io* io, int phases, cmlpl_stre
                       (!io->drop_mask || reinterpret_cast<uintptr_t>(io->drop_mask) % 16 == 0),
                   "train_step: feat / cube / drop_mask must be 16-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  StepStreams* ss = step_streams();
-  CMLPL_CHECK_ARG(ss, "train_step: could not create the side stream");
+  // the library's side stream (common.cuh) carries the step's two forks; its lock is held for the whole enqueue
+  SideStream* sd = side_stream();
+  CMLPL_CHECK_ARG(sd, "train_step: could not create the side stream");
+  std::lock_guard<std::mutex> lock(sd->mu);
   unsigned char* ws = static_cast<unsigned char*>(io->work);
   auto f32 = [&](size_t off) { return reinterpret_cast<float*>(ws + off); };
   auto f16 = [&](size_t off) { return reinterpret_cast<__half*>(ws + off); };
@@ -123,12 +108,12 @@ extern "C" int cmlpl_train_step(const cmlpl_train_io* io, int phases, cmlpl_stre
     }
     if ((rc = launch_train_conv0(a, w, st)) != CMLPL_OK) return rc;
     // fork: the spectral GEMM (needs only the noisy spectra of kernel 1) next to the conv trunk
-    CMLPL_CUDA(cudaEventRecord(ss->ev[0], st));
-    CMLPL_CUDA(cudaStreamWaitEvent(ss->side, ss->ev[0], 0));
-    if ((rc = launch_multi_gemm(mg, ss->side, "train_spectral_fwd")) != CMLPL_OK) return rc;
-    CMLPL_CUDA(cudaEventRecord(ss->ev[1], ss->side));
+    CMLPL_CUDA(cudaEventRecord(sd->fork[0], st));
+    CMLPL_CUDA(cudaStreamWaitEvent(sd->s, sd->fork[0], 0));
+    if ((rc = launch_multi_gemm(mg, sd->s, "train_spectral_fwd")) != CMLPL_OK) return rc;
+    CMLPL_CUDA(cudaEventRecord(sd->join[0], sd->s));
     if ((rc = launch_train_cnn(t, w, st)) != CMLPL_OK) return rc;
-    CMLPL_CUDA(cudaStreamWaitEvent(st, ss->ev[1], 0));
+    CMLPL_CUDA(cudaStreamWaitEvent(st, sd->join[0], 0));
     if ((rc = launch_head_fwd(ha, w, st)) != CMLPL_OK) return rc;
   }
 
@@ -196,15 +181,15 @@ extern "C" int cmlpl_train_step(const cmlpl_train_io* io, int phases, cmlpl_stre
       b0.g_w3[e][0] = io->net[e].g[2]; b0.g_w3[e][1] = io->net[e].g[4];
     }
     // fork: the head weight gradients (classifier, feat_spe) next to the conv backward chain
-    CMLPL_CUDA(cudaEventRecord(ss->ev[2], st));
-    CMLPL_CUDA(cudaStreamWaitEvent(ss->side, ss->ev[2], 0));
-    if ((rc = launch_head_wgrad(ha, w, ss->side)) != CMLPL_OK) return rc;
-    if ((rc = launch_multi_gemm(dws, ss->side, "train_spectral_wgrad")) != CMLPL_OK) return rc;
-    CMLPL_CUDA(cudaEventRecord(ss->ev[3], ss->side));
+    CMLPL_CUDA(cudaEventRecord(sd->fork[1], st));
+    CMLPL_CUDA(cudaStreamWaitEvent(sd->s, sd->fork[1], 0));
+    if ((rc = launch_head_wgrad(ha, w, sd->s)) != CMLPL_OK) return rc;
+    if ((rc = launch_multi_gemm(dws, sd->s, "train_spectral_wgrad")) != CMLPL_OK) return rc;
+    CMLPL_CUDA(cudaEventRecord(sd->join[1], sd->s));
     if ((rc = launch_train_conv_bwd(w / 2, b2, st)) != CMLPL_OK) return rc;      // conv2: 10 x 10 / 5 x 5
     if ((rc = launch_train_conv_bwd(w, b1, st)) != CMLPL_OK) return rc;          // conv1: 20 x 20 / 11 x 11
     if ((rc = launch_train_conv0_bwd(b0, w, st)) != CMLPL_OK) return rc;
-    CMLPL_CUDA(cudaStreamWaitEvent(st, ss->ev[3], 0));
+    CMLPL_CUDA(cudaStreamWaitEvent(st, sd->join[1], 0));
   }
 
   if (phases & 8) {

@@ -167,12 +167,6 @@ int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, int slab_ro
                         void* f0pad /* f16 [8, band_rows+w-1, cols+w-1, 8]: chunk-planar (8 channels per 16-B chunk) */, cmlpl_stream_t stream);
 int cmlpl_patch_cnn_f16(const void* f0pad, int cols, int w, int band_rows, const void* packed,
                         void* p2 /* f16 [band_rows*cols, (w/4)^2, 64] */, cmlpl_stream_t stream);
-int cmlpl_spectral_head_f32(const float* spectra, int64_t n, int num_features, int num_classes, int w,
-                            const void* packed, float* hidden /* f32 [chunk,1024] scratch */,
-                            int64_t chunk, float* spe_logits /* f32 [n, C] */, cmlpl_stream_t stream);
-int cmlpl_classify_f16(const void* p2, const float* spe_logits /* may be NULL */, int64_t n,
-                       int num_features, int num_classes, int w, const void* packed,
-                       uint8_t* labels, float* logits /* may be NULL */, cmlpl_stream_t stream);
 /* Dense (scene-level) conv tower, exact compute sharing of conv1 / conv2 / pools / classifier (SURVEY section 7;
  * tools/models.py:133-150 for all patches at once; csrc/conv1_scene_sm100.cu, csrc/conv2_scene_sm100.cu).
  * PR = band_rows+w-1, PC = cols+w-1, PR2 = (band_rows+w)/2, PC2 = (cols+w)/2; "planes" = the 4 parity planes
@@ -202,13 +196,9 @@ int cmlpl_pool2_cls_f16(const void* yq, int cols, int w, int band_rows, int num_
  *                                  quarter of the 1024 hidden features (tools/models.py:142-143,150), <= 32 classes
  *                                  (NC = 16 up to 16 classes, 32 for 17-32), as many bands as the kernel's input tiles
  *                                  fit shared memory for (cmlpl_scene_infer uses it up to 224)
- *   cmlpl_spectral_logits_raw_tc : the same from the raw cube (z-score folded into the fp16 conversion)
  *   cmlpl_head_sum_lmap          : 4 quarter partials + the 5 gathered conv partials + bias, argmax */
 int cmlpl_spectral_logits_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
                              const void* packed, void* x16, float* part, cmlpl_stream_t stream);
-int cmlpl_spectral_logits_raw_tc(const void* raw, int dtype, int64_t n, int num_features, int num_classes, int w,
-                                 const float* mu, const float* inv_sigma, const void* packed, void* x16, float* part,
-                                 cmlpl_stream_t stream);
 int cmlpl_head_sum_lmap(const float* part, const float* lmap, int cols, int band_rows, int num_features,
                         int num_classes, int w, const void* packed, uint8_t* labels, float* logits,
                         cmlpl_stream_t stream);
@@ -317,7 +307,8 @@ int cmlpl_comm_allreduce_confusion(cmlpl_comm* comm, int64_t* cm, int count, cml
 int cmlpl_comm_destroy(cmlpl_comm* comm);
 
 /* ------------------------------------------------------- fused training step --
- * One mutual-learning step of train.py:150-272 for BOTH BaseNet2 peers as ~17 kernel launches on `stream`
+ * One mutual-learning step of train.py:150-272 for BOTH BaseNet2 peers as 15 kernel launches (+ memsets of the gradient
+ * block) on `stream`
  * (CUDA-graph capturable: every per-step scalar lives in the device-side cmlpl_train_params block).
  * Contractions run on tcgen05 (fp16 operands = TF32's 11-bit significand, fp32 accumulate in TMEM): conv0 / conv1 /
  * conv2 forward (tools/models.py:132-140), their data gradients and weight gradients (train.py:267,271); gradient

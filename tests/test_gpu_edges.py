@@ -162,8 +162,8 @@ def test_raw_path_mid_size_matches_preprocessed_path(dev, B, K, dtype):
 
 
 def test_scene_infer_from_two_streams_interleaved(dev):
-    """cmlpl_scene_infer forks its spectral branch onto a per-device side stream (scene_infer.cu::side_stream).  Two
-    caller streams that issue scenes alternately share that side stream and its two events; every result must still be
+    """cmlpl_scene_infer forks its spectral branch onto the library's per-device side stream (api.cu::side_stream).  Two
+    caller streams that issue scenes alternately share that side stream and its events; every result must still be
     the one a lone call produces (bit-identical: the kernels are deterministic), and work queued on a caller stream
     after the call must see the labels."""
     from cmlpl_b200 import ops
@@ -193,3 +193,33 @@ def test_scene_infer_from_two_streams_interleaved(dev):
     torch.cuda.synchronize()
     for s in scenes:
         assert torch.equal(s["copy"], s["ref"]) and torch.equal(s["labels"], s["ref"])
+
+
+@pytest.mark.parametrize("case", ["band_outside_the_scene", "slab_misses_the_halo", "cube_not_16_byte_aligned"])
+def test_rejected_scene_call_leaves_workspace_and_labels_untouched(dev, case):
+    """A dense-path call that is rejected enqueues nothing, on the caller's stream or on the side stream: after a
+    device-wide synchronize (which waits on the side stream too) the workspace still holds its sentinel bytes and the
+    labels still read 255."""
+    from cmlpl_b200 import _lib, ops
+    R, C, B, K, w, rows = 40, 50, 103, 9, 20, 10
+    rng = np.random.default_rng(77)
+    cube = torch.from_numpy(rng.standard_normal((R, C, 60)).astype(np.float32)).to(dev)
+    spectra = torch.from_numpy(rng.standard_normal((rows * C, B)).astype(np.float32)).to(dev)
+    torch.manual_seed(77)
+    packed = ops.pack_basenet2({k: v.to(dev) for k, v in O.basenet2_init(B, K).items()}, B, K, w)
+    ws = ops.scene_workspace(rows, C, B, K, w, dev).fill_(0xA5)
+    labels = torch.full((rows * C,), 255, dtype=torch.uint8, device=dev)
+    kw = dict(band_rows=rows, scene_rows=R, workspace=ws, labels=labels)
+    if case == "band_outside_the_scene":
+        kw["band_row0"], match = R - 5, "band outside the scene"
+    elif case == "slab_misses_the_halo":
+        cube, kw["slab_row0"], match = cube[5:], 5, "do not cover the band's halo"     # rows 0..9 need scene row 0
+    else:
+        flat = torch.empty(R * C * 60 + 4, device=dev)
+        cube = flat[1:1 + R * C * 60].view(R, C, 60).copy_(cube)                       # 4 bytes past a 16-byte boundary
+        match = "cube must be 16-byte aligned"
+    torch.cuda.synchronize()
+    with pytest.raises(_lib.CmlplError, match=match):
+        ops.scene_infer(cube, spectra, packed, K, w, **kw)
+    torch.cuda.synchronize()
+    assert bool((ws == 0xA5).all()) and bool((labels == 255).all())
