@@ -221,13 +221,213 @@ conv0_tc_kernel(const T* __restrict__ in, int K, int KP, int nstage, int scene_r
   if (warp == 8) { tc_fence_after(); tmem_dealloc(tmem, 128); }
 }
 
+// K-sliced variant for the raw cube beyond 256 bands (split hi / lo operands only).  A tile's X operand no longer fits one
+// shared-memory stage, so it passes through a two-stage ring of 64-band slices [8 chunks][128 positions][8] (hi | lo):
+// the workers load and z-score slice j of a tile while the MMA thread consumes slice j-1, and the 3 x 4 tcgen05.mma of
+// every slice accumulate into the tile's TMEM slot.  The folded weights stay resident as fp16 hi + lo ([KC][64][8] each,
+// 128 KB at 512 bands).  Tile loop, TMEM slots, mirror index map and epilogue are those of conv0_tc_kernel.
+namespace c0k {
+constexpr int kSlice = 64, kSliceChunks = kSlice / 8;
+constexpr int XCH = 2064;                                     // chunk-plane stride of a slice (as conv0_tc_kernel's)
+constexpr int kXHalf = kSliceChunks * XCH;                    // one slice, hi or lo: 16 512 B
+constexpr int kMaxK = 512;
+}  // namespace c0k
+
+template <typename T>
+__global__ void __launch_bounds__(c0s::kThreads, 1)
+conv0_tc_sliced_kernel(const T* __restrict__ in, int K, int KP, int scene_rows, int cols, int slab_row0, int w, int band_row0,
+                       int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
+                       const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad) {
+  using namespace c0s;
+  using c0k::kSlice; using c0k::XCH; using c0k::kXHalf;
+  extern __shared__ __align__(128) unsigned char smem[];
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const uint32_t sbase = smem_u32(smem);
+  const int KC = KP / 8, nslice = (KP + kSlice - 1) / kSlice;
+  const int whalf = KC * 64 * 16;
+  const int S_W = 0, S_X = 2 * whalf, S_BIAS = S_X + 2 * 2 * kXHalf, S_MU = S_BIAS + 256, S_IS = S_MU + KP * 4,
+            S_BAR = S_IS + KP * 4;
+  const int S_TMEM = S_BAR + 64;
+  const uint32_t bars = sbase + S_BAR;
+  volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem + S_TMEM);
+  float* smu = reinterpret_cast<float*>(smem + S_MU);
+  float* sis = reinterpret_cast<float*>(smem + S_IS);
+  const int64_t plane = int64_t(prow_n) * pcol_n;
+  const int64_t ntiles = (plane + 127) / 128;
+  const int lo = window_lo(w);
+
+  // weights [K][64] f32 (times the band's sigma, see conv0_tc_kernel) -> fp16 hi / lo K-major B operands [KC][64 n][8 k]
+  {
+    __half* sw = reinterpret_cast<__half*>(smem + S_W);
+    for (int i = tid; i < KP * 64; i += kThreads) {
+      const int k = i >> 6, n = i & 63;
+      const float wv = k < K ? __ldg(wt + k * 64 + n) * (1.f / __ldg(inv_sigma + k)) : 0.f;
+      const __half hi = __float2half_rn(wv);
+      sw[((k >> 3) * 64 + n) * 8 + (k & 7)] = hi;
+      sw[whalf / 2 + ((k >> 3) * 64 + n) * 8 + (k & 7)] = __float2half_rn(wv - __half2float(hi));
+    }
+    if (tid < 64) reinterpret_cast<float*>(smem + S_BIAS)[tid] = __ldg(bias + tid);
+    for (int i = tid; i < KP; i += kThreads) {
+      smu[i] = i < K ? __ldg(mu + i) : 0.f;
+      sis[i] = i < K ? __ldg(inv_sigma + i) : 0.f;       // k >= K: the loaders write 0
+    }
+  }
+  if (tid == 0) {
+    for (int s = 0; s < 2; ++s) {
+      mbar_init(bars + 8 * (X_FULL0 + s), kWorkers);
+      mbar_init(bars + 8 * (X_EMPTY0 + s), 1);
+      mbar_init(bars + 8 * (D_FULL0 + s), 1);
+      mbar_init(bars + 8 * (D_EMPTY0 + s), kWorkers);
+    }
+    fence_barrier_init();
+  }
+  if (warp == 8) tmem_alloc(sbase + S_TMEM, 128);
+  fence_proxy_async();
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = *tmem_slot;
+  const int64_t t_first = blockIdx.x, t_step = gridDim.x;
+
+  if (warp == 8) {
+    const uint32_t kI = make_idesc_f16(128, 64);
+    int it = 0, g = 0;                                          // tile count, slice count (ring position)
+    for (int64_t t = t_first; t < ntiles; t += t_step, ++it) {
+      const int s = it & 1, ph = (it >> 1) & 1;                 // TMEM slot
+      mbar_wait(bars + 8 * (D_EMPTY0 + s), ph ^ 1, 91);
+      for (int j = 0; j < nslice; ++j, ++g) {
+        const int xs_ = g & 1;
+        mbar_wait(bars + 8 * (X_FULL0 + xs_), (g >> 1) & 1, 90);
+        tc_fence_after();
+        if (lane == 0) {
+          const uint32_t xa = sbase + S_X + xs_ * 2 * kXHalf, wa = sbase + S_W;
+          const int ksteps = (KP - j * kSlice < kSlice ? KP - j * kSlice : kSlice) / 16;
+          for (int ks = 0; ks < ksteps; ++ks) {
+            const uint32_t wk = wa + (j * (kSlice / 16) + ks) * 2 * 1024;
+            umma_f16(tmem + s * 64, make_desc(xa + ks * 2 * XCH, XCH, 128), make_desc(wk, 1024, 128), kI,
+                     (j | ks) != 0 ? 1u : 0u);
+            umma_f16(tmem + s * 64, make_desc(xa + ks * 2 * XCH, XCH, 128), make_desc(wk + whalf, 1024, 128), kI, 1u);
+            umma_f16(tmem + s * 64, make_desc(xa + kXHalf + ks * 2 * XCH, XCH, 128), make_desc(wk, 1024, 128), kI, 1u);
+          }
+          umma_commit(bars + 8 * (X_EMPTY0 + xs_));
+          if (j == nslice - 1) umma_commit(bars + 8 * (D_FULL0 + s));
+        }
+        __syncwarp();
+      }
+    }
+  } else {
+    const int q4 = warp & 3, chalf = warp >> 2;
+    const float* sb = reinterpret_cast<const float*>(smem + S_BIAS) + chalf * 32;
+    int g = 0;                                                  // slice count (ring position), as the MMA thread's
+    // all slices of tile t: a warp reads one pixel's 64 bands of the slice (two per lane), 8 pixels in flight per lane
+    auto load_tile = [&](int64_t t) {
+      const int64_t p0 = t * 128;
+      const T* src[16];
+#pragma unroll
+      for (int jj = 0; jj < 16; ++jj) {
+        int pp = int(p0) + warp + 8 * jj; if (pp >= int(plane)) pp = int(plane) - 1;     // plane < 2^31 (launcher)
+        const int pr = pp / pcol_n, pc = pp - pr * pcol_n;
+        const int sr = mirror_index(band_row0 + pr + lo, scene_rows) - slab_row0, sc = mirror_index(pc + lo, cols);
+        src[jj] = in + (int64_t(sr) * cols + sc) * K;
+      }
+#pragma unroll 1
+      for (int j = 0; j < nslice; ++j, ++g) {
+        const int s = g & 1;
+        mbar_wait(bars + 8 * (X_EMPTY0 + s), ((g >> 1) & 1) ^ 1, 92);
+        unsigned char* xs = smem + S_X + s * 2 * kXHalf;
+        const int k0 = j * kSlice + lane, k1 = k0 + 32;
+        const float m0 = smu[k0 < KP ? k0 : 0], i0 = k0 < KP ? sis[k0] : 0.f;
+        const float m1 = smu[k1 < KP ? k1 : 0], i1 = k1 < KP ? sis[k1] : 0.f;
+#pragma unroll
+        for (int h = 0; h < 16; h += 8) {
+          float v[8][2];
+#pragma unroll
+          for (int jj = 0; jj < 8; ++jj) {
+            v[jj][0] = k0 < K ? float(src[h + jj][k0]) : 0.f;
+            v[jj][1] = k1 < K ? float(src[h + jj][k1]) : 0.f;
+          }
+#pragma unroll
+          for (int jj = 0; jj < 8; ++jj) {
+            const int pos = warp + 8 * (h + jj);
+#pragma unroll
+            for (int m = 0; m < 2; ++m) {
+              const int kl = lane + 32 * m;                    // band within the slice
+              const float z = (v[jj][m] - (m ? m1 : m0)) * (m ? i1 : i0);       // 0 for k >= K
+              const __half hi = __float2half_rn(z);
+              unsigned char* d = xs + (kl >> 3) * XCH + pos * 16 + (kl & 7) * 2;
+              *reinterpret_cast<__half*>(d) = hi;
+              *reinterpret_cast<__half*>(d + kXHalf) = __float2half_rn(z - __half2float(hi));
+            }
+          }
+        }
+        fence_proxy_async();
+        mbar_arrive(bars + 8 * (X_FULL0 + s));
+      }
+    };
+    int it = 0;
+    if (t_first < ntiles) load_tile(t_first);
+    for (int64_t t = t_first; t < ntiles; t += t_step, ++it) {
+      if (t + t_step < ntiles) load_tile(t + t_step);           // its slices wait for the MMAs of this tile's last slices
+      const int s = it & 1;
+      mbar_wait(bars + 8 * (D_FULL0 + s), (it >> 1) & 1, 93);
+      tc_fence_after();
+      float v[32];
+      const uint32_t taddr = tmem + (uint32_t(q4 * 32) << 16) + s * 64 + chalf * 32;
+      tmem_ld16(taddr, v);
+      tmem_ld16(taddr + 16, v + 16);
+      tmem_ld_wait();
+      tc_fence_before();
+      mbar_arrive(bars + 8 * (D_EMPTY0 + s));
+      const int64_t p = t * 128 + q4 * 32 + lane;
+      if (p < plane) {
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          __half2 h[4];
+#pragma unroll
+          for (int j = 0; j < 4; ++j)
+            h[j] = __floats2half2_rn(v[c * 8 + 2 * j] + sb[c * 8 + 2 * j], v[c * 8 + 2 * j + 1] + sb[c * 8 + 2 * j + 1]);
+          *reinterpret_cast<uint4*>(f0pad + (int64_t(chalf * 4 + c) * plane + p) * 8) = *reinterpret_cast<uint4*>(h);
+        }
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 8) { tc_fence_after(); tmem_dealloc(tmem, 128); }
+}
+
+template <typename T>
+static int launch_conv0_tc_sliced(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0,
+                                  int prow_n, int pcol_n, const float* wt, const float* bias, const float* mu,
+                                  const float* inv_sigma, __half* f0pad, cudaStream_t s) {
+  const int KP = (K + 15) / 16 * 16;
+  CMLPL_CHECK_ARG(K <= c0k::kMaxK, "conv0: K=%d unsupported by the tensor-core kernel (at most %d)", K, c0k::kMaxK);
+  CMLPL_CHECK_ARG(mu && inv_sigma, "conv0: the K-sliced kernel needs the band means and 1/sigma");
+  const size_t smem = size_t(KP / 8) * 64 * 16 * 2 + 2 * 2 * c0k::kXHalf + 256 + 2 * size_t(KP) * 4 + 64 + 16 + 128;
+  CMLPL_CHECK_ARG(smem <= 227 * 1024, "conv0: K=%d does not fit shared memory", K);
+  auto kern = conv0_tc_sliced_kernel<T>;
+  CMLPL_MAX_DYN_SMEM(kern, int(smem));
+  const int64_t ntiles = (int64_t(prow_n) * pcol_n + 127) / 128;
+  int grid = sm_count();
+  if (grid > ntiles) grid = int(ntiles);
+  kern<<<grid, c0s::kThreads, smem, s>>>(in, K, KP, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
+                                         inv_sigma, f0pad);
+  CMLPL_CHECK_LAUNCH("conv0_tc_sliced");
+  return CMLPL_OK;
+}
+
 template <typename T, bool kVec4, bool kSplit>
 int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0, int prow_n, int pcol_n,
                     const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad, cudaStream_t s) {
   const int KP = (K + 15) / 16 * 16;
-  CMLPL_CHECK_ARG(KP <= 256 && (!kVec4 || (K % 4 == 0 && K <= 64)), "conv0: K=%d unsupported by the tensor-core kernel", K);
   CMLPL_CHECK_ARG(int64_t(prow_n) * pcol_n < (int64_t(1) << 31) - 256, "conv0: band of %d x %d padded positions is too large",
                   prow_n, pcol_n);
+  // beyond 256 bands (raw cube only) the X operand of a tile passes through shared memory in K-slices
+  if constexpr (kSplit && !kVec4)
+    if (KP > 256)
+      return launch_conv0_tc_sliced<T>(in, K, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
+                                       inv_sigma, f0pad, s);
+  CMLPL_CHECK_ARG(KP <= 256 && (!kVec4 || (K % 4 == 0 && K <= 64)), "conv0: K=%d unsupported by the tensor-core kernel", K);
   const int KC = KP / 8;
   const size_t xhalf = (size_t(KC) * 2064 + 127) / 128 * 128, mult = kSplit ? 2 : 1;
   const size_t fixed = size_t(KC) * 64 * 16 * mult + 256 + ((KP * 4 + 127) / 128) * 128 + 64 + 16 + 128;

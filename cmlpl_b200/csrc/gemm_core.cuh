@@ -14,6 +14,15 @@ struct StridedA {
   __device__ __forceinline__ void prep(int) {}
   __device__ __forceinline__ float at(int m, int k) const { return __ldg(p + m * rs + k * cs); }
 };
+// rows of the raw cube (uint16 / float32, row stride rs), z-scored on load: A(m,k) = (x[m][k] - mu[k]) * inv_sigma[k]
+template <typename T>
+struct RawZA {
+  const T* p; int64_t rs; const float* mu; const float* inv_sigma;
+  __device__ __forceinline__ void prep(int) {}
+  __device__ __forceinline__ float at(int m, int k) const {
+    return (float(__ldg(p + m * rs + k)) - __ldg(mu + k)) * __ldg(inv_sigma + k);
+  }
+};
 struct StridedB {  // B[k][n]
   const float* p; int64_t rs, cs;
   __device__ __forceinline__ float at(int n, int k) const { return __ldg(p + k * rs + n * cs); }

@@ -10,7 +10,8 @@
 //                    the avg-pool + conv columns of the classifier -> 25 class-partial maps (conv2_scene_sm100.cu)
 //   4. head          spectral columns of the classifier (models.py:150) + the pixel's 25 gathered conv
 //                    partials + bias, argmax (hyper_tools.py:426, first index wins ties)
-//   (<= 32 classes and <= 224 bands; otherwise the all-per-pixel patch_cnn_sm100.cu kernel + CUDA-core classify instead)
+//   (<= 32 classes and <= 224 bands; otherwise the all-per-pixel patch_cnn_sm100.cu kernel + CUDA-core classify instead,
+//   on both entry points; the raw entry point's CUDA-core spectral head reads the raw band, z-scored on load)
 #include "common.cuh"
 #include "gemm_core.cuh"
 
@@ -96,9 +97,12 @@ __global__ void argmax_kernel(const float* __restrict__ logits, int64_t n, int C
 }
 
 // Scene inference runs the tensor-core spectral branch (spectral_logits_kernel, head_sm100.cu) for <= 224 bands and <= 32
-// classes: on the dense path, and in path mode 0 for <= 16 classes or from the raw cube; otherwise the CUDA-core
-// spectral_head + classify kernels above run (same C ABI, same results contract).
+// classes: on the dense path, and in path mode 0 for <= 16 classes or from the raw cube; otherwise (beyond 224 bands on
+// either entry point, and in path mode 0 at 17-32 classes on the cube entry point) the CUDA-core spectral_head +
+// classify kernels below run (same C ABI, same results contract).
 static bool tc_spectral_fits(int B, int C) { return C <= 32 && ((B + 15) / 16) * 2 <= 28; }   // <= 224 bands
+// widest spectrum of the raw entry point (conv0_sm100.cu: the K-sliced kernel's resident weights)
+constexpr int kRawMaxBands = 512;
 
 // 1 (default): the exact-compute-sharing kernels where they apply; 0: the per-pixel tensor-core kernels everywhere (the
 // independent implementation the tests compare against).  Per host thread; the workspace layout follows the mode.
@@ -112,7 +116,7 @@ struct SceneWs {
 // tensor-core path: conv0 map, spectral tiles, partial spectral logits, pooled parity planes, the 9 half-pooled conv2
 // maps, the 5 class-partial row maps.  CUDA-core path: conv0 map, per-pixel pooled features, spectral logits, hidden
 // chunk.  Path mode 0 at 17-32 classes holds both spectral branches: the cube entry point runs the CUDA-core one, the raw
-// entry point (which has no other) the tensor-core one.
+// entry point the tensor-core one.  Beyond 224 bands both entry points run the CUDA-core one.
 static SceneWs scene_ws(int band_rows, int cols, int B, int C, int w) {
   SceneWs s;
   const int64_t n = int64_t(band_rows) * cols;
@@ -174,8 +178,9 @@ extern "C" int cmlpl_scene_workspace_layout(int band_rows, int cols, int num_fea
   return CMLPL_OK;
 }
 
-// Where a scene call reads the scene from.  The two entry points differ only in their first two launches, conv0 and the
-// spectral branch's conversion (and the raw entry point has no CUDA-core spectral head).
+// Where a scene call reads the scene from.  The two entry points differ only in their first two launches: conv0, and the
+// spectral branch's conversion or the CUDA-core spectral head's A operand (z-scored spectra, or the raw band z-scored on
+// load).
 struct SceneSrc {
   const char* fn;                          // the entry point, named in the error messages
   bool from_raw;
@@ -219,7 +224,8 @@ static int check_scene(const SceneSrc& src, int scene_rows, int cols, int slab_r
   CMLPL_CHECK_ARG(w == 20 || w == 11, "%s: w=%d unsupported (20, or 11 for the odd-window variant)", fn, w);
   CMLPL_CHECK_ARG(band_rows > 0 && cols > 0 && B > 0, "%s: bad dims (band_rows=%d cols=%d bands=%d)", fn, band_rows, cols, B);
   CMLPL_CHECK_ARG(C > 0 && C <= 32, "%s: needs 1..32 classes, got %d", fn, C);
-  CMLPL_CHECK_ARG(!src.from_raw || tc_spectral_fits(B, C), "%s: needs <= 224 bands, got %d", fn, B);
+  // the raw entry point: conv0 keeps the folded weights resident in shared memory as fp16 hi + lo, 128 KB at 512 bands
+  CMLPL_CHECK_ARG(!src.from_raw || B <= kRawMaxBands, "%s: needs <= %d bands, got %d", fn, kRawMaxBands, B);
   const int rc = check_band(fn, scene_rows, cols, slab_row0, slab_rows, w, band_row0, band_rows);
   if (rc != CMLPL_OK) return rc;
   CMLPL_CHECK_ARG(src.from_raw || reinterpret_cast<uintptr_t>(src.cube) % 16 == 0, "%s: cube must be 16-byte aligned", fn);
@@ -248,7 +254,9 @@ extern "C" int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, 
 
 // CUDA-core spectral head of the per-pixel path: spe_logits f32 [n][C] = Wc_spe . relu(Wspe . x + bspe), over chunks of
 // `chunk` pixels through the f32 scratch hidden [chunk][1024]
-static int spectral_head(const float* spectra, int64_t n, int num_features, int num_classes, int w, const void* packed,
+// `spectra` is StridedA over the z-scored f32 spectra, or RawZA over the raw band (z-scored on load); .p is advanced per chunk
+template <class FA>
+static int spectral_head(FA spectra, int64_t n, int num_features, int num_classes, int w, const void* packed,
                          float* hidden, int64_t chunk, float* spe_logits, cudaStream_t s) {
   const unsigned char* pk = static_cast<const unsigned char*>(packed);
   const PackedLayout L = packed_layout(num_features, num_classes, w);
@@ -258,8 +266,9 @@ static int spectral_head(const float* spectra, int64_t n, int num_features, int 
   for (int64_t s0 = 0; s0 < n; s0 += chunk) {
     const int m = int((n - s0) < chunk ? (n - s0) : chunk);
     // hidden = relu(X . Wspe^T + bspe)         (models.py:142-143)
-    int rc = launch_gemm(m, 1024, num_features, 1,
-                         StridedA{spectra + s0 * num_features, num_features, 1},
+    FA a = spectra;
+    a.p += s0 * num_features;
+    int rc = launch_gemm(m, 1024, num_features, 1, a,
                          StridedB{wspe, 1, num_features},
                          StridedC{hidden, 1024, 1, bspe, 1.f, 0.f, 1}, s, "spectral_hidden");
     if (rc != CMLPL_OK) return rc;
@@ -359,13 +368,23 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
     CMLPL_CUDA(cudaStreamWaitEvent(s, sd->join[0], 0));
     return cmlpl_head_sum_lmap(part, lmap, cols, band_rows, B, C, w, packed, labels, logits, stream);
   }
-  // per pixel: the tensor-core spectral branch, or the CUDA-core spectral head beyond 224 bands and in path mode 0 at
-  // 17-32 classes on the cube entry point (the raw entry point has only the tensor-core branch)
+  // per pixel: the tensor-core spectral branch; or the CUDA-core spectral head beyond 224 bands (both entry points) and in
+  // path mode 0 at 17-32 classes on the cube entry point, where the workspace holds both branches and the raw entry point
+  // runs the tensor-core one
   if ((rc = conv0()) != CMLPL_OK) return rc;
-  const bool tc = ws.tc || src.from_raw;
+  const bool tc = ws.tc || (src.from_raw && tc_spectral_fits(B, C));
   float* spe = reinterpret_cast<float*>(wsb + ws.spe);
-  rc = tc ? spectral_tc(s)
-          : spectral_head(src.spectra, n, B, C, w, packed, reinterpret_cast<float*>(wsb + ws.hidden), ws.chunk, spe, s);
+  float* hidden = reinterpret_cast<float*>(wsb + ws.hidden);
+  if (tc)
+    rc = spectral_tc(s);
+  else if (!src.from_raw)
+    rc = spectral_head(StridedA{src.spectra, B, 1}, n, B, C, w, packed, hidden, ws.chunk, spe, s);
+  else if (src.dtype == 0)
+    rc = spectral_head(RawZA<uint16_t>{static_cast<const uint16_t*>(band_spectra), B, src.mu, src.inv_sigma}, n, B, C, w,
+                       packed, hidden, ws.chunk, spe, s);
+  else
+    rc = spectral_head(RawZA<float>{static_cast<const float*>(band_spectra), B, src.mu, src.inv_sigma}, n, B, C, w, packed,
+                       hidden, ws.chunk, spe, s);
   if (rc != CMLPL_OK) return rc;
   if ((rc = cmlpl_patch_cnn_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.p2, stream)) != CMLPL_OK) return rc;
   return classify_launch(wsb + ws.p2, tc ? nullptr : spe, tc ? part : nullptr, ((n + 127) / 128) * 128, n, B, C, w, packed,

@@ -101,7 +101,16 @@ __device__ __forceinline__ uint4 philox_uniform4(unsigned long long seed, unsign
   return philox4x32_10(make_uint4(index, stream, uint32_t(offset), uint32_t(offset >> 32)),
                        make_uint2(uint32_t(seed), uint32_t(seed >> 32)));
 }
-enum { PHILOX_PATCH = 1, PHILOX_SPEC = 2, PHILOX_DROP = 3 };
+enum { PHILOX_PATCH = 1, PHILOX_SPEC = 2, PHILOX_DROP = 3, PHILOX_SPEC_HI = 4 };
+
+// Counter of the spectral noise of band quad j4 of sample s (four bands per draw).  Quads 0..63 keep the original
+// (PHILOX_SPEC, s*64 + j4), so every run up to 256 bands draws what it always drew; quad group g = j4 / 64 >= 1 (bands
+// 256..511) draws from its own stream PHILOX_SPEC_HI + g - 1 at s*64 + j4 % 64, disjoint from every other sample's
+// draws.  Valid up to 512 bands, the bound cmlpl_train_step checks.
+__device__ __forceinline__ uint2 spec_noise_counter(int s, int j4) {
+  const uint32_t g = uint32_t(j4) >> 6;
+  return make_uint2(g == 0 ? uint32_t(PHILOX_SPEC) : uint32_t(PHILOX_SPEC_HI) + g - 1u, uint32_t(s) * 64u + (uint32_t(j4) & 63u));
+}
 
 // power-of-two scale that puts gradients whose largest magnitude is `amax` near 2^12 in fp16 (max 65504, smallest
 // normal 6.1e-5): the data-gradient sums may grow by 2^4 and values 2^-26 below the maximum are still normal numbers

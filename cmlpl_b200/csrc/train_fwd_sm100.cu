@@ -84,7 +84,10 @@ train_conv0_kernel(Conv0Args a) {
     float* dst = a.ynoisy + int64_t(s) * a.bands;
     for (int j4 = tid; j4 * 4 < a.bands; j4 += THREADS) {
       float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (draw) z = philox_normal4(a.prm->seed, a.prm->offset, PHILOX_SPEC, uint32_t(s) * 64u + uint32_t(j4));
+      if (draw) {
+        const uint2 ctr = spec_noise_counter(s, j4);
+        z = philox_normal4(a.prm->seed, a.prm->offset, ctr.x, ctr.y);
+      }
       const float zz[4] = {z.x, z.y, z.z, z.w};
       for (int j = 0; j < 4 && j4 * 4 + j < a.bands; ++j) {
         const int b = j4 * 4 + j;

@@ -40,9 +40,11 @@ extern "C" int cmlpl_train_step(const cmlpl_train_io* io, int phases, cmlpl_stre
   CMLPL_CHECK_ARG(io, "train_step: null io");
   CMLPL_CHECK_ARG(io->w == 20 || io->w == 11, "train_step: w=%d unsupported (20 = the reference's BaseNet2, "
                   "tools/models.py:127; 11 = the odd window of ExtractPatches_for_base)", io->w);
-  CMLPL_CHECK_ARG(io->bs > 0 && io->btu > 0 && io->bands > 0 && io->bands <= 256 && io->classes > 0 && io->classes <= 32 &&
+  CMLPL_CHECK_ARG(io->bs > 0 && io->btu > 0 && io->bands > 0 && io->classes > 0 && io->classes <= 32 &&
                       io->queue > 0, "train_step: bad dims (bs=%d btu=%d bands=%d classes=%d queue=%d)", io->bs, io->btu,
                   io->bands, io->classes, io->queue);
+  // the spectral noise counter (train_common.cuh: spec_noise_counter) keeps its draws disjoint up to 512 bands
+  CMLPL_CHECK_ARG(io->bands <= 512, "train_step: needs <= 512 bands, got %d", io->bands);
   CMLPL_CHECK_ARG(io->params && io->work && io->spectra && io->labels && io->logits && io->feat && io->probs && io->mask &&
                       io->hist, "train_step: null pointer");
   CMLPL_CHECK_ARG(io->cube ? (io->pix != nullptr && io->scene_rows >= 10 && io->cols >= 10) : io->patch_noise != nullptr,

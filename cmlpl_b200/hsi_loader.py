@@ -14,7 +14,8 @@ import numpy as np
 import torch
 from torch.utils import data
 
-ROOTS = {1: "./dataset/PaviaU/", 2: "./dataset/Salinas/", 3: "./dataset/Houston/", 4: "./dataset/Indian_pines/"}
+ROOTS = {1: "./dataset/PaviaU/", 2: "./dataset/Salinas/", 3: "./dataset/Houston/", 4: "./dataset/Indian_pines/",
+         5: "./dataset/WHU_Hi_LongKou/", 6: "./dataset/WHU_Hi_HanChuan/", 7: "./dataset/WHU_Hi_HongHu/"}
 
 
 def _tile(arr, max_iters):

@@ -5,8 +5,8 @@
 * the PCA cube is stored once as ``XPCA.npy`` f32 [R,C,n_PC] (+ ``meta.npy`` = [w, R, C]) and the
   19.9 GB materialised ``XP.npy`` is only written with ``--materialize-xp`` (then through the device
   patch-gather kernel, chunked, bit-identical to hyper_tools.py:226-243);
-* ``--synthetic`` builds a PaviaU/Salinas/Houston/Indian-Pines *shaped* scene when the .mat files are
-  not available (they are not, offline).
+* ``--synthetic`` builds a PaviaU/Salinas/Houston/Indian-Pines/WHU-Hi *shaped* scene when the .mat files
+  are not available (they are not, offline).
 
 Splits reproduce sample_generation.py:43-65 exactly (numpy legacy seeds 2 and 0, the sorted
 ``set`` difference for ``unlabel_array``).
@@ -19,6 +19,11 @@ import os
 import numpy as np
 
 from .tools.hyper_tools import DATASETS, _MAT, PCANorm, _loadmat, featureNormalize
+
+
+# dataID -> the synth.SHAPES entry --synthetic builds
+SYNTHETIC = {1: "paviau", 2: "salinas", 3: "houston", 4: "indian_pines", 5: "whu_longkou", 6: "whu_hanchuan",
+             7: "whu_honghu"}
 
 
 def split_indices(Y, num_label):
@@ -44,8 +49,7 @@ def load_scene(dataID, root="./dataset/", synthetic=False, seed=1088):
     name, n_class, bands = DATASETS[dataID]
     if synthetic:
         from . import synth
-        shape = {1: synth.SHAPES["paviau"], 2: synth.SHAPES["salinas"], 3: synth.SHAPES["houston"],
-                 4: synth.SHAPES["indian_pines"]}[dataID]
+        shape = synth.SHAPES[SYNTHETIC[dataID]]
         return synth.synth_scene(*shape, seed=seed)
     fx, kx, fy, ky = _MAT[dataID]
     return _loadmat(os.path.join(root, fx))[kx], _loadmat(os.path.join(root, fy))[ky]

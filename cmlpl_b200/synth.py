@@ -9,6 +9,9 @@ SHAPES = {
     "indian_pines": (145, 145, 200, 16),
     "salinas": (512, 217, 204, 16),
     "houston": (349, 1905, 144, 15),
+    "whu_longkou": (550, 400, 270, 9),
+    "whu_hanchuan": (1217, 303, 274, 16),
+    "whu_honghu": (940, 475, 270, 22),
 }
 
 

@@ -12,11 +12,18 @@ import torch
 
 from .. import _lib, ops
 
-DATASETS = {1: ("PaviaU", 9, 103), 2: ("Salinas", 16, 204), 3: ("Houston", 15, 144), 4: ("Indian_pines", 16, 200)}
+# dataID -> (name, classes, bands).  5-7 are the WHU-Hi UAV scenes (LongKou 550 x 400, HanChuan 1217 x 303, HongHu
+# 940 x 475), wider than 256 bands
+DATASETS = {1: ("PaviaU", 9, 103), 2: ("Salinas", 16, 204), 3: ("Houston", 15, 144), 4: ("Indian_pines", 16, 200),
+            5: ("WHU_Hi_LongKou", 9, 270), 6: ("WHU_Hi_HanChuan", 16, 274), 7: ("WHU_Hi_HongHu", 22, 270)}
+# .mat file and variable names of the scene and of its ground truth (the WHU-Hi ones follow the public distribution)
 _MAT = {1: ("PaviaU.mat", "paviaU", "PaviaU_gt.mat", "paviaU_gt"),
         2: ("salinas.mat", "HSI_original", "salinas_gt.mat", "Data_gt"),
         3: ("Houston.mat", "Houston", "Houston_gt.mat", "Houston_gt"),
-        4: ("indian_pines_corrected.mat", "indian_pines_corrected", "indian_pines_gt.mat", "indian_pines_gt")}
+        4: ("indian_pines_corrected.mat", "indian_pines_corrected", "indian_pines_gt.mat", "indian_pines_gt"),
+        5: ("WHU_Hi_LongKou.mat", "WHU_Hi_LongKou", "WHU_Hi_LongKou_gt.mat", "WHU_Hi_LongKou_gt"),
+        6: ("WHU_Hi_HanChuan.mat", "WHU_Hi_HanChuan", "WHU_Hi_HanChuan_gt.mat", "WHU_Hi_HanChuan_gt"),
+        7: ("WHU_Hi_HongHu.mat", "WHU_Hi_HongHu", "WHU_Hi_HongHu_gt.mat", "WHU_Hi_HongHu_gt")}
 
 
 def _device():

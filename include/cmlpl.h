@@ -106,8 +106,9 @@ int cmlpl_l2norm_bwd_f32(const float* y, const float* norm, const float* dy, flo
  * spectral partials and takes the argmax.  This path takes up to 32 classes (class width 16 up to 16 classes, 32
  * beyond) and up to 224 bands.  The per-pixel path (patch_cnn_kernel: conv1 + conv2 per patch window staged in shared
  * memory, then the classifier heads) is the independent implementation selected by cmlpl_set_scene_path_mode(0); it
- * also serves > 224 bands in cmlpl_scene_infer, with the CUDA-core spectral head.  cmlpl_scene_infer / cmlpl_scene_infer_raw
- * refuse more than 32 classes, and cmlpl_scene_infer_raw more than 224 bands.
+ * also serves > 224 bands on both entry points, with the CUDA-core spectral head (cmlpl_scene_infer_raw reads it from
+ * the raw band, z-scored on load).  cmlpl_scene_infer / cmlpl_scene_infer_raw refuse more than 32 classes, and
+ * cmlpl_scene_infer_raw more than 512 bands.
  *
  * Packed weights: cmlpl_pack_basenet2() converts the reference state_dict tensors
  * (models.py:102-127: conv0/1/2.{weight,bias}, feat_spe.*, classifier.*) into the
@@ -150,10 +151,12 @@ int cmlpl_scene_infer(const float* cube, int scene_rows, int cols, int slab_row0
                       void* workspace, size_t workspace_bytes,
                       uint8_t* labels, float* logits, cmlpl_stream_t stream);
 
-/* The same from the RAW cube (dtype 0 = uint16, 1 = float32; <= 32 classes, <= 224 bands): the PCA
+/* The same from the RAW cube (dtype 0 = uint16, 1 = float32; <= 32 classes, <= 512 bands): the PCA
  * projection and both z-scores of tools/hyper_tools.py:285-292 are folded into conv0
- * (wf f32 [B][64] = (W0 . (U/s)^T)^T, bf f32 [64] = b0 - W0 . m/s) and into the fp16 conversion of the
- * spectral branch (mu, inv_sigma f32 [B]); neither the PCA cube nor the z-scored spectra touch HBM.
+ * (wf f32 [B][64] = (W0 . (U/s)^T)^T, bf f32 [64] = b0 - W0 . m/s) and into the spectral branch (mu, inv_sigma
+ * f32 [B]: the fp16 conversion of the tensor-core branch up to 224 bands, the operand loads of the CUDA-core spectral
+ * head beyond); neither the PCA cube nor the z-scored spectra touch HBM.  Above 256 bands conv0 streams each tile's
+ * bands through shared memory in 64-band slices.
  * raw [slab_rows*cols, B] holds scene rows slab_row0.. (halo included, like `cube` above). */
 int cmlpl_scene_infer_raw(const void* raw, int dtype, int scene_rows, int cols, int slab_row0, int slab_rows,
                           int num_features, int num_classes, int w, int band_row0, int band_rows,
@@ -347,7 +350,7 @@ typedef struct cmlpl_train_params {   /* lives in DEVICE memory; the host refres
 } cmlpl_train_params;
 
 typedef struct cmlpl_train_io {
-  int bs, btu, bands, classes, w, queue;      /* w = 20 or 11, classes <= 32, bands <= 256 */
+  int bs, btu, bands, classes, w, queue;      /* w = 20 or 11, classes <= 32, bands <= 512 */
   /* ---- inputs */
   const float* cube; int scene_rows, cols;    /* f32 [R, cols, 60] PCA cube, or NULL: patch_noise then HOLDS the input patches */
   const int64_t* pix;                         /* i64 [nb] raster pixel per row (both nets read the same pixels) */
