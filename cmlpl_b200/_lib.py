@@ -20,6 +20,7 @@ SIGNATURES = {
     "cmlpl_version": (I, []),
     "cmlpl_last_error": (c_char_p, []),
     "cmlpl_device_ok": (I, []),
+    "cmlpl_memcpy2d_async": (I, [P, Z, P, Z, Z, Z, P]),
     "cmlpl_patch_gather_f32": (I, [P, I, I, I, I, I, I, I, P, L, L, P, F, P, P]),
     "cmlpl_sgemm_f32": (I, [I, I, I, F, P, L, L, P, L, L, P, F, P, L, L, I, P]),
     "cmlpl_conv2d_f32": (I, [P, P, P, P, P, I, I, I, I, I, I, I, I, P]),
@@ -44,6 +45,7 @@ SIGNATURES = {
     "cmlpl_spectral_logits_tc": (I, [P, L, I, I, I, P, P, P, P]),
     "cmlpl_head_sum_lmap": (I, [P, P, I, I, I, I, I, P, P, P, P]),
     "cmlpl_argmax_u8": (I, [P, L, I, P, P]),
+    "cmlpl_preprocess_fit_cube_f64": (I, [P, I, I, I, I, P, P, P]),
     "cmlpl_preprocess_fit_f64": (I, [P, I, L, I, P, P, P]),
     "cmlpl_preprocess_apply": (I, [P, I, L, I, I, P, P, P, P, P, P, P]),
     "cmlpl_confusion_i64": (I, [P, P, L, I, P, P]),

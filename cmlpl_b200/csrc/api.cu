@@ -102,4 +102,15 @@ int cmlpl_device_ok(void) {
   return (major == 10 && minor == 0) ? 1 : 0;
 }
 
+int cmlpl_memcpy2d_async(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width_bytes, size_t height,
+                         cmlpl_stream_t stream) {
+  CMLPL_CHECK_ARG(dst && src, "memcpy2d_async: null pointer");
+  CMLPL_CHECK_ARG(width_bytes <= dpitch && width_bytes <= spitch, "memcpy2d_async: width %zu exceeds a pitch (%zu, %zu)",
+                  width_bytes, dpitch, spitch);
+  if (width_bytes == 0 || height == 0) return CMLPL_OK;
+  CMLPL_CUDA(cudaMemcpy2DAsync(dst, dpitch, src, spitch, width_bytes, height, cudaMemcpyDefault,
+                               static_cast<cudaStream_t>(stream)));
+  return CMLPL_OK;
+}
+
 }  // extern "C"

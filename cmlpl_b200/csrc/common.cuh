@@ -70,6 +70,34 @@ struct SideStream {
 // the current device's side stream, or nullptr if it cannot be created
 SideStream* side_stream();
 
+// Band-major raw slab (include/cmlpl.h: CMLPL_RAW_BIL / CMLPL_RAW_BSQ): the sample of slab row r, column c, band b is
+// at r * rs + c + b * bs (BIL: rs = B * cols, bs = cols; BSQ: rs = cols, bs = slab_rows * cols).
+struct BandMajor {
+  int cols;
+  int64_t rs, bs;
+};
+
+// The raw cube code (include/cmlpl.h): dtype = sample (CMLPL_RAW_U16 / F32 / I16) | interleave (CMLPL_RAW_BIP / BIL /
+// BSQ).  Bytes per sample:
+inline int raw_sample_bytes(int dtype) { return (dtype & 0x0f) == CMLPL_RAW_F32 ? 4 : 2; }
+// Checks a code and the alignment of the pointer `what` to its samples; `fn` names the entry point.  No CUDA call.
+inline int check_raw_code(const char* fn, const char* what, const void* p, int dtype) {
+  CMLPL_CHECK_ARG((dtype & ~0xff) == 0, "%s: dtype 0x%x has bits outside sample (0x0f) and interleave (0xf0)", fn,
+                  unsigned(dtype));
+  CMLPL_CHECK_ARG((dtype & 0x0f) <= CMLPL_RAW_I16, "%s: unknown sample type %d (0 = uint16, 1 = float32, 2 = int16)", fn,
+                  dtype & 0x0f);
+  CMLPL_CHECK_ARG((dtype & 0xf0) <= CMLPL_RAW_BSQ, "%s: unknown interleave 0x%x (0x00 = BIP, 0x10 = BIL, 0x20 = BSQ)", fn,
+                  unsigned(dtype & 0xf0));
+  CMLPL_CHECK_ARG(reinterpret_cast<uintptr_t>(p) % raw_sample_bytes(dtype) == 0, "%s: %s must be aligned to its %d-byte samples",
+                  fn, what, raw_sample_bytes(dtype));
+  return CMLPL_OK;
+}
+// Strides of a BIL / BSQ cube of B bands whose planes hold plane_rows rows of cols samples (BIP is not band-major)
+inline BandMajor band_major(int dtype, int B, int64_t plane_rows, int cols) {
+  return (dtype & 0xf0) == CMLPL_RAW_BSQ ? BandMajor{cols, int64_t(cols), plane_rows * cols}
+                                         : BandMajor{cols, int64_t(B) * cols, int64_t(cols)};
+}
+
 // a1 index map (tools/hyper_tools.py:35-55 == symmetric padding): single reflection.
 __host__ __device__ __forceinline__ int mirror_index(int o, int n) {
   return o < 0 ? -o - 1 : (o >= n ? 2 * n - 1 - o : o);

@@ -7,7 +7,8 @@
 // (mirrored index map, K contiguous values per pixel: fully coalesced), round to fp16 and write the UMMA K-major tile
 // [K/8 chunks][128 positions][8] straight into shared memory (two stages); one thread issues K/16 tcgen05.mma
 // (M=128, N=64) per tile into one of two TMEM slots; the same workers drain the previous tile (+bias -> fp16 -> F0,
-// 16-byte stores coalesced along positions) while their loads for the next tile are in flight.
+// 16-byte stores coalesced along positions) while their loads for the next tile are in flight.  A band-major raw slab
+// (BIL / BSQ) has its own loader: a thread owns one position and reads 8 bands per K-chunk, coalesced along columns.
 // Replaces the CUDA-core conv0_tiled_kernel of round 1 (L1-wavefront bound on the strided pixel rows).
 #include "common.cuh"
 #include "sm100_ptx.cuh"
@@ -22,14 +23,17 @@ enum { X_FULL0 = 0, X_EMPTY0 = 2, D_FULL0 = 4, D_EMPTY0 = 6 };
 // kSplit (raw cube): both operands are split into fp16 hi + lo parts and every K-step issues hi.hi + hi.lo + lo.hi
 // (~2^-21 relative error).  The folded PCA projection is ill-conditioned -- its noise components are differences of
 // band values ~10x larger than the result -- so single fp16 operands miss the 1e-3 logit bar (measured at B = 200).
-template <typename T, bool kVec4, bool kSplit>
-__global__ void __launch_bounds__(c0s::kThreads, 1)
-conv0_tc_kernel(const T* __restrict__ in, int K, int KP, int nstage, int scene_rows, int cols, int slab_row0, int w, int band_row0,
-                int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
-                const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad) {
+// kBM (raw cube, kSplit only): the slab is band-major (BIL / BSQ, addressed through bm) instead of pixel-major.  The
+// kernels read threadIdx.x and pass it in as tid, so the range their launch bounds give it still holds in the body.
+template <typename T, bool kVec4, bool kSplit, bool kBM>
+__device__ __forceinline__ void
+conv0_tc_body(const T* __restrict__ in, int K, int KP, int nstage, int scene_rows, int cols, int slab_row0, int w, int band_row0,
+              int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
+              const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad, BandMajor bm,
+              const int tid) {
   using namespace c0s;
   extern __shared__ __align__(128) unsigned char smem[];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem);
   const int KC = KP / 8;
   // X chunk planes are 2048 + 16 bytes apart (LBO = 2064): consecutive chunks start 16 B further along the banks, so
@@ -126,7 +130,47 @@ conv0_tc_kernel(const T* __restrict__ in, int K, int KP, int nstage, int scene_r
         const int sr = mirror_index(band_row0 + pr + lo, scene_rows) - slab_row0, sc = mirror_index(pc + lo, cols);
         return in + (int64_t(sr) * cols + sc) * K;
       };
-      if constexpr (kVec4) {
+      if constexpr (kBM) {
+        // band-major slab: a thread owns one of the tile's 128 positions and reads 8 consecutive bands per K-chunk (each
+        // load coalesced along the warp's consecutive columns), then stores the chunk as one 16-byte hi and one lo write.
+        // The z-score and the split are those of the pixel-major loader below, so the operand is the same byte for byte.
+        const int pos = tid & 127;
+        int pp = int(p0) + pos; if (pp >= int(plane)) pp = int(plane) - 1;
+        const int pr = pp / pcol_n, pc = pp - pr * pcol_n;
+        const int sr = mirror_index(band_row0 + pr + lo, scene_rows) - slab_row0, sc = mirror_index(pc + lo, cols);
+        const T* src = in + int64_t(sr) * bm.rs + sc;
+        const int kc_end = (K + 7) / 8;                         // chunks past it are K padding, written once above
+#pragma unroll 1
+        for (int c0 = tid >> 7; c0 < kc_end; c0 += 8) {        // 4 chunks (32 loads) in flight per thread
+          float v[4][8];
+#pragma unroll
+          for (int u = 0; u < 4; ++u)
+#pragma unroll
+            for (int e = 0; e < 8; ++e) {
+              const int k = (c0 + 2 * u) * 8 + e;
+              v[u][e] = k < K ? float(src[int64_t(k) * bm.bs]) : 0.f;
+            }
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            const int kc = c0 + 2 * u;
+            if (kc < kc_end) {
+              __half2 hi[4], lo2[4];
+#pragma unroll
+              for (int e = 0; e < 8; e += 2) {
+                const int k = kc * 8 + e;
+                const float z0 = k < K ? (v[u][e] - smu[k]) * __ldg(inv_sigma + k) : 0.f;
+                const float z1 = k + 1 < K ? (v[u][e + 1] - smu[k + 1]) * __ldg(inv_sigma + k + 1) : 0.f;
+                const __half h0 = __float2half_rn(z0), h1 = __float2half_rn(z1);
+                hi[e / 2] = __halves2half2(h0, h1);
+                lo2[e / 2] = __halves2half2(__float2half_rn(z0 - __half2float(h0)), __float2half_rn(z1 - __half2float(h1)));
+              }
+              unsigned char* d = xs + kc * XCH + pos * 16;
+              *reinterpret_cast<uint4*>(d) = *reinterpret_cast<const uint4*>(hi);
+              *reinterpret_cast<uint4*>(d + xhalf) = *reinterpret_cast<const uint4*>(lo2);
+            }
+          }
+        }
+      } else if constexpr (kVec4) {
         // K = 60 floats, 16-byte aligned pixels: a half-warp reads one pixel (15 float4 on 15 lanes), 8 pixels per lane
         // in flight; K % 4 == 0 and K <= 64
         const int hw = lane >> 4, q = lane & 15, Q = K / 4;
@@ -221,6 +265,26 @@ conv0_tc_kernel(const T* __restrict__ in, int K, int KP, int nstage, int scene_r
   if (warp == 8) { tc_fence_after(); tmem_dealloc(tmem, 128); }
 }
 
+template <typename T, bool kVec4, bool kSplit>
+__global__ void __launch_bounds__(c0s::kThreads, 1)
+conv0_tc_kernel(const T* __restrict__ in, int K, int KP, int nstage, int scene_rows, int cols, int slab_row0, int w, int band_row0,
+                int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
+                const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad) {
+  conv0_tc_body<T, kVec4, kSplit, false>(in, K, KP, nstage, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt,
+                                         bias, mu, inv_sigma, f0pad, BandMajor{}, threadIdx.x);
+}
+
+// the raw cube in BIL / BSQ (split operands)
+template <typename T>
+__global__ void __launch_bounds__(c0s::kThreads, 1)
+conv0_tc_bm_kernel(const T* __restrict__ in, int K, int KP, int nstage, int scene_rows, int cols, int slab_row0, int w,
+                   int band_row0, int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */,
+                   const float* __restrict__ bias, const float* __restrict__ mu, const float* __restrict__ inv_sigma,
+                   __half* __restrict__ f0pad, BandMajor bm) {
+  conv0_tc_body<T, false, true, true>(in, K, KP, nstage, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias,
+                                      mu, inv_sigma, f0pad, bm, threadIdx.x);
+}
+
 // K-sliced variant for the raw cube beyond 256 bands (split hi / lo operands only).  A tile's X operand no longer fits one
 // shared-memory stage, so it passes through a two-stage ring of 64-band slices [8 chunks][128 positions][8] (hi | lo):
 // the workers load and z-score slice j of a tile while the MMA thread consumes slice j-1, and the 3 x 4 tcgen05.mma of
@@ -233,15 +297,16 @@ constexpr int kXHalf = kSliceChunks * XCH;                    // one slice, hi o
 constexpr int kMaxK = 512;
 }  // namespace c0k
 
-template <typename T>
-__global__ void __launch_bounds__(c0s::kThreads, 1)
-conv0_tc_sliced_kernel(const T* __restrict__ in, int K, int KP, int scene_rows, int cols, int slab_row0, int w, int band_row0,
-                       int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
-                       const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad) {
+template <typename T, bool kBM>
+__device__ __forceinline__ void
+conv0_tc_sliced_body(const T* __restrict__ in, int K, int KP, int scene_rows, int cols, int slab_row0, int w, int band_row0,
+                     int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
+                     const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad,
+                     BandMajor bm, const int tid) {
   using namespace c0s;
   using c0k::kSlice; using c0k::XCH; using c0k::kXHalf;
   extern __shared__ __align__(128) unsigned char smem[];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem);
   const int KC = KP / 8, nslice = (KP + kSlice - 1) / kSlice;
   const int whalf = KC * 64 * 16;
@@ -322,46 +387,89 @@ conv0_tc_sliced_kernel(const T* __restrict__ in, int K, int KP, int scene_rows, 
     // all slices of tile t: a warp reads one pixel's 64 bands of the slice (two per lane), 8 pixels in flight per lane
     auto load_tile = [&](int64_t t) {
       const int64_t p0 = t * 128;
-      const T* src[16];
-#pragma unroll
-      for (int jj = 0; jj < 16; ++jj) {
-        int pp = int(p0) + warp + 8 * jj; if (pp >= int(plane)) pp = int(plane) - 1;     // plane < 2^31 (launcher)
+      if constexpr (kBM) {
+        // band-major slab: as in conv0_tc_kernel, a thread owns one position and reads 8 consecutive bands per K-chunk,
+        // 4 of a slice's 8 chunks; the z-score (0 for k >= K) and split are those of the pixel-major loader below
+        const int pos = tid & 127;
+        int pp = int(p0) + pos; if (pp >= int(plane)) pp = int(plane) - 1;
         const int pr = pp / pcol_n, pc = pp - pr * pcol_n;
         const int sr = mirror_index(band_row0 + pr + lo, scene_rows) - slab_row0, sc = mirror_index(pc + lo, cols);
-        src[jj] = in + (int64_t(sr) * cols + sc) * K;
-      }
+        const T* src = in + int64_t(sr) * bm.rs + sc;
 #pragma unroll 1
-      for (int j = 0; j < nslice; ++j, ++g) {
-        const int s = g & 1;
-        mbar_wait(bars + 8 * (X_EMPTY0 + s), ((g >> 1) & 1) ^ 1, 92);
-        unsigned char* xs = smem + S_X + s * 2 * kXHalf;
-        const int k0 = j * kSlice + lane, k1 = k0 + 32;
-        const float m0 = smu[k0 < KP ? k0 : 0], i0 = k0 < KP ? sis[k0] : 0.f;
-        const float m1 = smu[k1 < KP ? k1 : 0], i1 = k1 < KP ? sis[k1] : 0.f;
+        for (int j = 0; j < nslice; ++j, ++g) {
+          const int s = g & 1;
+          mbar_wait(bars + 8 * (X_EMPTY0 + s), ((g >> 1) & 1) ^ 1, 92);
+          unsigned char* xs = smem + S_X + s * 2 * kXHalf;
+          float v[4][8];
 #pragma unroll
-        for (int h = 0; h < 16; h += 8) {
-          float v[8][2];
+          for (int u = 0; u < 4; ++u)
 #pragma unroll
-          for (int jj = 0; jj < 8; ++jj) {
-            v[jj][0] = k0 < K ? float(src[h + jj][k0]) : 0.f;
-            v[jj][1] = k1 < K ? float(src[h + jj][k1]) : 0.f;
+            for (int e = 0; e < 8; ++e) {
+              const int k = j * kSlice + ((tid >> 7) + 2 * u) * 8 + e;
+              v[u][e] = k < K ? float(src[int64_t(k) * bm.bs]) : 0.f;
+            }
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            const int kl = ((tid >> 7) + 2 * u) * 8;             // first band of the chunk within the slice
+            __half2 hi[4], lo2[4];
+#pragma unroll
+            for (int e = 0; e < 8; e += 2) {
+              const int k = j * kSlice + kl + e;
+              const float z0 = (v[u][e] - smu[k < KP ? k : 0]) * (k < KP ? sis[k] : 0.f);
+              const float z1 = (v[u][e + 1] - smu[k + 1 < KP ? k + 1 : 0]) * (k + 1 < KP ? sis[k + 1] : 0.f);
+              const __half h0 = __float2half_rn(z0), h1 = __float2half_rn(z1);
+              hi[e / 2] = __halves2half2(h0, h1);
+              lo2[e / 2] = __halves2half2(__float2half_rn(z0 - __half2float(h0)), __float2half_rn(z1 - __half2float(h1)));
+            }
+            unsigned char* d = xs + (kl >> 3) * XCH + pos * 16;
+            *reinterpret_cast<uint4*>(d) = *reinterpret_cast<const uint4*>(hi);
+            *reinterpret_cast<uint4*>(d + kXHalf) = *reinterpret_cast<const uint4*>(lo2);
           }
+          fence_proxy_async();
+          mbar_arrive(bars + 8 * (X_FULL0 + s));
+        }
+      } else {
+        const T* src[16];
 #pragma unroll
-          for (int jj = 0; jj < 8; ++jj) {
-            const int pos = warp + 8 * (h + jj);
+        for (int jj = 0; jj < 16; ++jj) {
+          int pp = int(p0) + warp + 8 * jj; if (pp >= int(plane)) pp = int(plane) - 1;     // plane < 2^31 (launcher)
+          const int pr = pp / pcol_n, pc = pp - pr * pcol_n;
+          const int sr = mirror_index(band_row0 + pr + lo, scene_rows) - slab_row0, sc = mirror_index(pc + lo, cols);
+          src[jj] = in + (int64_t(sr) * cols + sc) * K;
+        }
+#pragma unroll 1
+        for (int j = 0; j < nslice; ++j, ++g) {
+          const int s = g & 1;
+          mbar_wait(bars + 8 * (X_EMPTY0 + s), ((g >> 1) & 1) ^ 1, 92);
+          unsigned char* xs = smem + S_X + s * 2 * kXHalf;
+          const int k0 = j * kSlice + lane, k1 = k0 + 32;
+          const float m0 = smu[k0 < KP ? k0 : 0], i0 = k0 < KP ? sis[k0] : 0.f;
+          const float m1 = smu[k1 < KP ? k1 : 0], i1 = k1 < KP ? sis[k1] : 0.f;
 #pragma unroll
-            for (int m = 0; m < 2; ++m) {
-              const int kl = lane + 32 * m;                    // band within the slice
-              const float z = (v[jj][m] - (m ? m1 : m0)) * (m ? i1 : i0);       // 0 for k >= K
-              const __half hi = __float2half_rn(z);
-              unsigned char* d = xs + (kl >> 3) * XCH + pos * 16 + (kl & 7) * 2;
-              *reinterpret_cast<__half*>(d) = hi;
-              *reinterpret_cast<__half*>(d + kXHalf) = __float2half_rn(z - __half2float(hi));
+          for (int h = 0; h < 16; h += 8) {
+            float v[8][2];
+#pragma unroll
+            for (int jj = 0; jj < 8; ++jj) {
+              v[jj][0] = k0 < K ? float(src[h + jj][k0]) : 0.f;
+              v[jj][1] = k1 < K ? float(src[h + jj][k1]) : 0.f;
+            }
+#pragma unroll
+            for (int jj = 0; jj < 8; ++jj) {
+              const int pos = warp + 8 * (h + jj);
+#pragma unroll
+              for (int m = 0; m < 2; ++m) {
+                const int kl = lane + 32 * m;                    // band within the slice
+                const float z = (v[jj][m] - (m ? m1 : m0)) * (m ? i1 : i0);       // 0 for k >= K
+                const __half hi = __float2half_rn(z);
+                unsigned char* d = xs + (kl >> 3) * XCH + pos * 16 + (kl & 7) * 2;
+                *reinterpret_cast<__half*>(d) = hi;
+                *reinterpret_cast<__half*>(d + kXHalf) = __float2half_rn(z - __half2float(hi));
+              }
             }
           }
+          fence_proxy_async();
+          mbar_arrive(bars + 8 * (X_FULL0 + s));
         }
-        fence_proxy_async();
-        mbar_arrive(bars + 8 * (X_FULL0 + s));
       }
     };
     int it = 0;
@@ -397,28 +505,57 @@ conv0_tc_sliced_kernel(const T* __restrict__ in, int K, int KP, int scene_rows, 
 }
 
 template <typename T>
+__global__ void __launch_bounds__(c0s::kThreads, 1)
+conv0_tc_sliced_kernel(const T* __restrict__ in, int K, int KP, int scene_rows, int cols, int slab_row0, int w, int band_row0,
+                       int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
+                       const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad) {
+  conv0_tc_sliced_body<T, false>(in, K, KP, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu, inv_sigma,
+                                 f0pad, BandMajor{}, threadIdx.x);
+}
+
+// the raw cube in BIL / BSQ
+template <typename T>
+__global__ void __launch_bounds__(c0s::kThreads, 1)
+conv0_tc_sliced_bm_kernel(const T* __restrict__ in, int K, int KP, int scene_rows, int cols, int slab_row0, int w,
+                          int band_row0, int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */,
+                          const float* __restrict__ bias, const float* __restrict__ mu, const float* __restrict__ inv_sigma,
+                          __half* __restrict__ f0pad, BandMajor bm) {
+  conv0_tc_sliced_body<T, true>(in, K, KP, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu, inv_sigma,
+                                f0pad, bm, threadIdx.x);
+}
+
+template <typename T>
 static int launch_conv0_tc_sliced(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0,
                                   int prow_n, int pcol_n, const float* wt, const float* bias, const float* mu,
-                                  const float* inv_sigma, __half* f0pad, cudaStream_t s) {
+                                  const float* inv_sigma, __half* f0pad, const BandMajor* bm, cudaStream_t s) {
   const int KP = (K + 15) / 16 * 16;
   CMLPL_CHECK_ARG(K <= c0k::kMaxK, "conv0: K=%d unsupported by the tensor-core kernel (at most %d)", K, c0k::kMaxK);
   CMLPL_CHECK_ARG(mu && inv_sigma, "conv0: the K-sliced kernel needs the band means and 1/sigma");
   const size_t smem = size_t(KP / 8) * 64 * 16 * 2 + 2 * 2 * c0k::kXHalf + 256 + 2 * size_t(KP) * 4 + 64 + 16 + 128;
   CMLPL_CHECK_ARG(smem <= 227 * 1024, "conv0: K=%d does not fit shared memory", K);
-  auto kern = conv0_tc_sliced_kernel<T>;
-  CMLPL_MAX_DYN_SMEM(kern, int(smem));
   const int64_t ntiles = (int64_t(prow_n) * pcol_n + 127) / 128;
   int grid = sm_count();
   if (grid > ntiles) grid = int(ntiles);
-  kern<<<grid, c0s::kThreads, smem, s>>>(in, K, KP, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
-                                         inv_sigma, f0pad);
+  if (bm) {
+    auto kern = conv0_tc_sliced_bm_kernel<T>;
+    CMLPL_MAX_DYN_SMEM(kern, int(smem));
+    kern<<<grid, c0s::kThreads, smem, s>>>(in, K, KP, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
+                                           inv_sigma, f0pad, *bm);
+  } else {
+    auto kern = conv0_tc_sliced_kernel<T>;
+    CMLPL_MAX_DYN_SMEM(kern, int(smem));
+    kern<<<grid, c0s::kThreads, smem, s>>>(in, K, KP, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
+                                           inv_sigma, f0pad);
+  }
   CMLPL_CHECK_LAUNCH("conv0_tc_sliced");
   return CMLPL_OK;
 }
 
+// bm: the raw slab is band-major (BIL / BSQ; split operands only), or nullptr for pixel-major
 template <typename T, bool kVec4, bool kSplit>
 int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0, int prow_n, int pcol_n,
-                    const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad, cudaStream_t s) {
+                    const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad,
+                    const BandMajor* bm, cudaStream_t s) {
   const int KP = (K + 15) / 16 * 16;
   CMLPL_CHECK_ARG(int64_t(prow_n) * pcol_n < (int64_t(1) << 31) - 256, "conv0: band of %d x %d padded positions is too large",
                   prow_n, pcol_n);
@@ -426,7 +563,8 @@ int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0,
   if constexpr (kSplit && !kVec4)
     if (KP > 256)
       return launch_conv0_tc_sliced<T>(in, K, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
-                                       inv_sigma, f0pad, s);
+                                       inv_sigma, f0pad, bm, s);
+  CMLPL_CHECK_ARG(!bm || (kSplit && !kVec4), "conv0: band-major input needs the split-operand kernel");
   CMLPL_CHECK_ARG(KP <= 256 && (!kVec4 || (K % 4 == 0 && K <= 64)), "conv0: K=%d unsupported by the tensor-core kernel", K);
   const int KC = KP / 8;
   const size_t xhalf = (size_t(KC) * 2064 + 127) / 128 * 128, mult = kSplit ? 2 : 1;
@@ -434,22 +572,34 @@ int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0,
   const int nstage = fixed + 2 * xhalf * mult <= 227 * 1024 ? 2 : 1;
   const size_t smem = fixed + nstage * xhalf * mult;
   CMLPL_CHECK_ARG(smem <= 227 * 1024, "conv0: K=%d does not fit shared memory", K);
-  auto kern = conv0_tc_kernel<T, kVec4, kSplit>;
-  CMLPL_MAX_DYN_SMEM(kern, int(smem));
   const int64_t ntiles = (int64_t(prow_n) * pcol_n + 127) / 128;
   int grid = sm_count();
   if (grid > ntiles) grid = int(ntiles);
+  if constexpr (kSplit && !kVec4) {
+    if (bm) {
+      auto kern = conv0_tc_bm_kernel<T>;
+      CMLPL_MAX_DYN_SMEM(kern, int(smem));
+      kern<<<grid, c0s::kThreads, smem, s>>>(in, K, KP, nstage, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt,
+                                             bias, mu, inv_sigma, f0pad, *bm);
+      CMLPL_CHECK_LAUNCH("conv0_tc_bm");
+      return CMLPL_OK;
+    }
+  }
+  auto kern = conv0_tc_kernel<T, kVec4, kSplit>;
+  CMLPL_MAX_DYN_SMEM(kern, int(smem));
   kern<<<grid, c0s::kThreads, smem, s>>>(in, K, KP, nstage, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
                                          inv_sigma, f0pad);
   CMLPL_CHECK_LAUNCH("conv0_tc");
   return CMLPL_OK;
 }
 
-template int launch_conv0_tc<float, true, false>(const float*, int, int, int, int, int, int, int, int, const float*, const float*,
-                                                 const float*, const float*, __half*, cudaStream_t);
-template int launch_conv0_tc<float, false, true>(const float*, int, int, int, int, int, int, int, int, const float*, const float*,
-                                                 const float*, const float*, __half*, cudaStream_t);
-template int launch_conv0_tc<uint16_t, false, true>(const uint16_t*, int, int, int, int, int, int, int, int, const float*,
-                                                    const float*, const float*, const float*, __half*, cudaStream_t);
+#define CMLPL_CONV0_INST(T, kVec4, kSplit)                                                                                 \
+  template int launch_conv0_tc<T, kVec4, kSplit>(const T*, int, int, int, int, int, int, int, int, const float*, const float*, \
+                                                 const float*, const float*, __half*, const BandMajor*, cudaStream_t);
+CMLPL_CONV0_INST(float, true, false)
+CMLPL_CONV0_INST(float, false, true)
+CMLPL_CONV0_INST(uint16_t, false, true)
+CMLPL_CONV0_INST(int16_t, false, true)
+#undef CMLPL_CONV0_INST
 
 }  // namespace cmlpl

@@ -23,6 +23,20 @@ struct RawZA {
     return (float(__ldg(p + m * rs + k)) - __ldg(mu + k)) * __ldg(inv_sigma + k);
   }
 };
+// the same from a band-major raw slab (BIL / BSQ): pixel m0 + m of the band is row (m0 + m) / cols, column
+// (m0 + m) % cols of the band's rows at p; the k order is RawZA's
+template <typename T>
+struct RawBandZA {
+  const T* p; BandMajor bm; int64_t m0; const float* mu; const float* inv_sigma;
+  int64_t off_;
+  __device__ __forceinline__ void prep(int m) {
+    const int64_t q = m0 + m, r = q / bm.cols;
+    off_ = r * bm.rs + (q - r * bm.cols);
+  }
+  __device__ __forceinline__ float at(int, int k) const {
+    return (float(__ldg(p + off_ + k * bm.bs)) - __ldg(mu + k)) * __ldg(inv_sigma + k);
+  }
+};
 struct StridedB {  // B[k][n]
   const float* p; int64_t rs, cs;
   __device__ __forceinline__ float at(int n, int k) const { return __ldg(p + k * rs + n * cs); }

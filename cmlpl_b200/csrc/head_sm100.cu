@@ -53,6 +53,31 @@ __global__ void x16_tile_raw_kernel(const T* __restrict__ X, int64_t n, int B, i
   }
 }
 
+// same from a band-major raw slab (BIL / BSQ, include/cmlpl.h): pixel p of the band is row p / cols, column p % cols of
+// the band's rows at X; with rows as the fastest index, a warp's loads of one band are consecutive columns
+template <typename T>
+__global__ void x16_tile_raw_bm_kernel(const T* __restrict__ X, BandMajor bm, int64_t n, int B, int KC, int64_t total,
+                                       const float* __restrict__ mu, const float* __restrict__ inv_sigma,
+                                       __half* __restrict__ out) {
+  for (int64_t t = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; t < total; t += int64_t(gridDim.x) * blockDim.x) {
+    const int row = int(t & 127);
+    const int64_t r = t >> 7;
+    const int kc = int(r % KC);
+    const int64_t p = (r / KC) * 128 + row;
+    const int64_t pr = p / bm.cols;
+    const T* x = X + pr * bm.rs + (p - pr * bm.cols);
+    __half2 h[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const int k = kc * 8 + 2 * e;
+      const float a = (p < n && k < B) ? (float(x[k * bm.bs]) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
+      const float b = (p < n && k + 1 < B) ? (float(x[(k + 1) * bm.bs]) - __ldg(mu + k + 1)) * __ldg(inv_sigma + k + 1) : 0.f;
+      h[e] = __floats2half2_rn(a, b);
+    }
+    *reinterpret_cast<uint4*>(out + t * 8) = *reinterpret_cast<uint4*>(h);
+  }
+}
+
 // ------------------------------------------------------------------ spectral logits: Wc_spe . relu(Wspe . x + b), hidden never in HBM
 // spectral_logits_kernel fuses the two GEMMs of the spectral branch (models.py:142-143 and the spectral columns of
 // models.py:150): a CTA owns one quarter (256) of the 1024 hidden features and walks pixel tiles of 128.
@@ -338,9 +363,11 @@ static bool spectral_logits_plan(int KC, int NC, int* nA, size_t* smem) {
 }
 
 // x16_tile(_raw) + spectral_logits_kernel: x16 is scratch for the fp16 input tiles, part f32 [4][ceil(n/128)*128][NC].
-int launch_spectral_logits(const void* x, int dtype /* -1 = preprocessed f32 spectra */, int64_t n, int num_features,
-                           int num_classes, int w, const float* mu, const float* inv_sigma, const void* packed, void* x16,
-                           float* part, cmlpl_stream_t stream) {
+// dtype: -1 = preprocessed f32 spectra, else the raw sample type (CMLPL_RAW_U16 / F32 / I16); bm: band-major raw rows, or
+// nullptr for pixel-major [n][B]
+int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_t n, int num_features, int num_classes,
+                           int w, const float* mu, const float* inv_sigma, const void* packed, void* x16, float* part,
+                           cmlpl_stream_t stream) {
   CMLPL_CHECK_ARG(x && packed && x16 && part, "spectral_logits_tc: null pointer");
   CMLPL_CHECK_ARG(n > 0 && num_features > 0, "spectral_logits_tc: bad dims");
   CMLPL_CHECK_ARG(num_classes <= 32, "spectral_logits_tc: needs <= 32 classes, got %d", num_classes);
@@ -351,12 +378,21 @@ int launch_spectral_logits(const void* x, int dtype /* -1 = preprocessed f32 spe
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const int64_t mtiles = (n + 127) / 128, total = mtiles * KC * 128;
   int64_t g = (total + 255) / 256; const int64_t cap = int64_t(sm_count()) * 16; if (g > cap) g = cap;
+  __half* o = static_cast<__half*>(x16);
   if (dtype < 0)
-    x16_tile_kernel<<<int(g), 256, 0, s>>>(static_cast<const float*>(x), n, num_features, KC, total, static_cast<__half*>(x16));
-  else if (dtype == 0)
-    x16_tile_raw_kernel<uint16_t><<<int(g), 256, 0, s>>>(static_cast<const uint16_t*>(x), n, num_features, KC, total, mu, inv_sigma, static_cast<__half*>(x16));
+    x16_tile_kernel<<<int(g), 256, 0, s>>>(static_cast<const float*>(x), n, num_features, KC, total, o);
+  else if (bm && dtype == CMLPL_RAW_U16)
+    x16_tile_raw_bm_kernel<uint16_t><<<int(g), 256, 0, s>>>(static_cast<const uint16_t*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, o);
+  else if (bm && dtype == CMLPL_RAW_I16)
+    x16_tile_raw_bm_kernel<int16_t><<<int(g), 256, 0, s>>>(static_cast<const int16_t*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, o);
+  else if (bm)
+    x16_tile_raw_bm_kernel<float><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, o);
+  else if (dtype == CMLPL_RAW_U16)
+    x16_tile_raw_kernel<uint16_t><<<int(g), 256, 0, s>>>(static_cast<const uint16_t*>(x), n, num_features, KC, total, mu, inv_sigma, o);
+  else if (dtype == CMLPL_RAW_I16)
+    x16_tile_raw_kernel<int16_t><<<int(g), 256, 0, s>>>(static_cast<const int16_t*>(x), n, num_features, KC, total, mu, inv_sigma, o);
   else
-    x16_tile_raw_kernel<float><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), n, num_features, KC, total, mu, inv_sigma, static_cast<__half*>(x16));
+    x16_tile_raw_kernel<float><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), n, num_features, KC, total, mu, inv_sigma, o);
   CMLPL_CHECK_LAUNCH("x16_tile");
   int grid = sm_count() / 4 * 4;
   if (grid > mtiles * 4) grid = int(mtiles * 4);
@@ -384,7 +420,7 @@ int launch_spectral_logits(const void* x, int dtype /* -1 = preprocessed f32 spe
 // scratch for the fp16 input tiles.
 extern "C" int cmlpl_spectral_logits_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
                                         const void* packed, void* x16, float* part, cmlpl_stream_t stream) {
-  return launch_spectral_logits(spectra, -1, n, num_features, num_classes, w, nullptr, nullptr, packed, x16, part, stream);
+  return launch_spectral_logits(spectra, -1, nullptr, n, num_features, num_classes, w, nullptr, nullptr, packed, x16, part, stream);
 }
 
 // Head of the dense path without a GEMM: quarter partials of cmlpl_spectral_logits_tc + the 5 gathered conv partials

@@ -25,14 +25,18 @@ namespace cmlpl {
 // logit bar).  PCA projection, both z-scores and conv0 are per-pixel affine maps, so they fold into one
 // F0 = Wf . (x - mu) + bf with Wf = W0 . (U/s)^T [64 x B] (SURVEY 8-f1).  Output: mirrored halo baked in, chunk-planar fp16
 // [8 chunks][prow_n][pcol_n][8].
+// bm: a band-major raw slab (BIL / BSQ), or nullptr for pixel-major
 template <typename T, bool kVec4, bool kSplit>
 int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0, int prow_n, int pcol_n,
-                    const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad, cudaStream_t s);
+                    const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad,
+                    const BandMajor* bm, cudaStream_t s);
 
 // x16_tile(_raw) + spectral_logits_kernel (head_sm100.cu): x is the f32 z-scored spectra (dtype -1) or the raw cube's
-// rows (dtype 0 = uint16, 1 = float32, z-scored with mu / inv_sigma in the conversion)
-int launch_spectral_logits(const void* x, int dtype, int64_t n, int num_features, int num_classes, int w, const float* mu,
-                           const float* inv_sigma, const void* packed, void* x16, float* part, cmlpl_stream_t stream);
+// rows (dtype = the sample type CMLPL_RAW_U16 / F32 / I16, z-scored with mu / inv_sigma in the conversion; band-major
+// through bm, else pixel-major)
+int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_t n, int num_features, int num_classes,
+                           int w, const float* mu, const float* inv_sigma, const void* packed, void* x16, float* part,
+                           cmlpl_stream_t stream);
 
 // ------------------------------------------------------------------ classifier + argmax
 // one warp per pixel; lanes stride over the K = P*64 pooled features in 8-half chunks.
@@ -186,7 +190,7 @@ struct SceneSrc {
   bool from_raw;
   const float* cube;                       // cmlpl_scene_infer: the PCA cube slab and the band's z-scored spectra
   const float* spectra;
-  const void* raw;                         // cmlpl_scene_infer_raw: the raw slab (dtype 0 = uint16, 1 = float32) and the
+  const void* raw;                         // cmlpl_scene_infer_raw: the raw slab (dtype = sample | interleave) and the
   int dtype;                               // preprocessing folded into conv0 and into the spectral branch (include/cmlpl.h)
   const float *wf, *bf, *mu, *inv_sigma;
 };
@@ -216,7 +220,10 @@ static int check_scene(const SceneSrc& src, int scene_rows, int cols, int slab_r
   CMLPL_CHECK_ARG(packed && workspace && labels &&
                       (src.from_raw ? src.raw && src.wf && src.bf && src.mu && src.inv_sigma : src.cube && src.spectra),
                   "%s: null pointer", fn);
-  CMLPL_CHECK_ARG(!src.from_raw || src.dtype == 0 || src.dtype == 1, "%s: dtype must be 0 (uint16) or 1 (float32)", fn);
+  if (src.from_raw) {
+    const int rc = check_raw_code(fn, "raw", src.raw, src.dtype);
+    if (rc != CMLPL_OK) return rc;
+  }
   // w = 20: the reference's BaseNet2 (classifier hard-wired to 2624 inputs, tools/models.py:127).  w = 11: the odd-window
   // variant BASELINE configs[4] names (ExtractPatches_for_base windows, hyper_tools.py:300-317; pooled 5 -> 2, classifier
   // over 64*2*2 + 1024 = 1280 inputs) -- a documented extension; its border classes and pooled cells are a subset of the
@@ -249,12 +256,14 @@ extern "C" int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, 
   const int prow_n = band_rows + w - 1, pcol_n = cols + w - 1;
   return launch_conv0_tc<float, true, false>(cube, 60, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n,
                                       reinterpret_cast<const float*>(pk + L.w0), reinterpret_cast<const float*>(pk + L.b0), nullptr,
-                                      nullptr, static_cast<__half*>(f0pad), static_cast<cudaStream_t>(stream));
+                                      nullptr, static_cast<__half*>(f0pad), nullptr, static_cast<cudaStream_t>(stream));
 }
 
 // CUDA-core spectral head of the per-pixel path: spe_logits f32 [n][C] = Wc_spe . relu(Wspe . x + bspe), over chunks of
 // `chunk` pixels through the f32 scratch hidden [chunk][1024]
-// `spectra` is StridedA over the z-scored f32 spectra, or RawZA over the raw band (z-scored on load); .p is advanced per chunk
+// `spectra` is StridedA over the z-scored f32 spectra, or RawZA / RawBandZA over the raw band (z-scored on load)
+template <class FA> static FA rows_from(FA a, int64_t s0) { a.p += s0 * a.rs; return a; }          // pixel-major rows
+template <typename T> static RawBandZA<T> rows_from(RawBandZA<T> a, int64_t s0) { a.m0 += s0; return a; }
 template <class FA>
 static int spectral_head(FA spectra, int64_t n, int num_features, int num_classes, int w, const void* packed,
                          float* hidden, int64_t chunk, float* spe_logits, cudaStream_t s) {
@@ -266,9 +275,7 @@ static int spectral_head(FA spectra, int64_t n, int num_features, int num_classe
   for (int64_t s0 = 0; s0 < n; s0 += chunk) {
     const int m = int((n - s0) < chunk ? (n - s0) : chunk);
     // hidden = relu(X . Wspe^T + bspe)         (models.py:142-143)
-    FA a = spectra;
-    a.p += s0 * num_features;
-    int rc = launch_gemm(m, 1024, num_features, 1, a,
+    int rc = launch_gemm(m, 1024, num_features, 1, rows_from(spectra, s0),
                          StridedB{wspe, 1, num_features},
                          StridedC{hidden, 1024, 1, bspe, 1.f, 0.f, 1}, s, "spectral_hidden");
     if (rc != CMLPL_OK) return rc;
@@ -328,12 +335,18 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const int64_t n = int64_t(band_rows) * cols;
   float* part = reinterpret_cast<float*>(wsb + ws.h16);
-  // the tensor-core spectral branch reads the band's z-scored spectra, or the band's rows of the raw slab
+  // the raw slab: sample type, and for BIL / BSQ its band-major strides (pixel-major BIP has row stride cols * B)
+  const int sample = src.dtype & 0x0f, il = src.dtype & 0xf0;
+  const BandMajor bmv = band_major(src.dtype, B, slab_rows, cols);
+  const BandMajor* bm = src.from_raw && il != CMLPL_RAW_BIP ? &bmv : nullptr;
+  // the spectral branch reads the band's z-scored spectra, or the band's rows of the raw slab: in every interleave they
+  // start band_row0 - slab_row0 rows (of cols * B samples; of cols samples in every plane for BSQ) into the slab
+  const int64_t row_stride = bm ? bm->rs : int64_t(cols) * B;
   const void* band_spectra =
-      src.from_raw ? static_cast<const unsigned char*>(src.raw) + size_t(band_row0 - slab_row0) * cols * B * (src.dtype == 0 ? 2 : 4)
+      src.from_raw ? static_cast<const unsigned char*>(src.raw) + (band_row0 - slab_row0) * row_stride * raw_sample_bytes(src.dtype)
                    : static_cast<const void*>(src.spectra);
   auto spectral_tc = [&](cudaStream_t st) {
-    return launch_spectral_logits(band_spectra, src.from_raw ? src.dtype : -1, n, B, C, w, src.mu, src.inv_sigma, packed,
+    return launch_spectral_logits(band_spectra, src.from_raw ? sample : -1, bm, n, B, C, w, src.mu, src.inv_sigma, packed,
                                   wsb + ws.x16, part, st);
   };
   auto conv0 = [&]() {
@@ -342,11 +355,14 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
                                  wsb + ws.f0pad, stream);
     const int prow_n = band_rows + w - 1, pcol_n = cols + w - 1;
     __half* f0 = reinterpret_cast<__half*>(wsb + ws.f0pad);
-    return src.dtype == 0
-        ? launch_conv0_tc<uint16_t, false, true>(static_cast<const uint16_t*>(src.raw), B, scene_rows, cols, slab_row0, w,
-                                                 band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, s)
-        : launch_conv0_tc<float, false, true>(static_cast<const float*>(src.raw), B, scene_rows, cols, slab_row0, w,
-                                              band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, s);
+    if (sample == CMLPL_RAW_U16)
+      return launch_conv0_tc<uint16_t, false, true>(static_cast<const uint16_t*>(src.raw), B, scene_rows, cols, slab_row0, w,
+                                                    band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, s);
+    if (sample == CMLPL_RAW_I16)
+      return launch_conv0_tc<int16_t, false, true>(static_cast<const int16_t*>(src.raw), B, scene_rows, cols, slab_row0, w,
+                                                   band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, s);
+    return launch_conv0_tc<float, false, true>(static_cast<const float*>(src.raw), B, scene_rows, cols, slab_row0, w,
+                                               band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, s);
   };
   if (ws.dense) {
     // The spectral branch (fp16 tiles of the spectra + the two spectral GEMMs) does not depend on the conv tower until
@@ -375,16 +391,23 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
   const bool tc = ws.tc || (src.from_raw && tc_spectral_fits(B, C));
   float* spe = reinterpret_cast<float*>(wsb + ws.spe);
   float* hidden = reinterpret_cast<float*>(wsb + ws.hidden);
+  // the CUDA-core spectral head's A operand from the raw band: z-scored on load, pixel-major or band-major
+  auto raw_head = [&](auto sample_type) {
+    using T = decltype(sample_type);
+    const T* x = static_cast<const T*>(band_spectra);
+    return bm ? spectral_head(RawBandZA<T>{x, *bm, 0, src.mu, src.inv_sigma, 0}, n, B, C, w, packed, hidden, ws.chunk, spe, s)
+              : spectral_head(RawZA<T>{x, B, src.mu, src.inv_sigma}, n, B, C, w, packed, hidden, ws.chunk, spe, s);
+  };
   if (tc)
     rc = spectral_tc(s);
   else if (!src.from_raw)
     rc = spectral_head(StridedA{src.spectra, B, 1}, n, B, C, w, packed, hidden, ws.chunk, spe, s);
-  else if (src.dtype == 0)
-    rc = spectral_head(RawZA<uint16_t>{static_cast<const uint16_t*>(band_spectra), B, src.mu, src.inv_sigma}, n, B, C, w,
-                       packed, hidden, ws.chunk, spe, s);
+  else if (sample == CMLPL_RAW_U16)
+    rc = raw_head(uint16_t{});
+  else if (sample == CMLPL_RAW_I16)
+    rc = raw_head(int16_t{});
   else
-    rc = spectral_head(RawZA<float>{static_cast<const float*>(band_spectra), B, src.mu, src.inv_sigma}, n, B, C, w, packed,
-                       hidden, ws.chunk, spe, s);
+    rc = raw_head(float{});
   if (rc != CMLPL_OK) return rc;
   if ((rc = cmlpl_patch_cnn_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.p2, stream)) != CMLPL_OK) return rc;
   return classify_launch(wsb + ws.p2, tc ? nullptr : spe, tc ? part : nullptr, ((n + 127) / 128) * 128, n, B, C, w, packed,
@@ -402,9 +425,9 @@ extern "C" int cmlpl_scene_infer(const float* cube, int scene_rows, int cols, in
 
 
 // ---------------------------------------------------------------------------------------------
-// Scene inference from the RAW cube (uint16 / float32): the preprocessing of
+// Scene inference from the RAW cube (uint16 / float32 / int16; BIP, BIL or BSQ): the preprocessing of
 // tools/hyper_tools.py:285-292 is folded into the first kernels (no PCA cube / z-scored spectra in HBM).
-//   raw       [slab_rows*cols, B]  raw scene rows slab_row0..  (dtype 0 = uint16, 1 = float32)
+//   raw       raw scene rows slab_row0..  (dtype = sample | interleave, include/cmlpl.h: CMLPL_RAW_*)
 //   wf f32 [B][64], bf f32 [64]    conv0 folded with the PCA projection and both z-scores
 //   mu, inv_sigma f32 [B]          band means / 1/std (z-score of the spectral branch)
 extern "C" int cmlpl_scene_infer_raw(const void* raw, int dtype, int scene_rows, int cols, int slab_row0, int slab_rows,

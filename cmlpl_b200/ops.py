@@ -209,22 +209,18 @@ def scene_infer(cube, spectra, packed, num_classes: int, w: int = 20, band_row0:
 def scene_infer_raw(raw, folded, packed, num_classes: int, cols: int, w: int = 20, band_row0: int = 0,
                     band_rows: int | None = None, scene_rows: int | None = None, slab_row0: int = 0,
                     want_logits: bool = False, workspace: torch.Tensor | None = None,
-                    labels: torch.Tensor | None = None):
-    """hyper_tools.py:285-292 + :416-437 from the RAW cube: raw uint16/f32 [slab_rows*cols, B] (scene rows
-    slab_row0..), ``folded`` = Preproc.folded_conv0(...) (conv0 folded with PCA + z-scores; band mean / 1/std).
-    Neither the PCA cube nor the z-scored spectra are materialised."""
+                    labels: torch.Tensor | None = None, interleave: str = "bip"):
+    """hyper_tools.py:285-292 + :416-437 from the RAW cube: raw uint16 / f32 / int16 holding scene rows slab_row0..
+    in the layout ``interleave`` -- "bip" [slab_rows*cols, B] or [slab_rows, cols, B], "bil" [slab_rows, B, cols],
+    "bsq" [B, slab_rows, cols] -- and ``folded`` = Preproc.folded_conv0(...) (conv0 folded with PCA + z-scores; band
+    mean / 1/std).  Neither the PCA cube nor the z-scored spectra are materialised.  Results do not depend on the
+    interleave."""
+    from . import preprocess
     if not raw.is_cuda or not raw.is_contiguous():
         raise _lib.CmlplError("raw must be a contiguous CUDA tensor (cmlpl_b200 has no CPU path)")
-    if raw.dtype == torch.uint16:
-        code = 0
-    elif raw.dtype == _f32:
-        code = 1
-    else:
-        raise _lib.CmlplError(f"raw scene must be uint16 or float32, got {raw.dtype}")
-    ns, B = raw.shape
-    if ns % cols:
-        raise _lib.CmlplError("raw rows are not a multiple of cols")
-    slab_rows = ns // cols
+    code = preprocess._dtype_code(raw)
+    slab_rows, _, B = preprocess.raw_geometry(raw.shape, interleave, cols=cols)
+    code |= preprocess.INTERLEAVE[interleave]
     scene_rows = slab_rows if scene_rows is None else scene_rows
     band_rows = scene_rows - band_row0 if band_rows is None else band_rows
     n = band_rows * cols

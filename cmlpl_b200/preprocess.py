@@ -43,22 +43,66 @@ class Preproc:
 
 
 def _dtype_code(x: torch.Tensor) -> int:
+    """The raw sample type code of include/cmlpl.h (CMLPL_RAW_U16 / F32 / I16)."""
     if x.dtype == torch.uint16:
         return 0
     if x.dtype == torch.float32:
         return 1
-    raise _lib.CmlplError(f"raw scene must be uint16 or float32, got {x.dtype}")
+    if x.dtype == torch.int16:
+        return 2
+    raise _lib.CmlplError(f"raw scene must be uint16, float32 or int16, got {x.dtype}")
 
 
-def fit(raw: torch.Tensor, n_PC: int = 60) -> Preproc:
-    """raw: CUDA tensor [N, B] (uint16 or float32).  Moments in float64 on device, SVD on the host."""
+# interleave codes of include/cmlpl.h (CMLPL_RAW_BIP / BIL / BSQ), or'ed into the sample type code
+INTERLEAVE = {"bip": 0x00, "bil": 0x10, "bsq": 0x20}
+
+
+def raw_geometry(shape, interleave: str = "bip", cols: int | None = None, bands: int | None = None):
+    """(rows, cols, bands) of a raw cube of this shape, checked against ``cols`` / ``bands`` when given:
+    BIP [rows*cols, B] or [rows, cols, B]; BIL [rows, B, cols]; BSQ [B, rows, cols].  A 2-D BIP cube without
+    ``cols`` is one row per pixel (rows = N, cols = 1).  Raises CmlplError on a mismatch."""
+    if interleave not in INTERLEAVE:
+        raise _lib.CmlplError(f"interleave must be one of {sorted(INTERLEAVE)}, got {interleave!r}")
+    shape = tuple(int(d) for d in shape)
+    if interleave == "bip" and len(shape) == 2:
+        n, B = shape
+        c = 1 if cols is None else cols
+        if c <= 0 or n % c:
+            raise _lib.CmlplError(f"raw BIP [rows*cols, B] = {list(shape)}: rows are not a multiple of cols = {cols}")
+        r = n // c
+    elif len(shape) == 3:
+        r, c, B = {"bip": (0, 1, 2), "bil": (0, 2, 1), "bsq": (1, 2, 0)}[interleave]
+        r, c, B = shape[r], shape[c], shape[B]
+        if cols is not None and c != cols:
+            raise _lib.CmlplError(f"raw {interleave.upper()} {list(shape)} has {c} columns, expected {cols}")
+    else:
+        want = {"bip": "[rows*cols, B] or [rows, cols, B]", "bil": "[rows, B, cols]", "bsq": "[B, rows, cols]"}
+        raise _lib.CmlplError(f"raw {interleave.upper()} must be {want[interleave]}, got {list(shape)}")
+    if bands is not None and B != bands:
+        raise _lib.CmlplError(f"raw {interleave.upper()} {list(shape)} has {B} bands, expected {bands}")
+    if r <= 0 or c <= 0 or B <= 0:
+        raise _lib.CmlplError(f"raw {interleave.upper()} {list(shape)} is empty")
+    if max(c, B) >= 2 ** 31 or (interleave != "bip" and r >= 2 ** 31):    # the C int arguments (BIP rows are int64)
+        raise _lib.CmlplError(f"raw {interleave.upper()} {list(shape)}: a dimension exceeds the library's int range")
+    return r, c, B
+
+
+def fit(raw: torch.Tensor, n_PC: int = 60, interleave: str = "bip") -> Preproc:
+    """raw: CUDA tensor (uint16, float32 or int16) in the layout ``interleave`` (see ``raw_geometry``).  Moments in
+    float64 on device, SVD on the host."""
     if not raw.is_cuda or not raw.is_contiguous():
         raise _lib.CmlplError("fit needs a contiguous CUDA tensor")
-    n, B = raw.shape
+    rows, cols, B = raw_geometry(raw.shape, interleave)
+    n = rows * cols
     mean = torch.empty(B, dtype=torch.float64, device=raw.device)
     gram = torch.empty(B, B, dtype=torch.float64, device=raw.device)
-    _lib.call("cmlpl_preprocess_fit_f64", raw.data_ptr(), _dtype_code(raw), n, B, mean.data_ptr(), gram.data_ptr(),
-              torch.cuda.current_stream().cuda_stream)
+    stream = torch.cuda.current_stream().cuda_stream
+    if interleave == "bip":                                       # one pixel per row: the int64 pixel count
+        _lib.call("cmlpl_preprocess_fit_f64", raw.data_ptr(), _dtype_code(raw), n, B, mean.data_ptr(), gram.data_ptr(),
+                  stream)
+    else:
+        _lib.call("cmlpl_preprocess_fit_cube_f64", raw.data_ptr(), _dtype_code(raw) | INTERLEAVE[interleave], rows, cols,
+                  B, mean.data_ptr(), gram.data_ptr(), stream)
     g = gram.cpu().numpy()
     g = np.triu(g) + np.triu(g, 1).T                              # the kernel fills upper tiles only
     mu = mean.cpu().numpy()
@@ -69,7 +113,7 @@ def fit(raw: torch.Tensor, n_PC: int = 60) -> Preproc:
 
 def apply(raw: torch.Tensor, pp: Preproc, want_spectra: bool = True, cube: torch.Tensor | None = None,
           spectra: torch.Tensor | None = None):
-    """raw CUDA [N, B] -> (cube f32 [N, n_PC], spectra f32 [N, B] or None)."""
+    """raw CUDA [N, B] (BIP) -> (cube f32 [N, n_PC], spectra f32 [N, B] or None)."""
     if not raw.is_cuda or not raw.is_contiguous():
         raise _lib.CmlplError("apply needs a contiguous CUDA tensor")
     n, B = raw.shape

@@ -243,17 +243,21 @@ class StreamedScene:
 
 
 class StreamedRawScene:
-    """Like StreamedScene, but from the RAW cube (uint16 / float32 [rows*cols, B], pinned host memory)
-    and a fitted ``cmlpl_b200.preprocess.Preproc``: each band's raw rows are copied on a side stream and fed
+    """Like StreamedScene, but from the RAW cube (uint16 / float32 / int16, pinned host memory) and a fitted
+    ``cmlpl_b200.preprocess.Preproc``: each band's raw rows are copied on a side stream and fed
     to cmlpl_scene_infer_raw, whose first kernels apply the preprocessing folded into conv0 / the fp16
     conversion of the spectra (``folded=`` from Preproc.folded_conv0; nothing preprocessed touches HBM) --
     42.7 MB over PCIe for a PaviaU scene instead of 135 MB.  Without ``folded`` the rows go through
-    cmlpl_preprocess_apply + cmlpl_scene_infer (materialised PCA cube / spectra).  Two sets of device
+    cmlpl_preprocess_apply + cmlpl_scene_infer (materialised PCA cube / spectra; BIP only).  Two sets of device
     buffers alternate between calls, so the copies of the next scene overlap the compute of the current one
-    when calls are issued back to back."""
+    when calls are issued back to back.
+
+    ``interleave`` is the host cube's layout, kept on the device: "bip" [(s1-s0)*cols, B], "bil" [s1-s0, B, cols]
+    (a row band is contiguous) or "bsq" [B, s1-s0, cols] (a row band is B plane segments, moved by one 2-D copy).
+    ``h2d_bytes`` is the number of bytes the last call copied to the device."""
 
     def __init__(self, preproc, scene_rows, cols, num_features, num_classes, w=20, nsplit=2, row0=0, rows=None,
-                 raw_dtype=torch.uint16, device=None):
+                 raw_dtype=torch.uint16, device=None, interleave="bip"):
         from .. import preprocess
         self._pp_mod, self.pp = preprocess, preproc
         self.R, self.C, self.B, self.K, self.w = scene_rows, cols, num_features, num_classes, w
@@ -266,7 +270,12 @@ class StreamedRawScene:
         ns = (self.s1 - self.s0) * cols
         n = (self.r1 - self.r0) * cols
         self._ns, self._dev = ns, dev
-        self.sets = [dict(raw=torch.empty((ns, num_features), dtype=raw_dtype, device=dev), cube=None, spectra=None,
+        sr = self.s1 - self.s0
+        shape = {"bip": (ns, num_features), "bil": (sr, num_features, cols), "bsq": (num_features, sr, cols)}
+        if interleave not in shape:
+            raise _lib.CmlplError(f"interleave must be one of {sorted(shape)}, got {interleave!r}")
+        self.interleave, self.h2d_bytes = interleave, 0
+        self.sets = [dict(raw=torch.empty(shape[interleave], dtype=raw_dtype, device=dev), cube=None, spectra=None,
                           labels=torch.empty((n,), dtype=torch.uint8, device=dev),
                           labels_host=torch.empty((n,), dtype=torch.uint8).pin_memory(),
                           done=torch.cuda.Event()) for _ in range(2)]
@@ -282,9 +291,17 @@ class StreamedRawScene:
         return self.sets[(self.calls - 1) & 1]["labels_host"]
 
     def __call__(self, packed, raw_host, d2h=True, folded=None):
-        """raw_host [(s1-s0)*cols, B] pinned: raw rows s0..s1 of the scene.  Returns uint8 labels of the band
-        (the pinned host tensor of this call's buffer set when d2h, else the CUDA tensor).  The D2H copy is
-        asynchronous: call ``wait()`` (or synchronise the stream) before reading the pinned tensor."""
+        """raw_host pinned: raw rows s0..s1 of the scene in the layout of ``interleave`` ([(s1-s0)*cols, B] for BIP).
+        Returns uint8 labels of the band (the pinned host tensor of this call's buffer set when d2h, else the CUDA
+        tensor).  The D2H copy is asynchronous: call ``wait()`` (or synchronise the stream) before reading the pinned
+        tensor."""
+        il = self.interleave
+        if folded is None and il != "bip":
+            raise _lib.CmlplError(f"StreamedRawScene: a {il.upper()} cube needs folded= (preprocess.apply reads BIP)")
+        want = self.sets[0]["raw"]
+        if il != "bip" and (raw_host.shape != want.shape or raw_host.dtype != want.dtype or not raw_host.is_contiguous()):
+            raise _lib.CmlplError(f"StreamedRawScene: raw_host must be contiguous {want.dtype} {list(want.shape)}, "
+                                  f"got {raw_host.dtype} {list(raw_host.shape)}")
         main = torch.cuda.current_stream()
         S, events = self.sets[self.calls & 1], self.events[self.calls & 1]
         self.calls += 1
@@ -293,14 +310,24 @@ class StreamedRawScene:
             S["spectra"] = torch.empty((self._ns, self.B), dtype=torch.float32, device=self._dev)
         lo, C = self.w // 2, self.C
         self.copy_stream.wait_event(S["done"])               # the call two scenes ago has consumed this set
-        copied, spans = self.s0, []
+        copied, spans, raw = self.s0, [], S["raw"]
+        esz, sr = raw.element_size(), self.s1 - self.s0
+        self.h2d_bytes = 0
         with torch.cuda.stream(self.copy_stream):
             for (a, b), ev in zip(self.bands, events):
                 upto = min(self.s1, b + (self.w - lo - 1))
                 spans.append((copied, upto))
                 if upto > copied:
-                    pa, pb = (copied - self.s0) * C, (upto - self.s0) * C
-                    S["raw"][pa:pb].copy_(raw_host[pa:pb], non_blocking=True)
+                    ra, rb = copied - self.s0, upto - self.s0
+                    if il == "bsq":                           # rows ra..rb of each of the B planes
+                        pitch, off, width = sr * C * esz, ra * C * esz, (rb - ra) * C * esz
+                        _lib.call("cmlpl_memcpy2d_async", raw.data_ptr() + off, pitch, raw_host.data_ptr() + off, pitch,
+                                  width, self.B, self.copy_stream.cuda_stream)
+                        self.h2d_bytes += width * self.B
+                    else:                                     # BIP pixels of rows ra..rb, or BIL rows ra..rb: one block
+                        src = raw_host[ra * C:rb * C] if il == "bip" else raw_host[ra:rb]
+                        (raw[ra * C:rb * C] if il == "bip" else raw[ra:rb]).copy_(src, non_blocking=True)
+                        self.h2d_bytes += src.nbytes
                     copied = upto
                 ev.record(self.copy_stream)
         for (a, b), ev, (c0, c1) in zip(self.bands, events, spans):
@@ -308,7 +335,8 @@ class StreamedRawScene:
             qa, qb = (a - self.r0) * C, (b - self.r0) * C
             if folded is not None:
                 ops.scene_infer_raw(S["raw"], folded, packed, self.K, C, self.w, band_row0=a, band_rows=b - a,
-                                    scene_rows=self.R, slab_row0=self.s0, workspace=self.ws, labels=S["labels"][qa:qb])
+                                    scene_rows=self.R, slab_row0=self.s0, workspace=self.ws, labels=S["labels"][qa:qb],
+                                    interleave=il)
                 continue
             if c1 > c0:                                       # preprocess the rows that just arrived
                 pa, pb = (c0 - self.s0) * C, (c1 - self.s0) * C

@@ -36,6 +36,10 @@ int cmlpl_version(void);
 const char* cmlpl_last_error(void);
 /* 1 if the device the current context runs on is sm_100 (B200), else 0 (or <0). */
 int cmlpl_device_ok(void);
+/* cudaMemcpy2DAsync (kind cudaMemcpyDefault): `height` rows of `width_bytes`, `spitch` / `dpitch` bytes apart, e.g. one
+ * row band of a host BSQ cube, B plane segments, into the same rows of a device slab. */
+int cmlpl_memcpy2d_async(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width_bytes, size_t height,
+                         cmlpl_stream_t stream);
 
 /* ------------------------------------------------------------------ patches --
  * tools/hyper_tools.py:35-55 (MirrowCut), :226-243 (ExtractPatches, even w) and
@@ -151,13 +155,26 @@ int cmlpl_scene_infer(const float* cube, int scene_rows, int cols, int slab_row0
                       void* workspace, size_t workspace_bytes,
                       uint8_t* labels, float* logits, cmlpl_stream_t stream);
 
-/* The same from the RAW cube (dtype 0 = uint16, 1 = float32; <= 32 classes, <= 512 bands): the PCA
- * projection and both z-scores of tools/hyper_tools.py:285-292 are folded into conv0
+/* Raw cube codes: dtype = sample | interleave.  Codes 0 and 1 are uint16 and float32 band-interleaved-by-pixel. */
+#define CMLPL_RAW_U16 0x00    /* sample types */
+#define CMLPL_RAW_F32 0x01
+#define CMLPL_RAW_I16 0x02
+#define CMLPL_RAW_BIP 0x00    /* interleave: band-interleaved-by-pixel, by line, band-sequential */
+#define CMLPL_RAW_BIL 0x10
+#define CMLPL_RAW_BSQ 0x20
+
+/* The same from the RAW cube (dtype = CMLPL_RAW_{U16,F32,I16} | CMLPL_RAW_{BIP,BIL,BSQ}; <= 32 classes, <= 512
+ * bands): the PCA projection and both z-scores of tools/hyper_tools.py:285-292 are folded into conv0
  * (wf f32 [B][64] = (W0 . (U/s)^T)^T, bf f32 [64] = b0 - W0 . m/s) and into the spectral branch (mu, inv_sigma
  * f32 [B]: the fp16 conversion of the tensor-core branch up to 224 bands, the operand loads of the CUDA-core spectral
  * head beyond); neither the PCA cube nor the z-scored spectra touch HBM.  Above 256 bands conv0 streams each tile's
  * bands through shared memory in 64-band slices.
- * raw [slab_rows*cols, B] holds scene rows slab_row0.. (halo included, like `cube` above). */
+ * raw holds scene rows slab_row0.. (halo included, like `cube` above), aligned to its sample size.  With
+ * sr = scene row - slab_row0, c = column, b = band, the sample is at
+ *   BIP  raw[(sr*cols + c)*B + b]          ([slab_rows*cols, B], a pixel's bands contiguous)
+ *   BIL  raw[(sr*B + b)*cols + c]          ([slab_rows, B, cols], AVIRIS-NG, Hyperion, PRISMA)
+ *   BSQ  raw[(b*slab_rows + sr)*cols + c]  ([B, slab_rows, cols]: the planes are the slab's, not the scene's)
+ * The band's spectra are read from the same slab.  Results do not depend on the interleave. */
 int cmlpl_scene_infer_raw(const void* raw, int dtype, int scene_rows, int cols, int slab_row0, int slab_rows,
                           int num_features, int num_classes, int w, int band_row0, int band_rows,
                           const float* wf, const float* bf, const float* mu, const float* inv_sigma,
@@ -211,11 +228,15 @@ int cmlpl_argmax_u8(const float* logits, int64_t n, int num_classes, uint8_t* la
 
 /* ------------------------------------------------------------- preprocessing --
  * tools/hyper_tools.py:8-32 (featureNormalize, PCANorm) as called at :289-292, on device (SURVEY 8-f1).
- * x: raw scene [n, B], dtype 0 = uint16, 1 = float32.
+ * x: raw scene [n, B] band-interleaved-by-pixel, dtype CMLPL_RAW_U16 / F32 / I16.
  * fit  : mean f64 [B] = column means, gram f64 [B,B] = sum_n (x-mean)(x-mean)^T, upper 32x32 tiles only
  *        (mirror on the host; np.cov = gram/(n-1), np.std^2 = diag(gram)/n).  The B x B SVD stays on the host.
+ *        cmlpl_preprocess_fit_cube_f64 takes a [rows, cols] cube in any raw code of cmlpl_scene_infer_raw (BIL needs
+ *        cols); cmlpl_preprocess_fit_f64 is the same for BIP [n, B] (rows = n, cols = 1).
  * apply: spectra f32 [n,B] = (x-mu)*inv_sigma (may be NULL);  cube f32 [n,npc] = (x-mu).Us - shift with
  *        Us f32 [B,npc] = U[:, :npc]/s and shift = m/s (m, s = mean/std of the projected data). */
+int cmlpl_preprocess_fit_cube_f64(const void* x, int dtype, int rows, int cols, int B, double* mean, double* gram,
+                                  cmlpl_stream_t stream);
 int cmlpl_preprocess_fit_f64(const void* x, int dtype, int64_t n, int B, double* mean, double* gram,
                              cmlpl_stream_t stream);
 int cmlpl_preprocess_apply(const void* x, int dtype, int64_t n, int B, int npc, const float* mu,
