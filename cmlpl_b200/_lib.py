@@ -29,8 +29,8 @@ SIGNATURES = {
     "cmlpl_avgpool2_bwd_f32": (I, [P, P, L, I, I, P]),
     "cmlpl_relu_bwd_f32": (I, [P, P, P, L, P]),
     "cmlpl_colsum_f32": (I, [P, P, L, L, P]),
-    "cmlpl_l2norm_f32": (I, [P, P, P, L, L, P]),
-    "cmlpl_l2norm_bwd_f32": (I, [P, P, P, P, L, L, P]),
+    "cmlpl_l2norm_f32": (I, [P, P, P, L, L, F, P]),
+    "cmlpl_l2norm_bwd_f32": (I, [P, P, P, P, L, L, F, P]),
     "cmlpl_packed_bytes": (Z, [I, I, I]),
     "cmlpl_pack_basenet2": (I, [P] * 10 + [I, I, I, P, P]),
     "cmlpl_scene_workspace_bytes": (Z, [I, I, I, I, I]),

@@ -86,7 +86,7 @@ int make_scene_tmap(CUtensorMap* out, const void* base, int outer, int rows, int
 
 extern "C" {
 
-int cmlpl_version(void) { return 100; }
+int cmlpl_version(void) { return 101; }
 
 const char* cmlpl_last_error(void) { return cmlpl::g_err; }
 

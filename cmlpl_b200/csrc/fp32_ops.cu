@@ -71,8 +71,10 @@ conv_bias_grad_kernel(const float* __restrict__ dy, float* __restrict__ db, int 
   }
 }
 
-// one warp per row
-__global__ void l2norm_kernel(const float* __restrict__ x, float* __restrict__ y, float* __restrict__ norm, int64_t rows, int64_t cols) {
+// one warp per row.  y = x / max(norm, eps); eps = 0 is models.py:88 (pow(1/2), no epsilon: a zero row gives NaN),
+// eps > 0 is F.normalize.  norm stores the unclamped norm.
+__global__ void l2norm_kernel(const float* __restrict__ x, float* __restrict__ y, float* __restrict__ norm, int64_t rows,
+                              int64_t cols, float eps) {
   const int64_t row = blockIdx.x * int64_t(blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= rows) return;
   const int lane = threadIdx.x & 31;
@@ -80,12 +82,14 @@ __global__ void l2norm_kernel(const float* __restrict__ x, float* __restrict__ y
   float s = 0.f;
   for (int64_t c = lane; c < cols; c += 32) s = fmaf(xr[c], xr[c], s);
   s = warp_sum(s);
-  const float nr = sqrtf(s);   // models.py:88 pow(1/2), no epsilon
+  const float nr = sqrtf(s);
   if (lane == 0 && norm) norm[row] = nr;
-  for (int64_t c = lane; c < cols; c += 32) y[row * cols + c] = xr[c] / nr;
+  const float d = nr < eps ? eps : nr;
+  for (int64_t c = lane; c < cols; c += 32) y[row * cols + c] = xr[c] / d;
 }
+// below eps the denominator is the constant eps (clamp_min passes no gradient): dx = dy / eps
 __global__ void l2norm_bwd_kernel(const float* __restrict__ y, const float* __restrict__ norm, const float* __restrict__ dy,
-                                  float* __restrict__ dx, int64_t rows, int64_t cols) {
+                                  float* __restrict__ dx, int64_t rows, int64_t cols, float eps) {
   const int64_t row = blockIdx.x * int64_t(blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= rows) return;
   const int lane = threadIdx.x & 31;
@@ -93,7 +97,9 @@ __global__ void l2norm_bwd_kernel(const float* __restrict__ y, const float* __re
   float s = 0.f;
   for (int64_t c = lane; c < cols; c += 32) s = fmaf(dr[c], yr[c], s);
   s = warp_sum(s);
-  const float inv = 1.f / norm[row];
+  const bool clamped = norm[row] < eps;
+  if (clamped) s = 0.f;
+  const float inv = 1.f / (clamped ? eps : norm[row]);
   for (int64_t c = lane; c < cols; c += 32) dx[row * cols + c] = (dr[c] - yr[c] * s) * inv;
 }
 
@@ -110,8 +116,10 @@ using namespace cmlpl;
 extern "C" int cmlpl_sgemm_f32(int M, int N, int K, float alpha, const float* A, int64_t a_rs, int64_t a_cs,
                                const float* B, int64_t b_rs, int64_t b_cs, const float* bias, float beta,
                                float* C, int64_t c_rs, int64_t c_cs, int act, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(A && B && C, "sgemm: null pointer");
   CMLPL_CHECK_ARG(M >= 0 && N >= 0 && K >= 0, "sgemm: negative dims");
+  // an operand without elements may be null (torch allocates nothing for it): K = 0 gives C = act(bias + beta*C)
+  CMLPL_CHECK_ARG((A || int64_t(M) * K == 0) && (B || int64_t(K) * N == 0) && (C || int64_t(M) * N == 0),
+                  "sgemm: null pointer");
   StridedA fa{A, a_rs, a_cs};
   StridedB fb{B, b_rs, b_cs};
   StridedC fc{C, c_rs, c_cs, bias, alpha, beta, act};
@@ -191,18 +199,19 @@ extern "C" int cmlpl_colsum_f32(const float* x, float* out, int64_t m, int64_t n
   CMLPL_CHECK_LAUNCH("colsum");
   return CMLPL_OK;
 }
-extern "C" int cmlpl_l2norm_f32(const float* x, float* y, float* norm, int64_t rows, int64_t cols, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(x && y && rows >= 0 && cols > 0, "l2norm: bad args");
+extern "C" int cmlpl_l2norm_f32(const float* x, float* y, float* norm, int64_t rows, int64_t cols, float eps,
+                                cmlpl_stream_t stream) {
+  CMLPL_CHECK_ARG(x && y && rows >= 0 && cols > 0 && eps >= 0.f, "l2norm: bad args");
   if (rows == 0) return CMLPL_OK;
-  l2norm_kernel<<<int((rows + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(x, y, norm, rows, cols);
+  l2norm_kernel<<<int((rows + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(x, y, norm, rows, cols, eps);
   CMLPL_CHECK_LAUNCH("l2norm");
   return CMLPL_OK;
 }
 extern "C" int cmlpl_l2norm_bwd_f32(const float* y, const float* norm, const float* dy, float* dx, int64_t rows,
-                                    int64_t cols, cmlpl_stream_t stream) {
-  CMLPL_CHECK_ARG(y && norm && dy && dx && rows >= 0 && cols > 0, "l2norm_bwd: bad args");
+                                    int64_t cols, float eps, cmlpl_stream_t stream) {
+  CMLPL_CHECK_ARG(y && norm && dy && dx && rows >= 0 && cols > 0 && eps >= 0.f, "l2norm_bwd: bad args");
   if (rows == 0) return CMLPL_OK;
-  l2norm_bwd_kernel<<<int((rows + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(y, norm, dy, dx, rows, cols);
+  l2norm_bwd_kernel<<<int((rows + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(y, norm, dy, dx, rows, cols, eps);
   CMLPL_CHECK_LAUNCH("l2norm_bwd");
   return CMLPL_OK;
 }

@@ -67,8 +67,10 @@ __global__ void softmax_entropy_kernel(const float* __restrict__ z, int64_t rows
 // ---------------------------------------------------------------- softmax JS divergence (trian_CCT.py:76-84)
 // loss = 0.5 * (kl_div(log_softmax(z), M, 'mean') + kl_div(log(t + 1e-5), M, 'mean')),  M = (softmax(z) + t) / 2,
 // 'mean' = over all rows*C elements.  One thread per row; gradient w.r.t. z in the same pass (t is a constant):
-//   f_k = 2 M log M - M log p - M log(t + eps);  g_k = df/dp_k = log M + 1 - log(p)/2 - M/p - log(t + eps)/2
-//   dz_j = p_j (g_j - sum_k g_k p_k) * scale * 0.5 / (rows*C)
+//   f_k = 2 M log M - M log p - M log(t + eps);  g_k = df/dp_k = h_k - M_k/p_k,  h_k = log M + 1 - log(p)/2 - log(t + eps)/2
+//   dz_j = p_j (g_j - sum_k g_k p_k) * cf = (p_j h_j - M_j - p_j sum_k (p_k h_k - M_k)) * cf,  cf = scale * 0.5 / (rows*C)
+// The second form has no M/p: where the softmax underflows (a logit ~88 or more below the row's max) p is 0 or a
+// denormal, and M/p would be inf or 0/0 and turn the whole row of dz into NaN.
 __global__ void js_kernel(const float* __restrict__ z, const float* __restrict__ t, int64_t rows, int C, float scale,
                           float* __restrict__ loss, float* __restrict__ dz) {
   __shared__ float red[32];
@@ -87,7 +89,7 @@ __global__ void js_kernel(const float* __restrict__ z, const float* __restrict__
       const float M = 0.5f * (p + tt), lt = logf(tt + 1e-5f);
       const float lM = M > 0.f ? logf(M) : 0.f;                // xlogy: 0 * log 0 = 0 (F.kl_div)
       li += M * (lM - lp) + M * (lM - lt);
-      gp += (lM + 1.f - 0.5f * lp - M / p - 0.5f * lt) * p;
+      gp += p * (lM + 1.f - 0.5f * lp - 0.5f * lt) - M;
     }
     if (dz) {
       const float cf = scale * 0.5f / (float(rows) * float(C));
@@ -95,7 +97,7 @@ __global__ void js_kernel(const float* __restrict__ z, const float* __restrict__
         const float lp = zr[c] - lse, p = expf(lp), tt = tr[c];
         const float M = 0.5f * (p + tt), lt = logf(tt + 1e-5f);
         const float lM = M > 0.f ? logf(M) : 0.f;
-        dz[r * C + c] = cf * p * ((lM + 1.f - 0.5f * lp - M / p - 0.5f * lt) - gp);
+        dz[r * C + c] = cf * (p * (lM + 1.f - 0.5f * lp - 0.5f * lt) - M - p * gp);
       }
     }
   }
@@ -387,7 +389,8 @@ extern "C" int cmlpl_adam_multi_f32(int n_tensors, float* const* p_host, const f
     for (int i = 0; i < t.count; ++i) {
       t.p[i] = p_host[base + i]; t.g[i] = g_host[base + i]; t.m[i] = m_host[base + i]; t.v[i] = v_host[base + i];
       t.n[i] = numel_host[base + i];
-      CMLPL_CHECK_ARG(t.p[i] && t.m[i] && t.v[i] && t.n[i] >= 0, "adam: null tensor %d", base + i);
+      // an empty tensor may have null pointers (torch allocates nothing for it); the kernel never touches them
+      CMLPL_CHECK_ARG(t.n[i] == 0 || (t.p[i] && t.m[i] && t.v[i] && t.n[i] > 0), "adam: null tensor %d", base + i);
       if (t.g[i] && t.n[i] > mx) mx = t.n[i];
     }
     if (mx == 0) continue;

@@ -54,14 +54,17 @@ def graph_contrast(f_row, f_col, probs1, probs, T, grad_side):
     return _GraphContrastFn.apply(f_row, f_col, probs1.detach(), probs.detach(), float(T), int(grad_side))
 
 
+_NORMALIZE_EPS = 1e-12                                # F.normalize's default eps
+
+
 class _NTXentFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, emb_i, emb_j, T):
         bs = emb_i.size(0)
         x = torch.cat([emb_i, emb_j], 0).contiguous()
-        z, norm = ops.l2norm(x)                       # F.normalize (models.py:23-24); eps only matters for zero rows
+        z, norm = ops.l2norm(x, _NORMALIZE_EPS)       # F.normalize (models.py:23-24): a zero row stays finite
         loss, dz = ops.ntxent(z, bs, T, True)
-        dx = ops.l2norm_bwd(z, norm, dz)
+        dx = ops.l2norm_bwd(z, norm, dz, _NORMALIZE_EPS)
         ctx.save_for_backward(dx)
         ctx.bs = bs
         return loss

@@ -140,20 +140,23 @@ def colsum(x):
     return out
 
 
-def l2norm(x):
+def l2norm(x, eps=0.0):
+    """x / max(||x||, eps) per row -> (y, unclamped norm).  eps = 0: models.py:87-90 Normalize (a zero row gives NaN);
+    eps = 1e-12: F.normalize."""
     _chk(x, name="x")
     rows, cols = x.shape
     y = torch.empty_like(x)
     norm = torch.empty((rows,), dtype=_f32, device=x.device)
-    _lib.call("cmlpl_l2norm_f32", x.data_ptr(), y.data_ptr(), norm.data_ptr(), rows, cols, _stream())
+    _lib.call("cmlpl_l2norm_f32", x.data_ptr(), y.data_ptr(), norm.data_ptr(), rows, cols, float(eps), _stream())
     return y, norm
 
 
-def l2norm_bwd(y, norm, dy):
+def l2norm_bwd(y, norm, dy, eps=0.0):
+    """Backward of l2norm(x, eps) given its outputs."""
     _chk(y, name="y"); _chk(dy, name="dy")
     dx = torch.empty_like(dy)
     _lib.call("cmlpl_l2norm_bwd_f32", y.data_ptr(), norm.data_ptr(), dy.data_ptr(), dx.data_ptr(),
-              y.shape[0], y.shape[1], _stream())
+              y.shape[0], y.shape[1], float(eps), _stream())
     return dx
 
 

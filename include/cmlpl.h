@@ -94,11 +94,13 @@ int cmlpl_relu_bwd_f32(const float* y, const float* dy, float* dx, int64_t n, cm
 /* column sums: out[n] = sum_m x[m,n] (bias gradients of nn.Linear). */
 int cmlpl_colsum_f32(const float* x, float* out, int64_t m, int64_t n, cmlpl_stream_t stream);
 
-/* models.py:87-90 Normalize: y = x / sqrt(sum x^2) per row (no epsilon), and its backward
- * dx = (dy - y * sum(dy*y)) / norm. */
-int cmlpl_l2norm_f32(const float* x, float* y, float* norm, int64_t rows, int64_t cols, cmlpl_stream_t stream);
+/* Row L2 normalisation: y = x / max(norm, eps), norm = sqrt(sum x^2) per row (stored unclamped), and its backward
+ * dx = (dy - y * sum(dy*y)) / norm, or dy / eps where norm < eps.  eps = 0 is models.py:87-90 Normalize (no epsilon:
+ * a zero row gives NaN); eps = 1e-12 is F.normalize (models.py:23-24, ContrastiveLoss). */
+int cmlpl_l2norm_f32(const float* x, float* y, float* norm, int64_t rows, int64_t cols, float eps,
+                     cmlpl_stream_t stream);
 int cmlpl_l2norm_bwd_f32(const float* y, const float* norm, const float* dy, float* dx,
-                         int64_t rows, int64_t cols, cmlpl_stream_t stream);
+                         int64_t rows, int64_t cols, float eps, cmlpl_stream_t stream);
 
 /* ------------------------------------------------------------ scene inference --
  * tools/hyper_tools.py:416-437 (test_whole) over a whole scene / row band without ever
