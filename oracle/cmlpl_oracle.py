@@ -172,6 +172,55 @@ def synth_cube_hard(R: int, C: int, B: int, K: int, seed: int = 1088, spread: fl
     return np.clip(cube, 0, 8000).astype(np.uint16), gt.astype(np.uint8)
 
 
+def sensor_scene(R: int, C: int, B: int, K: int, noise_dn: float = 8.0, seed: int = 1088, sample: str = "u16",
+                 dc: float = 0.0, block: int = 8):
+    """A scene conditioned like a real sensor's (PaviaU, AVIRIS, WHU-Hi) rather than like ``synth_cube``: every pixel is a
+    smooth mixture of K + 1 endmember spectra under a per-pixel illumination, plus ``noise_dn`` DN of sensor noise.  The
+    signal spans K + 1 dimensions and the noise floor is a few DN, so lambda_1 / lambda_60 of the band covariance is 1e5 to
+    1e8 (``synth_cube``: 1e3) and the trailing z-scored PCA components are small differences of large band values.
+
+    * endmembers: an offset plus four Gaussians over the band index (widths 5-30 % of the band range), 200-8000 DN;
+    * class map: blocky as in ``synth_cube``; abundances are the pixel's own class (weight 0.75-1) plus a share of the
+      classes half a block away in each direction;
+    * illumination: uniform in [0.7, 1.3] per pixel;
+    * ``sample``: "u16" (rounded, + ``dc`` DN, e.g. a 20 000 DN offset that makes the band means large next to their
+      standard deviations), "i16" (dark-subtracted: minus a dark level per band of about half the band's mean, so many
+      values are negative) or "f32" (reflectance-like: DN / 10 000, noise ``noise_dn`` / 10 000, not rounded).
+    -> (cube [R, C, B] of the sample type, gt uint8 [R, C] with 0 = unlabelled)."""
+    rng = np.random.default_rng(seed)
+    gb = rng.integers(0, K + 1, size=(-(-R // block), -(-C // block)))
+    gt = np.kron(gb, np.ones((block, block), dtype=np.int64))[:R, :C]
+    flat = gt.reshape(-1)
+    for k in range(1, K + 1):
+        if (flat == k).sum() < 32:
+            flat[rng.choice(flat.size, 32, replace=False)] = k
+    gt = flat.reshape(R, C)
+    t = np.arange(B) / max(B - 1, 1)
+    E = np.empty((K + 1, B))
+    for k in range(K + 1):
+        e = rng.uniform(200, 1200) + sum(rng.uniform(500, 2500) * np.exp(-0.5 * ((t - rng.uniform(-0.1, 1.1))
+                                                                                  / rng.uniform(0.05, 0.3)) ** 2)
+                                         for _ in range(4))
+        E[k] = np.clip(e, 200, 8000)
+    onehot = (gt[..., None] == np.arange(K + 1)).astype(np.float64)
+    h = max(block // 2, 1)
+    nb = sum(onehot[mirror_index(np.arange(R) + dr, R)][:, mirror_index(np.arange(C) + dc_, C)]
+             for dr, dc_ in ((-h, 0), (h, 0), (0, -h), (0, h))) / 4.0
+    own = rng.uniform(0.75, 1.0, size=(R, C, 1))
+    A = own * onehot + (1 - own) * nb
+    cube = rng.uniform(0.7, 1.3, size=(R, C, 1)) * (A @ E) + rng.normal(0, noise_dn, size=(R, C, B))
+    if sample == "u16":
+        cube = np.clip(np.rint(cube + dc), 0, 65535).astype(np.uint16)
+    elif sample == "i16":
+        dark = 0.5 * E.mean(0) * rng.uniform(0.8, 1.2, size=B)
+        cube = np.clip(np.rint(cube - dark), -32768, 32767).astype(np.int16)
+    elif sample == "f32":
+        cube = (cube / 1e4).astype(np.float32)
+    else:
+        raise ValueError(f"sample must be u16, i16 or f32, got {sample!r}")
+    return cube, gt.astype(np.uint8)
+
+
 def preprocess_params(cube_u16: np.ndarray, n_PC: int = 60):
     """The affine maps behind hyper_tools.py:285-292 as explicit float64 parameters:
     spectra = (X - mu) / sigma;  cubePCA = ((X - mu) @ U - pca_mu) / pca_sigma."""

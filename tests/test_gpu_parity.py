@@ -349,10 +349,11 @@ def test_device_preprocessing_matches_reference_numpy(dev):
     cube, spec = preprocess.apply(raw, pp)
     assert rel(spec.cpu(), ref_spec) < 1e-6
     got = cube.cpu().numpy().reshape(64, 50, 60)
-    # singular vectors are defined up to sign: align each component before comparing
+    # the host SVD of (almost) the same matrix gives every component the reference's sign: a net trained on the
+    # reference's preprocessing reads the device's unchanged
     sgn = np.sign((got * ref_cube).sum((0, 1)))
-    assert rel(got * sgn, ref_cube) < 2e-5
-    assert np.mean(sgn > 0) > 0.9                        # same LAPACK on (almost) the same matrix: same signs
+    assert np.all(sgn > 0)
+    assert rel(got, ref_cube) < 2e-5
     # float32 raw input path
     cube_f, _ = preprocess.apply(raw.float(), pp, want_spectra=False)
     assert rel(cube_f.cpu(), cube.cpu()) < 1e-6
