@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import c_char_p, c_float, c_int, c_int64, c_size_t, c_void_p
+from ctypes import c_char_p, c_double, c_float, c_int, c_int64, c_size_t, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libcmlpl_sm100.so")
@@ -36,6 +36,8 @@ SIGNATURES = {
     "cmlpl_scene_workspace_bytes": (Z, [I, I, I, I, I]),
     "cmlpl_scene_infer": (I, [P, I, I, I, I, P, I, I, I, I, I, P, P, Z, P, P, P]),
     "cmlpl_scene_infer_raw": (I, [P, I, I, I, I, I, I, I, I, I, I, P, P, P, P, P, P, Z, P, P, P]),
+    "cmlpl_scene_infer_raw_masked": (I, [P, I, I, I, I, I, I, I, I, I, I, P, P, P, P, P, P, P, Z, P, P, P]),
+    "cmlpl_valid_mask_u8": (I, [P, I, L, I, I, c_double, P, P, P, P]),
     "cmlpl_conv0_map_f16": (I, [P, I, I, I, I, I, I, I, P, P, P]),
     "cmlpl_patch_cnn_f16": (I, [P, I, I, I, P, P, P]),
     "cmlpl_scene_workspace_layout": (I, [I, I, I, I, I, P]),
@@ -48,6 +50,8 @@ SIGNATURES = {
     "cmlpl_preprocess_fit_cube_f64": (I, [P, I, I, I, I, P, P, P]),
     "cmlpl_preprocess_fit_f64": (I, [P, I, L, I, P, P, P]),
     "cmlpl_preprocess_apply": (I, [P, I, L, I, I, P, P, P, P, P, P, P]),
+    "cmlpl_preprocess_fit_masked_f64": (I, [P, I, L, I, I, P, P, P, P, P]),
+    "cmlpl_preprocess_apply_masked": (I, [P, I, L, I, I, P, P, P, P, P, P, P, P]),
     "cmlpl_confusion_i64": (I, [P, P, L, I, P, P]),
     "cmlpl_ce_fwd_bwd_f32": (I, [P, P, P, P, L, I, F, P, P, P]),
     "cmlpl_softmax_entropy_f32": (I, [P, L, I, F, P, P]),

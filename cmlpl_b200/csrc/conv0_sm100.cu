@@ -10,6 +10,9 @@
 // 16-byte stores coalesced along positions) while their loads for the next tile are in flight.  A band-major raw slab
 // (BIL / BSQ) has its own loader: a thread owns one position and reads 8 bands per K-chunk, coalesced along columns.
 // Replaces the CUDA-core conv0_tiled_kernel of round 1 (L1-wavefront bound on the strided pixel rows).
+// valid (raw cube only; u8 [slab_rows * cols] over the slab's pixels, or nullptr): a position whose mirrored source pixel
+// is no-data gets the z-scored operand 0 (hi and lo), i.e. the pixel stands in as its band means and F0 there is the
+// folded bias exactly.  The mask byte is read once per tile position; the sample loads keep their order.
 #include "common.cuh"
 #include "sm100_ptx.cuh"
 
@@ -30,7 +33,7 @@ __device__ __forceinline__ void
 conv0_tc_body(const T* __restrict__ in, int K, int KP, int nstage, int scene_rows, int cols, int slab_row0, int w, int band_row0,
               int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
               const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad, BandMajor bm,
-              const int tid) {
+              const uint8_t* __restrict__ valid, const int tid) {
   using namespace c0s;
   extern __shared__ __align__(128) unsigned char smem[];
   const int warp = tid >> 5, lane = tid & 31;
@@ -124,12 +127,13 @@ conv0_tc_body(const T* __restrict__ in, int K, int KP, int nstage, int scene_row
       mbar_wait(bars + 8 * (X_EMPTY0 + s), (nstage == 2 ? ((it >> 1) & 1) : (it & 1)) ^ 1, 82);
       unsigned char* xs = smem + S_X + s * xbytes;
       const int64_t p0 = t * 128;
-      auto src_of = [&](int pos) -> const T* {
+      auto pix_of = [&](int pos) -> int64_t {                   // the position's mirrored source pixel in the slab
         int pp = int(p0) + pos; if (pp >= int(plane)) pp = int(plane) - 1;      // plane < 2^31 (checked by the launcher)
         const int pr = pp / pcol_n, pc = pp - pr * pcol_n;
         const int sr = mirror_index(band_row0 + pr + lo, scene_rows) - slab_row0, sc = mirror_index(pc + lo, cols);
-        return in + (int64_t(sr) * cols + sc) * K;
+        return int64_t(sr) * cols + sc;
       };
+      auto src_of = [&](int pos) -> const T* { return in + pix_of(pos) * K; };
       if constexpr (kBM) {
         // band-major slab: a thread owns one of the tile's 128 positions and reads 8 consecutive bands per K-chunk (each
         // load coalesced along the warp's consecutive columns), then stores the chunk as one 16-byte hi and one lo write.
@@ -140,6 +144,7 @@ conv0_tc_body(const T* __restrict__ in, int K, int KP, int nstage, int scene_row
         const int sr = mirror_index(band_row0 + pr + lo, scene_rows) - slab_row0, sc = mirror_index(pc + lo, cols);
         const T* src = in + int64_t(sr) * bm.rs + sc;
         const int kc_end = (K + 7) / 8;                         // chunks past it are K padding, written once above
+        const bool ok = !valid || valid[int64_t(sr) * cols + sc];   // the source pixel has data
 #pragma unroll 1
         for (int c0 = tid >> 7; c0 < kc_end; c0 += 8) {        // 4 chunks (32 loads) in flight per thread
           float v[4][8];
@@ -158,8 +163,8 @@ conv0_tc_body(const T* __restrict__ in, int K, int KP, int nstage, int scene_row
 #pragma unroll
               for (int e = 0; e < 8; e += 2) {
                 const int k = kc * 8 + e;
-                const float z0 = k < K ? (v[u][e] - smu[k]) * __ldg(inv_sigma + k) : 0.f;
-                const float z1 = k + 1 < K ? (v[u][e + 1] - smu[k + 1]) * __ldg(inv_sigma + k + 1) : 0.f;
+                const float z0 = (ok && k < K) ? (v[u][e] - smu[k]) * __ldg(inv_sigma + k) : 0.f;
+                const float z1 = (ok && k + 1 < K) ? (v[u][e + 1] - smu[k + 1]) * __ldg(inv_sigma + k + 1) : 0.f;
                 const __half h0 = __float2half_rn(z0), h1 = __float2half_rn(z1);
                 hi[e / 2] = __halves2half2(h0, h1);
                 lo2[e / 2] = __halves2half2(__float2half_rn(z0 - __half2float(h0)), __float2half_rn(z1 - __half2float(h1)));
@@ -204,14 +209,17 @@ conv0_tc_body(const T* __restrict__ in, int K, int KP, int nstage, int scene_row
 #pragma unroll 1
         for (int j0 = 0; j0 < 16; j0 += 4) {                   // 4 pixels (up to 32 loads) in flight per lane
           float v[4][8];
+          bool ok[4];                                           // the source pixel has data
 #pragma unroll
           for (int jj = 0; jj < 4; ++jj) {
-            const T* src = src_of(warp + 8 * (j0 + jj));
+            const int64_t px = pix_of(warp + 8 * (j0 + jj));
+            const T* src = in + px * K;
 #pragma unroll
             for (int m = 0; m < 8; ++m) {
               const int k = lane + 32 * m;
               v[jj][m] = k < K ? float(src[k]) : 0.f;
             }
+            ok[jj] = !valid || valid[px];
           }
 #pragma unroll
           for (int jj = 0; jj < 4; ++jj) {
@@ -220,7 +228,7 @@ conv0_tc_body(const T* __restrict__ in, int K, int KP, int nstage, int scene_row
             for (int m = 0; m < 8; ++m) {
               const int k = lane + 32 * m;
               if (k < K) {
-                const float z = (v[jj][m] - mr[m]) * ir[m];
+                const float z = ok[jj] ? (v[jj][m] - mr[m]) * ir[m] : 0.f;
                 const __half hi = __float2half_rn(z);
                 unsigned char* d = xs + (k >> 3) * XCH + pos * 16 + (k & 7) * 2;
                 *reinterpret_cast<__half*>(d) = hi;
@@ -269,9 +277,10 @@ template <typename T, bool kVec4, bool kSplit>
 __global__ void __launch_bounds__(c0s::kThreads, 1)
 conv0_tc_kernel(const T* __restrict__ in, int K, int KP, int nstage, int scene_rows, int cols, int slab_row0, int w, int band_row0,
                 int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
-                const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad) {
+                const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad,
+                const uint8_t* __restrict__ valid) {
   conv0_tc_body<T, kVec4, kSplit, false>(in, K, KP, nstage, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt,
-                                         bias, mu, inv_sigma, f0pad, BandMajor{}, threadIdx.x);
+                                         bias, mu, inv_sigma, f0pad, BandMajor{}, valid, threadIdx.x);
 }
 
 // the raw cube in BIL / BSQ (split operands)
@@ -280,9 +289,9 @@ __global__ void __launch_bounds__(c0s::kThreads, 1)
 conv0_tc_bm_kernel(const T* __restrict__ in, int K, int KP, int nstage, int scene_rows, int cols, int slab_row0, int w,
                    int band_row0, int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */,
                    const float* __restrict__ bias, const float* __restrict__ mu, const float* __restrict__ inv_sigma,
-                   __half* __restrict__ f0pad, BandMajor bm) {
+                   __half* __restrict__ f0pad, BandMajor bm, const uint8_t* __restrict__ valid) {
   conv0_tc_body<T, false, true, true>(in, K, KP, nstage, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias,
-                                      mu, inv_sigma, f0pad, bm, threadIdx.x);
+                                      mu, inv_sigma, f0pad, bm, valid, threadIdx.x);
 }
 
 // K-sliced variant for the raw cube beyond 256 bands (split hi / lo operands only).  A tile's X operand no longer fits one
@@ -302,7 +311,7 @@ __device__ __forceinline__ void
 conv0_tc_sliced_body(const T* __restrict__ in, int K, int KP, int scene_rows, int cols, int slab_row0, int w, int band_row0,
                      int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
                      const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad,
-                     BandMajor bm, const int tid) {
+                     BandMajor bm, const uint8_t* __restrict__ valid, const int tid) {
   using namespace c0s;
   using c0k::kSlice; using c0k::XCH; using c0k::kXHalf;
   extern __shared__ __align__(128) unsigned char smem[];
@@ -395,6 +404,7 @@ conv0_tc_sliced_body(const T* __restrict__ in, int K, int KP, int scene_rows, in
         const int pr = pp / pcol_n, pc = pp - pr * pcol_n;
         const int sr = mirror_index(band_row0 + pr + lo, scene_rows) - slab_row0, sc = mirror_index(pc + lo, cols);
         const T* src = in + int64_t(sr) * bm.rs + sc;
+        const bool ok = !valid || valid[int64_t(sr) * cols + sc];   // the source pixel has data
 #pragma unroll 1
         for (int j = 0; j < nslice; ++j, ++g) {
           const int s = g & 1;
@@ -415,8 +425,8 @@ conv0_tc_sliced_body(const T* __restrict__ in, int K, int KP, int scene_rows, in
 #pragma unroll
             for (int e = 0; e < 8; e += 2) {
               const int k = j * kSlice + kl + e;
-              const float z0 = (v[u][e] - smu[k < KP ? k : 0]) * (k < KP ? sis[k] : 0.f);
-              const float z1 = (v[u][e + 1] - smu[k + 1 < KP ? k + 1 : 0]) * (k + 1 < KP ? sis[k + 1] : 0.f);
+              const float z0 = ok ? (v[u][e] - smu[k < KP ? k : 0]) * (k < KP ? sis[k] : 0.f) : 0.f;
+              const float z1 = ok ? (v[u][e + 1] - smu[k + 1 < KP ? k + 1 : 0]) * (k + 1 < KP ? sis[k + 1] : 0.f) : 0.f;
               const __half h0 = __float2half_rn(z0), h1 = __float2half_rn(z1);
               hi[e / 2] = __halves2half2(h0, h1);
               lo2[e / 2] = __halves2half2(__float2half_rn(z0 - __half2float(h0)), __float2half_rn(z1 - __half2float(h1)));
@@ -430,12 +440,14 @@ conv0_tc_sliced_body(const T* __restrict__ in, int K, int KP, int scene_rows, in
         }
       } else {
         const T* src[16];
+        unsigned okm = 0xffffu;                                 // bit jj: pixel jj's source pixel has data
 #pragma unroll
         for (int jj = 0; jj < 16; ++jj) {
           int pp = int(p0) + warp + 8 * jj; if (pp >= int(plane)) pp = int(plane) - 1;     // plane < 2^31 (launcher)
           const int pr = pp / pcol_n, pc = pp - pr * pcol_n;
           const int sr = mirror_index(band_row0 + pr + lo, scene_rows) - slab_row0, sc = mirror_index(pc + lo, cols);
           src[jj] = in + (int64_t(sr) * cols + sc) * K;
+          if (valid && !valid[int64_t(sr) * cols + sc]) okm &= ~(1u << jj);
         }
 #pragma unroll 1
         for (int j = 0; j < nslice; ++j, ++g) {
@@ -459,7 +471,7 @@ conv0_tc_sliced_body(const T* __restrict__ in, int K, int KP, int scene_rows, in
 #pragma unroll
               for (int m = 0; m < 2; ++m) {
                 const int kl = lane + 32 * m;                    // band within the slice
-                const float z = (v[jj][m] - (m ? m1 : m0)) * (m ? i1 : i0);       // 0 for k >= K
+                const float z = (okm >> (h + jj)) & 1 ? (v[jj][m] - (m ? m1 : m0)) * (m ? i1 : i0) : 0.f;   // 0 for k >= K
                 const __half hi = __float2half_rn(z);
                 unsigned char* d = xs + (kl >> 3) * XCH + pos * 16 + (kl & 7) * 2;
                 *reinterpret_cast<__half*>(d) = hi;
@@ -508,9 +520,10 @@ template <typename T>
 __global__ void __launch_bounds__(c0s::kThreads, 1)
 conv0_tc_sliced_kernel(const T* __restrict__ in, int K, int KP, int scene_rows, int cols, int slab_row0, int w, int band_row0,
                        int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
-                       const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad) {
+                       const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad,
+                       const uint8_t* __restrict__ valid) {
   conv0_tc_sliced_body<T, false>(in, K, KP, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu, inv_sigma,
-                                 f0pad, BandMajor{}, threadIdx.x);
+                                 f0pad, BandMajor{}, valid, threadIdx.x);
 }
 
 // the raw cube in BIL / BSQ
@@ -519,15 +532,16 @@ __global__ void __launch_bounds__(c0s::kThreads, 1)
 conv0_tc_sliced_bm_kernel(const T* __restrict__ in, int K, int KP, int scene_rows, int cols, int slab_row0, int w,
                           int band_row0, int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */,
                           const float* __restrict__ bias, const float* __restrict__ mu, const float* __restrict__ inv_sigma,
-                          __half* __restrict__ f0pad, BandMajor bm) {
+                          __half* __restrict__ f0pad, BandMajor bm, const uint8_t* __restrict__ valid) {
   conv0_tc_sliced_body<T, true>(in, K, KP, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu, inv_sigma,
-                                f0pad, bm, threadIdx.x);
+                                f0pad, bm, valid, threadIdx.x);
 }
 
 template <typename T>
 static int launch_conv0_tc_sliced(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0,
                                   int prow_n, int pcol_n, const float* wt, const float* bias, const float* mu,
-                                  const float* inv_sigma, __half* f0pad, const BandMajor* bm, cudaStream_t s) {
+                                  const float* inv_sigma, __half* f0pad, const BandMajor* bm, const uint8_t* valid,
+                                  cudaStream_t s) {
   const int KP = (K + 15) / 16 * 16;
   CMLPL_CHECK_ARG(K <= c0k::kMaxK, "conv0: K=%d unsupported by the tensor-core kernel (at most %d)", K, c0k::kMaxK);
   CMLPL_CHECK_ARG(mu && inv_sigma, "conv0: the K-sliced kernel needs the band means and 1/sigma");
@@ -540,22 +554,23 @@ static int launch_conv0_tc_sliced(const T* in, int K, int scene_rows, int cols, 
     auto kern = conv0_tc_sliced_bm_kernel<T>;
     CMLPL_MAX_DYN_SMEM(kern, int(smem));
     kern<<<grid, c0s::kThreads, smem, s>>>(in, K, KP, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
-                                           inv_sigma, f0pad, *bm);
+                                           inv_sigma, f0pad, *bm, valid);
   } else {
     auto kern = conv0_tc_sliced_kernel<T>;
     CMLPL_MAX_DYN_SMEM(kern, int(smem));
     kern<<<grid, c0s::kThreads, smem, s>>>(in, K, KP, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
-                                           inv_sigma, f0pad);
+                                           inv_sigma, f0pad, valid);
   }
   CMLPL_CHECK_LAUNCH("conv0_tc_sliced");
   return CMLPL_OK;
 }
 
-// bm: the raw slab is band-major (BIL / BSQ; split operands only), or nullptr for pixel-major
+// bm: the raw slab is band-major (BIL / BSQ; split operands only), or nullptr for pixel-major; valid: the slab's validity
+// mask (split operands only), or nullptr
 template <typename T, bool kVec4, bool kSplit>
 int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0, int prow_n, int pcol_n,
                     const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad,
-                    const BandMajor* bm, cudaStream_t s) {
+                    const BandMajor* bm, const uint8_t* valid, cudaStream_t s) {
   const int KP = (K + 15) / 16 * 16;
   CMLPL_CHECK_ARG(int64_t(prow_n) * pcol_n < (int64_t(1) << 31) - 256, "conv0: band of %d x %d padded positions is too large",
                   prow_n, pcol_n);
@@ -563,8 +578,9 @@ int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0,
   if constexpr (kSplit && !kVec4)
     if (KP > 256)
       return launch_conv0_tc_sliced<T>(in, K, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
-                                       inv_sigma, f0pad, bm, s);
+                                       inv_sigma, f0pad, bm, valid, s);
   CMLPL_CHECK_ARG(!bm || (kSplit && !kVec4), "conv0: band-major input needs the split-operand kernel");
+  CMLPL_CHECK_ARG(!valid || (kSplit && !kVec4), "conv0: a validity mask needs the raw-cube kernel");
   CMLPL_CHECK_ARG(KP <= 256 && (!kVec4 || (K % 4 == 0 && K <= 64)), "conv0: K=%d unsupported by the tensor-core kernel", K);
   const int KC = KP / 8;
   const size_t xhalf = (size_t(KC) * 2064 + 127) / 128 * 128, mult = kSplit ? 2 : 1;
@@ -580,7 +596,7 @@ int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0,
       auto kern = conv0_tc_bm_kernel<T>;
       CMLPL_MAX_DYN_SMEM(kern, int(smem));
       kern<<<grid, c0s::kThreads, smem, s>>>(in, K, KP, nstage, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt,
-                                             bias, mu, inv_sigma, f0pad, *bm);
+                                             bias, mu, inv_sigma, f0pad, *bm, valid);
       CMLPL_CHECK_LAUNCH("conv0_tc_bm");
       return CMLPL_OK;
     }
@@ -588,14 +604,15 @@ int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0,
   auto kern = conv0_tc_kernel<T, kVec4, kSplit>;
   CMLPL_MAX_DYN_SMEM(kern, int(smem));
   kern<<<grid, c0s::kThreads, smem, s>>>(in, K, KP, nstage, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
-                                         inv_sigma, f0pad);
+                                         inv_sigma, f0pad, valid);
   CMLPL_CHECK_LAUNCH("conv0_tc");
   return CMLPL_OK;
 }
 
 #define CMLPL_CONV0_INST(T, kVec4, kSplit)                                                                                 \
   template int launch_conv0_tc<T, kVec4, kSplit>(const T*, int, int, int, int, int, int, int, int, const float*, const float*, \
-                                                 const float*, const float*, __half*, const BandMajor*, cudaStream_t);
+                                                 const float*, const float*, __half*, const BandMajor*, const uint8_t*,   \
+                                                 cudaStream_t);
 CMLPL_CONV0_INST(float, true, false)
 CMLPL_CONV0_INST(float, false, true)
 CMLPL_CONV0_INST(uint16_t, false, true)

@@ -14,27 +14,30 @@ struct StridedA {
   __device__ __forceinline__ void prep(int) {}
   __device__ __forceinline__ float at(int m, int k) const { return __ldg(p + m * rs + k * cs); }
 };
-// rows of the raw cube (uint16 / float32, row stride rs), z-scored on load: A(m,k) = (x[m][k] - mu[k]) * inv_sigma[k]
+// rows of the raw cube (uint16 / float32, row stride rs), z-scored on load: A(m,k) = (x[m][k] - mu[k]) * inv_sigma[k];
+// valid (u8 per row, or nullptr): a no-data row stands in as its band means, a zero row
 template <typename T>
 struct RawZA {
-  const T* p; int64_t rs; const float* mu; const float* inv_sigma;
-  __device__ __forceinline__ void prep(int) {}
+  const T* p; int64_t rs; const float* mu; const float* inv_sigma; const uint8_t* valid;
+  bool ok_;
+  __device__ __forceinline__ void prep(int m) { ok_ = !valid || valid[m]; }
   __device__ __forceinline__ float at(int m, int k) const {
-    return (float(__ldg(p + m * rs + k)) - __ldg(mu + k)) * __ldg(inv_sigma + k);
+    return ok_ ? (float(__ldg(p + m * rs + k)) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
   }
 };
 // the same from a band-major raw slab (BIL / BSQ): pixel m0 + m of the band is row (m0 + m) / cols, column
-// (m0 + m) % cols of the band's rows at p; the k order is RawZA's
+// (m0 + m) % cols of the band's rows at p; the k order and the validity rows (valid[m0 + m]) are RawZA's
 template <typename T>
 struct RawBandZA {
-  const T* p; BandMajor bm; int64_t m0; const float* mu; const float* inv_sigma;
-  int64_t off_;
+  const T* p; BandMajor bm; int64_t m0; const float* mu; const float* inv_sigma; const uint8_t* valid;
+  int64_t off_; bool ok_;
   __device__ __forceinline__ void prep(int m) {
     const int64_t q = m0 + m, r = q / bm.cols;
     off_ = r * bm.rs + (q - r * bm.cols);
+    ok_ = !valid || valid[q];
   }
   __device__ __forceinline__ float at(int, int k) const {
-    return (float(__ldg(p + off_ + k * bm.bs)) - __ldg(mu + k)) * __ldg(inv_sigma + k);
+    return ok_ ? (float(__ldg(p + off_ + k * bm.bs)) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
   }
 };
 struct StridedB {  // B[k][n]

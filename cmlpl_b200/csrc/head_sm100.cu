@@ -6,6 +6,8 @@
 //                            contiguous block the loader moves with cp.async.bulk (UBLKCP) and tcgen05.mma reads as is
 //   spectral_logits_kernel : part = Wc_spe . relu(Wspe . x + b) per hidden quarter, the hidden features never in HBM
 //   head_sum_kernel        : logits = bc + spectral partials + the gathered conv partials of pool2_cls_kernel, argmax
+// valid (raw cube; u8 [n] over the band's pixels, or nullptr): the conversion writes zero rows for no-data pixels (their
+// band means, z-scored), and the head labels them CMLPL_NODATA_LABEL
 #include "common.cuh"
 #include "sm100_ptx.cuh"
 
@@ -35,18 +37,19 @@ __global__ void x16_tile_kernel(const float* __restrict__ X, int64_t n, int B, i
 template <typename T>
 __global__ void x16_tile_raw_kernel(const T* __restrict__ X, int64_t n, int B, int KC, int64_t total,
                                     const float* __restrict__ mu, const float* __restrict__ inv_sigma,
-                                    __half* __restrict__ out) {
+                                    const uint8_t* __restrict__ valid, __half* __restrict__ out) {
   for (int64_t t = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; t < total; t += int64_t(gridDim.x) * blockDim.x) {
     const int row = int(t & 127);
     const int64_t r = t >> 7;
     const int kc = int(r % KC);
     const int64_t p = (r / KC) * 128 + row;
+    const bool in = p < n && (!valid || valid[p]);
     __half2 h[4];
 #pragma unroll
     for (int e = 0; e < 4; ++e) {
       const int k = kc * 8 + 2 * e;
-      const float a = (p < n && k < B) ? (float(X[p * B + k]) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
-      const float b = (p < n && k + 1 < B) ? (float(X[p * B + k + 1]) - __ldg(mu + k + 1)) * __ldg(inv_sigma + k + 1) : 0.f;
+      const float a = (in && k < B) ? (float(X[p * B + k]) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
+      const float b = (in && k + 1 < B) ? (float(X[p * B + k + 1]) - __ldg(mu + k + 1)) * __ldg(inv_sigma + k + 1) : 0.f;
       h[e] = __floats2half2_rn(a, b);
     }
     *reinterpret_cast<uint4*>(out + t * 8) = *reinterpret_cast<uint4*>(h);
@@ -58,7 +61,7 @@ __global__ void x16_tile_raw_kernel(const T* __restrict__ X, int64_t n, int B, i
 template <typename T>
 __global__ void x16_tile_raw_bm_kernel(const T* __restrict__ X, BandMajor bm, int64_t n, int B, int KC, int64_t total,
                                        const float* __restrict__ mu, const float* __restrict__ inv_sigma,
-                                       __half* __restrict__ out) {
+                                       const uint8_t* __restrict__ valid, __half* __restrict__ out) {
   for (int64_t t = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; t < total; t += int64_t(gridDim.x) * blockDim.x) {
     const int row = int(t & 127);
     const int64_t r = t >> 7;
@@ -66,12 +69,13 @@ __global__ void x16_tile_raw_bm_kernel(const T* __restrict__ X, BandMajor bm, in
     const int64_t p = (r / KC) * 128 + row;
     const int64_t pr = p / bm.cols;
     const T* x = X + pr * bm.rs + (p - pr * bm.cols);
+    const bool in = p < n && (!valid || valid[p]);
     __half2 h[4];
 #pragma unroll
     for (int e = 0; e < 4; ++e) {
       const int k = kc * 8 + 2 * e;
-      const float a = (p < n && k < B) ? (float(x[k * bm.bs]) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
-      const float b = (p < n && k + 1 < B) ? (float(x[(k + 1) * bm.bs]) - __ldg(mu + k + 1)) * __ldg(inv_sigma + k + 1) : 0.f;
+      const float a = (in && k < B) ? (float(x[k * bm.bs]) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
+      const float b = (in && k + 1 < B) ? (float(x[(k + 1) * bm.bs]) - __ldg(mu + k + 1)) * __ldg(inv_sigma + k + 1) : 0.f;
       h[e] = __floats2half2_rn(a, b);
     }
     *reinterpret_cast<uint4*>(out + t * 8) = *reinterpret_cast<uint4*>(h);
@@ -297,7 +301,7 @@ template <int NC>
 __global__ void __launch_bounds__(256)
 head_sum_kernel(const float* __restrict__ part, int64_t mtiles, const float* __restrict__ lmap, int cols, int PR2, int PC2,
                 int64_t n, int C, int ncell /* pooled rows: 5 (w = 20) or 2 (w = 11) */, const float* __restrict__ bc,
-                uint8_t* __restrict__ labels, float* __restrict__ logits) {
+                const uint8_t* __restrict__ valid, uint8_t* __restrict__ labels, float* __restrict__ logits) {
   constexpr int NQ = NC / 4;                           // class quads per map entry
   const int64_t p = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
   if (p >= n) return;
@@ -341,7 +345,7 @@ head_sum_kernel(const float* __restrict__ part, int64_t mtiles, const float* __r
       if (z > best) { best = z; arg = c; }
     }
   }
-  labels[p] = uint8_t(arg);
+  labels[p] = (valid && !valid[p]) ? uint8_t(CMLPL_NODATA_LABEL) : uint8_t(arg);
 }
 
 }  // namespace cmlpl
@@ -364,10 +368,10 @@ static bool spectral_logits_plan(int KC, int NC, int* nA, size_t* smem) {
 
 // x16_tile(_raw) + spectral_logits_kernel: x16 is scratch for the fp16 input tiles, part f32 [4][ceil(n/128)*128][NC].
 // dtype: -1 = preprocessed f32 spectra, else the raw sample type (CMLPL_RAW_U16 / F32 / I16); bm: band-major raw rows, or
-// nullptr for pixel-major [n][B]
+// nullptr for pixel-major [n][B]; valid: u8 [n] of the raw rows (no-data pixels convert to zero rows), or nullptr
 int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_t n, int num_features, int num_classes,
-                           int w, const float* mu, const float* inv_sigma, const void* packed, void* x16, float* part,
-                           cmlpl_stream_t stream) {
+                           int w, const float* mu, const float* inv_sigma, const uint8_t* valid, const void* packed,
+                           void* x16, float* part, cmlpl_stream_t stream) {
   CMLPL_CHECK_ARG(x && packed && x16 && part, "spectral_logits_tc: null pointer");
   CMLPL_CHECK_ARG(n > 0 && num_features > 0, "spectral_logits_tc: bad dims");
   CMLPL_CHECK_ARG(num_classes <= 32, "spectral_logits_tc: needs <= 32 classes, got %d", num_classes);
@@ -382,17 +386,17 @@ int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_
   if (dtype < 0)
     x16_tile_kernel<<<int(g), 256, 0, s>>>(static_cast<const float*>(x), n, num_features, KC, total, o);
   else if (bm && dtype == CMLPL_RAW_U16)
-    x16_tile_raw_bm_kernel<uint16_t><<<int(g), 256, 0, s>>>(static_cast<const uint16_t*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, o);
+    x16_tile_raw_bm_kernel<uint16_t><<<int(g), 256, 0, s>>>(static_cast<const uint16_t*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, valid, o);
   else if (bm && dtype == CMLPL_RAW_I16)
-    x16_tile_raw_bm_kernel<int16_t><<<int(g), 256, 0, s>>>(static_cast<const int16_t*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, o);
+    x16_tile_raw_bm_kernel<int16_t><<<int(g), 256, 0, s>>>(static_cast<const int16_t*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, valid, o);
   else if (bm)
-    x16_tile_raw_bm_kernel<float><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, o);
+    x16_tile_raw_bm_kernel<float><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, valid, o);
   else if (dtype == CMLPL_RAW_U16)
-    x16_tile_raw_kernel<uint16_t><<<int(g), 256, 0, s>>>(static_cast<const uint16_t*>(x), n, num_features, KC, total, mu, inv_sigma, o);
+    x16_tile_raw_kernel<uint16_t><<<int(g), 256, 0, s>>>(static_cast<const uint16_t*>(x), n, num_features, KC, total, mu, inv_sigma, valid, o);
   else if (dtype == CMLPL_RAW_I16)
-    x16_tile_raw_kernel<int16_t><<<int(g), 256, 0, s>>>(static_cast<const int16_t*>(x), n, num_features, KC, total, mu, inv_sigma, o);
+    x16_tile_raw_kernel<int16_t><<<int(g), 256, 0, s>>>(static_cast<const int16_t*>(x), n, num_features, KC, total, mu, inv_sigma, valid, o);
   else
-    x16_tile_raw_kernel<float><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), n, num_features, KC, total, mu, inv_sigma, o);
+    x16_tile_raw_kernel<float><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), n, num_features, KC, total, mu, inv_sigma, valid, o);
   CMLPL_CHECK_LAUNCH("x16_tile");
   int grid = sm_count() / 4 * 4;
   if (grid > mtiles * 4) grid = int(mtiles * 4);
@@ -420,14 +424,15 @@ int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_
 // scratch for the fp16 input tiles.
 extern "C" int cmlpl_spectral_logits_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
                                         const void* packed, void* x16, float* part, cmlpl_stream_t stream) {
-  return launch_spectral_logits(spectra, -1, nullptr, n, num_features, num_classes, w, nullptr, nullptr, packed, x16, part, stream);
+  return launch_spectral_logits(spectra, -1, nullptr, n, num_features, num_classes, w, nullptr, nullptr, nullptr, packed, x16,
+                                part, stream);
 }
 
-// Head of the dense path without a GEMM: quarter partials of cmlpl_spectral_logits_tc + the 5 gathered conv partials
-// per pixel from lmap (cmlpl_pool2_cls_f16) + bias, argmax.  Pixels are the band's raster order.
-extern "C" int cmlpl_head_sum_lmap(const float* part, const float* lmap, int cols, int band_rows, int num_features,
-                                   int num_classes, int w, const void* packed, uint8_t* labels, float* logits,
-                                   cmlpl_stream_t stream) {
+namespace cmlpl {
+
+// head_sum_kernel over the band's pixels; valid: u8 [band_rows * cols] (no-data pixels get CMLPL_NODATA_LABEL) or nullptr
+int launch_head_sum(const float* part, const float* lmap, int cols, int band_rows, int num_features, int num_classes, int w,
+                    const void* packed, const uint8_t* valid, uint8_t* labels, float* logits, cmlpl_stream_t stream) {
   CMLPL_CHECK_ARG(part && lmap && packed && labels, "head_sum_lmap: null pointer");
   CMLPL_CHECK_ARG((w == 20 || w == 11) && cols > 0 && band_rows > 0, "head_sum_lmap: bad dims (w must be 20 or 11)");
   CMLPL_CHECK_ARG(num_classes > 0 && num_classes <= 32, "head_sum_lmap: needs 1..32 classes, got %d", num_classes);
@@ -439,9 +444,19 @@ extern "C" int cmlpl_head_sum_lmap(const float* part, const float* lmap, int col
   const int PR2 = (band_rows + w) / 2, PC2 = (cols + w) / 2, ncell = w == 20 ? 5 : 2;
   const float* bc = reinterpret_cast<const float*>(pk + L.bc);
   if (L.nc == 16)
-    head_sum_kernel<16><<<grid, 256, 0, s>>>(part, mtiles, lmap, cols, PR2, PC2, n, num_classes, ncell, bc, labels, logits);
+    head_sum_kernel<16><<<grid, 256, 0, s>>>(part, mtiles, lmap, cols, PR2, PC2, n, num_classes, ncell, bc, valid, labels, logits);
   else
-    head_sum_kernel<32><<<grid, 256, 0, s>>>(part, mtiles, lmap, cols, PR2, PC2, n, num_classes, ncell, bc, labels, logits);
+    head_sum_kernel<32><<<grid, 256, 0, s>>>(part, mtiles, lmap, cols, PR2, PC2, n, num_classes, ncell, bc, valid, labels, logits);
   CMLPL_CHECK_LAUNCH("head_sum");
   return CMLPL_OK;
+}
+
+}  // namespace cmlpl
+
+// Head of the dense path without a GEMM: quarter partials of cmlpl_spectral_logits_tc + the 5 gathered conv partials
+// per pixel from lmap (cmlpl_pool2_cls_f16) + bias, argmax.  Pixels are the band's raster order.
+extern "C" int cmlpl_head_sum_lmap(const float* part, const float* lmap, int cols, int band_rows, int num_features,
+                                   int num_classes, int w, const void* packed, uint8_t* labels, float* logits,
+                                   cmlpl_stream_t stream) {
+  return launch_head_sum(part, lmap, cols, band_rows, num_features, num_classes, w, packed, nullptr, labels, logits, stream);
 }

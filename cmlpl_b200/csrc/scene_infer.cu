@@ -12,6 +12,9 @@
 //                    partials + bias, argmax (hyper_tools.py:426, first index wins ties)
 //   (<= 32 classes and <= 224 bands; otherwise the all-per-pixel patch_cnn_sm100.cu kernel + CUDA-core classify instead,
 //   on both entry points; the raw entry point's CUDA-core spectral head reads the raw band, z-scored on load)
+// With a validity mask (cmlpl_scene_infer_raw_masked) a no-data pixel stands in as its band means wherever it is read:
+// conv0's loaders and the spectral branch's operands z-score it to 0 (so F0 there is the folded bias), and the heads label
+// it CMLPL_NODATA_LABEL.  Everything between conv0 and the heads is unchanged.
 #include "common.cuh"
 #include "gemm_core.cuh"
 
@@ -25,26 +28,30 @@ namespace cmlpl {
 // logit bar).  PCA projection, both z-scores and conv0 are per-pixel affine maps, so they fold into one
 // F0 = Wf . (x - mu) + bf with Wf = W0 . (U/s)^T [64 x B] (SURVEY 8-f1).  Output: mirrored halo baked in, chunk-planar fp16
 // [8 chunks][prow_n][pcol_n][8].
-// bm: a band-major raw slab (BIL / BSQ), or nullptr for pixel-major
+// bm: a band-major raw slab (BIL / BSQ), or nullptr for pixel-major; valid: the raw slab's validity mask, or nullptr
 template <typename T, bool kVec4, bool kSplit>
 int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0, int prow_n, int pcol_n,
                     const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad,
-                    const BandMajor* bm, cudaStream_t s);
+                    const BandMajor* bm, const uint8_t* valid, cudaStream_t s);
 
 // x16_tile(_raw) + spectral_logits_kernel (head_sm100.cu): x is the f32 z-scored spectra (dtype -1) or the raw cube's
 // rows (dtype = the sample type CMLPL_RAW_U16 / F32 / I16, z-scored with mu / inv_sigma in the conversion; band-major
-// through bm, else pixel-major)
+// through bm, else pixel-major; valid: the band's validity mask, or nullptr)
 int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_t n, int num_features, int num_classes,
-                           int w, const float* mu, const float* inv_sigma, const void* packed, void* x16, float* part,
-                           cmlpl_stream_t stream);
+                           int w, const float* mu, const float* inv_sigma, const uint8_t* valid, const void* packed,
+                           void* x16, float* part, cmlpl_stream_t stream);
+// head_sum_kernel (head_sm100.cu) behind cmlpl_head_sum_lmap; valid: the band's validity mask, or nullptr
+int launch_head_sum(const float* part, const float* lmap, int cols, int band_rows, int num_features, int num_classes, int w,
+                    const void* packed, const uint8_t* valid, uint8_t* labels, float* logits, cmlpl_stream_t stream);
 
 // ------------------------------------------------------------------ classifier + argmax
-// one warp per pixel; lanes stride over the K = P*64 pooled features in 8-half chunks.
+// one warp per pixel; lanes stride over the K = P*64 pooled features in 8-half chunks.  valid (u8 [n] or nullptr):
+// no-data pixels are labelled CMLPL_NODATA_LABEL
 template <int CMAX>
 __global__ void __launch_bounds__(256)
 classify_kernel(const __half* __restrict__ p2, const float* __restrict__ spe, const float* __restrict__ part,
                 int64_t part_stride, int part_width, int64_t n, int K, int C,
-                const float* __restrict__ wc, const float* __restrict__ bc,
+                const float* __restrict__ wc, const float* __restrict__ bc, const uint8_t* __restrict__ valid,
                 uint8_t* __restrict__ labels, float* __restrict__ logits) {
   const int lane = threadIdx.x & 31;
   const int64_t warp = blockIdx.x * int64_t(blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -87,7 +94,7 @@ classify_kernel(const __half* __restrict__ p2, const float* __restrict__ spe, co
         if (v > best) { best = v; arg = c; }   // strict '>' : first index wins ties
       }
     }
-    if (lane == 0) labels[p] = uint8_t(arg);
+    if (lane == 0) labels[p] = (valid && !valid[p]) ? uint8_t(CMLPL_NODATA_LABEL) : uint8_t(arg);
   }
 }
 
@@ -193,6 +200,8 @@ struct SceneSrc {
   const void* raw;                         // cmlpl_scene_infer_raw: the raw slab (dtype = sample | interleave) and the
   int dtype;                               // preprocessing folded into conv0 and into the spectral branch (include/cmlpl.h)
   const float *wf, *bf, *mu, *inv_sigma;
+  bool masked;                             // cmlpl_scene_infer_raw_masked: the slab's validity mask u8 [slab_rows * cols]
+  const uint8_t* valid;
 };
 
 // The conv0 map's conditions on the scene geometry (`fn` names the caller): the window fits the scene, the band lies
@@ -220,6 +229,7 @@ static int check_scene(const SceneSrc& src, int scene_rows, int cols, int slab_r
   CMLPL_CHECK_ARG(packed && workspace && labels &&
                       (src.from_raw ? src.raw && src.wf && src.bf && src.mu && src.inv_sigma : src.cube && src.spectra),
                   "%s: null pointer", fn);
+  CMLPL_CHECK_ARG(!src.masked || src.valid, "%s: null valid mask", fn);
   if (src.from_raw) {
     const int rc = check_raw_code(fn, "raw", src.raw, src.dtype);
     if (rc != CMLPL_OK) return rc;
@@ -256,13 +266,18 @@ extern "C" int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, 
   const int prow_n = band_rows + w - 1, pcol_n = cols + w - 1;
   return launch_conv0_tc<float, true, false>(cube, 60, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n,
                                       reinterpret_cast<const float*>(pk + L.w0), reinterpret_cast<const float*>(pk + L.b0), nullptr,
-                                      nullptr, static_cast<__half*>(f0pad), nullptr, static_cast<cudaStream_t>(stream));
+                                      nullptr, static_cast<__half*>(f0pad), nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 // CUDA-core spectral head of the per-pixel path: spe_logits f32 [n][C] = Wc_spe . relu(Wspe . x + bspe), over chunks of
 // `chunk` pixels through the f32 scratch hidden [chunk][1024]
 // `spectra` is StridedA over the z-scored f32 spectra, or RawZA / RawBandZA over the raw band (z-scored on load)
 template <class FA> static FA rows_from(FA a, int64_t s0) { a.p += s0 * a.rs; return a; }          // pixel-major rows
+template <typename T> static RawZA<T> rows_from(RawZA<T> a, int64_t s0) {
+  a.p += s0 * a.rs;
+  if (a.valid) a.valid += s0;
+  return a;
+}
 template <typename T> static RawBandZA<T> rows_from(RawBandZA<T> a, int64_t s0) { a.m0 += s0; return a; }
 template <class FA>
 static int spectral_head(FA spectra, int64_t n, int num_features, int num_classes, int w, const void* packed,
@@ -291,8 +306,8 @@ static int spectral_head(FA spectra, int64_t n, int num_features, int num_classe
 // classify_kernel over the per-pixel pooled features p2, adding the spectral logits spe_logits f32 [n][C] (CUDA-core
 // head) or the tensor-core branch's four quarter partials `part`
 static int classify_launch(const void* p2, const float* spe_logits, const float* part, int64_t part_stride, int64_t n,
-                           int num_features, int num_classes, int w, const void* packed, uint8_t* labels, float* logits,
-                           cudaStream_t s) {
+                           int num_features, int num_classes, int w, const void* packed, const uint8_t* valid,
+                           uint8_t* labels, float* logits, cudaStream_t s) {
   const int part_width = class_width(num_classes);        // row width of spectral_logits_kernel's partials
   const unsigned char* pk = static_cast<const unsigned char*>(packed);
   const PackedLayout L = packed_layout(num_features, num_classes, w);
@@ -304,10 +319,10 @@ static int classify_launch(const void* p2, const float* spe_logits, const float*
   if (grid > cap) grid = cap;
   if (num_classes <= 16)
     classify_kernel<16><<<int(grid), 256, 0, s>>>(static_cast<const __half*>(p2), spe_logits, part, part_stride, part_width, n,
-                                                  K, num_classes, wc, bc, labels, logits);
+                                                  K, num_classes, wc, bc, valid, labels, logits);
   else
     classify_kernel<32><<<int(grid), 256, 0, s>>>(static_cast<const __half*>(p2), spe_logits, part, part_stride, part_width, n,
-                                                  K, num_classes, wc, bc, labels, logits);
+                                                  K, num_classes, wc, bc, valid, labels, logits);
   CMLPL_CHECK_LAUNCH("classify");
   return CMLPL_OK;
 }
@@ -345,9 +360,11 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
   const void* band_spectra =
       src.from_raw ? static_cast<const unsigned char*>(src.raw) + (band_row0 - slab_row0) * row_stride * raw_sample_bytes(src.dtype)
                    : static_cast<const void*>(src.spectra);
+  // the band's validity: band pixel p is slab pixel (band_row0 - slab_row0) * cols + p
+  const uint8_t* band_valid = src.valid ? src.valid + int64_t(band_row0 - slab_row0) * cols : nullptr;
   auto spectral_tc = [&](cudaStream_t st) {
-    return launch_spectral_logits(band_spectra, src.from_raw ? sample : -1, bm, n, B, C, w, src.mu, src.inv_sigma, packed,
-                                  wsb + ws.x16, part, st);
+    return launch_spectral_logits(band_spectra, src.from_raw ? sample : -1, bm, n, B, C, w, src.mu, src.inv_sigma, band_valid,
+                                  packed, wsb + ws.x16, part, st);
   };
   auto conv0 = [&]() {
     if (!src.from_raw)
@@ -357,12 +374,12 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
     __half* f0 = reinterpret_cast<__half*>(wsb + ws.f0pad);
     if (sample == CMLPL_RAW_U16)
       return launch_conv0_tc<uint16_t, false, true>(static_cast<const uint16_t*>(src.raw), B, scene_rows, cols, slab_row0, w,
-                                                    band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, s);
+                                                    band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, src.valid, s);
     if (sample == CMLPL_RAW_I16)
       return launch_conv0_tc<int16_t, false, true>(static_cast<const int16_t*>(src.raw), B, scene_rows, cols, slab_row0, w,
-                                                   band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, s);
+                                                   band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, src.valid, s);
     return launch_conv0_tc<float, false, true>(static_cast<const float*>(src.raw), B, scene_rows, cols, slab_row0, w,
-                                               band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, s);
+                                               band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, src.valid, s);
   };
   if (ws.dense) {
     // The spectral branch (fp16 tiles of the spectra + the two spectral GEMMs) does not depend on the conv tower until
@@ -382,7 +399,7 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
     float* lmap = reinterpret_cast<float*>(wsb + ws.lmap);
     if ((rc = cmlpl_pool2_cls_f16(wsb + ws.yq, cols, w, band_rows, B, C, packed, lmap, stream)) != CMLPL_OK) return rc;
     CMLPL_CUDA(cudaStreamWaitEvent(s, sd->join[0], 0));
-    return cmlpl_head_sum_lmap(part, lmap, cols, band_rows, B, C, w, packed, labels, logits, stream);
+    return launch_head_sum(part, lmap, cols, band_rows, B, C, w, packed, band_valid, labels, logits, stream);
   }
   // per pixel: the tensor-core spectral branch; or the CUDA-core spectral head beyond 224 bands (both entry points) and in
   // path mode 0 at 17-32 classes on the cube entry point, where the workspace holds both branches and the raw entry point
@@ -395,8 +412,10 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
   auto raw_head = [&](auto sample_type) {
     using T = decltype(sample_type);
     const T* x = static_cast<const T*>(band_spectra);
-    return bm ? spectral_head(RawBandZA<T>{x, *bm, 0, src.mu, src.inv_sigma, 0}, n, B, C, w, packed, hidden, ws.chunk, spe, s)
-              : spectral_head(RawZA<T>{x, B, src.mu, src.inv_sigma}, n, B, C, w, packed, hidden, ws.chunk, spe, s);
+    return bm ? spectral_head(RawBandZA<T>{x, *bm, 0, src.mu, src.inv_sigma, band_valid, 0, false}, n, B, C, w, packed, hidden,
+                              ws.chunk, spe, s)
+              : spectral_head(RawZA<T>{x, B, src.mu, src.inv_sigma, band_valid, false}, n, B, C, w, packed, hidden, ws.chunk,
+                              spe, s);
   };
   if (tc)
     rc = spectral_tc(s);
@@ -411,7 +430,7 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
   if (rc != CMLPL_OK) return rc;
   if ((rc = cmlpl_patch_cnn_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.p2, stream)) != CMLPL_OK) return rc;
   return classify_launch(wsb + ws.p2, tc ? nullptr : spe, tc ? part : nullptr, ((n + 127) / 128) * 128, n, B, C, w, packed,
-                         labels, logits, s);
+                         band_valid, labels, logits, s);
 }
 
 extern "C" int cmlpl_scene_infer(const float* cube, int scene_rows, int cols, int slab_row0, int slab_rows,
@@ -436,6 +455,19 @@ extern "C" int cmlpl_scene_infer_raw(const void* raw, int dtype, int scene_rows,
                                      const void* packed, void* workspace, size_t workspace_bytes, uint8_t* labels,
                                      float* logits, cmlpl_stream_t stream) {
   const SceneSrc src{"scene_infer_raw", true, nullptr, nullptr, raw, dtype, wf, bf, mu, inv_sigma};
+  return scene_infer(src, scene_rows, cols, slab_row0, slab_rows, num_features, num_classes, w, band_row0, band_rows, packed,
+                     workspace, workspace_bytes, labels, logits, stream);
+}
+
+// The same with a validity mask valid u8 [slab_rows * cols] (1 = valid, 0 = no-data) over the slab's pixels in raster
+// order: a no-data pixel stands in as its band means wherever it is read (in its neighbours' windows, through the mirror
+// too, and as its own spectral input), and its label is CMLPL_NODATA_LABEL.  Same workspace size and layout.
+extern "C" int cmlpl_scene_infer_raw_masked(const void* raw, int dtype, int scene_rows, int cols, int slab_row0, int slab_rows,
+                                            int num_features, int num_classes, int w, int band_row0, int band_rows,
+                                            const float* wf, const float* bf, const float* mu, const float* inv_sigma,
+                                            const uint8_t* valid, const void* packed, void* workspace,
+                                            size_t workspace_bytes, uint8_t* labels, float* logits, cmlpl_stream_t stream) {
+  const SceneSrc src{"scene_infer_raw_masked", true, nullptr, nullptr, raw, dtype, wf, bf, mu, inv_sigma, true, valid};
   return scene_infer(src, scene_rows, cols, slab_row0, slab_rows, num_features, num_classes, w, band_row0, band_rows, packed,
                      workspace, workspace_bytes, labels, logits, stream);
 }

@@ -11,6 +11,9 @@ from . import _lib
 
 _f32 = torch.float32
 
+# label of a no-data pixel in scene_infer_raw(valid=...) (CMLPL_NODATA_LABEL: never a class, at most 32 classes)
+NODATA_LABEL = 255
+
 
 def _stream():
     return torch.cuda.current_stream().cuda_stream
@@ -212,12 +215,16 @@ def scene_infer(cube, spectra, packed, num_classes: int, w: int = 20, band_row0:
 def scene_infer_raw(raw, folded, packed, num_classes: int, cols: int, w: int = 20, band_row0: int = 0,
                     band_rows: int | None = None, scene_rows: int | None = None, slab_row0: int = 0,
                     want_logits: bool = False, workspace: torch.Tensor | None = None,
-                    labels: torch.Tensor | None = None, interleave: str = "bip"):
+                    labels: torch.Tensor | None = None, interleave: str = "bip", valid: torch.Tensor | None = None):
     """hyper_tools.py:285-292 + :416-437 from the RAW cube: raw uint16 / f32 / int16 holding scene rows slab_row0..
     in the layout ``interleave`` -- "bip" [slab_rows*cols, B] or [slab_rows, cols, B], "bil" [slab_rows, B, cols],
     "bsq" [B, slab_rows, cols] -- and ``folded`` = Preproc.folded_conv0(...) (conv0 folded with PCA + z-scores; band
     mean / 1/std).  Neither the PCA cube nor the z-scored spectra are materialised.  Results do not depend on the
-    interleave."""
+    interleave.
+
+    ``valid`` (u8 [slab_rows, cols], 1 = valid; preprocess.valid_mask or any mask of that layout): a no-data pixel
+    stands in as its band-mean spectrum wherever it is read -- in its neighbours' windows and as its own spectral input
+    -- and is labelled NODATA_LABEL; its logits, when asked for, are those of the imputed pixel."""
     from . import preprocess
     if not raw.is_cuda or not raw.is_contiguous():
         raise _lib.CmlplError("raw must be a contiguous CUDA tensor (cmlpl_b200 has no CPU path)")
@@ -236,10 +243,16 @@ def scene_infer_raw(raw, folded, packed, num_classes: int, cols: int, w: int = 2
     if labels is None:
         labels = torch.empty((n,), dtype=torch.uint8, device=raw.device)
     logits = torch.empty((n, num_classes), dtype=_f32, device=raw.device) if want_logits else None
-    _lib.call("cmlpl_scene_infer_raw", raw.data_ptr(), code, scene_rows, cols, slab_row0, slab_rows, B, num_classes, w,
-              band_row0, band_rows, folded["wf"].data_ptr(), folded["bf"].data_ptr(), folded["mu"].data_ptr(),
-              folded["inv_sigma"].data_ptr(), packed.data_ptr(), workspace.data_ptr(), workspace.numel(),
-              labels.data_ptr(), _p(logits), _stream())
+    pre = (folded["wf"].data_ptr(), folded["bf"].data_ptr(), folded["mu"].data_ptr(), folded["inv_sigma"].data_ptr())
+    post = (packed.data_ptr(), workspace.data_ptr(), workspace.numel(), labels.data_ptr(), _p(logits), _stream())
+    geom = (code, scene_rows, cols, slab_row0, slab_rows, B, num_classes, w, band_row0, band_rows)
+    if valid is None:
+        _lib.call("cmlpl_scene_infer_raw", raw.data_ptr(), *geom, *pre, *post)
+    else:
+        _chk(valid, torch.uint8, "valid")
+        if valid.numel() != slab_rows * cols:
+            raise _lib.CmlplError(f"valid has {valid.numel()} pixels, the slab {slab_rows} x {cols}")
+        _lib.call("cmlpl_scene_infer_raw_masked", raw.data_ptr(), *geom, *pre, valid.data_ptr(), *post)
     return (labels, logits) if want_logits else labels
 
 

@@ -87,9 +87,53 @@ def raw_geometry(shape, interleave: str = "bip", cols: int | None = None, bands:
     return r, c, B
 
 
-def fit(raw: torch.Tensor, n_PC: int = 60, interleave: str = "bip") -> Preproc:
+def _fill_value(raw: torch.Tensor, fill):
+    """The fill value of ``valid_mask`` as the library takes it: None is NaN (non-finite samples only) for float32 and an
+    error for integer cubes."""
+    if fill is None:
+        if raw.dtype != torch.float32:
+            raise _lib.CmlplError(f"valid_mask: a {raw.dtype} cube needs its fill value (fill=None means NaN / Inf only, "
+                                  "for float32)")
+        return float("nan")
+    return float(fill)
+
+
+def valid_mask(raw: torch.Tensor, fill=None, interleave: str = "bip", cols: int | None = None):
+    """No-data pixels of a raw CUDA cube in the layout ``interleave`` (see ``raw_geometry``; a 2-D BIP cube takes ``cols``).
+    A sample is missing when it equals ``fill`` in the sample type, and a float32 sample also when it is not finite (fill
+    None: only then); a pixel with any band missing is no-data.  One read of the cube on the device.
+    -> (valid u8 CUDA [rows, cols] with 1 = valid, n_valid, band_missing int64 [B] = pixels in which each band is missing)."""
+    if not raw.is_cuda or not raw.is_contiguous():
+        raise _lib.CmlplError("valid_mask needs a contiguous CUDA tensor")
+    rows, c, B = raw_geometry(raw.shape, interleave, cols=cols)
+    valid = torch.empty((rows, c), dtype=torch.uint8, device=raw.device)
+    counts = torch.empty(B + 1, dtype=torch.int64, device=raw.device)          # [n_valid, band_missing[B]]
+    mask_into(raw, fill, interleave, rows, c, B, valid, counts)
+    counts = counts.cpu().numpy()
+    return valid, int(counts[0]), counts[1:]
+
+
+def mask_into(raw: torch.Tensor, fill, interleave: str, rows: int, cols: int, B: int, valid: torch.Tensor,
+              counts: torch.Tensor):
+    """valid_mask without a host synchronisation, into caller buffers: valid u8 [rows * cols] and counts int64 [B + 1]
+    (n_valid, then band_missing), on the current stream.  ``raw`` holds the rows x cols pixels in ``interleave``."""
+    _lib.call("cmlpl_valid_mask_u8", raw.data_ptr(), _dtype_code(raw) | INTERLEAVE[interleave], rows, cols, B,
+              _fill_value(raw, fill), valid.data_ptr(), counts.data_ptr(), counts.data_ptr() + 8,
+              torch.cuda.current_stream().cuda_stream)
+
+
+def _check_valid(valid: torch.Tensor, n: int, what: str):
+    if not valid.is_cuda or valid.dtype != torch.uint8 or not valid.is_contiguous() or valid.numel() != n:
+        raise _lib.CmlplError(f"{what}: valid must be a contiguous uint8 CUDA mask of {n} pixels, got {valid.dtype} "
+                              f"{list(valid.shape)}")
+
+
+def fit(raw: torch.Tensor, n_PC: int = 60, interleave: str = "bip", valid: torch.Tensor | None = None,
+        fill=None) -> Preproc:
     """raw: CUDA tensor (uint16, float32 or int16) in the layout ``interleave`` (see ``raw_geometry``).  Moments in
-    float64 on device, SVD on the host."""
+    float64 on device, SVD on the host.  ``valid`` (u8 [rows, cols], ``valid_mask``) or ``fill`` (its mask is built
+    here): the moments of the valid pixels only.  Fewer than 2 valid pixels raise an error that names the bands missing
+    in every pixel (known when ``fill`` is given)."""
     if not raw.is_cuda or not raw.is_contiguous():
         raise _lib.CmlplError("fit needs a contiguous CUDA tensor")
     rows, cols, B = raw_geometry(raw.shape, interleave)
@@ -97,7 +141,22 @@ def fit(raw: torch.Tensor, n_PC: int = 60, interleave: str = "bip") -> Preproc:
     mean = torch.empty(B, dtype=torch.float64, device=raw.device)
     gram = torch.empty(B, B, dtype=torch.float64, device=raw.device)
     stream = torch.cuda.current_stream().cuda_stream
-    if interleave == "bip":                                       # one pixel per row: the int64 pixel count
+    band_missing = None
+    if fill is not None:
+        if valid is not None:
+            raise _lib.CmlplError("fit: pass valid= or fill=, not both")
+        valid, _, band_missing = valid_mask(raw, fill, interleave)
+    if valid is not None:
+        _check_valid(valid, n, "fit")
+        count = torch.empty(1, dtype=torch.int64, device=raw.device)
+        _lib.call("cmlpl_preprocess_fit_masked_f64", raw.data_ptr(), _dtype_code(raw) | INTERLEAVE[interleave], rows, cols,
+                  B, valid.data_ptr(), mean.data_ptr(), gram.data_ptr(), count.data_ptr(), stream)
+        n = int(count.item())
+        if n < 2:
+            every = [] if band_missing is None else [int(b) for b in np.flatnonzero(band_missing == rows * cols)]
+            raise _lib.CmlplError(f"fit: {n} valid pixels of {rows * cols}; the moments need at least 2"
+                                  + (f"; bands missing in every pixel: {every}" if every else ""))
+    elif interleave == "bip":                                     # one pixel per row: the int64 pixel count
         _lib.call("cmlpl_preprocess_fit_f64", raw.data_ptr(), _dtype_code(raw), n, B, mean.data_ptr(), gram.data_ptr(),
                   stream)
     else:
@@ -112,8 +171,9 @@ def fit(raw: torch.Tensor, n_PC: int = 60, interleave: str = "bip") -> Preproc:
 
 
 def apply(raw: torch.Tensor, pp: Preproc, want_spectra: bool = True, cube: torch.Tensor | None = None,
-          spectra: torch.Tensor | None = None):
-    """raw CUDA [N, B] (BIP) -> (cube f32 [N, n_PC], spectra f32 [N, B] or None)."""
+          spectra: torch.Tensor | None = None, valid: torch.Tensor | None = None):
+    """raw CUDA [N, B] (BIP) -> (cube f32 [N, n_PC], spectra f32 [N, B] or None).  ``valid`` (u8 [N] or [rows, cols]):
+    a no-data pixel is written as its band means, i.e. spectra row 0 and cube row -shift."""
     if not raw.is_cuda or not raw.is_contiguous():
         raise _lib.CmlplError("apply needs a contiguous CUDA tensor")
     n, B = raw.shape
@@ -123,7 +183,12 @@ def apply(raw: torch.Tensor, pp: Preproc, want_spectra: bool = True, cube: torch
         cube = torch.empty((n, npc), dtype=torch.float32, device=raw.device)
     if want_spectra and spectra is None:
         spectra = torch.empty((n, B), dtype=torch.float32, device=raw.device)
-    _lib.call("cmlpl_preprocess_apply", raw.data_ptr(), _dtype_code(raw), n, B, npc, d["mu"].data_ptr(),
-              d["inv_sigma"].data_ptr(), d["Us"].data_ptr(), d["shift"].data_ptr(), cube.data_ptr(),
-              spectra.data_ptr() if want_spectra else None, torch.cuda.current_stream().cuda_stream)
+    args = (raw.data_ptr(), _dtype_code(raw), n, B, npc, d["mu"].data_ptr(), d["inv_sigma"].data_ptr(), d["Us"].data_ptr(),
+            d["shift"].data_ptr())
+    outs = (cube.data_ptr(), spectra.data_ptr() if want_spectra else None, torch.cuda.current_stream().cuda_stream)
+    if valid is None:
+        _lib.call("cmlpl_preprocess_apply", *args, *outs)
+    else:
+        _check_valid(valid, n, "apply")
+        _lib.call("cmlpl_preprocess_apply_masked", *args, valid.data_ptr(), *outs)
     return cube, (spectra if want_spectra else None)

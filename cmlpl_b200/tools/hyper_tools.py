@@ -254,10 +254,15 @@ class StreamedRawScene:
 
     ``interleave`` is the host cube's layout, kept on the device: "bip" [(s1-s0)*cols, B], "bil" [s1-s0, B, cols]
     (a row band is contiguous) or "bsq" [B, s1-s0, cols] (a row band is B plane segments, moved by one 2-D copy).
-    ``h2d_bytes`` is the number of bytes the last call copied to the device."""
+    ``h2d_bytes`` is the number of bytes the last call copied to the device.
+
+    ``fill`` (a value of the sample type; NaN for float32 = non-finite samples only): the cube has no-data pixels.  The
+    slab's validity mask is built on the device from the rows each copy brought (BSQ: from the whole slab once its last
+    rows have landed, since a BSQ row band is not a cube of its own), so nothing more crosses PCIe; the calls run
+    cmlpl_scene_infer_raw_masked and need ``folded=``.  No-data pixels get ops.NODATA_LABEL."""
 
     def __init__(self, preproc, scene_rows, cols, num_features, num_classes, w=20, nsplit=2, row0=0, rows=None,
-                 raw_dtype=torch.uint16, device=None, interleave="bip"):
+                 raw_dtype=torch.uint16, device=None, interleave="bip", fill=None):
         from .. import preprocess
         self._pp_mod, self.pp = preprocess, preproc
         self.R, self.C, self.B, self.K, self.w = scene_rows, cols, num_features, num_classes, w
@@ -274,8 +279,12 @@ class StreamedRawScene:
         shape = {"bip": (ns, num_features), "bil": (sr, num_features, cols), "bsq": (num_features, sr, cols)}
         if interleave not in shape:
             raise _lib.CmlplError(f"interleave must be one of {sorted(shape)}, got {interleave!r}")
-        self.interleave, self.h2d_bytes = interleave, 0
+        self.interleave, self.h2d_bytes, self.fill = interleave, 0, fill
+        if fill is not None:
+            preprocess._fill_value(torch.empty(0, dtype=raw_dtype), fill)        # an integer cube needs a fill value
         self.sets = [dict(raw=torch.empty(shape[interleave], dtype=raw_dtype, device=dev), cube=None, spectra=None,
+                          valid=torch.empty((sr, cols), dtype=torch.uint8, device=dev) if fill is not None else None,
+                          counts=torch.empty(num_features + 1, dtype=torch.int64, device=dev),
                           labels=torch.empty((n,), dtype=torch.uint8, device=dev),
                           labels_host=torch.empty((n,), dtype=torch.uint8).pin_memory(),
                           done=torch.cuda.Event()) for _ in range(2)]
@@ -298,6 +307,8 @@ class StreamedRawScene:
         il = self.interleave
         if folded is None and il != "bip":
             raise _lib.CmlplError(f"StreamedRawScene: a {il.upper()} cube needs folded= (preprocess.apply reads BIP)")
+        if folded is None and self.fill is not None:
+            raise _lib.CmlplError("StreamedRawScene: a cube with a fill value needs folded= (cmlpl_scene_infer_raw_masked)")
         want = self.sets[0]["raw"]
         if il != "bip" and (raw_host.shape != want.shape or raw_host.dtype != want.dtype or not raw_host.is_contiguous()):
             raise _lib.CmlplError(f"StreamedRawScene: raw_host must be contiguous {want.dtype} {list(want.shape)}, "
@@ -330,13 +341,21 @@ class StreamedRawScene:
                         self.h2d_bytes += src.nbytes
                     copied = upto
                 ev.record(self.copy_stream)
-        for (a, b), ev, (c0, c1) in zip(self.bands, events, spans):
+        for i, ((a, b), ev, (c0, c1)) in enumerate(zip(self.bands, events, spans)):
             main.wait_event(ev)
             qa, qb = (a - self.r0) * C, (b - self.r0) * C
+            if self.fill is not None:                         # the validity of the rows that just arrived
+                ra, rb = c0 - self.s0, c1 - self.s0
+                if il == "bsq" and i == 0:
+                    main.wait_event(events[-1])
+                    self._pp_mod.mask_into(raw, self.fill, il, sr, C, self.B, S["valid"], S["counts"])
+                elif il != "bsq" and rb > ra:
+                    rows = raw[ra * C:rb * C] if il == "bip" else raw[ra:rb]
+                    self._pp_mod.mask_into(rows, self.fill, il, rb - ra, C, self.B, S["valid"][ra:rb], S["counts"])
             if folded is not None:
                 ops.scene_infer_raw(S["raw"], folded, packed, self.K, C, self.w, band_row0=a, band_rows=b - a,
                                     scene_rows=self.R, slab_row0=self.s0, workspace=self.ws, labels=S["labels"][qa:qb],
-                                    interleave=il)
+                                    interleave=il, valid=S["valid"])
                 continue
             if c1 > c0:                                       # preprocess the rows that just arrived
                 pa, pb = (c0 - self.s0) * C, (c1 - self.s0) * C

@@ -183,6 +183,37 @@ int cmlpl_scene_infer_raw(const void* raw, int dtype, int scene_rows, int cols, 
                           const void* packed, void* workspace, size_t workspace_bytes,
                           uint8_t* labels, float* logits, cmlpl_stream_t stream);
 
+/* No-data pixels of raw sensor cubes (swath edges, dropped scan lines, masked detectors).
+ *   missing sample  equal to the fill value, compared in the sample type; a float32 sample that is not finite is
+ *                   always missing
+ *   no-data pixel   a pixel with ANY band missing (every pixel is used whole or imputed whole)
+ *   validity mask   u8 [rows, cols] in raster order over the raw slab's rows, whatever the interleave: 1 = valid,
+ *                   0 = no-data.  Any mask of this layout works in its place (a cloud or water mask).
+ *   imputation      a no-data pixel stands in as its band-mean spectrum x = mu wherever it is read: in every
+ *                   neighbour's window (through the mirror at scene edges too), as its own spectral input (z-scored
+ *                   spectrum 0), and in cmlpl_preprocess_apply_masked's outputs (spectra row 0, PCA row -shift).  Its
+ *                   label is CMLPL_NODATA_LABEL; its logits, when requested, are those of the imputed pixel.
+ * At most 32 classes, so CMLPL_NODATA_LABEL is never a class and cmlpl_confusion_i64 never counts it. */
+#define CMLPL_NODATA_LABEL 255
+
+/* Validity mask of a raw cube of `rows` x `cols` pixels (any CMLPL_RAW_* code; BIP rows may be pixels with cols = 1,
+ * BSQ planes hold `rows` rows) in one read of the cube: valid u8 [rows*cols], *n_valid i64 = its number of valid
+ * pixels, band_missing i64 [B] (or NULL) = the number of pixels in which band b is missing, e.g. a band that is fill
+ * everywhere.  `fill` must be a value of the sample type (CMLPL_ERR_ARG otherwise, e.g. -9999 for uint16, 0.5 for
+ * int16); for float32, fill = NaN marks the non-finite samples only.  At most 8192 bands. */
+int cmlpl_valid_mask_u8(const void* raw, int dtype, int64_t rows, int cols, int B, double fill, uint8_t* valid,
+                        int64_t* n_valid, int64_t* band_missing, cmlpl_stream_t stream);
+
+/* cmlpl_scene_infer_raw with the slab's validity mask valid u8 [slab_rows*cols] (cmlpl_valid_mask_u8, or the caller's):
+ * no-data pixels are imputed as above and labelled CMLPL_NODATA_LABEL.  conv0's loaders and the spectral branch's
+ * operands read the mask; a pixel whose window (after mirroring) holds no no-data pixel gets exactly the logits of
+ * cmlpl_scene_infer_raw.  Same workspace, checks before anything is enqueued (a NULL valid included). */
+int cmlpl_scene_infer_raw_masked(const void* raw, int dtype, int scene_rows, int cols, int slab_row0, int slab_rows,
+                                 int num_features, int num_classes, int w, int band_row0, int band_rows,
+                                 const float* wf, const float* bf, const float* mu, const float* inv_sigma,
+                                 const uint8_t* valid, const void* packed, void* workspace, size_t workspace_bytes,
+                                 uint8_t* labels, float* logits, cmlpl_stream_t stream);
+
 /* Individual stages of cmlpl_scene_infer (exposed for tests / profiling). */
 int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, int slab_row0, int slab_rows,
                         int w, int band_row0, int band_rows, const void* packed,
@@ -241,9 +272,18 @@ int cmlpl_preprocess_fit_cube_f64(const void* x, int dtype, int rows, int cols, 
                                   cmlpl_stream_t stream);
 int cmlpl_preprocess_fit_f64(const void* x, int dtype, int64_t n, int B, double* mean, double* gram,
                              cmlpl_stream_t stream);
+/* The fit over the valid pixels only (valid u8 [rows*cols], cmlpl_valid_mask_u8): mean and Gram sum over the pixels
+ * with a nonzero byte, *n_valid i64 (device) = their number; np.cov = gram/(n_valid-1), sigma^2 = diag(gram)/n_valid.
+ * Any raw code, as cmlpl_preprocess_fit_cube_f64 (BIP: rows = pixels and cols = 1 works too). */
+int cmlpl_preprocess_fit_masked_f64(const void* raw, int dtype, int64_t rows, int cols, int B, const uint8_t* valid,
+                                    double* mean, double* gram, int64_t* n_valid, cmlpl_stream_t stream);
 int cmlpl_preprocess_apply(const void* x, int dtype, int64_t n, int B, int npc, const float* mu,
                            const float* inv_sigma, const float* Us, const float* shift, float* cube,
                            float* spectra, cmlpl_stream_t stream);
+/* apply with valid u8 [n]: a no-data pixel is written as its band means, spectra row 0 and cube row -shift. BIP only. */
+int cmlpl_preprocess_apply_masked(const void* x, int dtype, int64_t n, int B, int npc, const float* mu,
+                                  const float* inv_sigma, const float* Us, const float* shift, const uint8_t* valid,
+                                  float* cube, float* spectra, cmlpl_stream_t stream);
 
 /* ------------------------------------------------------------------ metrics --
  * tools/hyper_tools.py:208-223 (CalAccuracy): integer confusion matrix
