@@ -92,6 +92,14 @@ inline int check_raw_code(const char* fn, const char* what, const void* p, int d
                   fn, what, raw_sample_bytes(dtype));
   return CMLPL_OK;
 }
+// f(sample) with a value of the code's sample type: uint16_t, int16_t or float
+template <class F> auto with_sample(int dtype, F&& f) {
+  switch (dtype & 0x0f) {
+    case CMLPL_RAW_U16: return f(uint16_t{});
+    case CMLPL_RAW_I16: return f(int16_t{});
+    default: return f(float{});
+  }
+}
 // Strides of a BIL / BSQ cube of B bands whose planes hold plane_rows rows of cols samples (BIP is not band-major)
 inline BandMajor band_major(int dtype, int B, int64_t plane_rows, int cols) {
   return (dtype & 0xf0) == CMLPL_RAW_BSQ ? BandMajor{cols, int64_t(cols), plane_rows * cols}

@@ -1,7 +1,7 @@
 // Tensor-core head of the scene path (sm_100a): the spectral branch relu(feat_spe(x)) (tools/models.py:142-143)
 // and its classifier columns (models.py:150) as two chained tcgen05 GEMMs with fp16 operands / fp32 accumulate,
 // then the sum of all logit partials + argmax (models.py:144,150; hyper_tools.py:426).
-//   x16_tile(_raw)_kernel  : spectra (or the z-scored raw cube) -> fp16 A-operand tiles in the UMMA "no-swizzle
+//   x16_tile_kernel        : spectra (or the z-scored raw cube) -> fp16 A-operand tiles in the UMMA "no-swizzle
 //                            K-major" layout [m-tile][K/8 chunks][128 rows][8 halves], so that a tile is one
 //                            contiguous block the loader moves with cp.async.bulk (UBLKCP) and tcgen05.mma reads as is
 //   spectral_logits_kernel : part = Wc_spe . relu(Wspe . x + b) per hidden quarter, the hidden features never in HBM
@@ -14,68 +14,37 @@
 namespace cmlpl {
 
 // ------------------------------------------------------------------ spectra -> fp16 tiles
-__global__ void x16_tile_kernel(const float* __restrict__ X, int64_t n, int B, int KC, int64_t total,
-                                __half* __restrict__ out) {
+// kZ false: the preprocessed f32 spectra.  kZ: the raw cube, x16 = (raw - mu) * inv_sigma (featureNormalize(X, 1),
+// hyper_tools.py:292), zero rows for no-data pixels.  Band k of pixel p is at p * B + k (pixel-major), or for a
+// band-major slab (kBM: BIL / BSQ, include/cmlpl.h) at row p / cols, column p % cols of the band's rows at X, band
+// stride bm.bs; with rows as the fastest index, a warp's loads of one band are consecutive columns
+template <typename T, bool kBM, bool kZ>
+__global__ void x16_tile_kernel(const T* __restrict__ X, BandMajor bm, int64_t n, int B, int KC, int64_t total,
+                                const float* __restrict__ mu, const float* __restrict__ inv_sigma,
+                                const uint8_t* __restrict__ valid, __half* __restrict__ out) {
   for (int64_t t = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; t < total; t += int64_t(gridDim.x) * blockDim.x) {
     const int row = int(t & 127);
     const int64_t r = t >> 7;
     const int kc = int(r % KC);
     const int64_t p = (r / KC) * 128 + row;
-    __half2 h[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const int k = kc * 8 + 2 * e;
-      const float a = (p < n && k < B) ? __ldg(X + p * B + k) : 0.f;
-      const float b = (p < n && k + 1 < B) ? __ldg(X + p * B + k + 1) : 0.f;
-      h[e] = __floats2half2_rn(a, b);
+    const T* x;                                              // the pixel's band 0
+    if constexpr (kBM) {
+      const int64_t pr = p / bm.cols;
+      x = X + pr * bm.rs + (p - pr * bm.cols);
+    } else {
+      x = X + p * B;
     }
-    *reinterpret_cast<uint4*>(out + t * 8) = *reinterpret_cast<uint4*>(h);
-  }
-}
-
-// same from the raw cube: x16 = (raw - mu) * inv_sigma  (featureNormalize(X, 1), hyper_tools.py:292)
-template <typename T>
-__global__ void x16_tile_raw_kernel(const T* __restrict__ X, int64_t n, int B, int KC, int64_t total,
-                                    const float* __restrict__ mu, const float* __restrict__ inv_sigma,
-                                    const uint8_t* __restrict__ valid, __half* __restrict__ out) {
-  for (int64_t t = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; t < total; t += int64_t(gridDim.x) * blockDim.x) {
-    const int row = int(t & 127);
-    const int64_t r = t >> 7;
-    const int kc = int(r % KC);
-    const int64_t p = (r / KC) * 128 + row;
-    const bool in = p < n && (!valid || valid[p]);
+    const bool in = p < n && (!kZ || !valid || valid[p]);
+    auto at = [&](int k) -> float {                          // band k of the pixel, z-scored from the raw cube
+      if constexpr (!kZ) return __ldg(x + k);
+      else return (float(x[kBM ? k * bm.bs : k]) - __ldg(mu + k)) * __ldg(inv_sigma + k);
+    };
     __half2 h[4];
 #pragma unroll
     for (int e = 0; e < 4; ++e) {
       const int k = kc * 8 + 2 * e;
-      const float a = (in && k < B) ? (float(X[p * B + k]) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
-      const float b = (in && k + 1 < B) ? (float(X[p * B + k + 1]) - __ldg(mu + k + 1)) * __ldg(inv_sigma + k + 1) : 0.f;
-      h[e] = __floats2half2_rn(a, b);
-    }
-    *reinterpret_cast<uint4*>(out + t * 8) = *reinterpret_cast<uint4*>(h);
-  }
-}
-
-// same from a band-major raw slab (BIL / BSQ, include/cmlpl.h): pixel p of the band is row p / cols, column p % cols of
-// the band's rows at X; with rows as the fastest index, a warp's loads of one band are consecutive columns
-template <typename T>
-__global__ void x16_tile_raw_bm_kernel(const T* __restrict__ X, BandMajor bm, int64_t n, int B, int KC, int64_t total,
-                                       const float* __restrict__ mu, const float* __restrict__ inv_sigma,
-                                       const uint8_t* __restrict__ valid, __half* __restrict__ out) {
-  for (int64_t t = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; t < total; t += int64_t(gridDim.x) * blockDim.x) {
-    const int row = int(t & 127);
-    const int64_t r = t >> 7;
-    const int kc = int(r % KC);
-    const int64_t p = (r / KC) * 128 + row;
-    const int64_t pr = p / bm.cols;
-    const T* x = X + pr * bm.rs + (p - pr * bm.cols);
-    const bool in = p < n && (!valid || valid[p]);
-    __half2 h[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const int k = kc * 8 + 2 * e;
-      const float a = (in && k < B) ? (float(x[k * bm.bs]) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
-      const float b = (in && k + 1 < B) ? (float(x[(k + 1) * bm.bs]) - __ldg(mu + k + 1)) * __ldg(inv_sigma + k + 1) : 0.f;
+      const float a = (in && k < B) ? at(k) : 0.f;
+      const float b = (in && k + 1 < B) ? at(k + 1) : 0.f;
       h[e] = __floats2half2_rn(a, b);
     }
     *reinterpret_cast<uint4*>(out + t * 8) = *reinterpret_cast<uint4*>(h);
@@ -366,7 +335,7 @@ static bool spectral_logits_plan(int KC, int NC, int* nA, size_t* smem) {
   return false;
 }
 
-// x16_tile(_raw) + spectral_logits_kernel: x16 is scratch for the fp16 input tiles, part f32 [4][ceil(n/128)*128][NC].
+// x16_tile + spectral_logits_kernel: x16 is scratch for the fp16 input tiles, part f32 [4][ceil(n/128)*128][NC].
 // dtype: -1 = preprocessed f32 spectra, else the raw sample type (CMLPL_RAW_U16 / F32 / I16); bm: band-major raw rows, or
 // nullptr for pixel-major [n][B]; valid: u8 [n] of the raw rows (no-data pixels convert to zero rows), or nullptr
 int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_t n, int num_features, int num_classes,
@@ -384,19 +353,18 @@ int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_
   int64_t g = (total + 255) / 256; const int64_t cap = int64_t(sm_count()) * 16; if (g > cap) g = cap;
   __half* o = static_cast<__half*>(x16);
   if (dtype < 0)
-    x16_tile_kernel<<<int(g), 256, 0, s>>>(static_cast<const float*>(x), n, num_features, KC, total, o);
-  else if (bm && dtype == CMLPL_RAW_U16)
-    x16_tile_raw_bm_kernel<uint16_t><<<int(g), 256, 0, s>>>(static_cast<const uint16_t*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, valid, o);
-  else if (bm && dtype == CMLPL_RAW_I16)
-    x16_tile_raw_bm_kernel<int16_t><<<int(g), 256, 0, s>>>(static_cast<const int16_t*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, valid, o);
-  else if (bm)
-    x16_tile_raw_bm_kernel<float><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), *bm, n, num_features, KC, total, mu, inv_sigma, valid, o);
-  else if (dtype == CMLPL_RAW_U16)
-    x16_tile_raw_kernel<uint16_t><<<int(g), 256, 0, s>>>(static_cast<const uint16_t*>(x), n, num_features, KC, total, mu, inv_sigma, valid, o);
-  else if (dtype == CMLPL_RAW_I16)
-    x16_tile_raw_kernel<int16_t><<<int(g), 256, 0, s>>>(static_cast<const int16_t*>(x), n, num_features, KC, total, mu, inv_sigma, valid, o);
+    x16_tile_kernel<float, false, false><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), BandMajor{}, n, num_features, KC,
+                                                               total, nullptr, nullptr, nullptr, o);
   else
-    x16_tile_raw_kernel<float><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), n, num_features, KC, total, mu, inv_sigma, valid, o);
+    with_sample(dtype, [&](auto sample) {
+      using T = decltype(sample);
+      const T* xt = static_cast<const T*>(x);
+      if (bm)
+        x16_tile_kernel<T, true, true><<<int(g), 256, 0, s>>>(xt, *bm, n, num_features, KC, total, mu, inv_sigma, valid, o);
+      else
+        x16_tile_kernel<T, false, true><<<int(g), 256, 0, s>>>(xt, BandMajor{}, n, num_features, KC, total, mu, inv_sigma,
+                                                               valid, o);
+    });
   CMLPL_CHECK_LAUNCH("x16_tile");
   int grid = sm_count() / 4 * 4;
   if (grid > mtiles * 4) grid = int(mtiles * 4);

@@ -212,7 +212,7 @@ valid_mask_kernel(const T* __restrict__ x, int64_t n, int B, T fill, bool nan_on
 }
 
 // band-major (BIL / BSQ): a thread owns one pixel of a row and walks its bands, each load coalesced along the warp's
-// consecutive columns (as x16_tile_raw_bm_kernel); rows over blockIdx.y
+// consecutive columns (as x16_tile_kernel); rows over blockIdx.y
 template <typename T>
 __global__ void __launch_bounds__(256)
 valid_mask_bm_kernel(const T* __restrict__ x, BandMajor bm, int rows, int B, T fill, bool nan_only,
@@ -322,13 +322,14 @@ static int fit_cube(const char* fn, const void* x, int dtype, int64_t rows, int 
   CMLPL_CHECK_ARG(rows > 0 && cols > 0 && rows * cols > 1 && B > 0, "%s: bad dims (rows=%lld cols=%d bands=%d)", fn,
                   static_cast<long long>(rows), cols, B);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const int il = dtype & 0xf0, sample = dtype & 0x0f;
+  const int il = dtype & 0xf0;
   const BandMajor bmv = band_major(dtype, B, rows, cols);
   const BandMajor* bm = il == CMLPL_RAW_BIP ? nullptr : &bmv;
   const int64_t r = bm ? rows : rows * cols;                 // pixel-major: one row of cols * B samples per pixel
-  if (sample == CMLPL_RAW_U16) return fit_impl(static_cast<const uint16_t*>(x), bm, r, B, valid, mean, gram, n_valid, s);
-  if (sample == CMLPL_RAW_I16) return fit_impl(static_cast<const int16_t*>(x), bm, r, B, valid, mean, gram, n_valid, s);
-  return fit_impl(static_cast<const float*>(x), bm, r, B, valid, mean, gram, n_valid, s);
+  return with_sample(dtype, [&](auto sample) {
+    using T = decltype(sample);
+    return fit_impl(static_cast<const T*>(x), bm, r, B, valid, mean, gram, n_valid, s);
+  });
 }
 
 // widest spectrum of the mask kernels: their per-band histogram of missing samples sits in shared memory (32 KB)
@@ -371,12 +372,11 @@ static int apply_impl(const char* fn, const void* x, int dtype, int64_t n, int B
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   int64_t grid = (n + 7) / 8; const int64_t cap = int64_t(sm_count()) * 8; if (grid > cap) grid = cap;
   const size_t smem = sizeof(float) * 8 * B;
-  if (dtype == CMLPL_RAW_U16)
-    preprocess_apply_kernel<uint16_t><<<int(grid), 256, smem, s>>>(static_cast<const uint16_t*>(x), n, B, npc, mu, inv_sigma, Us, shift, valid, cube, spectra);
-  else if (dtype == CMLPL_RAW_I16)
-    preprocess_apply_kernel<int16_t><<<int(grid), 256, smem, s>>>(static_cast<const int16_t*>(x), n, B, npc, mu, inv_sigma, Us, shift, valid, cube, spectra);
-  else
-    preprocess_apply_kernel<float><<<int(grid), 256, smem, s>>>(static_cast<const float*>(x), n, B, npc, mu, inv_sigma, Us, shift, valid, cube, spectra);
+  with_sample(dtype, [&](auto sample) {
+    using T = decltype(sample);
+    preprocess_apply_kernel<T><<<int(grid), 256, smem, s>>>(static_cast<const T*>(x), n, B, npc, mu, inv_sigma, Us, shift, valid,
+                                                            cube, spectra);
+  });
   CMLPL_CHECK_LAUNCH("preprocess_apply");
   return CMLPL_OK;
 }
@@ -434,14 +434,12 @@ extern "C" int cmlpl_valid_mask_u8(const void* raw, int dtype, int64_t rows, int
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const BandMajor bmv = band_major(dtype, B, rows, cols);
   const BandMajor* bm = il == CMLPL_RAW_BIP ? nullptr : &bmv;
-  if (sample == CMLPL_RAW_U16)
-    return valid_mask_impl(static_cast<const uint16_t*>(raw), bm, rows, cols, B, uint16_t(fill), false, valid, n_valid,
-                           band_missing, s);
-  if (sample == CMLPL_RAW_I16)
-    return valid_mask_impl(static_cast<const int16_t*>(raw), bm, rows, cols, B, int16_t(fill), false, valid, n_valid,
-                           band_missing, s);
-  return valid_mask_impl(static_cast<const float*>(raw), bm, rows, cols, B, isnan(fill) ? 0.f : float(fill), bool(isnan(fill)),
-                         valid, n_valid, band_missing, s);
+  // (check_fill refuses a NaN fill for the integer types)
+  return with_sample(sample, [&](auto sample_type) {
+    using T = decltype(sample_type);
+    return valid_mask_impl(static_cast<const T*>(raw), bm, rows, cols, B, isnan(fill) ? T(0) : T(fill), bool(isnan(fill)), valid,
+                           n_valid, band_missing, s);
+  });
 }
 
 extern "C" int cmlpl_preprocess_fit_masked_f64(const void* raw, int dtype, int64_t rows, int cols, int B,

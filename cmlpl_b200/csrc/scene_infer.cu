@@ -34,7 +34,7 @@ int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0,
                     const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad,
                     const BandMajor* bm, const uint8_t* valid, cudaStream_t s);
 
-// x16_tile(_raw) + spectral_logits_kernel (head_sm100.cu): x is the f32 z-scored spectra (dtype -1) or the raw cube's
+// x16_tile + spectral_logits_kernel (head_sm100.cu): x is the f32 z-scored spectra (dtype -1) or the raw cube's
 // rows (dtype = the sample type CMLPL_RAW_U16 / F32 / I16, z-scored with mu / inv_sigma in the conversion; band-major
 // through bm, else pixel-major; valid: the band's validity mask, or nullptr)
 int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_t n, int num_features, int num_classes,
@@ -372,14 +372,11 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
                                  wsb + ws.f0pad, stream);
     const int prow_n = band_rows + w - 1, pcol_n = cols + w - 1;
     __half* f0 = reinterpret_cast<__half*>(wsb + ws.f0pad);
-    if (sample == CMLPL_RAW_U16)
-      return launch_conv0_tc<uint16_t, false, true>(static_cast<const uint16_t*>(src.raw), B, scene_rows, cols, slab_row0, w,
-                                                    band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, src.valid, s);
-    if (sample == CMLPL_RAW_I16)
-      return launch_conv0_tc<int16_t, false, true>(static_cast<const int16_t*>(src.raw), B, scene_rows, cols, slab_row0, w,
-                                                   band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, src.valid, s);
-    return launch_conv0_tc<float, false, true>(static_cast<const float*>(src.raw), B, scene_rows, cols, slab_row0, w,
-                                               band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, src.valid, s);
+    return with_sample(sample, [&](auto sample_type) {
+      using T = decltype(sample_type);
+      return launch_conv0_tc<T, false, true>(static_cast<const T*>(src.raw), B, scene_rows, cols, slab_row0, w, band_row0, prow_n,
+                                             pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, src.valid, s);
+    });
   };
   if (ws.dense) {
     // The spectral branch (fp16 tiles of the spectra + the two spectral GEMMs) does not depend on the conv tower until
@@ -421,12 +418,8 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
     rc = spectral_tc(s);
   else if (!src.from_raw)
     rc = spectral_head(StridedA{src.spectra, B, 1}, n, B, C, w, packed, hidden, ws.chunk, spe, s);
-  else if (sample == CMLPL_RAW_U16)
-    rc = raw_head(uint16_t{});
-  else if (sample == CMLPL_RAW_I16)
-    rc = raw_head(int16_t{});
   else
-    rc = raw_head(float{});
+    rc = with_sample(sample, raw_head);
   if (rc != CMLPL_OK) return rc;
   if ((rc = cmlpl_patch_cnn_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.p2, stream)) != CMLPL_OK) return rc;
   return classify_launch(wsb + ws.p2, tc ? nullptr : spe, tc ? part : nullptr, ((n + 127) / 128) * 128, n, B, C, w, packed,

@@ -8,7 +8,7 @@ In one session, alternating the variants round by round:
     makes them) on a WHU-Hi-HongHu-shaped scene, 940 x 475 x 270 with 22 classes, w = 20.  Both take the per-pixel path
     with the CUDA-core spectral head at 270 bands.
 Then, in a separate profiled pass (torch.profiler, CUDA activities), the device time of every kernel of one call of
-each entry point, which gives the raw conv0 stage (conv0_tc_sliced_kernel) on its own.  The scene inputs are seeded
+each entry point, which gives the raw conv0 stage (conv0_tc_kernel, 64-band slices) on its own.  The scene inputs are seeded
 random values: they do not change the work.  Each timing is one window of >= --seconds of back-to-back calls after
 warm-up.  The card's name and power limit are read in the same run.
 
