@@ -12,17 +12,13 @@ import torch
 import torch.nn.functional as F
 
 from oracle import cmlpl_oracle as O
+from scene_harness import rel
 
 pytestmark = pytest.mark.gpu
 REP = [0, 1, 4, 8, 9]
 cls = lambda i: 0 if i == 0 else (2 if i == 9 else 1)
 S = ((1, 2), (0, 1, 2), (0, 1))     # conv1 taps dy (dx) a top / mid / bottom (left / mid / right) patch border keeps
 AB = ((0, 1), (1, 1), (1, 2))       # conv1 border class of the two rows (columns) of a top / mid / bottom pooled cell
-
-
-def rel(a, b):
-    a = a.float(); b = b.float()
-    return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
 
 
 def conv1_pool_planes_ref(f0, W1, b1, PR, PC):

@@ -22,12 +22,11 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from fused_step_harness import assembled, init_nets, make_inputs, oracle_step, random_banks, set_banks, thr_for
 from oracle import cmlpl_oracle as O
 from oracle import golden
+from scene_harness import rel, relu_flips
 from test_fp32_kernels_cpu import U, js_inputs, product_bound, softmax_js_loss_ref
-from test_gpu_fused_step_shapes import random_banks, set_banks
-from test_gpu_train import rel, relu_flips
-import test_gpu_fused_step_w11 as W11
 
 pytestmark = pytest.mark.gpu
 
@@ -650,18 +649,18 @@ def test_fused_adam_many_tensors_empty_and_late(dev):
 # ------------------------------------------------------------------------------------------------ 6. fp32 mutual step
 def test_mutual_step_fp32_honghu_w11(dev, golden_dir):
     """One --fp32_step step at the WHU-Hi HongHu shape (270 bands, 22 classes) on 11 x 11 windows: train.mutual_step
-    against the oracle's ref_step, with the bars of test_gpu_train.py (its relu_flips docstring)."""
+    against the oracle's ref_step, with the bars of test_gpu_train.py (scene_harness.relu_flips's docstring)."""
     from cmlpl_b200 import train as T
     B, K, bs, btu, epoch, batch_index, ptrs, seed = 270, 22, 128, 128, 1, 5, (512, 768), 2711
     ti = golden.load(os.path.join(golden_dir, "train_infer.npz"))
     g = gen(seed)
-    inp = W11.make_inputs(ti, bs, btu, B, K, g)
-    sd, sd1 = W11.init_nets(B, K, seed)
+    inp = make_inputs(ti, bs, btu, B, K, g, 11)
+    sd, sd1 = init_nets(B, K, seed, 11)
     sa = O.StepArgs(num_epochs=20, labeled_batch_size=bs)
     ost = O.make_state(sd, sd1, K, sa)
     queues = random_banks(5 * bs * 2, K, g)
     set_banks(ost, queues, ptrs)
-    sa.thr = W11.thr_for(W11.oracle_step(copy.deepcopy(ost), inp, epoch, batch_index, sa), epoch, sa.num_epochs)
+    sa.thr = thr_for(oracle_step(copy.deepcopy(ost), inp, epoch, batch_index, sa), epoch, sa.num_epochs)
     args = argparse.Namespace(temperature=sa.temperature, thr=sa.thr, num_epochs=sa.num_epochs, queue_batch=sa.queue_batch,
                               alpha=sa.alpha, lr=sa.lr, labeled_batch_size=bs, dropout=0, noise=sa.noise)
     st = T.make_state(B, K, args, dev, w=11)
@@ -671,8 +670,8 @@ def test_mutual_step_fp32_honghu_w11(dev, golden_dir):
         dst.copy_(src)
     st.queue_ptr, st.queue_ptr1 = ptrs
     st.extras["keep_grads"] = True
-    r = W11.oracle_step(ost, inp, epoch, batch_index, sa)
-    patches, spectra = W11.assembled(inp, sa.noise)
+    r = oracle_step(ost, inp, epoch, batch_index, sa)
+    patches, spectra = assembled(inp, sa.noise)
     dd = lambda t: t.to(dev).contiguous()
     hist, aux = T.mutual_step(st, dd(patches[0]), dd(spectra[0]), dd(patches[1]), dd(spectra[1]), dd(inp["Y_l"]), epoch,
                               batch_index, args, drop_masks=(dd(inp["masks"][0]), dd(inp["masks"][1])))

@@ -9,10 +9,10 @@ Bars (north_star: 1e-3 for reduced-precision operands, stated as |d| <= bar * ma
   * convolution gradients end to end against the fp32 oracle: 3e-2.  An fp16-operand forward flips the ReLU mask of
     the few activations that are zero to within 2^-11 (counted and bounded below: < 1e-4 of all mask bits); one flip
     moves a weight gradient -- a sum of ~1e7 signed terms -- by a full term, so this figure measures the flips, not
-    the backward kernels.  (The fp32 path has the same effect at its own precision, see test_gpu_train.relu_flips.)
+    the backward kernels.  (The fp32 path has the same effect at its own precision, see scene_harness.relu_flips.)
 """
 import argparse
-import math
+import functools
 import os
 
 import numpy as np
@@ -20,143 +20,13 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from fused_step_harness import HEAD, compare_with_oracle, cube_mode_steps, make_fused
 from oracle import cmlpl_oracle as O
 from oracle import golden
+from scene_harness import rel
 from test_oracle_cpu import replay_step
 
 pytestmark = pytest.mark.gpu
-
-HEAD = ("feat_spe.weight", "feat_spe.bias", "classifier.weight", "classifier.bias")
-CONV = ("conv0.weight", "conv0.bias", "conv1.weight", "conv1.bias", "conv2.weight", "conv2.bias")
-
-
-def rel(a, b):
-    a = np.asarray(a.detach().cpu() if torch.is_tensor(a) else a, dtype=np.float64)
-    b = np.asarray(b.detach().cpu() if torch.is_tensor(b) else b, dtype=np.float64)
-    return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-30))
-
-
-def planes_to_nchw(buf, ns, npos, h):
-    t = buf.view(torch.float16)[: ns * 8 * npos * 8].view(ns, 8, npos, 8).float()
-    return t.permute(0, 1, 3, 2).reshape(ns, 64, h, h)
-
-
-def bits_to_mask(buf, ns, npos, h):
-    w = buf.view(torch.int32)[: ns * npos * 2].view(ns, npos, 2).cpu().numpy().astype(np.uint32)
-    bits = ((w[..., None] >> np.arange(32, dtype=np.uint32)) & 1).reshape(ns, npos, 64)
-    return torch.from_numpy(bits.astype(np.float32)).permute(0, 2, 1).reshape(ns, 64, h, h)
-
-
-def make_fused(dev, sd, sd1, B, K, queues, **kw):
-    from cmlpl_b200.fused_step import FusedMutualStep
-    from cmlpl_b200.tools.models import BaseNet2
-    nets = [BaseNet2(B, 0, K).to(dev) for _ in range(2)]
-    nets[0].load_state_dict({k: v.detach() for k, v in sd.items()}, strict=False)
-    nets[1].load_state_dict({k: v.detach() for k, v in sd1.items()}, strict=False)
-    fs = FusedMutualStep(nets[0], nets[1], **kw)
-    for dst, src in zip((fs.queue_feats[0], fs.queue_probs[0], fs.queue_feats[1], fs.queue_probs[1]), queues):
-        dst.copy_(src)
-    return fs
-
-
-def linearised_check(fs, w_before, nb, bar=1e-3):
-    """Every convolution-backward kernel against torch fp32 on the kernel's own inputs."""
-    dev = fs.dev
-    lay, ws, ns = fs.workspace_layout(), fs.work, 2 * nb
-    S = fs.grad_scale()
-    x16 = planes_to_nchw(ws[lay["x16"]:], ns, 400, 20)
-    a0 = planes_to_nchw(ws[lay["a0"]:], ns, 400, 20)
-    p1 = planes_to_nchw(ws[lay["p1"]:], ns, 100, 10)
-    m1 = bits_to_mask(ws[lay["m1"]:], ns, 400, 20).to(dev)
-    m2 = bits_to_mask(ws[lay["m2"]:], ns, 100, 10).to(dev)
-    dcat = ws[lay["dcat"]:lay["dcat"] + ns * 2624 * 4].view(torch.float32).view(ns, 2624)
-    dz2 = F.interpolate(dcat[:, :1600].reshape(ns, 64, 5, 5), scale_factor=2, mode="nearest") * 0.25 * m2
-    dz1_k = planes_to_nchw(ws[lay["dz1"]:], ns, 400, 20) / S
-    da0_k = planes_to_nchw(ws[lay["da0"]:], ns, 400, 20) / S
-    worst = {}
-    for e in range(2):
-        sl = slice(e * nb, (e + 1) * nb)
-        W0, W1, W2 = w_before[e]["conv0.weight"], w_before[e]["conv1.weight"], w_before[e]["conv2.weight"]
-        dp1 = F.conv_transpose2d(dz2[sl], W2, padding=1) + dz2[sl]                      # models.py:137-139 backward
-        dz1 = F.interpolate(dp1, scale_factor=2, mode="nearest") * 0.25 * m1[sl]        # :136 pool, :135 ReLU backward
-        da0 = F.conv_transpose2d(dz1_k[sl], W1, padding=1) + dz1_k[sl]                  # :133-135 backward
-        g = dict(zip(("conv0.weight", "conv0.bias", "conv1.weight", "conv1.bias", "conv2.weight", "conv2.bias"),
-                     [fs.grads[e][i] for i in range(6)]))
-        errs = {
-            "dz1": rel(dz1_k[sl], dz1), "da0": rel(da0_k[sl], da0),
-            "conv2.weight": rel(g["conv2.weight"], torch.nn.grad.conv2d_weight(p1[sl], W2.shape, dz2[sl], padding=1)),
-            "conv2.bias": rel(g["conv2.bias"], dz2[sl].sum((0, 2, 3))),
-            "conv1.weight": rel(g["conv1.weight"], torch.nn.grad.conv2d_weight(a0[sl], W1.shape, dz1_k[sl], padding=1)),
-            "conv1.bias": rel(g["conv1.bias"], dz1_k[sl].sum((0, 2, 3))),
-            "conv0.weight": rel(g["conv0.weight"], torch.nn.grad.conv2d_weight(x16[sl, :60], W0.shape, da0_k[sl])),
-            "conv0.bias": rel(g["conv0.bias"], da0_k[sl].sum((0, 2, 3))),
-        }
-        for k, v in errs.items():
-            worst[k] = max(worst.get(k, 0.0), v)
-    print("linearised backward errors:", {k: f"{v:.1e}" for k, v in worst.items()})
-    for k, v in worst.items():
-        assert v < bar, (k, v)
-    return m1, m2
-
-
-def mask_flips(fs, sds, patches, nb):
-    """ReLU-mask bits that differ between the fp16-operand forward and torch fp32 (fraction of all bits)."""
-    lay, ws, ns = fs.workspace_layout(), fs.work, 2 * nb
-    m1 = bits_to_mask(ws[lay["m1"]:], ns, 400, 20)
-    m2 = bits_to_mask(ws[lay["m2"]:], ns, 100, 10)
-    flips = 0
-    for e in range(2):
-        sd = sds[e]
-        a0 = F.conv2d(patches[e], sd["conv0.weight"], sd["conv0.bias"])
-        a1 = F.relu(F.conv2d(a0, sd["conv1.weight"], sd["conv1.bias"], padding=1) + a0)
-        p1 = F.avg_pool2d(a1, 2, 2)
-        a2 = F.relu(F.conv2d(p1, sd["conv2.weight"], sd["conv2.bias"], padding=1) + p1)
-        flips += int(((a1 > 0).float().cpu() != m1[e * nb:(e + 1) * nb]).sum())
-        flips += int(((a2 > 0).float().cpu() != m2[e * nb:(e + 1) * nb]).sum())
-    return flips, flips / float(m1.numel() + m2.numel())
-
-
-def compare_with_oracle(fs, hist, r, ost, w_before, patches, nb, sds_dev, adam=True):
-    """The step-1 bars.  ``adam=False`` skips the Adam block, which compares against the oracle's update from ITS
-    gradients and is only sound from a fresh Adam state (later steps: test_gpu_fused_step_shapes.check_adam_exact)."""
-    h = hist.cpu().numpy()
-    want = np.array([r["hist"][0], r["hist"][1], r["hist"][2], r["hist"][3], r["hist"][4], r["total1"], r["cls1"],
-                     r["con1"], r["lc1"]])
-    assert np.abs(h[:9] - want).max() <= 1e-3 * np.abs(want).max(), (h[:9], want)
-    assert rel(fs.logits[0], r["logits"]) < 1e-3 and rel(fs.logits[1], r["logits1"]) < 1e-3
-    assert rel(fs.feat[0], r["feat"]) < 1e-5 and rel(fs.feat[1], r["feat1"]) < 1e-5          # fp32 branch
-    assert rel(fs.probs[0], r["probs"]) < 1e-3 and rel(fs.probs[1], r["probs1"]) < 1e-3
-    # the threshold compares a max-probability with a constant: allow a flip only where the oracle's own score is
-    # within 1e-3 of the threshold
-    for got, ref_mask, p in ((fs.mask[0], r["mask"], r["probs"]), (fs.mask[1], r["masks"], r["probs1"])):
-        diff = (got.cpu() != ref_mask).nonzero().flatten()
-        for i in diff.tolist():
-            assert abs(float(p[i].max()) - fs.prm.adap_thr) < 1e-3 * fs.prm.adap_thr
-    flips, frac = mask_flips(fs, sds_dev, patches, nb)
-    print("ReLU mask bits differing from the fp32 forward: %d (%.2e of all)" % (flips, frac))
-    assert frac < 1e-4
-    g, g1 = r["grads"], r["grads1"]
-    from cmlpl_b200.fused_step import TENSORS
-    errs = [{k: rel(fs.grads[e][i], (g, g1)[e][k]) for i, k in enumerate(TENSORS)} for e in range(2)]
-    print("gradient errors vs the fp32 oracle:", [{k: f"{v:.1e}" for k, v in d.items()} for d in errs])
-    for d in errs:
-        for k in HEAD:
-            assert d[k] < 1e-3, (k, d[k])
-        for k in CONV:
-            assert d[k] < 3e-2, (k, d[k])
-    linearised_check(fs, w_before, nb)
-    # Adam: compare where the gradient is not ~0 (the first step moves every weight by ~lr*sign(g))
-    for e, sd_new in enumerate((ost.sd, ost.sd1) if adam else ()):
-        for i, k in enumerate(TENSORS):
-            gr = (g, g1)[e][k].numpy()
-            sel = np.abs(gr) > 5e-2 * np.abs(gr).max()
-            new = fs.params[e][i].detach().cpu().numpy()
-            assert np.abs(new - sd_new[k].detach().numpy())[sel].max() < 2e-5, k
-    # memory banks (incl. the queue_ptr1 quirk, train.py:237)
-    assert (fs.queue_ptr, fs.queue_ptr1) == (ost.queue_ptr, ost.queue_ptr1)
-    for t, (qf, qp) in enumerate(((ost.queue_feats, ost.queue_probs), (ost.queue_feats1, ost.queue_probs1))):
-        assert rel(fs.queue_feats[t], qf) < 1e-5 and rel(fs.queue_probs[t], qp) < 1e-3
-
 
 def test_fused_step_matches_oracle_and_fixture(dev, golden_dir):
     """The 128+128 step of tests/golden/step.npz (PaviaU shape, B=103, 9 classes, epoch 1, bank smoothing on)."""
@@ -177,7 +47,7 @@ def test_fused_step_matches_oracle_and_fixture(dev, golden_dir):
     hist = fs.step(inp["Y_l"].to(dev), 1, 0, patches=patches, spectra=spectra)
     # the frozen fixture and the oracle replayed now agree, so one comparison covers both
     assert np.abs(r["hist"] - z["hist"]).max() < 1e-6
-    compare_with_oracle(fs, hist, r, ost, w_before, patches, 256, w_before)
+    compare_with_oracle(fs, hist, r, ost, w_before, patches, 256)
 
 
 def test_both_steps_at_the_indian_pines_shape_with_dropout_masks(dev, golden_dir):
@@ -241,7 +111,7 @@ def test_both_steps_at_the_indian_pines_shape_with_dropout_masks(dev, golden_dir
     patches = torch.stack([XP_b, XP_e]).to(dev).contiguous()
     spectra = torch.stack([X_b, X_e]).to(dev).contiguous()
     hist = fs.step(d(Y_l), 3, 5, patches=patches, spectra=spectra, drop_masks=torch.stack(masks).to(dev))
-    compare_with_oracle(fs, hist, r, ost, w_before, patches, 256, w_before)
+    compare_with_oracle(fs, hist, r, ost, w_before, patches, 256)
 
 
 def test_fused_step_cube_mode_philox_and_graph(dev, golden_dir):
@@ -260,27 +130,7 @@ def test_fused_step_cube_mode_philox_and_graph(dev, golden_dir):
     torch.manual_seed(3)
     nets = [BaseNet2(103, 0.8, 9).to(dev) for _ in range(2)]
     sd0 = [{k: v.detach().clone() for k, v in n.state_dict().items()} for n in nets]
-
-    def run(noise, graph, steps=1, seed=1088, light=False, sync=False):
-        for n, s in zip(nets, sd0):
-            n.load_state_dict(s)
-        fs = FusedMutualStep(nets[0], nets[1], noise=noise, seed=seed, use_graph=graph, thr=0.5)
-        out = []
-        pix_d = pix.to(dev)
-        for it in range(steps):
-            fs.step(labels, 1, it, cube=cube, pix=pix_d, spectra=spectra)
-            if sync:
-                torch.cuda.synchronize()
-            if light:
-                continue
-            lay = fs.workspace_layout()
-            out.append(dict(x16=planes_to_nchw(fs.work[lay["x16"]:], 512, 400, 20).clone(), logits=fs.logits.clone(),
-                            hist=fs.hist.clone(),
-                            dmask=fs.work[lay["dmask"]:lay["dmask"] + 512 * 2624 * 4].view(torch.float32).clone(),
-                            y=fs.work[lay["ynoisy"]:lay["ynoisy"] + 512 * 103 * 4].view(torch.float32).view(512, 103).clone(),
-                            w=[p.detach().clone() for p in fs.params[0]]))
-        return out, fs
-
+    run = functools.partial(cube_mode_steps, nets, sd0, labels, cube, pix, spectra)
     want = torch.from_numpy(O.extract_patches_at(ti["cube_pca"], 20, pix.numpy()))
     clean, _ = run(0.0, False)
     x = clean[0]["x16"]

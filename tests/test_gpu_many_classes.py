@@ -12,36 +12,9 @@ import torch
 import torch.nn.functional as F
 
 from oracle import cmlpl_oracle as O
+from scene_harness import near_ties_only, path_mode, raw_scene, rel, scene_net
 
 pytestmark = pytest.mark.gpu
-
-
-def rel(a, b):
-    a = np.asarray(a, dtype=np.float64); b = np.asarray(b, dtype=np.float64)
-    return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-30))
-
-
-def near_ties_only(lab, lab_ref, log_ref, bar=2e-3):
-    """every label that differs from the reference sits on a reference top-2 margin below the bar"""
-    lab, lab_ref, log_ref = np.asarray(lab), np.asarray(lab_ref), np.asarray(log_ref, dtype=np.float64)
-    diff = lab != lab_ref
-    srt = np.sort(log_ref, 1)
-    return bool(np.all((srt[diff, -1] - srt[diff, -2]) <= bar * np.abs(log_ref).max()))
-
-
-class path_mode:
-    """cmlpl_set_scene_path_mode for a block (the mode is per host thread; 1 is the default)"""
-
-    def __init__(self, mode):
-        self.mode = mode
-
-    def __enter__(self):
-        from cmlpl_b200 import _lib
-        _lib.call("cmlpl_set_scene_path_mode", self.mode)
-
-    def __exit__(self, *exc):
-        from cmlpl_b200 import _lib
-        _lib.call("cmlpl_set_scene_path_mode", 1)
 
 
 def _dense_flag(R, C, B, K, w):
@@ -49,14 +22,6 @@ def _dense_flag(R, C, B, K, w):
     off = (ctypes.c_size_t * 12)()
     _lib.call("cmlpl_scene_workspace_layout", R, C, B, K, w, off)
     return int(off[11])
-
-
-def _net(B, K, w, seed, dev):
-    """random-init BaseNet2 (w = 11: the 1280-input classifier of the odd-window variant) and its cpu state dict"""
-    from cmlpl_b200.tools.models import BaseNet2
-    torch.manual_seed(seed)
-    net = BaseNet2(B, 0, K, w=w).to(dev).eval()
-    return net, {k: v.detach().cpu() for k, v in net.state_dict().items()}
 
 
 @pytest.mark.parametrize("w,B,K", [(20, 48, 20), (20, 103, 17), (20, 144, 24), (20, 224, 32), (11, 103, 20), (11, 224, 32)])
@@ -67,7 +32,7 @@ def test_dense_path_matches_oracle(dev, w, B, K):
     rng = np.random.default_rng(B * 100 + K)
     cube = rng.standard_normal((R, C, 60)).astype(np.float32)
     spectra = rng.standard_normal((R * C, B)).astype(np.float32)
-    net, sd = _net(B, K, w, B + K, dev)
+    net, sd = scene_net(B, K, w, B + K, dev)
     lab_ref, log_ref = O.test_whole(sd, cube, spectra, w, odd_mode=(w == 11), return_logits=True)
     labels, logits = ops.scene_infer(torch.from_numpy(cube).to(dev), torch.from_numpy(spectra).to(dev),
                                      net.packed_weights(w), K, w, want_logits=True)
@@ -85,7 +50,7 @@ def test_cube_path_dense_matches_mode0(dev, K):
     gen = torch.Generator(device=dev); gen.manual_seed(K)
     cube = torch.randn((R, C, 60), device=dev, generator=gen)
     spectra = torch.randn((R * C, B), device=dev, generator=gen)
-    net, _ = _net(B, K, w, K, dev)
+    net, _ = scene_net(B, K, w, K, dev)
     packed = net.packed_weights(w)
     lab1, log1 = ops.scene_infer(cube, spectra, packed, K, w, want_logits=True)
     with path_mode(0):
@@ -97,26 +62,12 @@ def test_cube_path_dense_matches_mode0(dev, K):
     assert near_ties_only(lab1.cpu().numpy(), lab0.cpu().numpy(), l0)
 
 
-def _raw_scene(dev, R, C, B, K, seed):
-    """synthetic raw scene, its float64 oracle preprocessing, and the device preprocessing with the oracle's PCA signs"""
-    from cmlpl_b200 import preprocess, synth
-    cube_u16, _ = synth.synth_scene(R, C, B, K, seed=seed)
-    ref_cube, ref_spec = O.preprocess(cube_u16, 60)
-    raw = torch.from_numpy(cube_u16.reshape(-1, B).copy()).to(dev)
-    pp = preprocess.fit(raw, 60)
-    cube, _ = preprocess.apply(raw, pp, want_spectra=False)
-    sgn = np.sign((cube.cpu().numpy().reshape(R, C, 60) * ref_cube).sum((0, 1)))   # singular vectors: up to sign
-    pp.U = pp.U * sgn[None, :]
-    pp._dev = None
-    return cube_u16, raw, pp, ref_cube.astype(np.float32), ref_spec.astype(np.float32)
-
-
 @pytest.mark.parametrize("K,dtype", [(20, "u16"), (32, "f32")])
 def test_raw_path_dense_and_mode0_match_oracle(dev, K, dtype):
     from cmlpl_b200 import ops
     R, C, B, w = 41, 37, 103, 20
-    _, raw, pp, ref_cube, ref_spec = _raw_scene(dev, R, C, B, K, seed=K)
-    net, sd = _net(B, K, w, 30 + K, dev)
+    _, raw, pp, ref_cube, ref_spec = raw_scene(dev, R, C, B, K, seed=K)
+    net, sd = scene_net(B, K, w, 30 + K, dev)
     packed = net.packed_weights(w)
     folded = pp.folded_conv0(sd["conv0.weight"], sd["conv0.bias"], dev)
     raw_in = raw if dtype == "u16" else raw.float()
@@ -140,14 +91,14 @@ def test_row_bands_are_bit_identical_at_32_classes(dev):
     gen = torch.Generator(device=dev); gen.manual_seed(5)
     cube = torch.randn((R, C, 60), device=dev, generator=gen)
     spectra = torch.randn((R * C, B), device=dev, generator=gen)
-    net, sd = _net(B, K, w, 5, dev)
+    net, sd = scene_net(B, K, w, 5, dev)
     packed = net.packed_weights(w)
     lab, lg = ops.scene_infer(cube, spectra, packed, K, w, want_logits=True)
     bands = [(0, 1), (1, 7), (7, 8), (8, 20), (20, 25), (25, 26)]
     parts = [ops.scene_infer(cube, spectra[a * C:b * C].contiguous(), packed, K, w, band_row0=a, band_rows=b - a, want_logits=True)
              for a, b in bands]
     assert torch.equal(torch.cat([p[0] for p in parts]), lab) and torch.equal(torch.cat([p[1] for p in parts]), lg)
-    _, raw, pp, _, _ = _raw_scene(dev, R, C, B, K, seed=6)
+    _, raw, pp, _, _ = raw_scene(dev, R, C, B, K, seed=6)
     folded = pp.folded_conv0(sd["conv0.weight"], sd["conv0.bias"], dev)
     lab_r, lg_r = ops.scene_infer_raw(raw, folded, packed, K, C, w, want_logits=True)
     parts = []
@@ -166,7 +117,7 @@ def test_pool2_cls_row_maps_match_torch(dev, K):
     R, C, B, w = 37, 45, 103, 20
     rng = np.random.default_rng(K)
     cube = torch.from_numpy(rng.standard_normal((R, C, 60)).astype(np.float32)).to(dev)
-    net, _ = _net(B, K, w, K, dev)
+    net, _ = scene_net(B, K, w, K, dev)
     packed = net.packed_weights(w)
     st = torch.cuda.current_stream().cuda_stream
     PR, PC, PR2, PC2 = R + w - 1, C + w - 1, (R + w) // 2, (C + w) // 2

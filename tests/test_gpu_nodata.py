@@ -16,8 +16,7 @@ import pytest
 import torch
 
 from oracle import cmlpl_oracle as O
-from test_gpu_many_classes import near_ties_only, path_mode, rel
-from test_gpu_raw_layouts import as_layout
+from scene_harness import as_layout, near_ties_only, path_mode, rel, scene_net
 from test_nodata_cpu import (NODATA, masked_params, nodata_pattern, scene_oracle, valid_mask,
                              window_touches, with_nodata)
 from test_sensor_scenes_cpu import apply_bound
@@ -154,13 +153,6 @@ CASES = [(103, 9, 20, 1, "u16", "bip", "wedge"),       # dense path, tensor-core
          (300, 9, 11, 1, "u16", "bil", "edge")]        # K-sliced band-major conv0, w = 11
 
 
-def _net(B, K, w, seed, dev):
-    from cmlpl_b200.tools.models import BaseNet2
-    torch.manual_seed(seed)
-    net = BaseNet2(B, 0, K, w=w).to(dev).eval()
-    return net, {k: v.detach().cpu() for k, v in net.state_dict().items()}
-
-
 @pytest.mark.parametrize("B,K,w,mode,sample,layout,kind", CASES)
 def test_masked_scene_against_the_oracle(dev, B, K, w, mode, sample, layout, kind):
     """4: against the oracle (impute, test_whole, 255): logits within 1e-3 of the largest (no-data pixels: those of the
@@ -171,7 +163,7 @@ def test_masked_scene_against_the_oracle(dev, B, K, w, mode, sample, layout, kin
     R, C = 60, 70
     dirty, valid, fill = _dirty_scene(R, C, B, K, sample, kind, B + K + w)
     ref_pp = masked_params(dirty, valid)
-    net, sd = _net(B, K, w, B * 7 + K, dev)
+    net, sd = scene_net(B, K, w, B * 7 + K, dev)
     lab_ref, log_ref = scene_oracle(sd, dirty, valid, ref_pp, w)
     raw = as_layout(dirty, layout, dev)
     vd = torch.from_numpy(valid).to(dev)
@@ -212,7 +204,7 @@ def test_row_bands_and_streamed_scene(dev, B, K, w, layout, sample):
     dirty, valid, fill = _dirty_scene(R, C, B, K, sample, "edge", B + w)
     dirty[R - 1, 5:9] = with_nodata(dirty[R - 1:, 5:9], np.ones((1, 4), bool), fill)[0]      # the bottom edge too
     valid = valid_mask(dirty, fill)[0]
-    net, _ = _net(B, K, w, B + K, dev)
+    net, _ = scene_net(B, K, w, B + K, dev)
     folded = _pp(masked_params(dirty, valid)).folded_conv0(net.conv0.weight, net.conv0.bias, dev)
     packed = net.packed_weights(w)
     one = ops.scene_infer_raw(as_layout(dirty, layout, dev), folded, packed, K, C, w, want_logits=True, interleave=layout,

@@ -11,13 +11,9 @@ import torch.nn.functional as F
 
 from oracle import cmlpl_oracle as O
 from oracle import golden
+from scene_harness import rel
 
 pytestmark = pytest.mark.gpu
-
-
-def rel(a, b):
-    a = np.asarray(a, dtype=np.float64); b = np.asarray(b, dtype=np.float64)
-    return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-30))
 
 
 def g(golden_dir, name):

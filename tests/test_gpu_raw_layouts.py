@@ -17,15 +17,11 @@ import numpy as np
 import pytest
 import torch
 
+from scene_harness import as_layout, fit_moments
+
 pytestmark = pytest.mark.gpu
 
 LAYOUTS = ("bip", "bil", "bsq")
-
-
-def as_layout(cube, interleave, dev):
-    """[rows, cols, B] numpy cube -> contiguous device tensor in the layout."""
-    a = {"bip": cube.reshape(-1, cube.shape[2]), "bil": cube.transpose(0, 2, 1), "bsq": cube.transpose(2, 0, 1)}[interleave]
-    return torch.from_numpy(np.ascontiguousarray(a)).to(dev)
 
 
 def scene(dev, R, C, B, K, w, seed):
@@ -98,20 +94,6 @@ def test_int16_matches_the_same_values(dev, B, K):
                     infer(as_layout(signed.astype(np.float32), il, dev), il, folded, packed, K, C, w))
         assert_same(infer(as_layout(cube, il, dev), il, folded, packed, K, C, w),
                     infer(as_layout(cube.astype(np.int16), il, dev), il, folded, packed, K, C, w))
-
-
-def fit_moments(raw, code, rows, cols, B):
-    from cmlpl_b200 import _lib
-    mean = torch.empty(B, dtype=torch.float64, device=raw.device)
-    gram = torch.empty(B, B, dtype=torch.float64, device=raw.device)
-    if cols is None:
-        _lib.call("cmlpl_preprocess_fit_f64", raw.data_ptr(), code, rows, B, mean.data_ptr(), gram.data_ptr(),
-                  torch.cuda.current_stream().cuda_stream)
-    else:
-        _lib.call("cmlpl_preprocess_fit_cube_f64", raw.data_ptr(), code, rows, cols, B, mean.data_ptr(), gram.data_ptr(),
-                  torch.cuda.current_stream().cuda_stream)
-    g = gram.cpu().numpy()
-    return mean.cpu().numpy(), np.triu(g) + np.triu(g, 1).T
 
 
 @pytest.mark.parametrize("B", [103, 270])

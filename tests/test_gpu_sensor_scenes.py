@@ -17,8 +17,7 @@ import pytest
 import torch
 
 from oracle import cmlpl_oracle as O
-from test_gpu_many_classes import near_ties_only, path_mode, rel
-from test_gpu_raw_layouts import as_layout, fit_moments
+from scene_harness import as_layout, fit_moments, near_ties_only, path_mode, rel
 from test_sensor_scenes_cpu import apply_bound, conv0_bar
 
 pytestmark = pytest.mark.gpu

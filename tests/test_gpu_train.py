@@ -12,35 +12,10 @@ import torch.nn.functional as F
 
 from oracle import cmlpl_oracle as O
 from oracle import golden
+from scene_harness import rel, relu_flips
 from test_oracle_cpu import replay_step
 
 pytestmark = pytest.mark.gpu
-
-
-def rel(a, b):
-    a = np.asarray(a, dtype=np.float64); b = np.asarray(b, dtype=np.float64)
-    return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-30))
-
-
-def relu_flips(sd, x, y, dev):
-    """Number of ReLU inputs whose sign differs between the CUDA fp32 forward and torch CPU fp32.
-    Summation order moves activations by ~2e-6; an activation that is zero to within that flips its
-    ReLU mask, and ONE flip moves a conv weight gradient (a sum of ~1e5 signed terms) by ~1e-3 of its
-    max.  Gradient bars are therefore 1e-4 when no mask differs and 5e-3 otherwise."""
-    from cmlpl_b200 import ops
-    d = lambda t: t.detach().to(dev).contiguous()
-    a0 = F.conv2d(x, sd["conv0.weight"], sd["conv0.bias"])
-    a1 = F.relu(F.conv2d(a0, sd["conv1.weight"], sd["conv1.bias"], padding=1) + a0)
-    p1 = F.avg_pool2d(a1, 2, 2)
-    a2 = F.relu(F.conv2d(p1, sd["conv2.weight"], sd["conv2.bias"], padding=1) + p1)
-    h = F.relu(F.linear(y, sd["feat_spe.weight"], sd["feat_spe.bias"]))
-    m0 = ops.conv2d(d(x), d(sd["conv0.weight"]), d(sd["conv0.bias"]))
-    m1 = ops.conv2d(m0, d(sd["conv1.weight"]), d(sd["conv1.bias"]), res=m0, relu=True)
-    mp1 = ops.avgpool2(m1)
-    m2 = ops.conv2d(mp1, d(sd["conv2.weight"]), d(sd["conv2.bias"]), res=mp1, relu=True)
-    mh = ops.sgemm(d(y), d(sd["feat_spe.weight"]), transB=True, bias=d(sd["feat_spe.bias"]), act=1)
-    assert rel(m1.cpu(), a1) < 1e-5 and rel(m2.cpu(), a2) < 1e-5 and rel(mh.cpu(), h) < 1e-5
-    return sum(int(((m.cpu() > 0) != (a > 0)).sum()) for m, a in ((m1, a1), (m2, a2), (mh, h)))
 
 
 def test_cross_entropy_hard_and_soft(dev):

@@ -9,13 +9,9 @@ import pytest
 import torch
 
 from oracle import cmlpl_oracle as O
+from scene_harness import rel
 
 pytestmark = pytest.mark.gpu
-
-
-def rel(a, b):
-    a = np.asarray(a, dtype=np.float64); b = np.asarray(b, dtype=np.float64)
-    return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-30))
 
 
 @pytest.mark.parametrize("shape,B,K", [((23, 31), 224, 16), ((12, 40), 103, 9)])

@@ -10,22 +10,13 @@ bands, and the WHU-Hi scenes through the CLIs.
     oracle, in row bands, and its conv0 map against torch;
   * sample_generation --dataID 7 --synthetic + train on a small HongHu-shaped scene, at w = 20 and w = 11.
 """
-import copy
-import math
-import os
-
 import numpy as np
 import pytest
 import torch
 
+from fused_step_harness import eight_steps_graph_replay, one_step_against_oracle
 from oracle import cmlpl_oracle as O
-from oracle import golden
-from test_gpu_fused_step import compare_with_oracle
-from test_gpu_fused_step_shapes import (assert_soft_ce_exercised, assembled, check_adam_exact, fused_for, fused_step,
-                                        make_inputs, on_fused_masks, oracle_state_of, oracle_step, random_banks,
-                                        set_banks, snapshot_adam, thr_in_widest_gap)
-import test_gpu_fused_step_w11 as W11
-from test_gpu_many_classes import near_ties_only, rel
+from scene_harness import near_ties_only, raw_scene, rel, scene_net
 from test_wide_bands_cpu import spectral_noise
 
 pytestmark = pytest.mark.gpu
@@ -77,109 +68,20 @@ STEP_SHAPES = {
 }
 
 
-def thr_for(r, epoch, num_epochs):
-    """args.thr whose adaptive threshold at ``epoch`` sits in the widest gap of this step's scores."""
-    return thr_in_widest_gap(r) / math.exp(-0.5 * ((epoch / num_epochs) ** 2))
-
-
 @pytest.mark.parametrize("case", list(STEP_SHAPES))
 def test_one_step_wide_bands(dev, golden_dir, case):
     bs, btu, B, K, w, epoch, batch_index, ptrs, seed = STEP_SHAPES[case]
-    ti = golden.load(os.path.join(golden_dir, "train_infer.npz"))
-    g = torch.Generator().manual_seed(seed)
-    mod_inputs = W11.make_inputs if w == 11 else make_inputs
-    inp = mod_inputs(ti, bs, btu, B, K, g)
-    torch.manual_seed(seed)
-    conv_feat = 256 if w == 11 else 1600
-    sd, sd1 = O.basenet2_init(B, K, conv_feat=conv_feat), O.basenet2_init(B, K, conv_feat=conv_feat)
-    sa = O.StepArgs(num_epochs=20, labeled_batch_size=bs)
-    ost = O.make_state(sd, sd1, K, sa)
-    queues = random_banks(5 * bs * 2, K, g)
-    set_banks(ost, queues, ptrs)
-    step = W11.oracle_step if w == 11 else oracle_step
-    sa.thr = thr_for(step(copy.deepcopy(ost), inp, epoch, batch_index, sa), epoch, sa.num_epochs)
-    ost_before = copy.deepcopy(ost)
-    r = step(ost, inp, epoch, batch_index, sa)
-    assert_soft_ce_exercised(r)
-    if w == 11:
-        fs = W11.make_fused(dev, sd, sd1, B, K, queues, ptrs, sa, bs=bs, btu=btu)
-        w_before = [{k: p.detach().clone() for k, p in n.named_parameters()} for n in fs.nets]
-        patches, spectra = (t.to(dev) for t in W11.assembled(inp, sa.noise))
-        hist = fs.step(inp["Y_l"].to(dev), epoch, batch_index, patches=patches, spectra=spectra,
-                       drop_masks=inp["masks"].to(dev))
-        r = W11.on_fused_masks(r, ost_before, inp, epoch, batch_index, sa, fs, bs + btu)
-        W11.compare_with_oracle(fs, hist, r, ost, w_before, patches, bs + btu)
-    else:
-        fs = fused_for(dev, sd, sd1, bs, btu, B, K, queues, ptrs, sa)
-        w_before = [{k: p.detach().clone() for k, p in n.named_parameters()} for n in fs.nets]
-        hist, patches = fused_step(fs, dev, inp, epoch, batch_index, sa.noise)
-        r = on_fused_masks(r, ost_before, inp, epoch, batch_index, sa, fs, bs + btu)
-        compare_with_oracle(fs, hist, r, ost, w_before, patches, bs + btu, w_before)
-    assert fs.B == B and fs.prm.smooth == 1
+    one_step_against_oracle(dev, golden_dir, w, bs, btu, B, K, epoch, batch_index, ptrs, "random", seed)
 
 
 def test_consecutive_steps_graph_replay_270_bands(dev, golden_dir):
     """Eight 128 + 128 steps at 270 bands / 22 classes of one FusedMutualStep captured once as a CUDA graph and replayed
-    on new inputs, re-anchored on the oracle before every step (test_gpu_fused_step_shapes): smoothing switches on at
-    batch 4, the bank pointer wraps at 1280, and Adam at steps 1..8 is checked exactly against float64."""
-    B, K, bs = 270, 22, 128
-    ti = golden.load(os.path.join(golden_dir, "train_infer.npz"))
-    torch.manual_seed(270)
-    sd, sd1 = O.basenet2_init(B, K), O.basenet2_init(B, K)
-    sa = O.StepArgs(num_epochs=20, queue_batch=3)
-    zero = [torch.zeros(1280, 1024), torch.zeros(1280, K)] * 2
-    fs = fused_for(dev, sd, sd1, bs, bs, B, K, zero, (0, 0), sa, use_graph=True)
-    patches = torch.zeros(2, 2 * bs, 60, 20, 20, device=dev)
-    spectra = torch.zeros(2, 2 * bs, B, device=dev)
-    masks = torch.zeros(2, 2 * bs, 2624, device=dev)
-    labels = torch.zeros(bs, dtype=torch.int64, device=dev)
-    g = torch.Generator().manual_seed(2702)
-    seen = []
-    for it in range(8):
-        inp = make_inputs(ti, bs, bs, B, K, g)
-        p_, s_ = assembled(inp, sa.noise)
-        patches.copy_(p_); spectra.copy_(s_); masks.copy_(inp["masks"]); labels.copy_(inp["Y_l"])
-        ost = oracle_state_of(fs, sa)
-        before = snapshot_adam(fs)
-        w_before = [{k: p.detach().clone() for k, p in n.named_parameters()} for n in fs.nets]
-        ptrs = (fs.queue_ptr, fs.queue_ptr1)
-        ost_before = copy.deepcopy(ost)
-        sa.thr = fs.thr = thr_in_widest_gap(oracle_step(copy.deepcopy(ost), inp, 0, it, sa))
-        r = oracle_step(ost, inp, 0, it, sa)
-        hist = fs.step(labels, 0, it, patches=patches, spectra=spectra, drop_masks=masks)
-        assert fs.adam_step == it + 1 and len(fs._graphs) == 1
-        assert fs.prm.smooth == int(it > 3)
-        r = on_fused_masks(r, ost_before, inp, 0, it, sa, fs, 2 * bs)
-        compare_with_oracle(fs, hist, r, ost, w_before, patches, 2 * bs, w_before, adam=it == 0)
-        worst = check_adam_exact(fs, before, it + 1)
-        seen.append((ptrs, (fs.queue_ptr, fs.queue_ptr1), float(r["mask"].mean()), worst))
-        print("step %d: pointers %s -> %s, mask fraction %.2f, Adam max rel error %.1e" % (it + 1, *seen[-1]))
-        assert 0.05 <= seen[-1][2] <= 0.95
-    assert [s[0][0] for s in seen] == [0, 256, 512, 768, 1024, 0, 256, 512]
+    on new inputs, re-anchored on the oracle before every step (fused_step_harness.eight_steps_graph_replay): smoothing
+    switches on at batch 4, the bank pointer wraps at 1280, and Adam at steps 1..8 is checked exactly against float64."""
+    eight_steps_graph_replay(dev, golden_dir, 20, 270, 22, 270, 2702)
 
 
 # ------------------------------------------------------------------------------------------ 3. raw entry point
-def _raw_scene(dev, R, C, B, K, seed):
-    """Synthetic raw scene, its float64 oracle preprocessing, and the device preprocessing with the oracle's PCA signs."""
-    from cmlpl_b200 import preprocess, synth
-    cube_u16, _ = synth.synth_scene(R, C, B, K, seed=seed)
-    ref_cube, ref_spec = O.preprocess(cube_u16, 60)
-    raw = torch.from_numpy(cube_u16.reshape(-1, B).copy()).to(dev)
-    pp = preprocess.fit(raw, 60)
-    cube, _ = preprocess.apply(raw, pp, want_spectra=False)
-    sgn = np.sign((cube.cpu().numpy().reshape(R, C, 60) * ref_cube).sum((0, 1)))   # singular vectors: up to sign
-    pp.U = pp.U * sgn[None, :]
-    pp._dev = None
-    return cube_u16, raw, pp, ref_cube.astype(np.float32), ref_spec.astype(np.float32)
-
-
-def _net(B, K, w, seed, dev):
-    from cmlpl_b200.tools.models import BaseNet2
-    torch.manual_seed(seed)
-    net = BaseNet2(B, 0, K, w=w).to(dev).eval()
-    return net, {k: v.detach().cpu() for k, v in net.state_dict().items()}
-
-
 @pytest.mark.parametrize("dtype", ["u16", "f32"])
 @pytest.mark.parametrize("B,K,w", [(240, 16, 20), (270, 22, 20), (425, 16, 20), (270, 9, 11)])
 def test_raw_entry_point_wide_bands(dev, B, K, w, dtype):
@@ -188,8 +90,8 @@ def test_raw_entry_point_wide_bands(dev, B, K, w, dtype):
     one-call labels and logits bit for bit."""
     from cmlpl_b200 import ops, preprocess
     R, C = 29, 37
-    _, raw, pp, ref_cube, ref_spec = _raw_scene(dev, R, C, B, K, seed=B + K)
-    net, sd = _net(B, K, w, B * 7 + K, dev)
+    _, raw, pp, ref_cube, ref_spec = raw_scene(dev, R, C, B, K, seed=B + K)
+    net, sd = scene_net(B, K, w, B * 7 + K, dev)
     packed = net.packed_weights(w)
     folded = pp.folded_conv0(sd["conv0.weight"], sd["conv0.bias"], dev)
     raw_in = raw if dtype == "u16" else raw.float()
@@ -221,8 +123,8 @@ def test_raw_conv0_map_matches_torch(dev, B):
     float64 torch evaluation of the folded 1x1 conv on the mirror-padded raw scene: 1e-3 of its largest entry."""
     from cmlpl_b200 import ops
     R, C, K, w = 23, 31, 22, 20
-    _, raw, pp, _, _ = _raw_scene(dev, R, C, B, K, seed=B)
-    net, sd = _net(B, K, w, B, dev)
+    _, raw, pp, _, _ = raw_scene(dev, R, C, B, K, seed=B)
+    net, sd = scene_net(B, K, w, B, dev)
     folded = pp.folded_conv0(sd["conv0.weight"], sd["conv0.bias"], dev)
     ws = ops.scene_workspace(R, C, B, K, w, dev)
     ops.scene_infer_raw(raw, folded, net.packed_weights(w), K, C, w, workspace=ws)
