@@ -17,15 +17,18 @@
 // conv1_pool_kernel does both in ONE kernel -- the fp32 variants G (2.3 KB per scene position) never touch
 // HBM.  It is a persistent, warp-specialised tcgen05 implicit GEMM over 4x30-position tiles (M=128 rows =
 // 4 rows x 32 columns incl. one halo column each side), taps = A-descriptor offsets in a row-major
-// zero-haloed shared-memory tile loaded by TMA:
-//   * the tensor core produces the nine single-tap-column sums  T[dy][dx] = sum_ci W1[dy,dx] . F0[p+(dy-1,dx-1)]
-//     separately (N = 32 channels at a time: sub-stage (h, dy) = T[dy][0..2] in 96 TMEM columns, ring of 5), so
-//     that all three column classes  R[dy][left|mid|right] = T1+T2 | T0+T1+T2 | T0+T1  are formed in the
-//     epilogue from one TMEM read (36 MMAs per 32 channels), and the row classes from them as
-//     top = R1+R2, mid = R0+R1+R2, bot = R0+R1;
-//   * a tile's 4 conv rows give 3 pooled rows and its 30 conv columns 29 pooled columns: the vertical 2x2
-//     partner (ty+1, tx) lives in another warp (TMEM lane quarter) and comes through a double-buffered
-//     shared-memory exchange, the horizontal partner (tx+1) through a warp shuffle;
+// zero-haloed shared-memory tile of 7 rows loaded by TMA:
+//   * the tensor core produces, per 32-channel half and tap column dx, four accumulators over two FRAMES of the
+//     same 4x32 lanes: frame 0 holds conv rows y0..y0+3 (one per TMEM lane quarter), frame 1 rows y0+1..y0+4,
+//     the same lanes one row down (its A rows are frame 0's plus one tile row).  A row offset s of the A tile
+//     feeds frame 0 tap dy = s and frame 1 tap dy = s-1, so
+//         U  = frame 0 taps dy 1+2 | D = frame 1 taps dy 0+1   (s = 1, 2: one N = 64 MMA each, B = [W1;W0] / [W2;W1])
+//         T0 = frame 0 tap  dy 0   | T2 = frame 1 tap  dy 2    (s = 0 / 3: one N = 32 MMA each)
+//     (48 MMAs in 384 TMEM columns per half).  The epilogue forms the column classes
+//     R[left|mid|right] = R1+R2 | R0+R1+R2 | R0+R1 of each, and the row classes  top = U, mid = T0+U  (frame 0)
+//     and  mid = D+T2, bot = D  (frame 1) from one TMEM read;
+//   * a tile emits 4 pooled rows x 29 pooled columns: the vertical 2x2 partner of frame 0's row is frame 1's row
+//     in the SAME lane, the horizontal partner (tx+1) comes through a warp shuffle -- no exchange between warps;
 //   * pooled cells go straight to the parity planes pmq (f16, chunk-planar), 8 channels = one 16-byte chunk
 //     per thread and pass.
 //   V[A][b]  = G[a0(A)][b](y,x) + G[a1(A)][b](y+1,x)                 (a0,a1 = top,mid | mid,mid | mid,bot)
@@ -37,22 +40,25 @@
 namespace cmlpl {
 
 namespace c1p {
-constexpr int TH = 4, TP = 32, OH = 3, OW = 29;      // conv rows, row pitch; pooled rows / columns per tile
-constexpr int CH = (TH + 2) * TP * 16;               // 3 072: one chunk plane of the conv0 tile, dense (written by TMA)
-constexpr int ABYTES = 8 * CH;
+constexpr int TH = 4, TP = 32, OH = 4, OW = 29;      // conv rows per frame, row pitch; pooled rows / columns per tile
+constexpr int AR = TH + 3;                           // 7 A-tile rows: frame 1 sits one row below frame 0, +1 halo row each side
+constexpr int CH = AR * TP * 16;                     // 3 584: one chunk plane of the conv0 tile, dense (written by TMA)
+constexpr int ABYTES = 8 * CH, NBUF = 3;
 constexpr int WBYTES = 3 * 8 * 192 * 16;
 constexpr int kEpi = 256, kThreads = kEpi + 64;      // warps 0-7 epilogue, warp 8 loader (one thread, TMA), warp 9 MMA issuer
 constexpr int kLoadWarp = kEpi / 32, kMmaWarp = kLoadWarp + 1;
-constexpr int XBYTES = 12 * kEpi * 16;               // exchange: 12 float4 (G[mid|bot][3 b][8 ch]) per epilogue thread
-constexpr int S_W = 0, S_A = WBYTES, S_X = S_A + 2 * ABYTES, S_BIAS = S_X + 2 * XBYTES, S_BAR = S_BIAS + 256,
-              S_TMEM = S_BAR + 128;
+constexpr int S_W = 0, S_A = WBYTES, S_BIAS = S_A + NBUF * ABYTES, S_BAR = S_BIAS + 256, S_TMEM = S_BAR + 128;
 constexpr int SMEM = (S_TMEM + 16 + 127) / 128 * 128;
-constexpr int NSUB = 5, SUBCOLS = 96;
+// TMEM columns of one channel half, per tap column dx (at dx * 128): [U | D] 0..63, T0 64..95, T2 96..127
+constexpr int HALFCOLS = 384, C_UD = 0, C_T0 = 64, C_T2 = 96;
+// weights in shared memory: [3 dx][8 kc][2 h][W2h W1h W0h: 96 rows][16 B], so [W2h;W1h] and [W1h;W0h] are contiguous
+// N = 64 operands.  In HBM (the packed layout patch_cnn_kernel shares) a (dx, kc) block is [(2-dy)*64 + n][16 B].
 constexpr int kWLbo = 192 * 16, kWDx = 8 * kWLbo;
-enum { A_FULL0 = 0, A_FULL1, A_EMPTY0, A_EMPTY1, S_FULL0 = 4, S_EMPTY0 = 4 + NSUB, W_FULL = 4 + 2 * NSUB };
+enum { A_FULL0 = 0, A_EMPTY0 = NBUF, S_FULL = 2 * NBUF, S_EMPTY, W_FULL };
 static_assert(SMEM <= 232448, "conv1_pool: shared memory over the 227 KB limit");
 static_assert(W_FULL < 16, "conv1_pool: barrier area too small");
 static_assert(S_A % 128 == 0 && ABYTES % 128 == 0, "conv1_pool: TMA destinations must be 128-byte aligned");
+static_assert(HALFCOLS <= 512, "conv1_pool: a channel half must fit tensor memory");
 }  // namespace c1p
 
 // f0: f16 chunk-planar [8][PR][PC][8];  pmq f16 [9 = A*3+B][4 planes][8 chunks][PR2][PC2][8]
@@ -68,19 +74,27 @@ conv1_pool_kernel(const __grid_constant__ CUtensorMap tm_f0, int PR, int PC, int
   const int tiles_c = (2 * PC2 + OW - 1) / OW, tiles_r = (2 * PR2 + OH - 1) / OH;
   const int ntiles = tiles_r * tiles_c;
   const int64_t psz = int64_t(PR2) * PC2;
+  // Tiles run from the bottom of the band up, so the planes written last -- still in L2 when the kernel ends -- are the
+  // top rows, which conv2_scene_kernel reads first.
 
   {
     uint4* z = reinterpret_cast<uint4*>(smem + S_A);
-    for (int i = tid; i < 2 * ABYTES / 16; i += kThreads) z[i] = make_uint4(0, 0, 0, 0);
+    for (int i = tid; i < NBUF * ABYTES / 16; i += kThreads) z[i] = make_uint4(0, 0, 0, 0);
   }
   if (tid < 64) sbias[tid] = b1g[tid];
   if (tid == 0) {
     mbar_init(bars + 8 * W_FULL, 1);
     fence_barrier_init();
-    bulk_weights_g2s(sbase + S_W, w1p, WBYTES, bars + 8 * W_FULL);
-    mbar_init(bars + 8 * A_FULL0, 1); mbar_init(bars + 8 * A_FULL1, 1);
-    mbar_init(bars + 8 * A_EMPTY0, 1 + kEpi); mbar_init(bars + 8 * A_EMPTY1, 1 + kEpi);
-    for (int s = 0; s < NSUB; ++s) { mbar_init(bars + 8 * (S_FULL0 + s), 1); mbar_init(bars + 8 * (S_EMPTY0 + s), kEpi); }
+    // 144 bulk copies of 512 B (32 rows of one (dx, kc, dy, h)) permute the weights into the half-interleaved order
+    mbar_arrive_expect_tx(bars + 8 * W_FULL, WBYTES);
+#pragma unroll 1
+    for (int i = 0; i < 3 * 8 * 6; ++i) {
+      const int blk = i / 6, dy = (i % 6) >> 1, h = i & 1;
+      bulk_g2s(sbase + S_W + (blk * 192 + h * 96 + (2 - dy) * 32) * 16, w1p + (blk * 192 + (2 - dy) * 64 + h * 32) * 16,
+               512, bars + 8 * W_FULL);
+    }
+    for (int b = 0; b < NBUF; ++b) { mbar_init(bars + 8 * (A_FULL0 + b), 1); mbar_init(bars + 8 * (A_EMPTY0 + b), 1 + kEpi); }
+    mbar_init(bars + 8 * S_FULL, 1); mbar_init(bars + 8 * S_EMPTY, kEpi);
     fence_barrier_init();
   }
   if (warp == kMmaWarp) tmem_alloc(sbase + S_TMEM, 512);
@@ -91,156 +105,140 @@ conv1_pool_kernel(const __grid_constant__ CUtensorMap tm_f0, int PR, int PC, int
   const uint32_t tmem = *reinterpret_cast<volatile uint32_t*>(smem + S_TMEM);
 
   if (warp == kLoadWarp) {
-    // ================================================================ loader: one TMA box per tile ((TH+2) x TP entries, zero outside the map)
+    // ================================================================ loader: one TMA box per tile (AR x TP entries, zero outside the map)
     if (lane == 0) {
       tma_prefetch_desc(&tm_f0);
-      uint32_t j = 0;
+      uint32_t j = 0, buf = 0, ph = 0;
       [[maybe_unused]] uint32_t ntr = 0;
       for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++j) {
-        const uint32_t buf = j & 1, ph = (j >> 1) & 1;
-        const int tr = t / tiles_c, tc = t - tr * tiles_c;
+        const int u = ntiles - 1 - t, tr = u / tiles_c, tc = u - tr * tiles_c;   // bottom tile rows first (see above)
         mbar_wait(bars + 8 * (A_EMPTY0 + buf), ph ^ 1, 81);
         CMLPL_TR(4, ntr, j);
         mbar_arrive_expect_tx(bars + 8 * (A_FULL0 + buf), ABYTES);
         tma_load_tile(sbase + S_A + buf * ABYTES, &tm_f0, tc * OW - 1, tr * OH - 1, 0, bars + 8 * (A_FULL0 + buf));
+        if (++buf == NBUF) { buf = 0; ph ^= 1; }
       }
     }
   } else if (warp == kMmaWarp) {
     // ================================================================ MMA issuer
     if (tmem != 0) { printf("conv1_pool: unexpected TMEM base %u\n", tmem); __trap(); }
     constexpr uint64_t kHi = (uint64_t(128 >> 4) | (uint64_t(1) << 14)) << 32;
-    constexpr uint32_t kI32 = make_idesc_f16(128, 32);
+    constexpr uint32_t kI32 = make_idesc_f16(128, 32), kI64 = make_idesc_f16(128, 64);
     const uint32_t w_lo = ((sbase + S_W) >> 4) | (uint32_t(kWLbo >> 4) << 16);
-    uint32_t j = 0, slot = 0, sph = 0;
+    uint32_t j = 0, buf = 0, ph = 0, sph = 0;
     [[maybe_unused]] uint32_t ntr = 0;
     mbar_wait(bars + 8 * W_FULL, 0, 80);                       // weights have landed
     for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++j) {
-      const uint32_t buf = j & 1, ph = (j >> 1) & 1;
-      // MMA row m of tap (dy,dx) reads tile entry m + dy*TP + dx - 1: descriptors start 16 B before the tile
+      // MMA row m at A row offset s, tap column dx reads tile entry m + s*TP + dx - 1: descriptors start 16 B before the tile
       const uint32_t a_lo = ((sbase + S_A + buf * ABYTES - 16) >> 4) | (uint32_t(CH >> 4) << 16);
       mbar_wait(bars + 8 * (A_FULL0 + buf), ph, 82);
 #pragma unroll 1
-      for (int hd = 0; hd < 6; ++hd) {                         // sub-stage = (channel half h, tap row dy)
-        const int h = hd / 3, dy = hd - h * 3;
-        if (lane == 0) CMLPL_TR(0, ntr, (j * 6 + hd) * 4);
-        mbar_wait(bars + 8 * (S_EMPTY0 + slot), sph ^ 1, 83);
+      for (int h = 0; h < 2; ++h) {                            // one channel half = one TMEM slot of 384 columns
+        if (lane == 0) CMLPL_TR(0, ntr, (j * 2 + h) * 4);
+        mbar_wait(bars + 8 * S_EMPTY, sph ^ 1, 83);
         tc_fence_after();
-        if (lane == 0) CMLPL_TR(0, ntr, (j * 6 + hd) * 4 + 1);
+        if (lane == 0) CMLPL_TR(0, ntr, (j * 2 + h) * 4 + 1);
         if (elect_one_sync()) {
 #pragma unroll
           for (int dx = 0; dx < 3; ++dx) {
-            const uint32_t d = slot * SUBCOLS + dx * 32;
+            const uint32_t d = dx * 128;
 #pragma unroll
             for (int ks = 0; ks < 4; ++ks) {
-              const uint32_t a = a_lo + uint32_t(dy * TP + dx) + uint32_t(ks * 2 * CH / 16);
-              const uint32_t bb = w_lo + uint32_t((dx * kWDx + ks * 2 * kWLbo) / 16) + uint32_t((2 - dy) * 64 + h * 32);
-              umma_f16(d, kHi | uint64_t(a), kHi | uint64_t(bb), kI32, ks ? 1u : 0u);
+              const uint32_t a = a_lo + uint32_t(dx) + uint32_t(ks * 2 * CH / 16);
+              const uint32_t bb = w_lo + uint32_t((dx * kWDx + ks * 2 * kWLbo) / 16) + uint32_t(h * 96);
+              const uint32_t acc = ks ? 1u : 0u;
+              umma_f16(d + C_UD, kHi | uint64_t(a + 1 * TP), kHi | uint64_t(bb + 32), kI64, acc);   // [U|D] += [W1;W0]
+              umma_f16(d + C_UD, kHi | uint64_t(a + 2 * TP), kHi | uint64_t(bb), kI64, 1u);         // [U|D] += [W2;W1]
+              umma_f16(d + C_T0, kHi | uint64_t(a), kHi | uint64_t(bb + 64), kI32, acc);            // T0 += W0
+              umma_f16(d + C_T2, kHi | uint64_t(a + 3 * TP), kHi | uint64_t(bb), kI32, acc);        // T2 += W2
             }
           }
-          umma_commit(bars + 8 * (S_FULL0 + slot));
-          if (hd == 5) umma_commit(bars + 8 * (A_EMPTY0 + buf));
+          umma_commit(bars + 8 * S_FULL);
+          if (h == 1) umma_commit(bars + 8 * (A_EMPTY0 + buf));
         }
         __syncwarp();
-        if (lane == 0) CMLPL_TR(0, ntr, (j * 6 + hd) * 4 + 2);
-        if (++slot == NSUB) { slot = 0; sph ^= 1; }
+        if (lane == 0) CMLPL_TR(0, ntr, (j * 2 + h) * 4 + 2);
+        sph ^= 1;
       }
+      if (++buf == NBUF) { buf = 0; ph ^= 1; }
     }
   } else {
-    // ================================================================ epilogue (warps 0-7)
+    // ================================================================ epilogue (warps 0-7, each on its own lane quarter)
     const int ty = warp & 3, tx = lane, chsel = warp >> 2;
     const uint32_t lane_addr = uint32_t(ty * 32) << 16;
-    const int nb = ty < 3 ? tid + 32 : tid;                   // exchange slot of the position one row below
-    uint32_t j = 0, slot = 0, sph = 0, xpar = 0;
+    uint32_t j = 0, buf = 0, ph = 0, sph = 0;
     [[maybe_unused]] uint32_t ntr = 0;
     const bool tracer = (warp == 0 || warp == 4) && lane == 0;
     for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++j) {
-      const uint32_t buf = j & 1;
-      const int tr = t / tiles_c, tc = t - tr * tiles_c;
+      const int u = ntiles - 1 - t, tr = u / tiles_c, tc = u - tr * tiles_c;   // bottom tile rows first (see above)
       const int pr = tr * OH + ty, pc = tc * OW + tx - 1;
-      const bool inplane = ty < OH && tx >= 1 && tx <= OW && (pr >> 1) < PR2 && (pc >> 1) < PC2;
+      const bool inplane = tx >= 1 && tx <= OW && (pr >> 1) < PR2 && (pc >> 1) < PC2;
       const bool cell = inplane && pr < PR - 1 && pc < PC - 1;
       const int64_t opos = inplane ? (int64_t((pr & 1) * 2 + (pc & 1)) * 8 * psz + int64_t(pr >> 1) * PC2 + (pc >> 1)) : 0;
-      mbar_wait(bars + 8 * (A_FULL0 + buf), (j >> 1) & 1, 84);
+      const unsigned char* abuf = smem + S_A + buf * ABYTES;
+      mbar_wait(bars + 8 * (A_FULL0 + buf), ph, 84);
 #pragma unroll 1
       for (int h = 0; h < 2; ++h) {
-        uint32_t sl[3];
         if (tracer) CMLPL_TR(1 + chsel, ntr, (j * 4 + h * 2) * 8);
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-          sl[k] = slot;
-          mbar_wait(bars + 8 * (S_FULL0 + slot), sph, 85);
-          if (++slot == NSUB) { slot = 0; sph ^= 1; }
-        }
+        mbar_wait(bars + 8 * S_FULL, sph, 85);
+        sph ^= 1;
         tc_fence_after();
         if (tracer) CMLPL_TR(1 + chsel, ntr, (j * 4 + h * 2) * 8 + 1);
 #pragma unroll 1
-        for (int pp = 0; pp < 2; ++pp, xpar ^= 1) {
+        for (int pp = 0; pp < 2; ++pp) {
           const int chunk = h * 4 + pp * 2 + chsel;
           const uint32_t col = uint32_t(pp * 16 + chsel * 8);
           typedef unsigned long long f2;                       // two packed fp32 channels (FADD2 / FMUL2)
-          f2 T[3][3][4];
+          f2 U[3][4], D[3][4], T0[3][4], T2[3][4];
 #pragma unroll
-          for (int dy = 0; dy < 3; ++dy)
-#pragma unroll
-            for (int dx = 0; dx < 3; ++dx) tmem_ld8_x2(lane_addr + sl[dy] * SUBCOLS + dx * 32 + col, T[dy][dx]);
+          for (int dx = 0; dx < 3; ++dx) {
+            const uint32_t ta = lane_addr + dx * 128 + col;
+            tmem_ld8_x2(ta + C_UD, U[dx]);
+            tmem_ld8_x2(ta + C_UD + 32, D[dx]);
+            tmem_ld8_x2(ta + C_T0, T0[dx]);
+            tmem_ld8_x2(ta + C_T2, T2[dx]);
+          }
           tmem_ld_wait();
           if (tracer) CMLPL_TR(1 + chsel, ntr, (j * 4 + h * 2 + pp) * 8 + 2);
-          if (pp == 1) {
+          if (pp == 1) {                                       // the MMAs of the next half may overwrite the slot
             tc_fence_before();
-#pragma unroll
-            for (int k = 0; k < 3; ++k) mbar_arrive(bars + 8 * (S_EMPTY0 + sl[k]));
+            mbar_arrive(bars + 8 * S_EMPTY);
           }
           {
-            // bias + residual (centre entry of the A tile) go into the centre tap, which every border class keeps
-            const uint4 rv = *reinterpret_cast<const uint4*>(smem + S_A + buf * ABYTES + chunk * CH + ((ty + 1) * TP + tx) * 16);
-            const __half2* hr = reinterpret_cast<const __half2*>(&rv);
+            // bias + residual (centre entry of the A tile, frame 0 row ty+1 / frame 1 row ty+2) go into the centre
+            // tap, which every border class keeps
+            const uint4 r0 = *reinterpret_cast<const uint4*>(abuf + chunk * CH + ((ty + 1) * TP + tx) * 16);
+            const uint4 r1 = *reinterpret_cast<const uint4*>(abuf + chunk * CH + ((ty + 2) * TP + tx) * 16);
+            const __half2* h0 = reinterpret_cast<const __half2*>(&r0);
+            const __half2* h1 = reinterpret_cast<const __half2*>(&r1);
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
-              const float2 f = __half22float2(hr[e]);
-              T[1][1][e] = f2_add(T[1][1][e], f2_pack(f.x + sbias[chunk * 8 + 2 * e], f.y + sbias[chunk * 8 + 2 * e + 1]));
+              const float b0 = sbias[chunk * 8 + 2 * e], b1 = sbias[chunk * 8 + 2 * e + 1];
+              const float2 f = __half22float2(h0[e]), g = __half22float2(h1[e]);
+              U[1][e] = f2_add(U[1][e], f2_pack(f.x + b0, f.y + b1));
+              D[1][e] = f2_add(D[1][e], f2_pack(g.x + b0, g.y + b1));
             }
           }
-          // G[a][b] = relu(b1 + F0 + sum of the taps the (row class a, column class b) border keeps)
-          f2 G[3][3][4];
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-            f2 R[3][3];
-#pragma unroll
-            for (int dy = 0; dy < 3; ++dy) {
-              const f2 s12 = f2_add(T[dy][1][c], T[dy][2][c]);
-              R[dy][0] = s12; R[dy][1] = f2_add(T[dy][0][c], s12); R[dy][2] = f2_add(T[dy][0][c], T[dy][1][c]);
-            }
-#pragma unroll
-            for (int b = 0; b < 3; ++b) {
-              const f2 top = f2_add(R[1][b], R[2][b]);
-              G[0][b][c] = f2_relu(top);
-              G[1][b][c] = f2_relu(f2_add(R[0][b], top));
-              G[2][b][c] = f2_relu(f2_add(R[0][b], R[1][b]));
-            }
-          }
-          // vertical partner through shared memory: this thread publishes its mid / bot variants
-          ulonglong2* xb = reinterpret_cast<ulonglong2*>(smem + S_X + xpar * XBYTES);
-#pragma unroll
-          for (int a = 1; a < 3; ++a)
-#pragma unroll
-            for (int b = 0; b < 3; ++b)
-#pragma unroll
-              for (int q = 0; q < 2; ++q)
-                xb[(((a - 1) * 3 + b) * 2 + q) * kEpi + tid] = make_ulonglong2(G[a][b][2 * q], G[a][b][2 * q + 1]);
-          if (tracer) CMLPL_TR(1 + chsel, ntr, (j * 4 + h * 2 + pp) * 8 + 3);
-          named_bar_sync(1, kEpi);
-          if (tracer) CMLPL_TR(1 + chsel, ntr, (j * 4 + h * 2 + pp) * 8 + 4);
+          // G[a][b] = relu(b1 + F0 + sum of the taps the (row class a, column class b) border keeps), and the
+          // vertical pool  V[A][b] = G0[a0(A)][b] + G1[a1(A)][b]  in the same lane
           f2 V[3][3][4];                                       // [A][b]
 #pragma unroll
-          for (int b = 0; b < 3; ++b)
+          for (int c = 0; c < 4; ++c) {
 #pragma unroll
-            for (int q = 0; q < 2; ++q) {
-              const ulonglong2 m = xb[((0 * 3 + b) * 2 + q) * kEpi + nb];
-              const ulonglong2 o = xb[((1 * 3 + b) * 2 + q) * kEpi + nb];
-              V[0][b][2 * q] = f2_add(G[0][b][2 * q], m.x); V[0][b][2 * q + 1] = f2_add(G[0][b][2 * q + 1], m.y);
-              V[1][b][2 * q] = f2_add(G[1][b][2 * q], m.x); V[1][b][2 * q + 1] = f2_add(G[1][b][2 * q + 1], m.y);
-              V[2][b][2 * q] = f2_add(G[1][b][2 * q], o.x); V[2][b][2 * q + 1] = f2_add(G[1][b][2 * q + 1], o.y);
+            for (int b = 0; b < 3; ++b) {
+              // column class b of a tap-column triple: left = 1+2, mid = 0+1+2, right = 0+1
+              auto cls = [&](const f2 (&X)[3][4]) {
+                return b == 0 ? f2_add(X[1][c], X[2][c])
+                              : b == 1 ? f2_add(X[0][c], f2_add(X[1][c], X[2][c])) : f2_add(X[0][c], X[1][c]);
+              };
+              const f2 u = cls(U), d = cls(D);
+              const f2 g0top = f2_relu(u), g0mid = f2_relu(f2_add(cls(T0), u));
+              const f2 g1mid = f2_relu(f2_add(cls(T2), d)), g1bot = f2_relu(d);
+              V[0][b][c] = f2_add(g0top, g1mid);
+              V[1][b][c] = f2_add(g0mid, g1mid);
+              V[2][b][c] = f2_add(g0mid, g1bot);
             }
+          }
           // horizontal partner (tx+1) by shuffle, scale (0 for plane cells without a pooled value), round, store
           const f2 sc = f2_pack(cell ? 0.25f : 0.f, cell ? 0.25f : 0.f);
 #pragma unroll
@@ -261,10 +259,11 @@ conv1_pool_kernel(const __grid_constant__ CUtensorMap tm_f0, int PR, int PC, int
               if (ncls > 2) *reinterpret_cast<uint4*>(dst + int64_t(64) * psz * 8) = *reinterpret_cast<uint4*>(o2);
             }
           }
-          if (tracer) CMLPL_TR(1 + chsel, ntr, (j * 4 + h * 2 + pp) * 8 + 5);
+          if (tracer) CMLPL_TR(1 + chsel, ntr, (j * 4 + h * 2 + pp) * 8 + 3);
         }
       }
       mbar_arrive(bars + 8 * (A_EMPTY0 + buf));               // residual reads (and the MMAs, by their commit) done with A
+      if (++buf == NBUF) { buf = 0; ph ^= 1; }
     }
   }
   tc_fence_before();
@@ -290,7 +289,7 @@ extern "C" int cmlpl_conv1_pool_planes_f16(const void* f0pad, int cols, int w, i
   const int ntiles = ((2 * PR2 + c1p::OH - 1) / c1p::OH) * ((2 * PC2 + c1p::OW - 1) / c1p::OW);
   int grid = sm_count(); if (grid > ntiles) grid = ntiles;
   CUtensorMap tm_f0;
-  const int trc = make_scene_tmap(&tm_f0, f0pad, 1, PR, PC, c1p::TH + 2, c1p::TP);
+  const int trc = make_scene_tmap(&tm_f0, f0pad, 1, PR, PC, c1p::AR, c1p::TP);
   if (trc != CMLPL_OK) return trc;
   conv1_pool_kernel<<<grid, c1p::kThreads, c1p::SMEM, static_cast<cudaStream_t>(stream)>>>(
       tm_f0, PR, PC, PR2, PC2, w == 11 ? 2 : 3, pk + L.w1, reinterpret_cast<const float*>(pk + L.b1), static_cast<__half*>(pmq));

@@ -469,6 +469,8 @@ pool2_cls_kernel(const __grid_constant__ CUtensorMap tm_y, int PR2, int PC2, int
   const int tiles_c = (PC2 + TW - 1) / TW, tiles_r = (PR2 + TH - 1) / TH;
   const int tiles_p = tiles_r * tiles_c, ntiles = 4 * tiles_p;
   const int64_t psz = int64_t(PR2) * PC2;
+  // Tiles run in the reverse of conv2_scene_kernel's order (last parity plane, bottom rows first): the maps conv2 wrote
+  // last are still in L2 when this kernel starts, and it reads them before they are evicted.
   // w = 11: pooled cells I, J in {0, 1} only -> row classes Al = 0, 1 and pooled columns J = 0, 1 (the weights of every
   // other cell are zero in wcq, their maps are neither loaded nor multiplied)
   const int nAl = ncell >= 5 ? 3 : 2, nJ = ncell >= 5 ? 5 : 2;
@@ -498,7 +500,7 @@ pool2_cls_kernel(const __grid_constant__ CUtensorMap tm_y, int PR2, int PC2, int
       tma_prefetch_desc(&tm_y);
       uint32_t slot = 0, ph = 0;
       for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
-        const int pl = t / tiles_p, tt = t - pl * tiles_p;
+        const int u = ntiles - 1 - t, pl = u / tiles_p, tt = u - pl * tiles_p;   // last plane, bottom rows first (see above)
         const int tr = tt / tiles_c, tc = tt - tr * tiles_c;
 #pragma unroll 1
         for (int q = 0; q < 15; ++q) {
@@ -565,7 +567,7 @@ pool2_cls_kernel(const __grid_constant__ CUtensorMap tm_y, int PR2, int PC2, int
     const int m0 = half ? 3 : 0, m1 = half ? 5 : 3;
     uint32_t tj = 0;
     for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++tj) {
-      const int pl = t / tiles_p, tt = t - pl * tiles_p;
+      const int u = ntiles - 1 - t, pl = u / tiles_p, tt = u - pl * tiles_p;   // last plane, bottom rows first (see above)
       const int tr = tt / tiles_c, tc = tt - tr * tiles_c;
       const int y = tr * TH + ty, x = tc * TW + tx;
       const bool valid = tx < TW && y < PR2 && x < PC2;

@@ -380,9 +380,12 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
   };
   if (ws.dense) {
     // The spectral branch (fp16 tiles of the spectra + the two spectral GEMMs) does not depend on the conv tower until
-    // the head: forked onto the side stream, its conversion kernel shares the SMs with conv0 and its tail with the head
-    // of conv1_pool.  Then conv1 (9 border classes) -> pooled parity planes -> conv2 (25 classes) -> pool + conv
-    // classifier columns, and the head joins the branch: spectral partials + gathered conv partials + argmax.
+    // the head: forked onto the side stream, its conversion kernel shares the SMs with conv0.  The main stream joins it
+    // before conv1_pool, so that each kernel reads what its predecessor has just written while much of it is still in
+    // L2: spectral_logits the fp16 tiles (47 MB on PaviaU; beside conv1_pool they were evicted by its 200 MB of
+    // stores), conv2 the pooled conv1 planes (conv1_pool writes the rows conv2 reads first last).
+    // Then conv1 (9 border classes) -> pooled parity planes -> conv2 (25 classes) -> pool + conv classifier columns ->
+    // head: spectral partials + gathered conv partials + argmax.
     SideStream* sd = side_stream();
     CMLPL_CHECK_ARG(sd, "%s: cannot create the side stream", src.fn);
     std::lock_guard<std::mutex> lock(sd->mu);
@@ -391,11 +394,11 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
     if ((rc = spectral_tc(sd->s)) != CMLPL_OK) return rc;
     CMLPL_CUDA(cudaEventRecord(sd->join[0], sd->s));
     if ((rc = conv0()) != CMLPL_OK) return rc;
+    CMLPL_CUDA(cudaStreamWaitEvent(s, sd->join[0], 0));
     if ((rc = cmlpl_conv1_pool_planes_f16(wsb + ws.f0pad, cols, w, band_rows, packed, wsb + ws.pm, stream)) != CMLPL_OK) return rc;
     if ((rc = cmlpl_conv2_scene_f16(wsb + ws.pm, cols, w, band_rows, packed, wsb + ws.yq, stream)) != CMLPL_OK) return rc;
     float* lmap = reinterpret_cast<float*>(wsb + ws.lmap);
     if ((rc = cmlpl_pool2_cls_f16(wsb + ws.yq, cols, w, band_rows, B, C, packed, lmap, stream)) != CMLPL_OK) return rc;
-    CMLPL_CUDA(cudaStreamWaitEvent(s, sd->join[0], 0));
     return launch_head_sum(part, lmap, cols, band_rows, B, C, w, packed, band_valid, labels, logits, stream);
   }
   // per pixel: the tensor-core spectral branch; or the CUDA-core spectral head beyond 224 bands (both entry points) and in

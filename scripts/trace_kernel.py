@@ -75,15 +75,15 @@ if which == "conv2":
         r = t >> 2
         return f"item kap{r // 3} it{r % 3} " + ["wait", "ready", "done"][t & 3]
 elif which == "conv1":
-    m = [c for c, n, t in ev if n == "mma" and t % 24 == 0]
+    m = [c for c, n, t in ev if n == "mma" and t % 8 == 0]
     print("cycles per tile (MMA loop):", [m[i + 1] - m[i] for i in range(5, min(17, len(m) - 1))])
 
     def desc(n, t):
         if n == "mma":
-            return f"tile {t // 24} sub-stage {(t // 4) % 6} " + ["loop", "slot free", "issued"][t & 3]
+            return f"tile {t // 8} half {(t // 4) % 2} " + ["loop", "slot free", "issued"][t & 3]
         if n == "load":
             return f"tile {t} tma issued"
-        return f"tile {t // 32} pass {(t // 8) % 4} " + ["wait T", "T full", "T in regs", "published", "past barrier", "stored"][t & 7]
+        return f"tile {t // 32} pass {(t // 8) % 4} " + ["wait slot", "slot full", "in regs", "stored"][t & 7]
 else:
     m1 = [c for c, n, t in ev if n == "mma1" and (t & 3) == 0]
     print("cycles per unit (MMA1 loop):", [m1[i + 1] - m1[i] for i in range(20, 40)])
