@@ -10,7 +10,11 @@ from oracle import cmlpl_oracle as O
 
 
 def rel(a, b):
-    """max|a - b| / max|b| in float64; a and b may be numpy arrays or tensors on any device."""
+    """max|a - b| / max|b| in float64; a and b may be numpy arrays or tensors on any device (two tensors on one device
+    are compared there).  NaN in a gives NaN, which fails every bar."""
+    if torch.is_tensor(a) and torch.is_tensor(b) and a.device == b.device:
+        a, b = a.detach().double(), b.detach().double()
+        return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
     a = np.asarray(a.detach().cpu() if torch.is_tensor(a) else a, dtype=np.float64)
     b = np.asarray(b.detach().cpu() if torch.is_tensor(b) else b, dtype=np.float64)
     return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-30))

@@ -9,8 +9,8 @@ import ctypes
 import numpy as np
 import pytest
 import torch
-import torch.nn.functional as F
 
+import dense_refs as D
 from oracle import cmlpl_oracle as O
 from scene_harness import near_ties_only, path_mode, raw_scene, rel, scene_net
 
@@ -112,7 +112,8 @@ def test_row_bands_are_bit_identical_at_32_classes(dev):
 @pytest.mark.parametrize("K", [24, 32])
 def test_pool2_cls_row_maps_match_torch(dev, K):
     """pool2_cls_kernel<32> on the kernel's own half-pooled conv2 maps yq: M[I][y', x'] = sum_J L[I][J][y', x' + 2J]
-    with the remaining 2x2 pool of the middle classes, against torch in fp32 on the same fp16 inputs and weights."""
+    with the remaining 2x2 pool of the middle classes, against the float64 reference of tests/dense_refs.py on the same
+    fp16 inputs and weights: within its bound on every entry the head reads, and within 1e-4 * max|ref|."""
     from cmlpl_b200 import _lib
     R, C, B, w = 37, 45, 103, 20
     rng = np.random.default_rng(K)
@@ -130,22 +131,16 @@ def test_pool2_cls_row_maps_match_torch(dev, K):
     _lib.call("cmlpl_conv2_scene_f16", pmq.data_ptr(), C, w, R, packed.data_ptr(), yq.data_ptr(), st)
     _lib.call("cmlpl_pool2_cls_f16", yq.data_ptr(), C, w, R, B, K, packed.data_ptr(), lmap.data_ptr(), st)
     torch.cuda.synchronize()
-    yz = torch.nan_to_num(yq.permute(0, 1, 2, 5, 3, 4).reshape(9, 4, 64, PR2, PC2).float())
-    Wc = net.classifier.weight.detach()[:, :1600].reshape(K, 64, 5, 5).half().float()
+    YP = torch.nan_to_num(D.dense_planes(yq, PR2, PC2).to(D.F64))
+    Wconv = net.classifier.weight.detach()[:, :1600].reshape(K, 64, 5, 5)
+    M_ref, M_a = D.pool2_ref(YP, Wconv, w, K)
+    Mk = D.dense_lmap(lmap, 32, PR2, PC2)[:, :, :K]
+    use = torch.from_numpy(D.consumed(R, C, w)[0]).to(dev)[:, :, None].expand(4, 5, K, PR2, PC2)
+    assert not torch.isnan(Mk[use]).any()
+    assert D.ratio(Mk, M_ref, D.bound(M_ref, M_a, D.N_POOL2, False), use) <= 1.0
     for I in range(5):
-        Al = 0 if I == 0 else (2 if I == 4 else 1)
-        ref = torch.zeros(4, K, PR2, PC2, device=dev)
-        for J in range(5):
-            Be = 0 if J == 0 else (2 if J == 4 else 1)
-            us = [0, 1] if Al == 1 else [0]
-            vs = [0, 1] if Be == 1 else [0]
-            for u in us:
-                for v in vs:
-                    sh = F.pad(yz[Al * 3 + Be], (0, 2 * J + 1, 0, 1))[:, :, u:u + PR2, 2 * J + v:2 * J + v + PC2]
-                    ref += torch.einsum("kc,pcyx->pkyx", Wc[:, :, I, J], sh) / (len(us) * len(vs))
-        got = lmap[:, I].permute(0, 1, 4, 2, 3).reshape(4, 32, PR2, PC2)[:, :K]
         # map I is read at y' = r' + 2I >= 2I, x' = c' <= PC2 - 11 only: compare where every input exists
-        g, r = got[:, :, 2 * I:PR2 - 1, :PC2 - 10], ref[:, :, 2 * I:PR2 - 1, :PC2 - 10]
+        g, r = Mk[:, I, :, 2 * I:PR2 - 1, :PC2 - 10], M_ref[:, I, :, 2 * I:PR2 - 1, :PC2 - 10]
         assert not torch.isnan(g).any(), I
         assert rel(g.cpu(), r.cpu()) < 1e-4, I
 

@@ -16,9 +16,10 @@ import numpy as np
 import pytest
 import torch
 
+import dense_refs as D
 from oracle import cmlpl_oracle as O
 from scene_harness import as_layout, fit_moments, near_ties_only, path_mode, rel
-from test_sensor_scenes_cpu import apply_bound, conv0_bar
+from test_sensor_scenes_cpu import apply_bound
 
 pytestmark = pytest.mark.gpu
 
@@ -111,39 +112,10 @@ def test_raw_conv0_map_on_sensor_scenes(dev, B, nd, sample, dc, layout):
     BIP), its band-major instantiation (224 BSQ), and the K-sliced kernel (270 BIL, 512 BIP), against the folded 1x1 conv
     in float64 on the mirror-padded scene: per position and channel within conv0_bar (half an fp16 ulp + the hi / lo
     cancellation term), and 1e-3 of the largest entry overall."""
-    from cmlpl_b200 import ops, preprocess
-    from cmlpl_b200.tools.models import BaseNet2
-    R, C, K, w = 23, 31, 9, 20
-    cube, _, _ = _scene(R, C, B, K, nd, sample, dc)
-    pp = preprocess.fit(as_layout(cube, "bip", dev), 60)
-    torch.manual_seed(B)
-    net = BaseNet2(B, 0, K, w=w).to(dev).eval()
-    folded = pp.folded_conv0(net.conv0.weight, net.conv0.bias, dev)
-    W0 = net.conv0.weight.detach().double().cpu().numpy().reshape(64, 60)
-    wf64 = (pp.U / pp.pca_sigma[None]) @ W0.T
-    bf64 = net.conv0.bias.detach().double().cpu().numpy() - W0 @ (pp.pca_mu / pp.pca_sigma)
-    ws = ops.scene_workspace(R, C, B, K, w, dev)
-    ops.scene_infer_raw(as_layout(cube, layout, dev), folded, net.packed_weights(w), K, C, w, workspace=ws,
-                        interleave=layout)
-    torch.cuda.synchronize()
-    PR, PC = R + w - 1, C + w - 1
-    got = ws[:8 * PR * PC * 16].view(torch.float16).view(8, PR, PC, 8).permute(1, 2, 0, 3).reshape(-1, 64).double().cpu().numpy()
-    rr = O.mirror_index(np.arange(PR) - w // 2, R)
-    cc = O.mirror_index(np.arange(PC) - w // 2, C)
-    Xp = cube[rr][:, cc].reshape(-1, B).astype(np.float64)
-    ref = (Xp - pp.mu) @ wf64 + bf64
-    bar, T = conv0_bar(Xp, folded["mu"].cpu().numpy(), pp.mu, folded["inv_sigma"].cpu().numpy(),
-                       folded["wf"].cpu().numpy(), wf64, bf64, ref)
-    err = np.abs(got - ref)
-    r = err / bar
-    i = np.argmax(r)
-    print("B = %d, %s, %s, %.0f DN: conv0 map error / max|F0| %.1e; worst element: error %.2e, bar %.2e (half ulp "
-          "%.2e), ratio %.3f; sum|z||w| / |F0| there %.1e" % (B, sample, layout, nd, err.max() / np.abs(ref).max(),
-                                                              err.flat[i], bar.flat[i],
-                                                              0.5 * np.spacing(np.float16(abs(ref.flat[i]))),
-                                                              r.max(), T.flat[i] / abs(ref.flat[i])))
-    assert np.all(err <= bar)
-    assert err.max() < 1e-3 * np.abs(ref).max()
+    q, e = D.raw_conv0_map_check(dev, 23, 31, B, 9, 20, nd, sample, dc, layout)
+    print("B = %d, %s, %s, %.0f DN: conv0 map error / max|F0| %.1e; worst error / bar %.3f" % (B, sample, layout, nd, e, q))
+    assert q <= 1.0
+    assert e < 1e-3
 
 
 # --------------------------------------------------------------------------------------- 4. raw entry point, oracle
