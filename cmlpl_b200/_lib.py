@@ -38,6 +38,10 @@ SIGNATURES = {
     "cmlpl_scene_infer_raw": (I, [P, I, I, I, I, I, I, I, I, I, I, P, P, P, P, P, P, Z, P, P, P]),
     "cmlpl_scene_infer_raw_masked": (I, [P, I, I, I, I, I, I, I, I, I, I, P, P, P, P, P, P, P, Z, P, P, P]),
     "cmlpl_valid_mask_u8": (I, [P, I, L, I, I, c_double, P, P, P, P]),
+    "cmlpl_valid_mask_sel_u8": (I, [P, I, L, I, I, P, I, c_double, P, P, P, P]),
+    "cmlpl_preprocess_fit_sel_f64": (I, [P, I, L, I, I, P, I, P, P, P, P, P]),
+    "cmlpl_preprocess_apply_sel": (I, [P, I, L, I, P, I, I, P, P, P, P, P, P, P, P]),
+    "cmlpl_scene_infer_raw_sel": (I, [P, I, I, I, I, I, I, P, I, I, I, I, I, P, P, P, P, P, P, P, Z, P, P, P]),
     "cmlpl_conv0_map_f16": (I, [P, I, I, I, I, I, I, I, P, P, P]),
     "cmlpl_patch_cnn_f16": (I, [P, I, I, I, P, P, P]),
     "cmlpl_scene_workspace_layout": (I, [I, I, I, I, I, P]),

@@ -77,6 +77,57 @@ struct BandMajor {
   int64_t rs, bs;
 };
 
+// Band selection (include/cmlpl.h, the *_sel entry points): which raw band every reader of raw samples reads as feature
+// k.  AllBands is the whole cube (feature k = band k, the entry points without a list); BandList<N> carries a strictly
+// increasing list of n <= N raw bands by value in the kernel parameters (checked on the host, captured by CUDA graphs,
+// no device buffer); SmemBands is such a list staged in shared memory, for readers whose lanes index it divergently
+// (the constant bank serialises divergent reads).  Every reader maps a feature to its raw band with raw_band().
+struct AllBands {
+  static constexpr bool kSel = false;
+  __host__ __device__ __forceinline__ int operator[](int k) const { return k; }
+};
+template <int N> struct BandList {
+  static constexpr bool kSel = true;
+  int n;
+  uint16_t b[N];
+  __host__ __device__ __forceinline__ int operator[](int k) const { return b[k]; }
+};
+struct SmemBands {
+  static constexpr bool kSel = true;
+  const uint16_t* b;
+  __device__ __forceinline__ int operator[](int k) const { return b[k]; }
+};
+template <class Sel> __host__ __device__ __forceinline__ int raw_band(const Sel& sel, int k) { return sel[k]; }
+// the scene path's list (<= 512 selected bands, 1 KB of parameters) and the preprocessing's (<= 8192, 16 KB)
+constexpr int kSceneMaxSel = 512, kRawMaxBandsSel = 8192;
+using SceneBands = BandList<kSceneMaxSel>;
+using PreBands = BandList<kRawMaxBandsSel>;
+// stage `sel` into tab [n] (block-wide; the caller synchronises before reading it): a SmemBands view, or AllBands as is
+template <int N> __device__ __forceinline__ SmemBands stage_bands(const BandList<N>& sel, uint16_t* tab) {
+  for (int i = threadIdx.x; i < sel.n; i += blockDim.x) tab[i] = sel.b[i];
+  return SmemBands{tab};
+}
+__device__ __forceinline__ AllBands stage_bands(const AllBands& sel, uint16_t*) { return sel; }
+
+// Checks a host band list (the *_sel entry points) and copies it into *out: 1 <= nsel <= max_sel entries, strictly
+// increasing, inside [0, B), B <= kRawMaxBandsSel.  `fn` names the entry point.  No CUDA call.
+template <int N>
+inline int check_band_list(const char* fn, int B, const int* bands_host, int nsel, int max_sel, BandList<N>* out) {
+  CMLPL_CHECK_ARG(bands_host, "%s: null band list", fn);
+  CMLPL_CHECK_ARG(B > 0 && B <= kRawMaxBandsSel, "%s: raw band count %d outside 1..%d", fn, B, kRawMaxBandsSel);
+  CMLPL_CHECK_ARG(nsel > 0, "%s: empty band list", fn);
+  CMLPL_CHECK_ARG(nsel <= max_sel && nsel <= N, "%s: band list of %d bands, at most %d", fn, nsel, max_sel < N ? max_sel : N);
+  for (int k = 0; k < nsel; ++k) {
+    CMLPL_CHECK_ARG(bands_host[k] >= 0 && bands_host[k] < B, "%s: band list entry %d = %d outside [0, %d)", fn, k,
+                    bands_host[k], B);
+    CMLPL_CHECK_ARG(k == 0 || bands_host[k] > bands_host[k - 1], "%s: band list not strictly increasing at entry %d (%d after %d)",
+                    fn, k, bands_host[k], bands_host[k - 1]);
+    out->b[k] = uint16_t(bands_host[k]);
+  }
+  out->n = nsel;
+  return CMLPL_OK;
+}
+
 // The raw cube code (include/cmlpl.h): dtype = sample (CMLPL_RAW_U16 / F32 / I16) | interleave (CMLPL_RAW_BIP / BIL /
 // BSQ).  Bytes per sample:
 inline int raw_sample_bytes(int dtype) { return (dtype & 0x0f) == CMLPL_RAW_F32 ? 4 : 2; }

@@ -17,6 +17,9 @@
 // valid (raw cube only; u8 [slab_rows * cols] over the slab's pixels, or nullptr): a position whose mirrored source pixel
 // is no-data gets the z-scored operand 0 (hi and lo), i.e. the pixel stands in as its band means and F0 there is the
 // folded bias exactly.  The mask byte is read once per tile position; the sample loads keep their order.
+// Band selection (Sel = SceneBands, include/cmlpl.h cmlpl_scene_infer_raw_sel): channel k is raw band raw_band(sel, k) of
+// pixels of ld samples (pixel-major) or of the band-major slab; the list is staged in shared memory, where the
+// pixel-major loaders' lanes index it divergently.  K, the plan and the operands follow the selected count.
 #include <type_traits>
 
 #include "common.cuh"
@@ -38,20 +41,20 @@ enum { kLoadVec4, kLoadPixel, kLoadPixelSlice, kLoadBandMajor };
 
 // Shared memory of conv0_tc_kernel, the same for the launcher (its size) and the kernel (its offsets): fp16 weights
 // [KC][64 n][8 k] (hi | lo when split), the ring of nstage X slice buffers [S/8 chunks][128 positions][8] (hi | lo),
-// bias, band means, barriers and the TMEM address.
+// bias, band means, the band list (u16 [KP], only with a list), barriers and the TMEM address.
 struct Conv0Plan {
   int KP, S, nslice, nstage;
   int whalf, xhalf, xstage;                // bytes: weights hi, a slice buffer's hi, a slice buffer
-  int x, bias, mu, bar, tmem, bytes;       // offsets; the dynamic shared memory in all
+  int x, bias, mu, sel, bar, tmem, bytes;  // offsets; the dynamic shared memory in all
 };
 __host__ __device__ inline int conv0_xhalf(int S) { return (S / 8 * c0s::XCH + 127) / 128 * 128; }
-__host__ __device__ inline Conv0Plan conv0_plan(int K, bool split) {
+__host__ __device__ inline Conv0Plan conv0_plan(int K, bool split, bool sel) {
   Conv0Plan P;
   const int mult = split ? 2 : 1;
   P.KP = (K + 15) / 16 * 16;
   P.whalf = P.KP / 8 * 64 * 16;
-  const int mu_bytes = (P.KP * 4 + 127) / 128 * 128;
-  const int fixed = P.whalf * mult + 256 + mu_bytes + 64 + 16 + 128;    // + barriers, TMEM address, alignment
+  const int mu_bytes = (P.KP * 4 + 127) / 128 * 128, sel_bytes = sel ? (P.KP * 2 + 127) / 128 * 128 : 0;
+  const int fixed = P.whalf * mult + 256 + mu_bytes + sel_bytes + 64 + 16 + 128;    // + barriers, TMEM address, alignment
   if (P.KP <= 256) {
     P.S = P.KP;
     P.nstage = fixed + 2 * conv0_xhalf(P.S) * mult <= 227 * 1024 ? 2 : 1;
@@ -65,7 +68,8 @@ __host__ __device__ inline Conv0Plan conv0_plan(int K, bool split) {
   P.x = P.whalf * mult;
   P.bias = P.x + P.nstage * P.xstage;
   P.mu = P.bias + 256;
-  P.bar = P.mu + mu_bytes;
+  P.sel = P.mu + mu_bytes;
+  P.bar = P.sel + sel_bytes;
   P.tmem = P.bar + 64;
   P.bytes = fixed + P.nstage * P.xstage;
   return P;
@@ -74,19 +78,20 @@ __host__ __device__ inline Conv0Plan conv0_plan(int K, bool split) {
 // Split operands (raw cube): both operands are split into fp16 hi + lo parts and every K-step issues hi.hi + hi.lo +
 // lo.hi (~2^-21 relative error).  The folded PCA projection is ill-conditioned -- its noise components are differences
 // of band values ~10x larger than the result -- so single fp16 operands miss the 1e-3 logit bar (measured at B = 200).
-// bm: the band-major slab's strides (kLoadBandMajor only).
-template <typename T, int kLoad>
+// bm: the band-major slab's strides (kLoadBandMajor only); ld: samples per pixel of a pixel-major input (K without a list).
+template <typename T, int kLoad, class Sel>
 __global__ void __launch_bounds__(c0s::kThreads, 1)
-conv0_tc_kernel(const T* __restrict__ in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0, int prow_n,
-                int pcol_n, const float* __restrict__ wt /* [K][64] */, const float* __restrict__ bias,
-                const float* __restrict__ mu, const float* __restrict__ inv_sigma, __half* __restrict__ f0pad, BandMajor bm,
-                const uint8_t* __restrict__ valid) {
+conv0_tc_kernel(const T* __restrict__ in, int K, int ld, Sel sel, int scene_rows, int cols, int slab_row0, int w,
+                int band_row0, int prow_n, int pcol_n, const float* __restrict__ wt /* [K][64] */,
+                const float* __restrict__ bias, const float* __restrict__ mu, const float* __restrict__ inv_sigma,
+                __half* __restrict__ f0pad, BandMajor bm, const uint8_t* __restrict__ valid) {
   using namespace c0s;
   constexpr bool kSplit = kLoad != kLoadVec4;
   extern __shared__ __align__(128) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t sbase = smem_u32(smem);
-  const Conv0Plan P = conv0_plan(K, kSplit);
+  const Conv0Plan P = conv0_plan(K, kSplit, Sel::kSel);
+  const auto bands = stage_bands(sel, reinterpret_cast<uint16_t*>(smem + P.sel));   // read after the __syncthreads below
   const int KP = P.KP, sh = P.nstage - 1;                       // slice g of the ring: buffer g & sh, phase (g >> sh) & 1
   const uint32_t bars = sbase + P.bar;
   volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem + P.tmem);
@@ -210,11 +215,13 @@ conv0_tc_kernel(const T* __restrict__ in, int K, int scene_rows, int cols, int s
         // (per-lane mean / 1/sigma of its k's stay in registers), 4 pixels (up to 32 loads) in flight per lane
         for_slices([&](int, unsigned char* xs) {
           float mr[8], ir[8];
+          int rb[8];                                            // raw band of each of the lane's k's (AllBands: k itself)
 #pragma unroll
           for (int m = 0; m < 8; ++m) {
             const int k = lane + 32 * m;
             mr[m] = k < K ? smu[k] : 0.f;
             ir[m] = (inv_sigma && k < K) ? __ldg(inv_sigma + k) : 1.f;
+            rb[m] = k < K ? raw_band(bands, k) : 0;
           }
 #pragma unroll 1
           for (int j0 = 0; j0 < 16; j0 += 4) {
@@ -224,11 +231,11 @@ conv0_tc_kernel(const T* __restrict__ in, int K, int scene_rows, int cols, int s
             for (int jj = 0; jj < 4; ++jj) {
               const int2 sp = src_pixel(p0, warp + 8 * (j0 + jj));
               const int64_t px = int64_t(sp.x) * cols + sp.y;
-              const T* src = in + px * K;
+              const T* src = in + px * ld;
 #pragma unroll
               for (int m = 0; m < 8; ++m) {
                 const int k = lane + 32 * m;
-                v[jj][m] = k < K ? float(src[k]) : 0.f;
+                v[jj][m] = k < K ? float(src[Sel::kSel ? rb[m] : k]) : 0.f;
               }
               ok[jj] = !valid || valid[px];
             }
@@ -257,20 +264,21 @@ conv0_tc_kernel(const T* __restrict__ in, int K, int scene_rows, int cols, int s
         for (int jj = 0; jj < 16; ++jj) {
           const int2 sp = src_pixel(p0, warp + 8 * jj);
           const int64_t px = int64_t(sp.x) * cols + sp.y;
-          src[jj] = in + px * K;
+          src[jj] = in + px * ld;
           if (valid && !valid[px]) okm &= ~(1u << jj);
         }
         for_slices([&](int j, unsigned char* xs) {
           const int k0 = j * kSlice + lane, k1 = k0 + 32;
           const float m0 = smu[k0 < KP ? k0 : 0], i0 = k0 < K ? __ldg(inv_sigma + k0) : 0.f;
           const float m1 = smu[k1 < KP ? k1 : 0], i1 = k1 < K ? __ldg(inv_sigma + k1) : 0.f;
+          const int b0 = k0 < K ? raw_band(bands, k0) : 0, b1 = k1 < K ? raw_band(bands, k1) : 0;
 #pragma unroll
           for (int h = 0; h < 16; h += 8) {
             float v[8][2];
 #pragma unroll
             for (int jj = 0; jj < 8; ++jj) {
-              v[jj][0] = k0 < K ? float(src[h + jj][k0]) : 0.f;
-              v[jj][1] = k1 < K ? float(src[h + jj][k1]) : 0.f;
+              v[jj][0] = k0 < K ? float(src[h + jj][Sel::kSel ? b0 : k0]) : 0.f;
+              v[jj][1] = k1 < K ? float(src[h + jj][Sel::kSel ? b1 : k1]) : 0.f;
             }
 #pragma unroll
             for (int jj = 0; jj < 8; ++jj) {
@@ -306,7 +314,7 @@ conv0_tc_kernel(const T* __restrict__ in, int K, int scene_rows, int cols, int s
 #pragma unroll
               for (int e = 0; e < 8; ++e) {
                 const int k = kb + (c0 + 2 * u) * 8 + e;
-                v[u][e] = k < K ? float(src[int64_t(k) * bm.bs]) : 0.f;
+                v[u][e] = k < K ? float(src[int64_t(raw_band(bands, k)) * bm.bs]) : 0.f;
               }
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
@@ -364,16 +372,18 @@ conv0_tc_kernel(const T* __restrict__ in, int K, int scene_rows, int cols, int s
 }
 
 // kVec4 (PCA cube) with plain operands, or the raw cube with split operands.  bm: the raw slab is band-major (BIL /
-// BSQ), or nullptr for pixel-major; valid: the raw slab's validity mask, or nullptr
-template <typename T, bool kVec4, bool kSplit>
-int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0, int prow_n, int pcol_n,
-                    const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad,
-                    const BandMajor* bm, const uint8_t* valid, cudaStream_t s) {
+// BSQ), or nullptr for pixel-major with ld samples per pixel; valid: the raw slab's validity mask, or nullptr; sel: the
+// raw bands of the K channels (AllBands: channel k is band k)
+template <typename T, bool kVec4, bool kSplit, class Sel>
+int launch_conv0_tc(const T* in, int K, int ld, const Sel& sel, int scene_rows, int cols, int slab_row0, int w, int band_row0,
+                    int prow_n, int pcol_n, const float* wt, const float* bias, const float* mu, const float* inv_sigma,
+                    __half* f0pad, const BandMajor* bm, const uint8_t* valid, cudaStream_t s) {
   static_assert(kVec4 != kSplit, "conv0 reads the PCA cube with plain operands and the raw cube with split ones");
+  static_assert(!(kVec4 && Sel::kSel), "a band list selects raw bands");
   using namespace c0s;
   CMLPL_CHECK_ARG(int64_t(prow_n) * pcol_n < (int64_t(1) << 31) - 256, "conv0: band of %d x %d padded positions is too large",
                   prow_n, pcol_n);
-  const Conv0Plan P = conv0_plan(K, kSplit);
+  const Conv0Plan P = conv0_plan(K, kSplit, Sel::kSel);
   if (kSplit && P.KP > 256) {
     CMLPL_CHECK_ARG(K <= kMaxK, "conv0: K=%d unsupported by the tensor-core kernel (at most %d)", K, kMaxK);
     CMLPL_CHECK_ARG(mu && inv_sigma, "conv0: the K-sliced kernel needs the band means and 1/sigma");
@@ -388,10 +398,10 @@ int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0,
   if (grid > ntiles) grid = int(ntiles);
   // one instantiation of run per kernel, so that the shared-memory opt-in CMLPL_MAX_DYN_SMEM caches is that kernel's
   auto run = [&](auto load) {
-    auto kern = conv0_tc_kernel<T, decltype(load)::value>;
+    auto kern = conv0_tc_kernel<T, decltype(load)::value, Sel>;
     CMLPL_MAX_DYN_SMEM(kern, P.bytes);
-    kern<<<grid, kThreads, P.bytes, s>>>(in, K, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu, inv_sigma,
-                                         f0pad, bm ? *bm : BandMajor{}, valid);
+    kern<<<grid, kThreads, P.bytes, s>>>(in, K, ld, sel, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n, wt, bias, mu,
+                                         inv_sigma, f0pad, bm ? *bm : BandMajor{}, valid);
     CMLPL_CHECK_LAUNCH("conv0_tc");
     return CMLPL_OK;
   };
@@ -401,14 +411,17 @@ int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0,
   else return run(std::integral_constant<int, kLoadPixel>{});
 }
 
-#define CMLPL_CONV0_INST(T, kVec4, kSplit)                                                                                 \
-  template int launch_conv0_tc<T, kVec4, kSplit>(const T*, int, int, int, int, int, int, int, int, const float*, const float*, \
-                                                 const float*, const float*, __half*, const BandMajor*, const uint8_t*,   \
-                                                 cudaStream_t);
-CMLPL_CONV0_INST(float, true, false)
-CMLPL_CONV0_INST(float, false, true)
-CMLPL_CONV0_INST(uint16_t, false, true)
-CMLPL_CONV0_INST(int16_t, false, true)
+#define CMLPL_CONV0_INST(T, kVec4, kSplit, Sel)                                                                             \
+  template int launch_conv0_tc<T, kVec4, kSplit, Sel>(const T*, int, int, const Sel&, int, int, int, int, int, int, int,    \
+                                                      const float*, const float*, const float*, const float*, __half*,      \
+                                                      const BandMajor*, const uint8_t*, cudaStream_t);
+CMLPL_CONV0_INST(float, true, false, AllBands)
+CMLPL_CONV0_INST(float, false, true, AllBands)
+CMLPL_CONV0_INST(uint16_t, false, true, AllBands)
+CMLPL_CONV0_INST(int16_t, false, true, AllBands)
+CMLPL_CONV0_INST(float, false, true, SceneBands)
+CMLPL_CONV0_INST(uint16_t, false, true, SceneBands)
+CMLPL_CONV0_INST(int16_t, false, true, SceneBands)
 #undef CMLPL_CONV0_INST
 
 }  // namespace cmlpl

@@ -14,30 +14,33 @@ struct StridedA {
   __device__ __forceinline__ void prep(int) {}
   __device__ __forceinline__ float at(int m, int k) const { return __ldg(p + m * rs + k * cs); }
 };
-// rows of the raw cube (uint16 / float32, row stride rs), z-scored on load: A(m,k) = (x[m][k] - mu[k]) * inv_sigma[k];
-// valid (u8 per row, or nullptr): a no-data row stands in as its band means, a zero row
-template <typename T>
+// rows of the raw cube (uint16 / float32, row stride rs), z-scored on load: A(m,k) = (x[m][b] - mu[k]) * inv_sigma[k] with
+// b = raw_band(sel, k) (Sel: common.cuh; a warp's lanes share k); valid (u8 per row, or nullptr): a no-data row stands in
+// as its band means, a zero row
+template <typename T, class Sel = AllBands>
 struct RawZA {
   const T* p; int64_t rs; const float* mu; const float* inv_sigma; const uint8_t* valid;
   bool ok_;
+  Sel sel;
   __device__ __forceinline__ void prep(int m) { ok_ = !valid || valid[m]; }
   __device__ __forceinline__ float at(int m, int k) const {
-    return ok_ ? (float(__ldg(p + m * rs + k)) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
+    return ok_ ? (float(__ldg(p + m * rs + raw_band(sel, k))) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
   }
 };
 // the same from a band-major raw slab (BIL / BSQ): pixel m0 + m of the band is row (m0 + m) / cols, column
-// (m0 + m) % cols of the band's rows at p; the k order and the validity rows (valid[m0 + m]) are RawZA's
-template <typename T>
+// (m0 + m) % cols of the band's rows at p; the k order, the band list and the validity rows (valid[m0 + m]) are RawZA's
+template <typename T, class Sel = AllBands>
 struct RawBandZA {
   const T* p; BandMajor bm; int64_t m0; const float* mu; const float* inv_sigma; const uint8_t* valid;
   int64_t off_; bool ok_;
+  Sel sel;
   __device__ __forceinline__ void prep(int m) {
     const int64_t q = m0 + m, r = q / bm.cols;
     off_ = r * bm.rs + (q - r * bm.cols);
     ok_ = !valid || valid[q];
   }
   __device__ __forceinline__ float at(int, int k) const {
-    return ok_ ? (float(__ldg(p + off_ + k * bm.bs)) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
+    return ok_ ? (float(__ldg(p + off_ + raw_band(sel, k) * bm.bs)) - __ldg(mu + k)) * __ldg(inv_sigma + k) : 0.f;
   }
 };
 struct StridedB {  // B[k][n]

@@ -17,10 +17,11 @@ namespace cmlpl {
 // kZ false: the preprocessed f32 spectra.  kZ: the raw cube, x16 = (raw - mu) * inv_sigma (featureNormalize(X, 1),
 // hyper_tools.py:292), zero rows for no-data pixels.  Band k of pixel p is at p * B + k (pixel-major), or for a
 // band-major slab (kBM: BIL / BSQ, include/cmlpl.h) at row p / cols, column p % cols of the band's rows at X, band
-// stride bm.bs; with rows as the fastest index, a warp's loads of one band are consecutive columns
-template <typename T, bool kBM, bool kZ>
-__global__ void x16_tile_kernel(const T* __restrict__ X, BandMajor bm, int64_t n, int B, int KC, int64_t total,
-                                const float* __restrict__ mu, const float* __restrict__ inv_sigma,
+// stride bm.bs; with rows as the fastest index, a warp's loads of one band are consecutive columns.  Pixel-major rows hold ld
+// samples; feature k is raw band raw_band(sel, k) (warp-uniform: a warp's 32 rows share their K-chunk)
+template <typename T, bool kBM, bool kZ, class Sel>
+__global__ void x16_tile_kernel(const T* __restrict__ X, BandMajor bm, int64_t n, int B, int ld, Sel sel, int KC,
+                                int64_t total, const float* __restrict__ mu, const float* __restrict__ inv_sigma,
                                 const uint8_t* __restrict__ valid, __half* __restrict__ out) {
   for (int64_t t = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; t < total; t += int64_t(gridDim.x) * blockDim.x) {
     const int row = int(t & 127);
@@ -32,12 +33,15 @@ __global__ void x16_tile_kernel(const T* __restrict__ X, BandMajor bm, int64_t n
       const int64_t pr = p / bm.cols;
       x = X + pr * bm.rs + (p - pr * bm.cols);
     } else {
-      x = X + p * B;
+      x = X + p * ld;
     }
     const bool in = p < n && (!kZ || !valid || valid[p]);
     auto at = [&](int k) -> float {                          // band k of the pixel, z-scored from the raw cube
       if constexpr (!kZ) return __ldg(x + k);
-      else return (float(x[kBM ? k * bm.bs : k]) - __ldg(mu + k)) * __ldg(inv_sigma + k);
+      else {
+        const int b = raw_band(sel, k);
+        return (float(x[kBM ? b * bm.bs : b]) - __ldg(mu + k)) * __ldg(inv_sigma + k);
+      }
     };
     __half2 h[4];
 #pragma unroll
@@ -337,10 +341,11 @@ static bool spectral_logits_plan(int KC, int NC, int* nA, size_t* smem) {
 
 // x16_tile + spectral_logits_kernel: x16 is scratch for the fp16 input tiles, part f32 [4][ceil(n/128)*128][NC].
 // dtype: -1 = preprocessed f32 spectra, else the raw sample type (CMLPL_RAW_U16 / F32 / I16); bm: band-major raw rows, or
-// nullptr for pixel-major [n][B]; valid: u8 [n] of the raw rows (no-data pixels convert to zero rows), or nullptr
-int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_t n, int num_features, int num_classes,
-                           int w, const float* mu, const float* inv_sigma, const uint8_t* valid, const void* packed,
-                           void* x16, float* part, cmlpl_stream_t stream) {
+// nullptr for pixel-major [n][ld]; sel: the raw bands of the num_features features, or nullptr for bands 0..; valid: u8 [n]
+// of the raw rows (no-data pixels convert to zero rows), or nullptr
+int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int ld, const SceneBands* sel, int64_t n,
+                           int num_features, int num_classes, int w, const float* mu, const float* inv_sigma,
+                           const uint8_t* valid, const void* packed, void* x16, float* part, cmlpl_stream_t stream) {
   CMLPL_CHECK_ARG(x && packed && x16 && part, "spectral_logits_tc: null pointer");
   CMLPL_CHECK_ARG(n > 0 && num_features > 0, "spectral_logits_tc: bad dims");
   CMLPL_CHECK_ARG(num_classes <= 32, "spectral_logits_tc: needs <= 32 classes, got %d", num_classes);
@@ -353,17 +358,21 @@ int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_
   int64_t g = (total + 255) / 256; const int64_t cap = int64_t(sm_count()) * 16; if (g > cap) g = cap;
   __half* o = static_cast<__half*>(x16);
   if (dtype < 0)
-    x16_tile_kernel<float, false, false><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), BandMajor{}, n, num_features, KC,
-                                                               total, nullptr, nullptr, nullptr, o);
+    x16_tile_kernel<float, false, false><<<int(g), 256, 0, s>>>(static_cast<const float*>(x), BandMajor{}, n, num_features,
+                                                               num_features, AllBands{}, KC, total, nullptr, nullptr, nullptr, o);
   else
     with_sample(dtype, [&](auto sample) {
       using T = decltype(sample);
       const T* xt = static_cast<const T*>(x);
-      if (bm)
-        x16_tile_kernel<T, true, true><<<int(g), 256, 0, s>>>(xt, *bm, n, num_features, KC, total, mu, inv_sigma, valid, o);
-      else
-        x16_tile_kernel<T, false, true><<<int(g), 256, 0, s>>>(xt, BandMajor{}, n, num_features, KC, total, mu, inv_sigma,
-                                                               valid, o);
+      auto run = [&](auto bands) {
+        if (bm)
+          x16_tile_kernel<T, true, true><<<int(g), 256, 0, s>>>(xt, *bm, n, num_features, ld, bands, KC, total, mu, inv_sigma,
+                                                                valid, o);
+        else
+          x16_tile_kernel<T, false, true><<<int(g), 256, 0, s>>>(xt, BandMajor{}, n, num_features, ld, bands, KC, total, mu,
+                                                                 inv_sigma, valid, o);
+      };
+      if (sel) run(*sel); else run(AllBands{});
     });
   CMLPL_CHECK_LAUNCH("x16_tile");
   int grid = sm_count() / 4 * 4;
@@ -392,8 +401,8 @@ int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_
 // scratch for the fp16 input tiles.
 extern "C" int cmlpl_spectral_logits_tc(const float* spectra, int64_t n, int num_features, int num_classes, int w,
                                         const void* packed, void* x16, float* part, cmlpl_stream_t stream) {
-  return launch_spectral_logits(spectra, -1, nullptr, n, num_features, num_classes, w, nullptr, nullptr, nullptr, packed, x16,
-                                part, stream);
+  return launch_spectral_logits(spectra, -1, nullptr, num_features, nullptr, n, num_features, num_classes, w, nullptr, nullptr,
+                                nullptr, packed, x16, part, stream);
 }
 
 namespace cmlpl {

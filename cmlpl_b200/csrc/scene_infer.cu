@@ -15,6 +15,8 @@
 // With a validity mask (cmlpl_scene_infer_raw_masked) a no-data pixel stands in as its band means wherever it is read:
 // conv0's loaders and the spectral branch's operands z-score it to 0 (so F0 there is the folded bias), and the heads label
 // it CMLPL_NODATA_LABEL.  Everything between conv0 and the heads is unchanged.
+#include <type_traits>
+
 #include "common.cuh"
 #include "gemm_core.cuh"
 
@@ -28,18 +30,20 @@ namespace cmlpl {
 // logit bar).  PCA projection, both z-scores and conv0 are per-pixel affine maps, so they fold into one
 // F0 = Wf . (x - mu) + bf with Wf = W0 . (U/s)^T [64 x B] (SURVEY 8-f1).  Output: mirrored halo baked in, chunk-planar fp16
 // [8 chunks][prow_n][pcol_n][8].
-// bm: a band-major raw slab (BIL / BSQ), or nullptr for pixel-major; valid: the raw slab's validity mask, or nullptr
-template <typename T, bool kVec4, bool kSplit>
-int launch_conv0_tc(const T* in, int K, int scene_rows, int cols, int slab_row0, int w, int band_row0, int prow_n, int pcol_n,
-                    const float* wt, const float* bias, const float* mu, const float* inv_sigma, __half* f0pad,
-                    const BandMajor* bm, const uint8_t* valid, cudaStream_t s);
+// bm: a band-major raw slab (BIL / BSQ), or nullptr for pixel-major with ld samples per pixel; valid: the raw slab's
+// validity mask, or nullptr; sel: the raw bands of the K channels (AllBands, or SceneBands from a band list)
+template <typename T, bool kVec4, bool kSplit, class Sel>
+int launch_conv0_tc(const T* in, int K, int ld, const Sel& sel, int scene_rows, int cols, int slab_row0, int w, int band_row0,
+                    int prow_n, int pcol_n, const float* wt, const float* bias, const float* mu, const float* inv_sigma,
+                    __half* f0pad, const BandMajor* bm, const uint8_t* valid, cudaStream_t s);
 
 // x16_tile + spectral_logits_kernel (head_sm100.cu): x is the f32 z-scored spectra (dtype -1) or the raw cube's
 // rows (dtype = the sample type CMLPL_RAW_U16 / F32 / I16, z-scored with mu / inv_sigma in the conversion; band-major
-// through bm, else pixel-major; valid: the band's validity mask, or nullptr)
-int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int64_t n, int num_features, int num_classes,
-                           int w, const float* mu, const float* inv_sigma, const uint8_t* valid, const void* packed,
-                           void* x16, float* part, cmlpl_stream_t stream);
+// through bm, else pixel-major rows of ld samples; sel: the listed raw bands, or nullptr; valid: the band's validity mask,
+// or nullptr)
+int launch_spectral_logits(const void* x, int dtype, const BandMajor* bm, int ld, const SceneBands* sel, int64_t n,
+                           int num_features, int num_classes, int w, const float* mu, const float* inv_sigma,
+                           const uint8_t* valid, const void* packed, void* x16, float* part, cmlpl_stream_t stream);
 // head_sum_kernel (head_sm100.cu) behind cmlpl_head_sum_lmap; valid: the band's validity mask, or nullptr
 int launch_head_sum(const float* part, const float* lmap, int cols, int band_rows, int num_features, int num_classes, int w,
                     const void* packed, const uint8_t* valid, uint8_t* labels, float* logits, cmlpl_stream_t stream);
@@ -202,6 +206,8 @@ struct SceneSrc {
   const float *wf, *bf, *mu, *inv_sigma;
   bool masked;                             // cmlpl_scene_infer_raw_masked: the slab's validity mask u8 [slab_rows * cols]
   const uint8_t* valid;
+  int raw_bands;                           // cmlpl_scene_infer_raw_sel: the slab's band count and the list of the features'
+  const SceneBands* sel;                   // raw bands (else the features are the slab's bands)
 };
 
 // The conv0 map's conditions on the scene geometry (`fn` names the caller): the window fits the scene, the band lies
@@ -264,7 +270,7 @@ extern "C" int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, 
   const PackedLayout L = packed_layout(1, 1, w);  // w0/b0 offsets do not depend on B, C
   const unsigned char* pk = static_cast<const unsigned char*>(packed);
   const int prow_n = band_rows + w - 1, pcol_n = cols + w - 1;
-  return launch_conv0_tc<float, true, false>(cube, 60, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n,
+  return launch_conv0_tc<float, true, false>(cube, 60, 60, AllBands{}, scene_rows, cols, slab_row0, w, band_row0, prow_n, pcol_n,
                                       reinterpret_cast<const float*>(pk + L.w0), reinterpret_cast<const float*>(pk + L.b0), nullptr,
                                       nullptr, static_cast<__half*>(f0pad), nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
@@ -273,12 +279,12 @@ extern "C" int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, 
 // `chunk` pixels through the f32 scratch hidden [chunk][1024]
 // `spectra` is StridedA over the z-scored f32 spectra, or RawZA / RawBandZA over the raw band (z-scored on load)
 template <class FA> static FA rows_from(FA a, int64_t s0) { a.p += s0 * a.rs; return a; }          // pixel-major rows
-template <typename T> static RawZA<T> rows_from(RawZA<T> a, int64_t s0) {
+template <typename T, class Sel> static RawZA<T, Sel> rows_from(RawZA<T, Sel> a, int64_t s0) {
   a.p += s0 * a.rs;
   if (a.valid) a.valid += s0;
   return a;
 }
-template <typename T> static RawBandZA<T> rows_from(RawBandZA<T> a, int64_t s0) { a.m0 += s0; return a; }
+template <typename T, class Sel> static RawBandZA<T, Sel> rows_from(RawBandZA<T, Sel> a, int64_t s0) { a.m0 += s0; return a; }
 template <class FA>
 static int spectral_head(FA spectra, int64_t n, int num_features, int num_classes, int w, const void* packed,
                          float* hidden, int64_t chunk, float* spe_logits, cudaStream_t s) {
@@ -350,21 +356,23 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const int64_t n = int64_t(band_rows) * cols;
   float* part = reinterpret_cast<float*>(wsb + ws.h16);
-  // the raw slab: sample type, and for BIL / BSQ its band-major strides (pixel-major BIP has row stride cols * B)
+  // the raw slab: sample type, and for BIL / BSQ its band-major strides (pixel-major BIP has row stride cols * RB) over its
+  // RB bands, the B features' bands with a band list
   const int sample = src.dtype & 0x0f, il = src.dtype & 0xf0;
-  const BandMajor bmv = band_major(src.dtype, B, slab_rows, cols);
+  const int RB = src.sel ? src.raw_bands : B;
+  const BandMajor bmv = band_major(src.dtype, RB, slab_rows, cols);
   const BandMajor* bm = src.from_raw && il != CMLPL_RAW_BIP ? &bmv : nullptr;
   // the spectral branch reads the band's z-scored spectra, or the band's rows of the raw slab: in every interleave they
-  // start band_row0 - slab_row0 rows (of cols * B samples; of cols samples in every plane for BSQ) into the slab
-  const int64_t row_stride = bm ? bm->rs : int64_t(cols) * B;
+  // start band_row0 - slab_row0 rows (of cols * RB samples; of cols samples in every plane for BSQ) into the slab
+  const int64_t row_stride = bm ? bm->rs : int64_t(cols) * RB;
   const void* band_spectra =
       src.from_raw ? static_cast<const unsigned char*>(src.raw) + (band_row0 - slab_row0) * row_stride * raw_sample_bytes(src.dtype)
                    : static_cast<const void*>(src.spectra);
   // the band's validity: band pixel p is slab pixel (band_row0 - slab_row0) * cols + p
   const uint8_t* band_valid = src.valid ? src.valid + int64_t(band_row0 - slab_row0) * cols : nullptr;
   auto spectral_tc = [&](cudaStream_t st) {
-    return launch_spectral_logits(band_spectra, src.from_raw ? sample : -1, bm, n, B, C, w, src.mu, src.inv_sigma, band_valid,
-                                  packed, wsb + ws.x16, part, st);
+    return launch_spectral_logits(band_spectra, src.from_raw ? sample : -1, bm, RB, src.sel, n, B, C, w, src.mu, src.inv_sigma,
+                                  band_valid, packed, wsb + ws.x16, part, st);
   };
   auto conv0 = [&]() {
     if (!src.from_raw)
@@ -374,8 +382,12 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
     __half* f0 = reinterpret_cast<__half*>(wsb + ws.f0pad);
     return with_sample(sample, [&](auto sample_type) {
       using T = decltype(sample_type);
-      return launch_conv0_tc<T, false, true>(static_cast<const T*>(src.raw), B, scene_rows, cols, slab_row0, w, band_row0, prow_n,
-                                             pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, src.valid, s);
+      auto run = [&](const auto& bands) {
+        return launch_conv0_tc<T, false, true>(static_cast<const T*>(src.raw), B, RB, bands, scene_rows, cols, slab_row0, w,
+                                               band_row0, prow_n, pcol_n, src.wf, src.bf, src.mu, src.inv_sigma, f0, bm, src.valid,
+                                               s);
+      };
+      return src.sel ? run(*src.sel) : run(AllBands{});
     });
   };
   if (ws.dense) {
@@ -412,10 +424,14 @@ static int scene_infer(const SceneSrc& src, int scene_rows, int cols, int slab_r
   auto raw_head = [&](auto sample_type) {
     using T = decltype(sample_type);
     const T* x = static_cast<const T*>(band_spectra);
-    return bm ? spectral_head(RawBandZA<T>{x, *bm, 0, src.mu, src.inv_sigma, band_valid, 0, false}, n, B, C, w, packed, hidden,
-                              ws.chunk, spe, s)
-              : spectral_head(RawZA<T>{x, B, src.mu, src.inv_sigma, band_valid, false}, n, B, C, w, packed, hidden, ws.chunk,
-                              spe, s);
+    auto run = [&](const auto& bands) {
+      using Sel = std::decay_t<decltype(bands)>;
+      return bm ? spectral_head(RawBandZA<T, Sel>{x, *bm, 0, src.mu, src.inv_sigma, band_valid, 0, false, bands}, n, B, C, w,
+                                packed, hidden, ws.chunk, spe, s)
+                : spectral_head(RawZA<T, Sel>{x, RB, src.mu, src.inv_sigma, band_valid, false, bands}, n, B, C, w, packed,
+                                hidden, ws.chunk, spe, s);
+    };
+    return src.sel ? run(*src.sel) : run(AllBands{});
   };
   if (tc)
     rc = spectral_tc(s);
@@ -466,4 +482,21 @@ extern "C" int cmlpl_scene_infer_raw_masked(const void* raw, int dtype, int scen
   const SceneSrc src{"scene_infer_raw_masked", true, nullptr, nullptr, raw, dtype, wf, bf, mu, inv_sigma, true, valid};
   return scene_infer(src, scene_rows, cols, slab_row0, slab_rows, num_features, num_classes, w, band_row0, band_rows, packed,
                      workspace, workspace_bytes, labels, logits, stream);
+}
+
+// The same over the listed raw bands (include/cmlpl.h): raw holds B bands, the model reads the nsel bands of bands_host
+// (the features), valid is the slab's validity mask or NULL.  The list is checked with every other condition before
+// anything is enqueued; the path and the workspace follow nsel.
+extern "C" int cmlpl_scene_infer_raw_sel(const void* raw, int dtype, int scene_rows, int cols, int slab_row0, int slab_rows,
+                                         int B, const int* bands_host, int nsel, int num_classes, int w, int band_row0,
+                                         int band_rows, const float* wf, const float* bf, const float* mu,
+                                         const float* inv_sigma, const uint8_t* valid, const void* packed, void* workspace,
+                                         size_t workspace_bytes, uint8_t* labels, float* logits, cmlpl_stream_t stream) {
+  const char* fn = "scene_infer_raw_sel";
+  SceneBands sel;
+  const int rc = check_band_list(fn, B, bands_host, nsel, kRawMaxBands, &sel);
+  if (rc != CMLPL_OK) return rc;
+  const SceneSrc src{fn, true, nullptr, nullptr, raw, dtype, wf, bf, mu, inv_sigma, valid != nullptr, valid, B, &sel};
+  return scene_infer(src, scene_rows, cols, slab_row0, slab_rows, nsel, num_classes, w, band_row0, band_rows, packed, workspace,
+                     workspace_bytes, labels, logits, stream);
 }

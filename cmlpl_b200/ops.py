@@ -224,7 +224,11 @@ def scene_infer_raw(raw, folded, packed, num_classes: int, cols: int, w: int = 2
 
     ``valid`` (u8 [slab_rows, cols], 1 = valid; preprocess.valid_mask or any mask of that layout): a no-data pixel
     stands in as its band-mean spectrum wherever it is read -- in its neighbours' windows and as its own spectral input
-    -- and is labelled NODATA_LABEL; its logits, when asked for, are those of the imputed pixel."""
+    -- and is labelled NODATA_LABEL; its logits, when asked for, are those of the imputed pixel.
+
+    A ``folded`` from a Preproc fitted with ``bands`` carries that list: the call reads only those raw bands of ``raw``
+    (which must have the fit's ``raw_bands``), and the model, the path and the workspace see len(bands) features; the
+    results equal those of the same call on ``raw`` holding only the listed bands."""
     from . import preprocess
     if not raw.is_cuda or not raw.is_contiguous():
         raise _lib.CmlplError("raw must be a contiguous CUDA tensor (cmlpl_b200 has no CPU path)")
@@ -236,22 +240,32 @@ def scene_infer_raw(raw, folded, packed, num_classes: int, cols: int, w: int = 2
     n = band_rows * cols
     for k in ("wf", "bf", "mu", "inv_sigma"):
         _chk(folded[k], name=k)
-    if folded["wf"].shape != (B, 64):
-        raise _lib.CmlplError(f"folded conv0 weight must be [{B}, 64]")
+    sel = folded.get("bands")
+    if sel is not None:
+        sel = preprocess.band_list(sel)
+        if B != folded["raw_bands"]:
+            raise _lib.CmlplError(f"raw has {B} bands, the band list of folded= selects from {folded['raw_bands']}")
+    nf = B if sel is None else sel.size
+    if folded["wf"].shape != (nf, 64):
+        raise _lib.CmlplError(f"folded conv0 weight must be [{nf}, 64]")
     if workspace is None:
-        workspace = scene_workspace(band_rows, cols, B, num_classes, w, raw.device)
+        workspace = scene_workspace(band_rows, cols, nf, num_classes, w, raw.device)
     if labels is None:
         labels = torch.empty((n,), dtype=torch.uint8, device=raw.device)
     logits = torch.empty((n, num_classes), dtype=_f32, device=raw.device) if want_logits else None
     pre = (folded["wf"].data_ptr(), folded["bf"].data_ptr(), folded["mu"].data_ptr(), folded["inv_sigma"].data_ptr())
     post = (packed.data_ptr(), workspace.data_ptr(), workspace.numel(), labels.data_ptr(), _p(logits), _stream())
     geom = (code, scene_rows, cols, slab_row0, slab_rows, B, num_classes, w, band_row0, band_rows)
-    if valid is None:
-        _lib.call("cmlpl_scene_infer_raw", raw.data_ptr(), *geom, *pre, *post)
-    else:
+    if valid is not None:
         _chk(valid, torch.uint8, "valid")
         if valid.numel() != slab_rows * cols:
             raise _lib.CmlplError(f"valid has {valid.numel()} pixels, the slab {slab_rows} x {cols}")
+    if sel is not None:
+        _lib.call("cmlpl_scene_infer_raw_sel", raw.data_ptr(), *geom[:6], sel.ctypes.data, sel.size, *geom[6:], *pre,
+                  _p(valid), *post)
+    elif valid is None:
+        _lib.call("cmlpl_scene_infer_raw", raw.data_ptr(), *geom, *pre, *post)
+    else:
         _lib.call("cmlpl_scene_infer_raw_masked", raw.data_ptr(), *geom, *pre, valid.data_ptr(), *post)
     return (labels, logits) if want_logits else labels
 

@@ -259,13 +259,23 @@ class StreamedRawScene:
     ``fill`` (a value of the sample type; NaN for float32 = non-finite samples only): the cube has no-data pixels.  The
     slab's validity mask is built on the device from the rows each copy brought (BSQ: from the whole slab once its last
     rows have landed, since a BSQ row band is not a cube of its own), so nothing more crosses PCIe; the calls run
-    cmlpl_scene_infer_raw_masked and need ``folded=``.  No-data pixels get ops.NODATA_LABEL."""
+    cmlpl_scene_infer_raw_masked and need ``folded=``.  No-data pixels get ops.NODATA_LABEL.
+
+    A ``preproc`` fitted with ``bands`` (``num_features`` = the host cube's band count, its ``raw_bands``) makes every call
+    read only those bands, and the model sees len(bands) features.  A BSQ cube copies only the listed planes, one 2-D copy
+    per run of consecutive bands (``h2d_bytes`` shrinks to nsel / B of the whole); BIP and BIL copy whole rows and the
+    kernels select the bands on the device."""
 
     def __init__(self, preproc, scene_rows, cols, num_features, num_classes, w=20, nsplit=2, row0=0, rows=None,
                  raw_dtype=torch.uint16, device=None, interleave="bip", fill=None):
         from .. import preprocess
         self._pp_mod, self.pp = preprocess, preproc
         self.R, self.C, self.B, self.K, self.w = scene_rows, cols, num_features, num_classes, w
+        self.sel = None if preproc is None else preproc.bands
+        if self.sel is not None and preproc.raw_bands != num_features:
+            raise _lib.CmlplError(f"StreamedRawScene: the Preproc's band list selects from {preproc.raw_bands} bands, the "
+                                  f"cube has num_features = {num_features}")
+        self.nf = num_features if self.sel is None else self.sel.size          # the model's features
         self.r0 = row0
         self.r1 = scene_rows if rows is None else row0 + rows
         dev = _device() if device is None else device
@@ -280,17 +290,26 @@ class StreamedRawScene:
         if interleave not in shape:
             raise _lib.CmlplError(f"interleave must be one of {sorted(shape)}, got {interleave!r}")
         self.interleave, self.h2d_bytes, self.fill = interleave, 0, fill
+        self.host_shape = shape[interleave]
+        # BSQ with a band list: the device slab holds the listed planes only, copied as runs (first raw band, first slab
+        # plane, count) of consecutive bands; the kernels then read all of its planes
+        sel = np.arange(num_features) if self.sel is None else self.sel
+        self.runs = [(int(r[0]), int(np.searchsorted(sel, r[0])), len(r))
+                     for r in np.split(sel, np.flatnonzero(np.diff(sel) != 1) + 1)]
+        self.compact = interleave == "bsq" and self.sel is not None
+        if self.compact:
+            shape["bsq"] = (self.nf, sr, cols)
         if fill is not None:
             preprocess._fill_value(torch.empty(0, dtype=raw_dtype), fill)        # an integer cube needs a fill value
         self.sets = [dict(raw=torch.empty(shape[interleave], dtype=raw_dtype, device=dev), cube=None, spectra=None,
                           valid=torch.empty((sr, cols), dtype=torch.uint8, device=dev) if fill is not None else None,
-                          counts=torch.empty(num_features + 1, dtype=torch.int64, device=dev),
+                          counts=torch.empty(self.nf + 1, dtype=torch.int64, device=dev),
                           labels=torch.empty((n,), dtype=torch.uint8, device=dev),
                           labels_host=torch.empty((n,), dtype=torch.uint8).pin_memory(),
                           done=torch.cuda.Event()) for _ in range(2)]
         per = -(-(self.r1 - self.r0) // nsplit)
         self.bands = [(a, min(a + per, self.r1)) for a in range(self.r0, self.r1, per)]
-        self.ws = ops.scene_workspace(per, cols, num_features, num_classes, w, dev)
+        self.ws = ops.scene_workspace(per, cols, self.nf, num_classes, w, dev)
         self.copy_stream = torch.cuda.Stream(device=dev)
         self.events = [[torch.cuda.Event() for _ in self.bands] for _ in range(2)]
         self.calls = 0
@@ -310,15 +329,22 @@ class StreamedRawScene:
         if folded is None and self.fill is not None:
             raise _lib.CmlplError("StreamedRawScene: a cube with a fill value needs folded= (cmlpl_scene_infer_raw_masked)")
         want = self.sets[0]["raw"]
-        if il != "bip" and (raw_host.shape != want.shape or raw_host.dtype != want.dtype or not raw_host.is_contiguous()):
-            raise _lib.CmlplError(f"StreamedRawScene: raw_host must be contiguous {want.dtype} {list(want.shape)}, "
+        if il != "bip" and (tuple(raw_host.shape) != self.host_shape or raw_host.dtype != want.dtype
+                            or not raw_host.is_contiguous()):
+            raise _lib.CmlplError(f"StreamedRawScene: raw_host must be contiguous {want.dtype} {list(self.host_shape)}, "
                                   f"got {raw_host.dtype} {list(raw_host.shape)}")
+        if folded is not None:
+            fb = folded.get("bands")
+            if (fb is None) != (self.sel is None) or (fb is not None and not np.array_equal(fb, self.sel)):
+                raise _lib.CmlplError("StreamedRawScene: folded= has another band list than the Preproc")
+            if self.compact:                                  # the device planes are the listed bands
+                folded = dict(folded, bands=None, raw_bands=self.nf)
         main = torch.cuda.current_stream()
         S, events = self.sets[self.calls & 1], self.events[self.calls & 1]
         self.calls += 1
         if folded is None and S["cube"] is None:
             S["cube"] = torch.empty((self.s1 - self.s0, self.C, 60), dtype=torch.float32, device=self._dev)
-            S["spectra"] = torch.empty((self._ns, self.B), dtype=torch.float32, device=self._dev)
+            S["spectra"] = torch.empty((self._ns, self.nf), dtype=torch.float32, device=self._dev)
         lo, C = self.w // 2, self.C
         self.copy_stream.wait_event(S["done"])               # the call two scenes ago has consumed this set
         copied, spans, raw = self.s0, [], S["raw"]
@@ -330,11 +356,13 @@ class StreamedRawScene:
                 spans.append((copied, upto))
                 if upto > copied:
                     ra, rb = copied - self.s0, upto - self.s0
-                    if il == "bsq":                           # rows ra..rb of each of the B planes
+                    if il == "bsq":                           # rows ra..rb of each (listed) plane, a 2-D copy per run
                         pitch, off, width = sr * C * esz, ra * C * esz, (rb - ra) * C * esz
-                        _lib.call("cmlpl_memcpy2d_async", raw.data_ptr() + off, pitch, raw_host.data_ptr() + off, pitch,
-                                  width, self.B, self.copy_stream.cuda_stream)
-                        self.h2d_bytes += width * self.B
+                        for b0, k0, cnt in self.runs:
+                            _lib.call("cmlpl_memcpy2d_async", raw.data_ptr() + k0 * pitch + off, pitch,
+                                      raw_host.data_ptr() + b0 * pitch + off, pitch, width, cnt,
+                                      self.copy_stream.cuda_stream)
+                            self.h2d_bytes += width * cnt
                     else:                                     # BIP pixels of rows ra..rb, or BIL rows ra..rb: one block
                         src = raw_host[ra * C:rb * C] if il == "bip" else raw_host[ra:rb]
                         (raw[ra * C:rb * C] if il == "bip" else raw[ra:rb]).copy_(src, non_blocking=True)
@@ -348,10 +376,12 @@ class StreamedRawScene:
                 ra, rb = c0 - self.s0, c1 - self.s0
                 if il == "bsq" and i == 0:
                     main.wait_event(events[-1])
-                    self._pp_mod.mask_into(raw, self.fill, il, sr, C, self.B, S["valid"], S["counts"])
+                    self._pp_mod.mask_into(raw, self.fill, il, sr, C, raw.shape[0], S["valid"], S["counts"],
+                                           None if self.compact else self.sel)
                 elif il != "bsq" and rb > ra:
                     rows = raw[ra * C:rb * C] if il == "bip" else raw[ra:rb]
-                    self._pp_mod.mask_into(rows, self.fill, il, rb - ra, C, self.B, S["valid"][ra:rb], S["counts"])
+                    self._pp_mod.mask_into(rows, self.fill, il, rb - ra, C, self.B, S["valid"][ra:rb], S["counts"],
+                                           self.sel)
             if folded is not None:
                 ops.scene_infer_raw(S["raw"], folded, packed, self.K, C, self.w, band_row0=a, band_rows=b - a,
                                     scene_rows=self.R, slab_row0=self.s0, workspace=self.ws, labels=S["labels"][qa:qb],

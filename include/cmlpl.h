@@ -214,6 +214,37 @@ int cmlpl_scene_infer_raw_masked(const void* raw, int dtype, int scene_rows, int
                                  const uint8_t* valid, const void* packed, void* workspace, size_t workspace_bytes,
                                  uint8_t* labels, float* logits, cmlpl_stream_t stream);
 
+/* Band selection: the raw cube keeps all B bands, and a host list bands_host i32 [nsel] of strictly increasing raw band
+ * indices in [0, B) (B <= 8192) names the bands the call reads; feature k is raw band bands_host[k].  The model, the
+ * preprocessing, the choice of path and the workspace see nsel bands; results are bit-identical to the same call without
+ * a list on a cube that holds only the listed bands, in the same order.  The list is checked on the host before anything
+ * is enqueued (CMLPL_ERR_ARG: empty, unsorted or duplicate, out of range, too long) and travels by value in the kernel
+ * parameters: it needs no device buffer and is captured by a CUDA graph.  Use it to leave out water-absorption,
+ * uncalibrated (zero-filled) or dead detector bands.
+ *   cmlpl_valid_mask_sel_u8       cmlpl_valid_mask_u8 deciding on the listed bands only: band_missing i64 [nsel] (or NULL)
+ *                                 per listed band; nsel <= 8192
+ *   cmlpl_preprocess_fit_sel_f64  the fit of cmlpl_preprocess_fit_cube_f64 (valid NULL) or _masked_f64 (valid u8
+ *                                 [rows*cols], *n_valid i64 then required) over the listed bands, in any raw code:
+ *                                 mean f64 [nsel], gram f64 [nsel, nsel] (upper 32x32 tiles); nsel <= 8192
+ *   cmlpl_preprocess_apply_sel    cmlpl_preprocess_apply (valid NULL) or _masked over the listed bands of x [n, B] (BIP):
+ *                                 mu, inv_sigma f32 [nsel], Us f32 [nsel, npc], spectra f32 [n, nsel]; nsel <= 1024
+ *   cmlpl_scene_infer_raw_sel     cmlpl_scene_infer_raw (valid NULL) or _masked with num_features = nsel <= 512: wf f32
+ *                                 [nsel][64], mu / inv_sigma f32 [nsel], workspace of cmlpl_scene_workspace_bytes(...,
+ *                                 nsel, ...); raw holds B bands in its interleave (e.g. 196 of Hyperion's 242 bands run
+ *                                 the dense path of <= 224 bands). */
+int cmlpl_valid_mask_sel_u8(const void* raw, int dtype, int64_t rows, int cols, int B, const int* bands_host, int nsel,
+                            double fill, uint8_t* valid, int64_t* n_valid, int64_t* band_missing, cmlpl_stream_t stream);
+int cmlpl_preprocess_fit_sel_f64(const void* raw, int dtype, int64_t rows, int cols, int B, const int* bands_host, int nsel,
+                                 const uint8_t* valid, double* mean, double* gram, int64_t* n_valid, cmlpl_stream_t stream);
+int cmlpl_preprocess_apply_sel(const void* x, int dtype, int64_t n, int B, const int* bands_host, int nsel, int npc,
+                               const float* mu, const float* inv_sigma, const float* Us, const float* shift,
+                               const uint8_t* valid, float* cube, float* spectra, cmlpl_stream_t stream);
+int cmlpl_scene_infer_raw_sel(const void* raw, int dtype, int scene_rows, int cols, int slab_row0, int slab_rows, int B,
+                              const int* bands_host, int nsel, int num_classes, int w, int band_row0, int band_rows,
+                              const float* wf, const float* bf, const float* mu, const float* inv_sigma,
+                              const uint8_t* valid, const void* packed, void* workspace, size_t workspace_bytes,
+                              uint8_t* labels, float* logits, cmlpl_stream_t stream);
+
 /* Individual stages of cmlpl_scene_infer (exposed for tests / profiling). */
 int cmlpl_conv0_map_f16(const float* cube, int scene_rows, int cols, int slab_row0, int slab_rows,
                         int w, int band_row0, int band_rows, const void* packed,
